@@ -1,7 +1,10 @@
 #!/usr/bin/env python
 """bench.py -- motif x contig-bp scored / second on B200 (BASELINE.json metric).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
+
+The inputs are seeded: two runs with the same arguments score the same data, so the counts that --dump-outputs
+writes can be compared output for output between two builds.
 
 Workload (config.workload = "cfg3"): BASELINE.json configs[2], the synthetic metagenome of SURVEY.md 8d --
 300 bins x 5 Mbp = 1.5 Gbp in ~23 k contigs, per-bin GC in U(0.3, 0.7), 1-5 planted motifs per bin, a depth-30
@@ -45,6 +48,7 @@ import time
 
 import numpy as np
 
+sys.dont_write_bytecode = True  # the tree may be read-only: the bench leaves no bytecode cache in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -399,9 +403,10 @@ class Resident:
         return out
 
 
-def run_schedule(res: Resident, launches, outs, world, scan_events=None, pending=None):
+def run_schedule(res: Resident, launches, outs, world, scan_events=None, pending=None, keep=None):
     """One pass over a schedule: per launch compile the motif records, zero the count tensor, scan, and (N > 1)
-    start the all-reduce of the counts, which overlaps the next launch's scan (two count tensors alternate)."""
+    start the all-reduce of the counts, which overlaps the next launch's scan (two count tensors alternate).
+    `keep`, one [rows, 4] tensor per launch, replaces the alternating tensors so that every launch's counts remain."""
     import torch.distributed as dist
 
     from nanomotif_b200.device import scan_count
@@ -412,7 +417,7 @@ def run_schedule(res: Resident, launches, outs, world, scan_events=None, pending
         if pending[slot] is not None:
             pending[slot].wait()  # the collective that last used this count tensor
             pending[slot] = None
-        out = outs[slot][:L["rows"]]
+        out = outs[slot][:L["rows"]] if keep is None else keep[i]
         out.zero_()
         if L["progs"] is not None:
             L["progs"].compile()  # motif records -> scan programs (device kernel)
@@ -647,7 +652,17 @@ def main():
     ap.add_argument("--bins", type=int, default=N_BINS, help="cfg3 bins (debug: smaller assemblies)")
     ap.add_argument("--ref-bins", type=int, default=2, help="--impl reference: bins held by the CPU pool")
     ap.add_argument("--ref-tasks-per-core", type=int, default=8, help="--impl reference: tasks per core and step")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the counts of the last timed step to DIR/counts.npy: float64 [rows, 4] = n_mod '+', "
+                         "n_nomod '+', n_mod '-', n_nomod '-'; rows round by round, within a round the (bin, mod type) "
+                         "jobs in order, within a job its motifs of the round in work-list order")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the counts of the b200 path")
+    if args.dump_outputs and (args.only_stream or args.only_sweep):
+        ap.error("--dump-outputs needs the timed frontier schedule, which --only-stream / --only-sweep skip")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     # stdout carries exactly ONE line (the JSON): anything a library prints there (e.g. "NCCL version ...") goes to stderr
     global _JSON_FD
@@ -748,12 +763,17 @@ def main():
     step_ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     scan_ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps * n_scans)]
     scan_ev_all = list(scan_ev)
+    keep = None
+    if args.dump_outputs:  # the last step scans into one block of rows per launch, so that all of its counts remain
+        launch_rows = [L["rows"] for L in head]
+        last_counts = torch.zeros((sum(launch_rows), 4), dtype=torch.int64, device=device)
+        keep = list(torch.split(last_counts, launch_rows))
     barrier()
     t_wall = time.perf_counter()
     torch.cuda.nvtx.range_push("timed")  # ncu --nvtx --nvtx-include "timed/" profiles exactly the timed region
     for i in range(args.steps):
         step_ev[i][0].record()
-        run_schedule(res, head, outs, world, scan_ev, pending)
+        run_schedule(res, head, outs, world, scan_ev, pending, keep if i == args.steps - 1 else None)
         if i == args.steps - 1:
             drain(pending)
         step_ev[i][1].record()
@@ -764,6 +784,9 @@ def main():
     dev_ms = max_over_ranks(step_ev[0][0].elapsed_time(step_ev[-1][1]))  # first record to last record, device clock
     scan_ms = float(np.mean([a.elapsed_time(b) for a, b in scan_ev_all])) if scan_ev_all else 0.0
     value = units_per_step * args.steps / (dev_ms * 1e-3)
+    if keep is not None and rank == 0:  # after the all-reduce of the last step rank 0 holds the counts of every rank
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "counts.npy"), last_counts.cpu().numpy().astype(np.float64))
 
     peak, peak_kind = measured_peak_gbs()
 
@@ -823,7 +846,7 @@ def main():
 
         for _ in range(2):
             e2e_step(e2e_counts)
-        e2e_steps = max(3, args.steps)  # the same number of steps as the device-timed leg
+        e2e_steps = args.steps  # the same number of steps as the device-timed leg
         barrier()
         t0 = time.perf_counter()
         for _ in range(e2e_steps):

@@ -6,6 +6,7 @@ import subprocess
 import sys
 
 import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -53,3 +54,38 @@ def test_e2e_host_table_helpers():
         for kids in rounds:
             assert 1 <= len(kids) <= bench.WIDTH and len({p for _, p in kids} | {len(m) for m, _ in kids}) <= 2 * len(kids)
     assert bench.table_bytes(table) > 40 * table.num_rows
+
+
+def test_steps_below_one_are_refused():
+    res = subprocess.run([sys.executable, "bench.py", "--steps", "0"], capture_output=True, text=True, cwd=ROOT, timeout=120)
+    assert res.returncode == 2 and "--steps must be at least 1" in res.stderr
+
+
+@pytest.mark.gpu
+def test_dump_outputs_holds_the_counts_of_the_last_timed_step(tmp_path):
+    """--steps sets the timed steps of both timed legs, and --dump-outputs writes the counts of the last one: the
+    inputs are seeded, so they do not depend on the number of steps."""
+    import torch
+
+    if not torch.cuda.is_available():
+        pytest.skip("no CUDA device")
+    sys.path.insert(0, ROOT)
+    import bench
+
+    lists = bench.job_worklists(bench.load_synth(), range(2))
+    n_rows = sum(len(kids) for rounds in lists.values() for kids in rounds)
+    dumped = []
+    for steps in (1, 2):
+        out = tmp_path / f"steps{steps}"
+        res = subprocess.run([sys.executable, "bench.py", "--bins", "2", "--e2e-bins", "1", "--no-extras",
+                              "--no-cpu-baseline", "--steps", str(steps), "--warmup", "0", "--dump-outputs", str(out)],
+                             capture_output=True, text=True, cwd=ROOT, timeout=900)
+        assert res.returncode == 0, res.stderr[-2000:]
+        line = json.loads(res.stdout)
+        assert line["steps"] == steps and line["e2e"]["steps"] == steps
+        assert sorted(os.listdir(out)) == ["counts.npy"]
+        counts = np.load(out / "counts.npy")
+        assert counts.dtype == np.float64 and counts.shape == (n_rows, 4)
+        assert (counts >= 0).all() and (counts == np.round(counts)).all() and counts.sum() > 0
+        dumped.append(counts)
+    np.testing.assert_array_equal(dumped[0], dumped[1])

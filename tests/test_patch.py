@@ -46,16 +46,34 @@ def test_install_swaps_every_name_and_uninstall_restores():
     assert all(getattr(getattr(pkg, m), n) is f for (m, n), f in before.items())
 
 
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="reference tree not mounted")
-def test_spawned_interpreter_gets_the_backend_through_the_import_hook():
+def _write_stand_in_package(parent) -> None:
+    """An importable `nanomotif` with the reference's module layout where the hook acts on it: find_motifs_bin
+    imports subseq_indices from nanomotif.utils BY NAME (find_motifs_bin.py:18)."""
+    pkg = parent / "nanomotif"
+    pkg.mkdir()
+    stub = "def {}(*args, **kwargs):\n    raise NotImplementedError\n\n\n"
+    (pkg / "__init__.py").write_text("from . import find_motifs_bin, utils  # noqa: F401\n")
+    (pkg / "utils.py").write_text(stub.format("subseq_indices"))
+    (pkg / "find_motifs_bin.py").write_text("from nanomotif.utils import subseq_indices  # noqa: F401\n\n\n" + "".join(
+        stub.format(n) for n in ("methylated_motif_occourances", "motif_model_contig", "motif_model_bin", "get_parent_scores")))
+
+
+def test_spawned_interpreter_gets_the_backend_through_the_import_hook(tmp_path):
     """What a worker of get_context("spawn") sees: a fresh interpreter whose environment was prepared by
-    enable_for_workers() patches nanomotif while importing it."""
+    enable_for_workers() patches nanomotif while importing it -- the reference package where its tree is mounted,
+    otherwise a stand-in package written to a temporary directory."""
     env = dict(os.environ)
+    if ref_shim.reference_available():
+        load = "from oracle import ref_shim; nm = ref_shim.load_reference()"
+    else:
+        _write_stand_in_package(tmp_path)
+        env["PYTHONPATH"] = os.pathsep.join(p for p in (str(tmp_path), env.get("PYTHONPATH")) if p)
+        load = "import nanomotif as nm"
     code = ("import os, sys; sys.path.insert(0, %r); from nanomotif_b200 import patch; patch.enable_for_workers(); "
             "print(os.environ['PYTHONPATH']); print(os.environ['NMB200_PATCH'])" % ROOT)
     out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, check=True).stdout.split("\n")
     env["PYTHONPATH"], env["NMB200_PATCH"] = out[0], out[1]
-    child = ("from oracle import ref_shim; nm = ref_shim.load_reference(); f = nm.find_motifs_bin; "
+    child = (load + "; f = nm.find_motifs_bin; "
              "print(f.motif_model_bin.__module__, f.subseq_indices.__module__, nm.utils.subseq_indices.__module__, "
              "f.methylated_motif_occourances.__module__, f.get_parent_scores.__module__)")
     got = subprocess.run([sys.executable, "-c", child], capture_output=True, text=True, env=env, cwd=ROOT)
