@@ -49,7 +49,7 @@
 extern "C" {
 #endif
 
-#define NMB_ABI_VERSION 4 /* 2: lane-interleaved tile records (NMB_WORD_SLOT), chunk_info flag bits 28-30; 3: table ingest; 4: nmb_pack_motifs */
+#define NMB_ABI_VERSION 5 /* 2: lane-interleaved tile records (NMB_WORD_SLOT), chunk_info flag bits 28-30; 3: table ingest; 4: nmb_pack_motifs; 5: per-bin sweep slots */
 
 #if defined(__GNUC__)
 #define NMB_API __attribute__((visibility("default")))
@@ -516,6 +516,51 @@ NMB_API int nmb_sweep_expand(const uint32_t *src, uint32_t *dst, int64_t outer, 
  * = number of hits, of which at most `capacity` are written. */
 NMB_API int nmb_sweep_filter(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n, double min_mean,
                              int64_t min_mod, int64_t *out_index, int64_t capacity, int64_t *n_out, void *stream);
+
+/* ---- K8 per bin: many histograms ("slots", e.g. one per bin) from ONE pass, stacked at nmb_sweep_hist_size() /
+ *      nmb_sweep_bipartite_size() counters per slot ----
+ * contig_slot[c] (device int32, one entry per contig of the assembly) = the slot that the rows under the windows of
+ * contig c count into; -1 (or any value outside [0, n_slots)) skips the contig.  A window never leaves its contig, so
+ * contigs of different slots may share tiles.  The counters ADD like those of nmb_sweep_hist; nmb_sweep_hist /
+ * nmb_sweep_bipartite are the one-slot case of the same kernel (contig range instead of a map). */
+NMB_API int nmb_sweep_hist_slots(const nmb_assembly *assembly_h, const uint32_t *class_records_of_modtype,
+                                 int32_t tile_begin, int32_t tile_count, const int32_t *contig_slot, int32_t n_slots,
+                                 uint32_t *hist, void *stream);
+NMB_API int nmb_sweep_bipartite_slots(const nmb_assembly *assembly_h, const uint32_t *class_records_of_modtype,
+                                      int32_t tile_begin, int32_t tile_count, const int32_t *contig_slot, int32_t n_slots,
+                                      uint32_t *hist, void *stream);
+/* nmb_sweep_finalize / nmb_sweep_bipartite_finalize of n_slots (1..65535) stacked raw histograms, in place. */
+NMB_API int nmb_sweep_finalize_slots(uint32_t *hist, int32_t n_slots, void *stream);
+NMB_API int nmb_sweep_bipartite_finalize_slots(uint32_t *hist, int32_t n_slots, void *stream);
+/* nmb_sweep_slice of n_slots (1..65535) sources src + s * src_slot_stride -> dst stacked [slot][n_out]. */
+NMB_API int nmb_sweep_slice_slots(const uint32_t *src, int64_t src_slot_stride, int32_t n_slots, uint32_t *dst,
+                                  int64_t n_out, int64_t axis_stride, int32_t digit, void *stream);
+
+/* One candidate of the per-slot filters: table index (IUPAC) or counter index in the slot's bipartite histogram. */
+typedef struct nmb_sweep_hit {
+    int32_t slot;
+    uint32_t index;
+    uint32_t n_mod;
+    uint32_t n_nomod;
+} nmb_sweep_hit; /* 16 bytes */
+
+/* The LAST nmb_sweep_expand pass of a (k, mod_pos) table fused with nmb_sweep_filter: n_mod / n_nomod are stacked
+ * [n_slots][5][inner], inner = 15^(k-2) (every axis but the most significant one already expanded); the kernel
+ * expands that axis in registers and records every entry with n_mod >= min_mod and posterior mean (5 + n_mod) /
+ * (10 + n_mod + n_nomod) >= min_mean -- nmb_sweep_filter's test, bit for bit -- as (slot, table index of the
+ * 15^(k-1) table, n_mod, n_nomod).  Motifs in canonical form only: no N as the first or last letter (the modified
+ * position's own letter, at mod_pos 0 or k-1, is the fixed base and never N).  The 15^(k-1) table is not written.
+ * *n_out (device int64) = number of hits, in no particular order, of which at most `capacity` are written. */
+NMB_API int nmb_sweep_expand_filter(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots, int64_t inner,
+                                    int32_t k, int32_t mod_pos, double min_mean, int64_t min_mod, nmb_sweep_hit *out,
+                                    int64_t capacity, int64_t *n_out, void *stream);
+/* Candidates of n_slots FINISHED bipartite histograms stacked at nmb_sweep_bipartite_size(): the n_mod counters
+ * (class 0) whose concrete letter at the counter's offset o is `canonical` (A=0 T=1 G=2 C=3) and that pass the test
+ * above; index = the n_mod counter's position in its slot's histogram (n_nomod sits 4^(a+b) counters later).
+ * *n_out / capacity as for nmb_sweep_expand_filter. */
+NMB_API int nmb_sweep_bipartite_filter(const uint32_t *hist, int32_t n_slots, int32_t canonical, double min_mean,
+                                       int64_t min_mod, nmb_sweep_hit *out, int64_t capacity, int64_t *n_out,
+                                       void *stream);
 
 /* ---- host helper: CPython's random.sample(range(n), k) on a transplanted MT19937 state (the reference draws its
  *      background windows with random.sample, nanomotif/seq.py:202-225; its picks depend only on n, k and the

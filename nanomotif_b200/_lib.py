@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libnmb200.so")
 
 # ---- constants mirrored from include/nmb200.h -------------------------------------------------
-ABI_VERSION = 4
+ABI_VERSION = 5
 CHUNK_WORDS = 16
 CHUNK_BP = 512
 TILE_WORDS = 2048
@@ -76,6 +76,9 @@ JOB_DTYPE = np.dtype(
 )
 assert JOB_DTYPE.itemsize == 48
 
+SWEEP_HIT_DTYPE = np.dtype([("slot", np.int32), ("index", np.uint32), ("n_mod", np.uint32), ("n_nomod", np.uint32)])
+assert SWEEP_HIT_DTYPE.itemsize == 16
+
 _P = C.c_void_p
 _I32 = C.c_int32
 _I64 = C.c_int64
@@ -109,6 +112,13 @@ SIGNATURES = {
     "nmb_sweep_slice": (C.c_int, [_P, _P, _I64, _I64, _I32, _P]),
     "nmb_sweep_expand": (C.c_int, [_P, _P, _I64, _I64, _P]),
     "nmb_sweep_filter": (C.c_int, [_P, _P, _I64, _F64, _I64, _P, _I64, _P, _P]),
+    "nmb_sweep_hist_slots": (C.c_int, [C.POINTER(NmbAssembly), _P, _I32, _I32, _P, _I32, _P, _P]),
+    "nmb_sweep_bipartite_slots": (C.c_int, [C.POINTER(NmbAssembly), _P, _I32, _I32, _P, _I32, _P, _P]),
+    "nmb_sweep_finalize_slots": (C.c_int, [_P, _I32, _P]),
+    "nmb_sweep_bipartite_finalize_slots": (C.c_int, [_P, _I32, _P]),
+    "nmb_sweep_slice_slots": (C.c_int, [_P, _I64, _I32, _P, _I64, _I64, _I32, _P]),
+    "nmb_sweep_expand_filter": (C.c_int, [_P, _P, _I64, _I64, _I32, _I32, _F64, _I64, _P, _I64, _P, _P]),
+    "nmb_sweep_bipartite_filter": (C.c_int, [_P, _I32, _I32, _F64, _I64, _P, _I64, _P, _P]),
     "nmb_add_class_planes_compact": (C.c_int, [_P, _P, _P, _P, _I64, _I32, _I32, C.POINTER(NmbAssembly), _I32, _P, _P]),
     "nmb_filter_coverage": (C.c_int, [_P, _I64, _I64, _P, _P]),
     "nmb_filter_min_mod_frequency": (C.c_int, [_P, _P, _I64, _I32, _F64, _F64, _I64, _P, _P, _P]),

@@ -37,11 +37,14 @@ __host__ __device__ constexpr int64_t sweep_hist_offset(int k) {
 }
 constexpr int64_t kSweepHistSize = sweep_hist_offset(kSweepMaxK + 1);  // 7 567 500 counters
 
+// contig_slot == nullptr: one histogram, contigs [contig_begin, contig_end) counted.  Otherwise a chunk of contig c
+// counts into histogram slot contig_slot[c] (skipped when outside [0, n_slots)), slots stacked at the histogram size.
 struct SweepParams {
     const uint32_t *seq_records, *nonacgt, *cls;  // cls: the class records of ONE mod type
     const int64_t *contig_start, *contig_len;
     uint32_t *hist;
-    int tile_begin, n_tiles_total, contig_begin, contig_end;
+    const int32_t *contig_slot;
+    int tile_begin, n_tiles_total, contig_begin, contig_end, n_slots;
 };
 
 // word w (0..16) of chunk t in a lane-interleaved plane; word 16 = first word of chunk t + 1
@@ -146,8 +149,10 @@ __device__ __forceinline__ void bip_add_gap(uint32_t *hist, uint64_t X, uint64_t
 
 // One CTA per tile, one lane per 512-bp chunk, positions in order: the 8-letter window code slides by one letter
 // per position (base-5 digits, most significant first; the reverse-complement code slides the other way).
+// The minimum-blocks bound keeps the register counts the kernels had before slot routing (48 / 56: 10 / 9 CTAs per SM);
+// unbounded, the routed histogram pointer costs the IUPAC variant 6 registers and one resident CTA.
 template <bool BIPARTITE>
-__global__ void __launch_bounds__(kTileChunks) sweep_hist_kernel(const SweepParams p) {
+__global__ void __launch_bounds__(kTileChunks, BIPARTITE ? 9 : 10) sweep_hist_kernel(const SweepParams p) {
     // The records are read straight from global memory / L2 (the lane-interleaved layout keeps the lanes' words
     // adjacent): every word is used once, and without a 50 KB tile per CTA in shared memory three times as many
     // warps are resident to cover the latency of the divergent REDs (ncu on the staged version: issue-active 16 %,
@@ -159,7 +164,16 @@ __global__ void __launch_bounds__(kTileChunks) sweep_hist_kernel(const SweepPara
     const int info = reinterpret_cast<const int32_t *>(sy + kSeqPlaneWords)[tid];
     if (info < 0) return;
     const int contig = info & kChunkIdMask;
-    if (contig < p.contig_begin || contig >= p.contig_end) return;
+    // A lane's chunk lies in one contig and no window leaves its contig, so routing per lane keeps bins apart even
+    // when their contigs share a tile.
+    uint32_t *hist = p.hist;
+    if (p.contig_slot) {
+        const int slot = __ldg(p.contig_slot + contig);
+        if (slot < 0 || slot >= p.n_slots) return;
+        hist += (size_t)slot * (BIPARTITE ? kBipHistSize : kSweepHistSize);
+    } else if (contig < p.contig_begin || contig >= p.contig_end) {
+        return;
+    }
     const uint32_t *scls = p.cls + (size_t)tile * kClsRecWords;
     const int64_t chunk_pos = ((int64_t)tile * kTileChunks + tid) * NMB_CHUNK_BP;
     const int64_t contig_start_pos = __ldg(p.contig_start + contig);
@@ -210,18 +224,18 @@ __global__ void __launch_bounds__(kTileChunks) sweep_hist_kernel(const SweepPara
         if (BIPARTITE) {  // spans of 10..16 letters: bits b .. b + 15 of the pairs
             const int rem16 = (int)min((int64_t)16, contig_end_pos - (chunk_pos + s));
             if ((C0 | C2) >> b & 0xFFFF) {
-                bip_add_gap<4>(p.hist, X, Y, N, C0, C2, b, 0, rem16, left_n);
-                bip_add_gap<5>(p.hist, X, Y, N, C0, C2, b, 0, rem16, left_n);
-                bip_add_gap<6>(p.hist, X, Y, N, C0, C2, b, 0, rem16, left_n);
-                bip_add_gap<7>(p.hist, X, Y, N, C0, C2, b, 0, rem16, left_n);
-                bip_add_gap<8>(p.hist, X, Y, N, C0, C2, b, 0, rem16, left_n);
+                bip_add_gap<4>(hist, X, Y, N, C0, C2, b, 0, rem16, left_n);
+                bip_add_gap<5>(hist, X, Y, N, C0, C2, b, 0, rem16, left_n);
+                bip_add_gap<6>(hist, X, Y, N, C0, C2, b, 0, rem16, left_n);
+                bip_add_gap<7>(hist, X, Y, N, C0, C2, b, 0, rem16, left_n);
+                bip_add_gap<8>(hist, X, Y, N, C0, C2, b, 0, rem16, left_n);
             }
             if ((C1 | C3) >> b & 0xFFFF) {
-                bip_add_gap<4>(p.hist, X, Y, N, C1, C3, b, 1, rem16, left_n);
-                bip_add_gap<5>(p.hist, X, Y, N, C1, C3, b, 1, rem16, left_n);
-                bip_add_gap<6>(p.hist, X, Y, N, C1, C3, b, 1, rem16, left_n);
-                bip_add_gap<7>(p.hist, X, Y, N, C1, C3, b, 1, rem16, left_n);
-                bip_add_gap<8>(p.hist, X, Y, N, C1, C3, b, 1, rem16, left_n);
+                bip_add_gap<4>(hist, X, Y, N, C1, C3, b, 1, rem16, left_n);
+                bip_add_gap<5>(hist, X, Y, N, C1, C3, b, 1, rem16, left_n);
+                bip_add_gap<6>(hist, X, Y, N, C1, C3, b, 1, rem16, left_n);
+                bip_add_gap<7>(hist, X, Y, N, C1, C3, b, 1, rem16, left_n);
+                bip_add_gap<8>(hist, X, Y, N, C1, C3, b, 1, rem16, left_n);
             }
             left_n = (N >> b) & 1;
             continue;
@@ -230,8 +244,8 @@ __global__ void __launch_bounds__(kTileChunks) sweep_hist_kernel(const SweepPara
         const unsigned mp = (unsigned)(C0 >> b) & 0xFF, np = (unsigned)(C1 >> b) & 0xFF;  // rows under the window, '+'
         const unsigned mm = (unsigned)(C2 >> b) & 0xFF, nm = (unsigned)(C3 >> b) & 0xFF;  // '-'
         if (rem >= kSweepMaxK) {  // the common case: the 8-window lies inside the contig
-            if (mp | mm) sweep_add<8>(p.hist, code8, rc8, mp, mm, 0, rem);
-            if (np | nm) sweep_add<8>(p.hist, code8, rc8, np, nm, 1, rem);
+            if (mp | mm) sweep_add<8>(hist, code8, rc8, mp, mm, 0, rem);
+            if (np | nm) sweep_add<8>(hist, code8, rc8, np, nm, 1, rem);
         }
         // k < 8 comes from marginalising k + 1 (nmb_sweep_finalize) except for the windows without an extension inside
         // the contig: '+' rows under the k-window that ENDS at the contig end (rem == k), '-' rows under the k-window
@@ -242,8 +256,8 @@ __global__ void __launch_bounds__(kTileChunks) sweep_hist_kernel(const SweepPara
             {                                                                                                    \
                 const unsigned pm = rem == K ? mp : 0u, pn = rem == K ? np : 0u;                                 \
                 const unsigned qm = at_start ? mm : 0u, qn = at_start ? nm : 0u;                                 \
-                if (pm | qm) sweep_add<K>(p.hist, code8, rc8, pm, qm, 0, rem);                                   \
-                if (pn | qn) sweep_add<K>(p.hist, code8, rc8, pn, qn, 1, rem);                                   \
+                if (pm | qm) sweep_add<K>(hist, code8, rc8, pm, qm, 0, rem);                                     \
+                if (pn | qn) sweep_add<K>(hist, code8, rc8, pn, qn, 1, rem);                                     \
             }
             NMB_EDGE(4) NMB_EDGE(5) NMB_EDGE(6) NMB_EDGE(7)
 #undef NMB_EDGE
@@ -257,8 +271,9 @@ __global__ void __launch_bounds__(kTileChunks) sweep_hist_kernel(const SweepPara
 }
 
 // hist[k][o][c][w] += sum_{j < 5} hist[k + 1][o][c][5 w + j] for o < k: a k-letter motif is the prefix of its five
-// one-letter extensions (the trailing letter is the least significant base-5 digit).
+// one-letter extensions (the trailing letter is the least significant base-5 digit).  blockIdx.y = histogram slot.
 __global__ void __launch_bounds__(256) sweep_marginalise_kernel(uint32_t *__restrict__ hist, int k) {
+    hist += (size_t)blockIdx.y * kSweepHistSize;
     int n5 = 1;
     for (int i = 0; i < k; ++i) n5 *= 5;
     const int64_t n = (int64_t)k * 2 * n5;
@@ -276,7 +291,9 @@ __global__ void __launch_bounds__(256) sweep_marginalise_kernel(uint32_t *__rest
 
 // Bipartite marginals (see bip_add_gap).  mode 0: shape (a, b) += sum over the LAST right letter of shape (a, b + 1),
 // same offsets; mode 1: shape (a, b) += sum over the FIRST left letter of shape (a + 1, b), offset o <- o + 1.
+// blockIdx.y = histogram slot.
 __global__ void __launch_bounds__(256) bip_marginalise_kernel(uint32_t *__restrict__ hist, int g, int a, int b, int mode) {
+    hist += (size_t)blockIdx.y * kBipHistSize;
     const int n_code = 1 << (2 * (a + b));
     const int64_t n = (int64_t)(a + b) * 2 * n_code;
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -298,6 +315,19 @@ __global__ void __launch_bounds__(256) bip_marginalise_kernel(uint32_t *__restri
     hist[bip_offset(a, g, b) + i] += sum;
 }
 
+// The 15 IUPAC sums of the 5 letter states s[0], s[inner], ..., s[4 * inner] (A T G C other).
+__device__ __forceinline__ void iupac_sums(const uint32_t *s, int64_t inner, uint32_t v[15]) {
+    const uint32_t a = s[0], t = s[inner], g = s[2 * inner], c = s[3 * inner], x = s[4 * inner];
+    // A T G C R Y S W K M B D H V; N also takes the "other" state: the regex wildcard matches non-ACGT letters
+    v[0] = a; v[1] = t; v[2] = g; v[3] = c;
+    v[4] = a + g; v[5] = c + t; v[6] = g + c; v[7] = a + t; v[8] = g + t; v[9] = a + c;
+    v[10] = c + g + t; v[11] = a + g + t; v[12] = a + c + t; v[13] = a + c + g; v[14] = a + c + g + t + x;
+}
+
+__device__ __forceinline__ bool sweep_pass(uint32_t m, uint32_t n, double min_mean, uint32_t min_mod) {
+    return m >= min_mod && (5.0 + m) / (10.0 + m + n) >= min_mean;
+}
+
 // dst[outer][15][inner] = subset sums of src[outer][5][inner] over the letters of each IUPAC code.
 // Letter states: A T G C other; IUPAC order = nanomotif/constants.py:2 (A T G C R Y S W K M B D H V N).
 __global__ void __launch_bounds__(256) sweep_expand_kernel(const uint32_t *__restrict__ src, uint32_t *__restrict__ dst,
@@ -306,31 +336,94 @@ __global__ void __launch_bounds__(256) sweep_expand_kernel(const uint32_t *__res
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
         const int64_t o = i / inner, r = i - o * inner;
-        const uint32_t *s = src + o * 5 * inner + r;
-        const uint32_t a = s[0], t = s[inner], g = s[2 * inner], c = s[3 * inner], x = s[4 * inner];
+        uint32_t v[15];
+        iupac_sums(src + o * 5 * inner + r, inner, v);
         uint32_t *d = dst + o * 15 * inner + r;
-        d[0] = a; d[inner] = t; d[2 * inner] = g; d[3 * inner] = c;
-        d[4 * inner] = a + g;           // R
-        d[5 * inner] = c + t;           // Y
-        d[6 * inner] = g + c;           // S
-        d[7 * inner] = a + t;           // W
-        d[8 * inner] = g + t;           // K
-        d[9 * inner] = a + c;           // M
-        d[10 * inner] = c + g + t;      // B
-        d[11 * inner] = a + g + t;      // D
-        d[12 * inner] = a + c + t;      // H
-        d[13 * inner] = a + c + g;      // V
-        d[14 * inner] = a + c + g + t + x;  // N: the regex wildcard also matches non-ACGT letters
+        for (int l = 0; l < 15; ++l) d[l * inner] = v[l];
     }
 }
 
 // dst[...] = src[... with the digit of axis `axis_stride` fixed to `digit` ...]: drops one base-5 axis.
-__global__ void __launch_bounds__(256) sweep_slice_kernel(const uint32_t *__restrict__ src, uint32_t *__restrict__ dst,
-                                                          int64_t n_out, int64_t axis_stride, int digit) {
+// blockIdx.y = slot: src at slot * src_slot_stride, dst stacked [slot][n_out].
+__global__ void __launch_bounds__(256) sweep_slice_kernel(const uint32_t *__restrict__ src, int64_t src_slot_stride,
+                                                          uint32_t *__restrict__ dst, int64_t n_out, int64_t axis_stride,
+                                                          int digit) {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_out) return;
+    src += blockIdx.y * src_slot_stride;
+    dst += blockIdx.y * n_out;
     const int64_t hi = i / axis_stride, lo = i - hi * axis_stride;
     dst[i] = src[(hi * 5 + digit) * axis_stride + lo];
+}
+
+// The last expansion pass fused with the filter: the most significant table axis of src[slot][5][inner] is expanded to
+// the 15 IUPAC letters in registers and every entry that passes sweep_filter_kernel's test (same arithmetic) is
+// appended as (slot, table index = letter * inner + r, n_mod, n_nomod); the expanded table is never written.  Motifs
+// whose first or last letter is N are skipped (canonical form) unless that letter is the modified position's fixed
+// base.  *n_out counts all hits, at most `capacity` are written.
+__global__ void __launch_bounds__(256) sweep_expand_filter_kernel(const uint32_t *__restrict__ n_mod,
+                                                                  const uint32_t *__restrict__ n_nomod, int64_t n_slots,
+                                                                  int64_t inner, bool skip_first_n, bool skip_last_n,
+                                                                  double min_mean, uint32_t min_mod,
+                                                                  nmb_sweep_hit *__restrict__ out, int64_t capacity,
+                                                                  unsigned long long *__restrict__ n_out) {
+    const int64_t n = n_slots * inner;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const int64_t slot = i / inner, r = i - slot * inner;
+        uint32_t m[15], u[15];
+        iupac_sums(n_mod + slot * 5 * inner + r, inner, m);
+        uint32_t hits = 0;  // bit d: letter d passes
+        const int last = skip_last_n && r % 15 == 14 ? 0 : 15;
+        for (int d = 0; d < last; ++d)
+            if (m[d] >= min_mod) hits |= 1u << d;
+        if (skip_first_n) hits &= ~(1u << 14);
+        if (!hits) continue;
+        iupac_sums(n_nomod + slot * 5 * inner + r, inner, u);
+        for (int d = 0; d < 15; ++d)
+            if ((hits >> d & 1) && !sweep_pass(m[d], u[d], min_mean, min_mod)) hits &= ~(1u << d);
+        if (!hits) continue;
+        unsigned long long at = atomicAdd(n_out, (unsigned long long)__popc(hits));
+        for (int d = 0; d < 15; ++d) {
+            if (!(hits >> d & 1)) continue;
+            if ((int64_t)at < capacity)
+                out[at] = nmb_sweep_hit{(int32_t)slot, (uint32_t)(d * inner + r), m[d], u[d]};
+            ++at;
+        }
+    }
+}
+
+// Candidates of finished bipartite histograms stacked [slot][kBipHistSize]: every n_mod counter (class 0) whose
+// concrete letter at the counter's offset is `canonical` (A=0 T=1 G=2 C=3) and that passes the test of
+// sweep_filter_kernel; index = the counter's position in its slot's histogram.
+__global__ void __launch_bounds__(256) bip_filter_kernel(const uint32_t *__restrict__ hist, int64_t n_slots, int canonical,
+                                                         double min_mean, uint32_t min_mod, nmb_sweep_hit *__restrict__ out,
+                                                         int64_t capacity, unsigned long long *__restrict__ n_out) {
+    constexpr int64_t b33 = bip_block(3, 3), b34 = bip_block(3, 4), b43 = bip_block(4, 3);
+    constexpr int64_t per_gap = bip_offset(3, kBipMinGap + 1, 3);
+    const int64_t n = n_slots * kBipHistSize;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const uint32_t m = hist[i];
+        if (m < min_mod) continue;
+        const int64_t slot = i / kBipHistSize, j = i - slot * kBipHistSize;
+        int64_t rem = j % per_gap;
+        int a, b;
+        if (rem < b33) { a = 3; b = 3; }
+        else if (rem < b33 + b34) { a = 3; b = 4; rem -= b33; }
+        else if (rem < b33 + b34 + b43) { a = 4; b = 3; rem -= b33 + b34; }
+        else { a = 4; b = 4; rem -= b33 + b34 + b43; }
+        const int bits = 2 * (a + b);
+        const int oc = (int)(rem >> bits), code = (int)(rem & ((1 << bits) - 1));
+        if (oc & 1) continue;  // an n_nomod counter
+        const int o = oc >> 1;
+        const int xbit = o < a ? o : 2 * a + (o - a), ybit = o < a ? a + o : 2 * a + b + (o - a);
+        if ((((code >> xbit) & 1) << 1 | ((code >> ybit) & 1)) != canonical) continue;
+        const uint32_t u = hist[i + (1 << bits)];
+        if (!sweep_pass(m, u, min_mean, min_mod)) continue;
+        const unsigned long long at = atomicAdd(n_out, 1ull);
+        if ((int64_t)at < capacity) out[at] = nmb_sweep_hit{(int32_t)slot, (uint32_t)j, m, u};
+    }
 }
 
 // Candidates of one finished table pair: posterior mean (5 + n_mod) / (10 + n_mod + n_nomod) >= min_mean and
@@ -341,10 +434,7 @@ __global__ void __launch_bounds__(256) sweep_filter_kernel(const uint32_t *__res
                                                            int64_t capacity, unsigned long long *__restrict__ n_out) {
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-        const uint32_t m = n_mod[i];
-        if (m < min_mod) continue;
-        const double mean = (5.0 + m) / (10.0 + m + n_nomod[i]);
-        if (mean < min_mean) continue;
+        if (!sweep_pass(n_mod[i], n_nomod[i], min_mean, min_mod)) continue;
         const unsigned long long slot = atomicAdd(n_out, 1ull);
         if ((int64_t)slot < capacity) out[slot] = i;
     }
@@ -359,28 +449,45 @@ int64_t nmb_sweep_hist_size(void) { return nmb::kSweepHistSize; }
 int64_t nmb_sweep_bipartite_size(void) { return nmb::kBipHistSize; }
 
 static int sweep_launch(bool bipartite, const nmb_assembly *a, const uint32_t *class_records_of_modtype,
-                        int32_t tile_begin, int32_t tile_count, int32_t contig_begin, int32_t contig_end, uint32_t *hist,
-                        void *stream);
+                        int32_t tile_begin, int32_t tile_count, int32_t contig_begin, int32_t contig_end,
+                        const int32_t *contig_slot, int32_t n_slots, uint32_t *hist, void *stream);
 
 int nmb_sweep_hist(const nmb_assembly *a, const uint32_t *class_records_of_modtype, int32_t tile_begin,
                    int32_t tile_count, int32_t contig_begin, int32_t contig_end, uint32_t *hist, void *stream) {
-    return sweep_launch(false, a, class_records_of_modtype, tile_begin, tile_count, contig_begin, contig_end, hist, stream);
+    return sweep_launch(false, a, class_records_of_modtype, tile_begin, tile_count, contig_begin, contig_end, nullptr, 1,
+                        hist, stream);
 }
 
 int nmb_sweep_bipartite(const nmb_assembly *a, const uint32_t *class_records_of_modtype, int32_t tile_begin,
                         int32_t tile_count, int32_t contig_begin, int32_t contig_end, uint32_t *hist, void *stream) {
-    return sweep_launch(true, a, class_records_of_modtype, tile_begin, tile_count, contig_begin, contig_end, hist, stream);
+    return sweep_launch(true, a, class_records_of_modtype, tile_begin, tile_count, contig_begin, contig_end, nullptr, 1,
+                        hist, stream);
+}
+
+int nmb_sweep_hist_slots(const nmb_assembly *a, const uint32_t *class_records_of_modtype, int32_t tile_begin,
+                         int32_t tile_count, const int32_t *contig_slot, int32_t n_slots, uint32_t *hist, void *stream) {
+    NMB_REQUIRE(contig_slot && n_slots > 0, "nmb_sweep_hist_slots: bad slot map");
+    return sweep_launch(false, a, class_records_of_modtype, tile_begin, tile_count, 0, 0, contig_slot, n_slots, hist,
+                        stream);
+}
+
+int nmb_sweep_bipartite_slots(const nmb_assembly *a, const uint32_t *class_records_of_modtype, int32_t tile_begin,
+                              int32_t tile_count, const int32_t *contig_slot, int32_t n_slots, uint32_t *hist,
+                              void *stream) {
+    NMB_REQUIRE(contig_slot && n_slots > 0, "nmb_sweep_bipartite_slots: bad slot map");
+    return sweep_launch(true, a, class_records_of_modtype, tile_begin, tile_count, 0, 0, contig_slot, n_slots, hist,
+                        stream);
 }
 
 static int sweep_launch(bool bipartite, const nmb_assembly *a, const uint32_t *class_records_of_modtype,
-                        int32_t tile_begin, int32_t tile_count, int32_t contig_begin, int32_t contig_end, uint32_t *hist,
-                        void *stream) {
+                        int32_t tile_begin, int32_t tile_count, int32_t contig_begin, int32_t contig_end,
+                        const int32_t *contig_slot, int32_t n_slots, uint32_t *hist, void *stream) {
     NMB_REQUIRE(a && class_records_of_modtype && hist, "nmb_sweep_hist: null argument");
     NMB_REQUIRE(tile_begin >= 0 && tile_count >= 0 && tile_begin + tile_count <= a->n_tiles,
                 "nmb_sweep_hist: tiles [%d, %d) outside the assembly", tile_begin, tile_begin + tile_count);
     if (tile_count == 0) return NMB_OK;
     nmb::SweepParams p{a->seq_records, a->nonacgt, class_records_of_modtype, a->contig_start, a->contig_len, hist,
-                       tile_begin, a->n_tiles, contig_begin, contig_end};
+                       contig_slot, tile_begin, a->n_tiles, contig_begin, contig_end, n_slots};
     if (bipartite)
         nmb::sweep_hist_kernel<true><<<tile_count, nmb::kTileChunks, 0, (cudaStream_t)stream>>>(p);
     else
@@ -389,21 +496,25 @@ static int sweep_launch(bool bipartite, const nmb_assembly *a, const uint32_t *c
     return NMB_OK;
 }
 
-int nmb_sweep_finalize(uint32_t *hist, void *stream) {
-    NMB_REQUIRE(hist, "nmb_sweep_finalize: null argument");
+int nmb_sweep_finalize_slots(uint32_t *hist, int32_t n_slots, void *stream) {
+    NMB_REQUIRE(hist && n_slots > 0 && n_slots <= 65535, "nmb_sweep_finalize: bad argument");
     for (int k = nmb::kSweepMaxK - 1; k >= nmb::kSweepMinK; --k) {  // 8 -> 7, then 7 -> 6, ... each level complete first
         const int64_t n = (int64_t)k * 2 * nmb::pow5(k);
-        nmb::sweep_marginalise_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(hist, k);
+        const dim3 grid((unsigned)((n + 255) / 256), (unsigned)n_slots);
+        nmb::sweep_marginalise_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(hist, k);
         NMB_CUDA(cudaGetLastError());
     }
     return NMB_OK;
 }
 
-int nmb_sweep_bipartite_finalize(uint32_t *hist, void *stream) {
-    NMB_REQUIRE(hist, "nmb_sweep_bipartite_finalize: null argument");
+int nmb_sweep_finalize(uint32_t *hist, void *stream) { return nmb_sweep_finalize_slots(hist, 1, stream); }
+
+int nmb_sweep_bipartite_finalize_slots(uint32_t *hist, int32_t n_slots, void *stream) {
+    NMB_REQUIRE(hist && n_slots > 0 && n_slots <= 65535, "nmb_sweep_bipartite_finalize: bad argument");
     auto run = [&](int g, int a, int b, int mode) {
         const int64_t n = (int64_t)(a + b) * 2 * (1ll << (2 * (a + b)));
-        nmb::bip_marginalise_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(hist, g, a, b, mode);
+        const dim3 grid((unsigned)((n + 255) / 256), (unsigned)n_slots);
+        nmb::bip_marginalise_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(hist, g, a, b, mode);
     };
     for (int g = nmb::kBipMinGap; g <= nmb::kBipMaxGap; ++g) {
         run(g, 4, 3, 0);  // (4,g,3) from (4,g,4): last letter
@@ -414,11 +525,59 @@ int nmb_sweep_bipartite_finalize(uint32_t *hist, void *stream) {
     return NMB_OK;
 }
 
+int nmb_sweep_bipartite_finalize(uint32_t *hist, void *stream) {
+    return nmb_sweep_bipartite_finalize_slots(hist, 1, stream);
+}
+
+int nmb_sweep_slice_slots(const uint32_t *src, int64_t src_slot_stride, int32_t n_slots, uint32_t *dst, int64_t n_out,
+                          int64_t axis_stride, int32_t digit, void *stream) {
+    NMB_REQUIRE(src && dst && n_out > 0 && axis_stride > 0 && digit >= 0 && digit < 5 && n_slots > 0 &&
+                    n_slots <= 65535 && src_slot_stride >= 0,
+                "nmb_sweep_slice: bad argument");
+    const dim3 grid((unsigned)((n_out + 255) / 256), (unsigned)n_slots);
+    nmb::sweep_slice_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(src, src_slot_stride, dst, n_out, axis_stride, digit);
+    NMB_CUDA(cudaGetLastError());
+    return NMB_OK;
+}
+
 int nmb_sweep_slice(const uint32_t *src, uint32_t *dst, int64_t n_out, int64_t axis_stride, int32_t digit,
                     void *stream) {
-    NMB_REQUIRE(src && dst && n_out > 0 && axis_stride > 0 && digit >= 0 && digit < 5, "nmb_sweep_slice: bad argument");
-    nmb::sweep_slice_kernel<<<(unsigned)((n_out + 255) / 256), 256, 0, (cudaStream_t)stream>>>(src, dst, n_out,
-                                                                                             axis_stride, digit);
+    return nmb_sweep_slice_slots(src, 0, 1, dst, n_out, axis_stride, digit, stream);
+}
+
+static uint32_t clamp_min_mod(int64_t min_mod) { return (uint32_t)(min_mod > 0xFFFFFFFFll ? 0xFFFFFFFFll : min_mod); }
+
+int nmb_sweep_expand_filter(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots, int64_t inner, int32_t k,
+                            int32_t mod_pos, double min_mean, int64_t min_mod, nmb_sweep_hit *out, int64_t capacity,
+                            int64_t *n_out, void *stream) {
+    NMB_REQUIRE(n_mod && n_nomod && n_out && n_slots >= 0 && inner >= 15 && capacity >= 0 && min_mod >= 0 &&
+                    k >= nmb::kSweepMinK && k <= nmb::kSweepMaxK && mod_pos >= 0 && mod_pos < k,
+                "nmb_sweep_expand_filter: bad argument");
+    NMB_REQUIRE(capacity == 0 || out, "nmb_sweep_expand_filter: null output");
+    NMB_CUDA(cudaMemsetAsync(n_out, 0, sizeof(int64_t), (cudaStream_t)stream));
+    if (n_slots == 0) return NMB_OK;
+    int64_t blocks = (n_slots * inner + 255) / 256;
+    if (blocks > 148 * 32) blocks = 148 * 32;
+    // the first motif letter is the expanded (most significant) axis unless it is the modified position; the last one
+    // is the least significant digit of r unless it is the modified position
+    nmb::sweep_expand_filter_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+        n_mod, n_nomod, n_slots, inner, mod_pos != 0, mod_pos != k - 1, min_mean, clamp_min_mod(min_mod), out, capacity,
+        (unsigned long long *)n_out);
+    NMB_CUDA(cudaGetLastError());
+    return NMB_OK;
+}
+
+int nmb_sweep_bipartite_filter(const uint32_t *hist, int32_t n_slots, int32_t canonical, double min_mean,
+                               int64_t min_mod, nmb_sweep_hit *out, int64_t capacity, int64_t *n_out, void *stream) {
+    NMB_REQUIRE(hist && n_out && n_slots >= 0 && canonical >= 0 && canonical < 4 && capacity >= 0 && min_mod >= 0,
+                "nmb_sweep_bipartite_filter: bad argument");
+    NMB_REQUIRE(capacity == 0 || out, "nmb_sweep_bipartite_filter: null output");
+    NMB_CUDA(cudaMemsetAsync(n_out, 0, sizeof(int64_t), (cudaStream_t)stream));
+    if (n_slots == 0) return NMB_OK;
+    int64_t blocks = ((int64_t)n_slots * nmb::kBipHistSize + 255) / 256;
+    if (blocks > 148 * 32) blocks = 148 * 32;
+    nmb::bip_filter_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+        hist, n_slots, canonical, min_mean, clamp_min_mod(min_mod), out, capacity, (unsigned long long *)n_out);
     NMB_CUDA(cudaGetLastError());
     return NMB_OK;
 }
@@ -441,7 +600,7 @@ int nmb_sweep_filter(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n, 
     int64_t blocks = (n + 255) / 256;
     if (blocks > 148 * 32) blocks = 148 * 32;
     nmb::sweep_filter_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
-        n_mod, n_nomod, n, min_mean, (uint32_t)(min_mod > 0xFFFFFFFFll ? 0xFFFFFFFFll : min_mod), out_index, capacity,
+        n_mod, n_nomod, n, min_mean, clamp_min_mod(min_mod), out_index, capacity,
         (unsigned long long *)n_out);
     NMB_CUDA(cudaGetLastError());
     return NMB_OK;

@@ -8,6 +8,13 @@ position, from one histogram pass over the assembly plus a subset-sum transform 
     index.counts("GRNGAAGY", 5)                                    # one motif's counts (table lookup)
     index.candidates(k, mod_pos, "A", min_mean=0.7, min_mod=50)    # motifs above a posterior-mean / support bar
 
+The same per bin, for all bins of a MultiBinScorer at once (one histogram launch for all of them):
+
+    sw = BinSweep(scorer, "a")                                     # per-bin histograms, IUPAC + bipartite
+    sw.counts("bin_3", "GRNGAAGY", 5)                              # == scorer.context("bin_3", "a").score(...)
+    sw.index("bin_3")                                              # SweepIndex over that bin's histograms
+    sw.candidates(min_mean=0.7, min_mod=50)                        # pandas frame: every bin's candidates
+
 Letters of a motif are indexed in the order of nanomotif/constants.py:2 (A T G C R Y S W K M B D H V N); the
 modified position's own letter is fixed to the concrete canonical base and left out of the table index (a pileup
 row of mod type 'a' only exists under an A, so every other letter there gives zero or a duplicate).
@@ -15,6 +22,7 @@ row of mod type 'a' only exists under an A, so every other letter there gives ze
 from __future__ import annotations
 
 import ctypes as C
+import re
 
 import numpy as np
 import torch
@@ -87,12 +95,21 @@ class SweepIndex:
         self._bip = None
         return self
 
+    @classmethod
+    def of_finished(cls, assembly: DeviceAssembly, pileup: DevicePileup, modtype_index: int, hist: torch.Tensor,
+                    bip: torch.Tensor | None = None) -> "SweepIndex":
+        """An index over histograms finished elsewhere (one bin's slice of a BinSweep): tables, counts and candidates
+        read `hist` / `bip`; there is no raw histogram, so add() and all_reduce() do not apply."""
+        self = cls.__new__(cls)
+        self.asm, self.pileup, self.modtype = assembly, pileup, int(modtype_index)
+        self.raw, self._hist, self.bip_raw, self._bip = None, hist, None, bip
+        self._tables = {}
+        return self
+
     @property
     def bip(self):
         """The finished bipartite histogram (nmb_sweep_bipartite_finalize applied to a copy of the raw one), or None."""
-        if self.bip_raw is None:
-            return None
-        if self._bip is None:
+        if self._bip is None and self.bip_raw is not None:
             with torch.cuda.device(self.asm.device):
                 h = self.bip_raw.clone()
                 check(lib.nmb_sweep_bipartite_finalize(ptr(h), _stream()), "nmb_sweep_bipartite_finalize")
@@ -226,3 +243,268 @@ class SweepIndex:
                 continue
             out.append((s, x, y))
         return out
+
+
+# ---- per-bin sweep ----
+HIST_SIZE = int(lib.nmb_sweep_hist_size())  # counters of one IUPAC histogram (7 567 500)
+BIP_SIZE = int(lib.nmb_sweep_bipartite_size())  # counters of one bipartite histogram (7 782 400)
+_IUPAC_BYTES = np.frombuffer(IUPAC_ORDER.encode(), dtype=np.uint8)
+_ACGT_BYTES = np.frombuffer(b"ATGC", dtype=np.uint8)  # letter code x << 1 | y, as in _BASE_DIGIT
+_BIP_SHAPES = ((3, 3), (3, 4), (4, 3), (4, 4))  # storage order within one gap
+_BIPARTITE = re.compile(r"([ACGT]{3,4})(N{4,8})([ACGT]{3,4})")
+
+
+def decode_motifs(k: int, mod_pos: int, index, canonical: str = "A") -> np.ndarray:
+    """Vectorised SweepIndex.index_motif: table indices of the (k, mod_pos) table -> numpy array of motif strings."""
+    rest = np.asarray(index, dtype=np.int64).copy()
+    letters = np.empty((rest.size, k), dtype=np.uint8)
+    for i in reversed(range(k)):
+        if i == mod_pos:
+            letters[:, i] = ord(canonical)
+        else:
+            letters[:, i] = _IUPAC_BYTES[rest % 15]
+            rest //= 15
+    return letters.view(f"S{k}").ravel().astype(str)
+
+
+def decode_bipartite(counter) -> tuple[np.ndarray, np.ndarray]:
+    """Positions of n_mod counters in a bipartite histogram -> (motif strings left + "N" * gap + right, mod_position).
+    Inverts SweepIndex.bipartite_block / bipartite_index."""
+    counter = np.asarray(counter, dtype=np.int64)
+    motifs = np.empty(counter.size, dtype=object)
+    mod_pos = np.empty(counter.size, dtype=np.int64)
+    per_gap = SweepIndex.bipartite_block(3, 5, 3)[0]
+    gap, rem = counter // per_gap + 4, counter % per_gap
+    for a, b in _BIP_SHAPES:
+        first, n = SweepIndex.bipartite_block(a, 4, b)
+        inside = (rem >= first) & (rem < first + (a + b) * 2 * n)
+        for g in range(4, 9):
+            sel = np.flatnonzero(inside & (gap == g))
+            if not sel.size:
+                continue
+            r = rem[sel] - first
+            o, code = r // (2 * n), r % n
+            bits = lambda at: (code >> at) & 1
+            letters = np.full((sel.size, a + g + b), ord("N"), dtype=np.uint8)
+            for i in range(a):
+                letters[:, i] = _ACGT_BYTES[bits(i) << 1 | bits(a + i)]
+            for i in range(b):
+                letters[:, a + g + i] = _ACGT_BYTES[bits(2 * a + i) << 1 | bits(2 * a + b + i)]
+            motifs[sel] = letters.view(f"S{a + g + b}").ravel().astype(str)
+            mod_pos[sel] = np.where(o < a, o, o + g)
+    return motifs, mod_pos
+
+
+def table_scratch_bytes(k: int) -> int:
+    """Device bytes per bin of one (k, mod_pos) candidate pass: the largest expansion step's input + output, both
+    classes (the fused last step writes no table).  k = 8: 607.5 MB."""
+    sizes = [5 ** (k - 1)] + [5 ** (k - 2 - s) * 15 ** (s + 1) for s in range(k - 2)]
+    return 2 * 4 * max(x + y for x, y in zip(sizes, sizes[1:]))
+
+
+class BinSweep:
+    """The sweep of every listed bin of a MultiBinScorer for one mod type: one histogram per bin ("slot"), all of
+    them filled by ONE launch over the bins' tiles (+ one for the bipartite shapes).  Answers "which motifs are
+    methylated in which bin" for every IUPAC motif of length 4..8 and every bipartite X{3,4} N{4..8} Y{3,4} motif.
+
+    Device memory per bin: 30.3 MB of raw IUPAC counters and 31.1 MB of raw bipartite ones (400 bins: 12.1 + 12.5
+    GB), and the same again for the finished copies once tables or candidates are read; `bins=` sweeps a subset.
+    candidates() needs `scratch_bytes` more (at least table_scratch_bytes(max k) per bin of a chunk)."""
+
+    def __init__(self, scorer, mod_type, bins=None, bipartite: bool = True):
+        from .search import CANONICAL
+
+        self.asm, self.pileup, self.mod_type = scorer.assembly, scorer.pileup, mod_type
+        self.modtype = list(scorer.mod_types).index(mod_type)
+        self.canonical = CANONICAL[str(mod_type)]
+        self.bins = list(scorer._ranges) if bins is None else list(bins)
+        self.slot = {}
+        for b in self.bins:
+            if b not in scorer._ranges:
+                raise KeyError(b)
+            if b in self.slot:
+                raise ValueError(f"bin {b!r} listed twice")
+            self.slot[b] = len(self.slot)
+        asm = self.asm
+        contig_slot = np.full(asm.n_contigs, -1, dtype=np.int32)
+        first, last = asm.n_tiles, 0
+        for b, s in self.slot.items():
+            lo, hi = scorer._ranges[b]
+            contig_slot[lo:hi] = s
+            t0, n = asm.tile_span(lo, hi)
+            if n:
+                first, last = min(first, t0), max(last, t0 + n)
+        self.tile_begin, self.tile_count = (first, last - first) if last > first else (0, 0)
+        n = len(self.bins)
+        with torch.cuda.device(asm.device):
+            self.contig_slot = torch.from_numpy(np.append(contig_slot, np.int32(-1))).to(asm.device)
+            self.raw = torch.zeros(n * HIST_SIZE, dtype=torch.int32, device=asm.device)
+            self.bip_raw = torch.zeros(n * BIP_SIZE, dtype=torch.int32, device=asm.device) if bipartite else None
+        self._hist = self._bip = None
+        self.add()
+        if bipartite:
+            self.add_bipartite()
+
+    def _launch(self, fn, hist, what):
+        if not self.bins:
+            return
+        base = ptr(self.pileup.class_records) + self.modtype * self.asm.n_tiles * _lib.CLS_REC_WORDS * 4
+        with torch.cuda.device(self.asm.device):
+            check(fn(C.byref(self.asm.view()), base, self.tile_begin, self.tile_count, ptr(self.contig_slot),
+                     len(self.bins), ptr(hist), _stream()), what)
+
+    def add(self) -> "BinSweep":
+        """One more pass over the listed bins into the raw IUPAC histograms (counters add)."""
+        self._launch(lib.nmb_sweep_hist_slots, self.raw, "nmb_sweep_hist_slots")
+        self._hist = None
+        return self
+
+    def add_bipartite(self) -> "BinSweep":
+        """One more pass into the raw bipartite histograms (counters add)."""
+        if self.bip_raw is None:
+            raise ValueError("this BinSweep was made with bipartite=False")
+        self._launch(lib.nmb_sweep_bipartite_slots, self.bip_raw, "nmb_sweep_bipartite_slots")
+        self._bip = None
+        return self
+
+    @property
+    def hist(self) -> torch.Tensor:
+        """Finished IUPAC histograms [bin][HIST_SIZE] (nmb_sweep_finalize_slots on a copy of the raw ones)."""
+        if self._hist is None:
+            with torch.cuda.device(self.asm.device):
+                h = self.raw.clone()
+                if self.bins:
+                    check(lib.nmb_sweep_finalize_slots(ptr(h), len(self.bins), _stream()), "nmb_sweep_finalize_slots")
+            self._hist = h
+        return self._hist.view(-1, HIST_SIZE)
+
+    @property
+    def bip(self):
+        """Finished bipartite histograms [bin][BIP_SIZE], or None without bipartite."""
+        if self.bip_raw is None:
+            return None
+        if self._bip is None:
+            with torch.cuda.device(self.asm.device):
+                h = self.bip_raw.clone()
+                if self.bins:
+                    check(lib.nmb_sweep_bipartite_finalize_slots(ptr(h), len(self.bins), _stream()),
+                          "nmb_sweep_bipartite_finalize_slots")
+            self._bip = h
+        return self._bip.view(-1, BIP_SIZE)
+
+    def index(self, bin_name) -> SweepIndex:
+        """SweepIndex over one bin's finished histograms: table / counts / candidates / bipartite_* as for a
+        SweepIndex of that bin's contig range."""
+        s = self.slot[bin_name]
+        return SweepIndex.of_finished(self.asm, self.pileup, self.modtype, self.hist[s],
+                                      None if self.bip_raw is None else self.bip[s])
+
+    def counts(self, bin_name, motif_iupac: str, mod_pos: int) -> tuple[int, int]:
+        """(n_mod, n_nomod) of one motif in one bin: an IUPAC motif of length 4..8, or left + "N" * gap + right of a
+        bipartite shape."""
+        index = self.index(bin_name)
+        m = _BIPARTITE.fullmatch(motif_iupac)
+        if m and len(motif_iupac) > MAX_K:
+            return index.bipartite_counts(m.group(1), len(m.group(2)), m.group(3), mod_pos)
+        return index.counts(motif_iupac, mod_pos, keep=False)
+
+    def candidates(self, min_mean: float = 0.7, min_mod: int = 50, ks=range(MIN_K, MAX_K + 1), bipartite: bool = True,
+                   scratch_bytes: int = 8 << 30, capacity: int = 1 << 20):
+        """Every bin's motifs with posterior mean (5 + n_mod) / (10 + n_mod + n_nomod) >= min_mean and n_mod >=
+        min_mod, as SweepIndex.candidates finds them per (k, mod_pos), plus the bipartite ones whose modified position
+        holds the canonical base.  pandas frame with columns bin, mod_type, motif (IUPAC; bipartite as left + "N" *
+        gap + right), mod_position, n_mod, n_nomod, mean; rows in bin order, then k, then mod_position, then table
+        index, the bipartite shapes after k = 8 (by gap, then (3,3) (3,4) (4,3) (4,4), then mod_position, then
+        index).  Bins are processed in chunks of max(1, scratch_bytes // table_scratch_bytes(max k)); `capacity` is
+        the initial number of hit records per pass (a pass with more hits runs again with the exact count)."""
+        if min_mod < 1:
+            raise ValueError("min_mod must be >= 1: every motif without rows has the prior mean 0.5")
+        ks = sorted(set(int(k) for k in ks))
+        if any(not MIN_K <= k <= MAX_K for k in ks):
+            raise ValueError("ks must lie in 4..8")
+        if bipartite and self.bip_raw is None:
+            raise ValueError("this BinSweep was made with bipartite=False")
+        groups = [(k, mp) for k in ks for mp in range(k)]
+        d, n_bins = self.asm.device, len(self.bins)
+        state = {"cap": max(int(capacity), 1)}
+        parts = []  # (group, hit records)
+
+        def collect(group, launch, slot0=0):
+            with torch.cuda.device(d):
+                n_out = torch.zeros(1, dtype=torch.int64, device=d)
+                if "buf" not in state or state["buf"].numel() < state["cap"] * 16:
+                    state["buf"] = torch.empty(state["cap"] * 16, dtype=torch.uint8, device=d)
+                launch(ptr(state["buf"]), state["cap"], ptr(n_out))
+                m = int(n_out.item())
+                if m > state["cap"]:  # count-then-fill: run again with room for every hit
+                    state["cap"] = m
+                    state["buf"] = torch.empty(m * 16, dtype=torch.uint8, device=d)
+                    launch(ptr(state["buf"]), m, ptr(n_out))
+                hits = state["buf"][:m * 16].cpu().numpy().view(_lib.SWEEP_HIT_DTYPE)
+                hits["slot"] += slot0
+                parts.append((group, hits))
+
+        if groups and n_bins:
+            chunk = max(1, int(scratch_bytes) // table_scratch_bytes(ks[-1]))
+            hist = self.hist.view(-1)
+            for s0 in range(0, n_bins, chunk):
+                ns = min(chunk, n_bins - s0)
+                for group, (k, mp) in enumerate(groups):
+                    with torch.cuda.device(d):
+                        n5 = 5 ** (k - 1)
+                        tab = []
+                        for cls in (0, 1):
+                            src = hist[s0 * HIST_SIZE + hist_offset(k) + (mp * 2 + cls) * 5 ** k:]
+                            t = torch.empty(ns * n5, dtype=torch.int32, device=d)
+                            check(lib.nmb_sweep_slice_slots(ptr(src), HIST_SIZE, ns, ptr(t), n5, 5 ** (k - 1 - mp),
+                                                            _BASE_DIGIT[self.canonical], _stream()),
+                                  "nmb_sweep_slice_slots")
+                            tab.append(t)
+                        for step in range(k - 2):  # every axis but the most significant one, as in SweepIndex.table
+                            outer, inner = ns * 5 ** (k - 2 - step), 15 ** step
+                            nxt = []
+                            for t in tab:
+                                e = torch.empty(outer * 15 * inner, dtype=torch.int32, device=d)
+                                check(lib.nmb_sweep_expand(ptr(t), ptr(e), outer, inner, _stream()), "nmb_sweep_expand")
+                                nxt.append(e)
+                            tab = nxt
+                    def launch(out, cap, n_out, tab=tab, ns=ns, k=k, mp=mp):
+                        check(lib.nmb_sweep_expand_filter(ptr(tab[0]), ptr(tab[1]), ns, 15 ** (k - 2), k, mp,
+                                                          float(min_mean), int(min_mod), out, cap, n_out, _stream()),
+                              "nmb_sweep_expand_filter")
+
+                    collect(group, launch, s0)
+                    del tab
+        if bipartite and n_bins:
+            def launch_bip(out, cap, n_out):
+                check(lib.nmb_sweep_bipartite_filter(ptr(self.bip), n_bins, _BASE_DIGIT[self.canonical],
+                                                     float(min_mean), int(min_mod), out, cap, n_out, _stream()),
+                      "nmb_sweep_bipartite_filter")
+
+            collect(len(groups), launch_bip)
+        return self._frame(parts, groups)
+
+    def _frame(self, parts, groups):
+        import pandas as pd
+
+        group = np.concatenate([np.full(len(h), g, dtype=np.int64) for g, h in parts]) if parts else np.zeros(0, np.int64)
+        hits = np.concatenate([h for _, h in parts]) if parts else np.zeros(0, _lib.SWEEP_HIT_DTYPE)
+        key = (hits["slot"].astype(np.int64) * (len(groups) + 1) + group) << 32 | hits["index"].astype(np.int64)
+        order = np.argsort(key, kind="stable")
+        hits, group = hits[order], group[order]
+        motif = np.empty(len(hits), dtype=object)
+        mod_position = np.empty(len(hits), dtype=np.int64)
+        for g in np.unique(group):
+            sel = np.flatnonzero(group == g)
+            if g < len(groups):
+                k, mp = groups[g]
+                motif[sel] = decode_motifs(k, mp, hits["index"][sel], self.canonical)
+                mod_position[sel] = mp
+            else:
+                motif[sel], mod_position[sel] = decode_bipartite(hits["index"][sel])
+        n_mod, n_nomod = hits["n_mod"].astype(np.int64), hits["n_nomod"].astype(np.int64)
+        names = np.empty(len(self.bins), dtype=object)
+        names[:] = self.bins
+        return pd.DataFrame({"bin": names[hits["slot"]], "mod_type": np.full(len(hits), self.mod_type, dtype=object),
+                             "motif": motif, "mod_position": mod_position, "n_mod": n_mod, "n_nomod": n_nomod,
+                             "mean": (5.0 + n_mod) / (10.0 + n_mod + n_nomod)})
