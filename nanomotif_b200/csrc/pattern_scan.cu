@@ -367,7 +367,9 @@ __global__ void __launch_bounds__(kPatThreads, 4) pattern_scan_kernel(const __gr
             if (warp_n) {
                 LaneSeq<H, true> q;
                 load_xyn<H>(sx, sy, tid, p.nonacgt + kHalo + (size_t)tile * kTileWords + tid * NW - H, q);
-                const LaneEdge edge = {0, false, false};
+                // motifs are unstripped: a flanking '.' is never tested against the n plane, so clip to the contig
+                const LaneEdge edge = lane_edge(true, info, (int64_t)tile * kTileChunks + tid, p.contig_start,
+                                                p.contig_len);
                 pattern_motifs<H, true>(p, mblk, q, edge, sv, s_pref, wq, rank_p, rank_m, contig, c0);
             } else {
                 LaneSeq<H, false> q;

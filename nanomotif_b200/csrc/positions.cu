@@ -29,7 +29,8 @@ __global__ void __launch_bounds__(kTileChunks) match_plane_kernel(
         if (warp_n) {
             LaneSeq<H, true> q;
             load_xyn<H>(px, py, tid, nonacgt + kHalo + (size_t)tile * kTileWords + tid * NW - H, q);
-            const LaneEdge edge = {0, false, false};
+            // programs may be unstripped: a flanking '.' is never tested against the n plane, so clip to the contig
+            const LaneEdge edge = lane_edge(true, info, (int64_t)tile * kTileChunks + tid, contig_start, contig_len);
             match_words<H, true>(pv, q, m, edge);
         } else {
             LaneSeq<H, false> q;

@@ -20,7 +20,9 @@
 //   XYN  additionally the non-ACGT plane n, ANDed out of every indicator so that such letters fail every
 //        constrained position and only match '.', the regex semantics of the reference (SURVEY.md
 //        Appendix B item 5).  One extra logic op per word and step; used only by warps whose chunks (or
-//        neighbouring chunks) hold a non-ACGT letter of a contig -- rare.
+//        neighbouring chunks) hold a non-ACGT letter of a contig -- rare.  Padding fails every constrained
+//        position here too, but a flanking '.' of an unstripped motif (K3, K5) is never tested, so callers
+//        that may see one clip these chains as well (LaneEdge with edge set); K2's stripped motifs need not.
 // The branch on the base is uniform across the CTA (it depends on the motif only).
 #pragma once
 #include "common.cuh"
@@ -163,7 +165,7 @@ __device__ __forceinline__ void run_chain(const ProgramView &pv, const LaneSeq<H
                 break;
         }
     }
-    if (!HASN && edge.edge) clip_start_aligned<H>(c, edge, pv.len);
+    if (edge.edge) clip_start_aligned<H>(c, edge, pv.len);
 }
 
 // Allowed-set of the complementary bases: A<->T (bits 0,1), G<->C (bits 2,3).
@@ -274,7 +276,7 @@ __device__ __forceinline__ bool run_chain_pair(const ProgramView &pv, const Lane
         }
     }
     if (pv.n >= 8 && !chains_alive<H>(c, d)) return false;
-    if (!HASN && edge.edge) {  // warp-uniform
+    if (edge.edge) {  // warp-uniform
         clip_start_aligned<H>(c, edge, pv.len);
         clip_end_aligned_rev<H>(d, edge, pv.len);
     }
