@@ -43,6 +43,14 @@ def _one_hot_to_masks(one_hot: np.ndarray) -> np.ndarray:
     return rec
 
 
+def _window_width(padding: int) -> int:
+    """2 * padding + 1, refused with ValueError when it is not a window the device can hold (1..MAX_WINDOW)."""
+    width = 2 * int(padding) + 1
+    if padding < 0 or width > _lib.MAX_WINDOW:
+        raise ValueError(f"window width {width} (padding {padding}) is outside 1..{_lib.MAX_WINDOW}")
+    return width
+
+
 class DeviceDNAarray:
     """Drop-in for the reference's ``DNAarray`` as the motif search uses it: ``shape``, ``copy()``,
     ``filter_sequence_matches(one_hot, keep_matches)`` and ``pssm()``.  Rows live on the GPU as
@@ -63,6 +71,7 @@ class DeviceDNAarray:
         """Windows of +-padding around forward-strand positions (strand 1 = reverse-complemented).
         Positions violating the reference's strict bound padding < i < len - padding must already have
         been dropped (see `methylation_windows`)."""
+        width = _window_width(padding)
         d = assembly.device
         ci = np.asarray(contig_index, dtype=np.int64)
         gpos = assembly.starts[ci] + np.asarray(position, dtype=np.int64)
@@ -76,7 +85,7 @@ class DeviceDNAarray:
                 check(lib.nmb_extract_windows(C.byref(view), ptr(g), ptr(st), n, int(padding), ptr(win), _stream()),
                       "nmb_extract_windows")
                 torch.cuda.current_stream().synchronize()
-        return cls(win, 2 * padding + 1)
+        return cls(win, width)
 
     # -- DNAarray surface -----------------------------------------------------------------------
     @property
@@ -254,6 +263,7 @@ def methylation_windows(assembly: DeviceAssembly, contig_id, position, strand, f
     """Windows around confidently methylated sites in the reference's row order: per contig, '+' sites
     then reverse-complemented '-' sites (find_motifs_bin.py:625-672).  Columns as numpy arrays;
     contig_id indexes the assembly, strand is 0/1."""
+    _window_width(padding)
     ci, pos, st = window_rows(assembly.lengths, contig_id, position, strand, fraction_mod, high, padding)
     if len(pos) == 0:
         return None
@@ -355,7 +365,7 @@ def prepare_searches(scorer, mod_type, padding: int, high: float, bin_names=None
     d = asm.device
     names = list(scorer._ranges) if bin_names is None else list(bin_names)
     mti = scorer.mod_types.index(mod_type)
-    width = 2 * padding + 1
+    width = _window_width(padding)
     if not scorer.rows:
         raise ValueError("the scorer keeps no pileup rows (built with keep_rows=False or from_device)")
     from .search import CANONICAL
