@@ -49,7 +49,7 @@
 extern "C" {
 #endif
 
-#define NMB_ABI_VERSION 5 /* 2: lane-interleaved tile records (NMB_WORD_SLOT), chunk_info flag bits 28-30; 3: table ingest; 4: nmb_pack_motifs; 5: per-bin sweep slots */
+#define NMB_ABI_VERSION 6 /* 2: lane-interleaved tile records (NMB_WORD_SLOT), chunk_info flag bits 28-30; 3: table ingest; 4: nmb_pack_motifs; 5: per-bin sweep slots; 6: degenerate bipartite sweep */
 
 #if defined(__GNUC__)
 #define NMB_API __attribute__((visibility("default")))
@@ -561,6 +561,30 @@ NMB_API int nmb_sweep_expand_filter(const uint32_t *n_mod, const uint32_t *n_nom
 NMB_API int nmb_sweep_bipartite_filter(const uint32_t *hist, int32_t n_slots, int32_t canonical, double min_mean,
                                        int64_t min_mod, nmb_sweep_hit *out, int64_t capacity, int64_t *n_out,
                                        void *stream);
+
+/* ---- K8 degenerate bipartite motifs (ABI 6): X{a} N{g} Y{b} whose halves use the 14 IUPAC letters other than N
+ *      (A T G C R Y S W K M B D H V, the order of nmb_sweep_expand without N), from the FINISHED bipartite
+ *      histograms.  Exact: such a letter matches only ACGT contig letters, and the bipartite histograms skip every
+ *      window with a non-ACGT letter in a half, so a motif's count is the sum of the ACGT counters of the concrete
+ *      motifs it stands for.  N in a half is not covered (it would need a non-ACGT state in the histogram pass). ----
+ * Slice: dst[slot][w] (4^(a+b-1) uint32 per slot) = the class-`cls` counters (0 methylated, 1 unmethylated) of shape
+ * (a, g, b) with the modified base at motif position mod_pos (inside X or Y, gap counted) for the n_slots (1..65535)
+ * finished histograms stacked at nmb_sweep_bipartite_size(); the letter at mod_pos is fixed to `canonical` (A=0 T=1
+ * G=2 C=3) and w holds the other a + b - 1 letters as base-4 digits in that code, first motif letter most
+ * significant. */
+NMB_API int nmb_sweep_bip_iupac_slice(const uint32_t *hist, int32_t n_slots, int32_t a, int32_t g, int32_t b,
+                                      int32_t mod_pos, int32_t cls, int32_t canonical, uint32_t *dst, void *stream);
+/* dst[outer][14][inner] = sums of src[outer][4][inner] over the concrete letters of each of the 14 letters.  Applied
+ * to the a + b - 1 axes of a slice, last axis first, it gives the table of all 14^(a+b-1) motifs, index = the letters
+ * other than the modified one as base-14 digits, first letter most significant. */
+NMB_API int nmb_sweep_bip_iupac_expand(const uint32_t *src, uint32_t *dst, int64_t outer, int64_t inner, void *stream);
+/* The last nmb_sweep_bip_iupac_expand pass fused with the filter of nmb_sweep_expand_filter: n_mod / n_nomod stacked
+ * [n_slots][4][inner] (inner = 14^(a+b-2), every axis but the first expanded); records (slot, table index, n_mod,
+ * n_nomod) of every motif with n_mod >= min_mod and posterior mean >= min_mean; the table is not written.
+ * *n_out / capacity as for nmb_sweep_expand_filter. */
+NMB_API int nmb_sweep_bip_iupac_expand_filter(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots,
+                                              int64_t inner, double min_mean, int64_t min_mod, nmb_sweep_hit *out,
+                                              int64_t capacity, int64_t *n_out, void *stream);
 
 /* ---- host helper: CPython's random.sample(range(n), k) on a transplanted MT19937 state (the reference draws its
  *      background windows with random.sample, nanomotif/seq.py:202-225; its picks depend only on n, k and the

@@ -315,13 +315,19 @@ __global__ void __launch_bounds__(256) bip_marginalise_kernel(uint32_t *__restri
     hist[bip_offset(a, g, b) + i] += sum;
 }
 
+// The sums of the 4 concrete letter states over the 14 IUPAC letters other than N: A T G C R Y S W K M B D H V.
+__device__ __forceinline__ void acgt_sums(uint32_t a, uint32_t t, uint32_t g, uint32_t c, uint32_t *v) {
+    v[0] = a; v[1] = t; v[2] = g; v[3] = c;
+    v[4] = a + g; v[5] = c + t; v[6] = g + c; v[7] = a + t; v[8] = g + t; v[9] = a + c;
+    v[10] = c + g + t; v[11] = a + g + t; v[12] = a + c + t; v[13] = a + c + g;
+}
+
 // The 15 IUPAC sums of the 5 letter states s[0], s[inner], ..., s[4 * inner] (A T G C other).
 __device__ __forceinline__ void iupac_sums(const uint32_t *s, int64_t inner, uint32_t v[15]) {
     const uint32_t a = s[0], t = s[inner], g = s[2 * inner], c = s[3 * inner], x = s[4 * inner];
-    // A T G C R Y S W K M B D H V; N also takes the "other" state: the regex wildcard matches non-ACGT letters
-    v[0] = a; v[1] = t; v[2] = g; v[3] = c;
-    v[4] = a + g; v[5] = c + t; v[6] = g + c; v[7] = a + t; v[8] = g + t; v[9] = a + c;
-    v[10] = c + g + t; v[11] = a + g + t; v[12] = a + c + t; v[13] = a + c + g; v[14] = a + c + g + t + x;
+    // N also takes the "other" state: the regex wildcard matches non-ACGT letters
+    acgt_sums(a, t, g, c, v);
+    v[14] = a + c + g + t + x;
 }
 
 __device__ __forceinline__ bool sweep_pass(uint32_t m, uint32_t n, double min_mean, uint32_t min_mod) {
@@ -423,6 +429,83 @@ __global__ void __launch_bounds__(256) bip_filter_kernel(const uint32_t *__restr
         if (!sweep_pass(m, u, min_mean, min_mod)) continue;
         const unsigned long long at = atomicAdd(n_out, 1ull);
         if ((int64_t)at < capacity) out[at] = nmb_sweep_hit{(int32_t)slot, (uint32_t)j, m, u};
+    }
+}
+
+// ---- degenerate bipartite halves: X{a} N{g} Y{b} with any of the 14 IUPAC letters other than N in X and Y ----
+// A half letter other than N matches only the four concrete contig letters, and bip_add skips every window with a
+// non-ACGT letter in a half, so the count of such a motif is the sum of the finished ACGT counters over the concrete
+// letters each of its letters stands for: a 4-state -> 14-letter subset sum, one axis per letter, on the bit-planar
+// blocks.  N in a half would need a fifth ("other") state in the histogram pass.
+
+// dst[slot][w] = the (shape (a, b), offset o, class cls) block of slot `slot` of finished bipartite histograms stacked
+// at kBipHistSize (`block` = bip_offset(a, g, b)), with the letter at offset o fixed to `canonical` and the other
+// a + b - 1 letters written as base-4 digits w (A=0 T=1 G=2 C=3), first letter most significant.  blockIdx.y = slot.
+__global__ void __launch_bounds__(256) bip_iupac_slice_kernel(const uint32_t *__restrict__ hist, int64_t block, int a,
+                                                              int b, int o, int cls, int canonical,
+                                                              uint32_t *__restrict__ dst) {
+    const int n_out = 1 << (2 * (a + b - 1));
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n_out) return;
+    const uint32_t *h = hist + (size_t)blockIdx.y * kBipHistSize + block + (size_t)(o * 2 + cls) * (1u << (2 * (a + b)));
+    unsigned code = 0;
+    for (int p = a + b - 1, w = i; p >= 0; --p) {  // last letter = least significant digit
+        int d = canonical;
+        if (p != o) { d = w & 3; w >>= 2; }
+        const int xbit = p < a ? p : 2 * a + (p - a), ybit = p < a ? a + p : 2 * a + b + (p - a);
+        code |= (unsigned)(d >> 1) << xbit | (unsigned)(d & 1) << ybit;
+    }
+    dst[(size_t)blockIdx.y * n_out + i] = h[code];
+}
+
+// dst[outer][14][inner] = sums of src[outer][4][inner] over the concrete letters of each IUPAC letter but N.
+__global__ void __launch_bounds__(256) bip_iupac_expand_kernel(const uint32_t *__restrict__ src, uint32_t *__restrict__ dst,
+                                                               int64_t outer, int64_t inner) {
+    const int64_t n = outer * inner;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const int64_t o = i / inner, r = i - o * inner;
+        const uint32_t *s = src + o * 4 * inner + r;
+        uint32_t v[14];
+        acgt_sums(s[0], s[inner], s[2 * inner], s[3 * inner], v);
+        uint32_t *d = dst + o * 14 * inner + r;
+        for (int l = 0; l < 14; ++l) d[l * inner] = v[l];
+    }
+}
+
+// The last bip_iupac_expand pass fused with the filter, as sweep_expand_filter_kernel does for the contiguous tables:
+// src[slot][4][inner] -> the 14 letters of the most significant axis in registers, every entry that passes
+// sweep_pass appended as (slot, index = letter * inner + r, n_mod, n_nomod).  *n_out counts all hits, at most
+// `capacity` are written.
+__global__ void __launch_bounds__(256) bip_iupac_expand_filter_kernel(const uint32_t *__restrict__ n_mod,
+                                                                      const uint32_t *__restrict__ n_nomod,
+                                                                      int64_t n_slots, int64_t inner, double min_mean,
+                                                                      uint32_t min_mod, nmb_sweep_hit *__restrict__ out,
+                                                                      int64_t capacity,
+                                                                      unsigned long long *__restrict__ n_out) {
+    const int64_t n = n_slots * inner;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const int64_t slot = i / inner, r = i - slot * inner;
+        const uint32_t *s = n_mod + slot * 4 * inner + r;
+        uint32_t m[14], u[14];
+        acgt_sums(s[0], s[inner], s[2 * inner], s[3 * inner], m);
+        uint32_t hits = 0;  // bit d: letter d passes
+        for (int d = 0; d < 14; ++d)
+            if (m[d] >= min_mod) hits |= 1u << d;
+        if (!hits) continue;
+        s = n_nomod + slot * 4 * inner + r;
+        acgt_sums(s[0], s[inner], s[2 * inner], s[3 * inner], u);
+        for (int d = 0; d < 14; ++d)
+            if ((hits >> d & 1) && !sweep_pass(m[d], u[d], min_mean, min_mod)) hits &= ~(1u << d);
+        if (!hits) continue;
+        unsigned long long at = atomicAdd(n_out, (unsigned long long)__popc(hits));
+        for (int d = 0; d < 14; ++d) {
+            if (!(hits >> d & 1)) continue;
+            if ((int64_t)at < capacity)
+                out[at] = nmb_sweep_hit{(int32_t)slot, (uint32_t)(d * inner + r), m[d], u[d]};
+            ++at;
+        }
     }
 }
 
@@ -578,6 +661,49 @@ int nmb_sweep_bipartite_filter(const uint32_t *hist, int32_t n_slots, int32_t ca
     if (blocks > 148 * 32) blocks = 148 * 32;
     nmb::bip_filter_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
         hist, n_slots, canonical, min_mean, clamp_min_mod(min_mod), out, capacity, (unsigned long long *)n_out);
+    NMB_CUDA(cudaGetLastError());
+    return NMB_OK;
+}
+
+int nmb_sweep_bip_iupac_slice(const uint32_t *hist, int32_t n_slots, int32_t a, int32_t g, int32_t b, int32_t mod_pos,
+                              int32_t cls, int32_t canonical, uint32_t *dst, void *stream) {
+    NMB_REQUIRE((a == 3 || a == 4) && (b == 3 || b == 4) && g >= nmb::kBipMinGap && g <= nmb::kBipMaxGap,
+                "nmb_sweep_bip_iupac_slice: shape (%d, %d, %d) is not X{3,4} N{4..8} Y{3,4}", a, g, b);
+    NMB_REQUIRE(mod_pos >= 0 && mod_pos < a + g + b && !(mod_pos >= a && mod_pos < a + g),
+                "nmb_sweep_bip_iupac_slice: modified position %d outside the halves", mod_pos);
+    NMB_REQUIRE(hist && dst && n_slots > 0 && n_slots <= 65535 && (cls == 0 || cls == 1) && canonical >= 0 &&
+                    canonical < 4,
+                "nmb_sweep_bip_iupac_slice: bad argument");
+    const int n_out = 1 << (2 * (a + b - 1));
+    const dim3 grid((unsigned)((n_out + 255) / 256), (unsigned)n_slots);
+    nmb::bip_iupac_slice_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(
+        hist, nmb::bip_offset(a, g, b), a, b, mod_pos < a ? mod_pos : mod_pos - g, cls, canonical, dst);
+    NMB_CUDA(cudaGetLastError());
+    return NMB_OK;
+}
+
+int nmb_sweep_bip_iupac_expand(const uint32_t *src, uint32_t *dst, int64_t outer, int64_t inner, void *stream) {
+    NMB_REQUIRE(src && dst && outer > 0 && inner > 0, "nmb_sweep_bip_iupac_expand: bad argument");
+    int64_t blocks = (outer * inner + 255) / 256;
+    if (blocks > 148 * 64) blocks = 148 * 64;
+    nmb::bip_iupac_expand_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(src, dst, outer, inner);
+    NMB_CUDA(cudaGetLastError());
+    return NMB_OK;
+}
+
+int nmb_sweep_bip_iupac_expand_filter(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots, int64_t inner,
+                                      double min_mean, int64_t min_mod, nmb_sweep_hit *out, int64_t capacity,
+                                      int64_t *n_out, void *stream) {
+    NMB_REQUIRE(n_mod && n_nomod && n_out && n_slots >= 0 && inner > 0 && inner <= 0xFFFFFFFFll / 14 &&
+                    capacity >= 0 && min_mod >= 0,
+                "nmb_sweep_bip_iupac_expand_filter: bad argument");
+    NMB_REQUIRE(capacity == 0 || out, "nmb_sweep_bip_iupac_expand_filter: null output");
+    NMB_CUDA(cudaMemsetAsync(n_out, 0, sizeof(int64_t), (cudaStream_t)stream));
+    if (n_slots == 0) return NMB_OK;
+    int64_t blocks = (n_slots * inner + 255) / 256;
+    if (blocks > 148 * 32) blocks = 148 * 32;
+    nmb::bip_iupac_expand_filter_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+        n_mod, n_nomod, n_slots, inner, min_mean, clamp_min_mod(min_mod), out, capacity, (unsigned long long *)n_out);
     NMB_CUDA(cudaGetLastError());
     return NMB_OK;
 }

@@ -14,6 +14,8 @@ The same per bin, for all bins of a MultiBinScorer at once (one histogram launch
     sw.counts("bin_3", "GRNGAAGY", 5)                              # == scorer.context("bin_3", "a").score(...)
     sw.index("bin_3")                                              # SweepIndex over that bin's histograms
     sw.candidates(min_mean=0.7, min_mod=50)                        # pandas frame: every bin's candidates
+    sw.candidates(bipartite_letters="IUPAC")                       # bipartite halves over every IUPAC letter but N
+    sw.bipartite_iupac_counts("bin_3", "GAA", 6, "RTCG", 2)        # GAANNNNNNRTCG, modified A at position 2
 
 Letters of a motif are indexed in the order of nanomotif/constants.py:2 (A T G C R Y S W K M B D H V N); the
 modified position's own letter is fixed to the concrete canonical base and left out of the table index (a pileup
@@ -32,6 +34,7 @@ from ._lib import check, lib, ptr
 from .device import DeviceAssembly, DevicePileup, _stream
 
 IUPAC_ORDER = "ATGCRYSWKMBDHVN"
+BIP_LETTERS = IUPAC_ORDER[:-1]  # letters of the halves of degenerate bipartite motifs: every IUPAC letter but N
 _BASE_DIGIT = {"A": 0, "T": 1, "G": 2, "C": 3}
 MIN_K, MAX_K = 4, 8
 
@@ -93,6 +96,7 @@ class SweepIndex:
             check(lib.nmb_sweep_bipartite(C.byref(view), base, tile_begin, tile_count, contig_begin, contig_end,
                                           ptr(self.bip_raw), _stream()), "nmb_sweep_bipartite")
         self._bip = None
+        self._tables = {k: v for k, v in self._tables.items() if k[0] != "bip"}
         return self
 
     @classmethod
@@ -148,6 +152,62 @@ class SweepIndex:
         """(n_mod, n_nomod) of the motif left + N*gap + right with the modified base at mod_pos."""
         n_mod, n_nomod = self.bipartite_table(len(left), gap, len(right), mod_pos)
         i = self.bipartite_index(left, right)
+        return int(n_mod[i].item()) & 0xFFFFFFFF, int(n_nomod[i].item()) & 0xFFFFFFFF
+
+    # ---- degenerate bipartite motifs: the halves use the 14 IUPAC letters other than N (BIP_LETTERS) ----
+    def bipartite_iupac_table(self, a: int, g: int, b: int, mod_pos: int, canonical: str = "A", keep: bool = False):
+        """(n_mod, n_nomod) device views over all 14^(a+b-1) motifs of shape X{a} N{g} Y{b} whose halves use
+        BIP_LETTERS, with `canonical` at motif position mod_pos (inside X or Y).  Entry index:
+        bipartite_iupac_index(left, right, offset of mod_pos in left + right)."""
+        self.bipartite_block(a, g, b)
+        if a <= mod_pos < a + g or not 0 <= mod_pos < a + g + b:
+            raise ValueError("the modified position must lie in one of the two concrete parts")
+        if canonical not in _BASE_DIGIT:
+            raise ValueError("the modified position must hold a concrete base")
+        if self.bip is None:
+            raise ValueError("no bipartite histogram: call add_bipartite() first")
+        key = ("bip", a, g, b, mod_pos, canonical)
+        if key in self._tables:
+            return self._tables[key]
+        d, n = self.asm.device, a + b - 1
+        out = []
+        with torch.cuda.device(d):
+            for cls in (0, 1):
+                t = torch.empty(4 ** n, dtype=torch.int32, device=d)
+                check(lib.nmb_sweep_bip_iupac_slice(ptr(self.bip), 1, a, g, b, mod_pos, cls, _BASE_DIGIT[canonical],
+                                                    ptr(t), _stream()), "nmb_sweep_bip_iupac_slice")
+                for step in range(n):  # last axis first, as in table()
+                    outer, inner = 4 ** (n - 1 - step), 14 ** step
+                    e = torch.empty(outer * 14 * inner, dtype=torch.int32, device=d)
+                    check(lib.nmb_sweep_bip_iupac_expand(ptr(t), ptr(e), outer, inner, _stream()),
+                          "nmb_sweep_bip_iupac_expand")
+                    t = e
+                out.append(t)
+        if keep:
+            self._tables[key] = tuple(out)
+        return tuple(out)
+
+    @staticmethod
+    def bipartite_iupac_index(left: str, right: str, offset: int) -> int:
+        """Index in bipartite_iupac_table of the motif with halves left / right whose modified base is letter
+        `offset` of left + right (the gap not counted): the other letters as base-14 digits (BIP_LETTERS), first
+        letter most significant."""
+        idx = 0
+        for i, ch in enumerate(left + right):
+            if i != offset:
+                idx = idx * 14 + BIP_LETTERS.index(ch)
+        return idx
+
+    def bipartite_iupac_counts(self, left: str, gap: int, right: str, mod_pos: int, keep: bool = True) -> tuple[int, int]:
+        """(n_mod, n_nomod) of the motif left + N*gap + right, halves over BIP_LETTERS, modified base at mod_pos."""
+        if any(ch not in BIP_LETTERS for ch in left + right):
+            raise ValueError(f"half letters must be among {BIP_LETTERS}")
+        a = len(left)
+        offset = mod_pos if mod_pos < a else mod_pos - gap
+        if a <= mod_pos < a + gap or not 0 <= offset < a + len(right):
+            raise ValueError("the modified position must lie in one of the two concrete parts")
+        n_mod, n_nomod = self.bipartite_iupac_table(a, gap, len(right), mod_pos, (left + right)[offset], keep=keep)
+        i = self.bipartite_iupac_index(left, right, offset)
         return int(n_mod[i].item()) & 0xFFFFFFFF, int(n_nomod[i].item()) & 0xFFFFFFFF
 
     def all_reduce(self) -> "SweepIndex":
@@ -295,6 +355,32 @@ def decode_bipartite(counter) -> tuple[np.ndarray, np.ndarray]:
     return motifs, mod_pos
 
 
+def decode_bipartite_iupac(a: int, g: int, b: int, mod_pos: int, index, canonical: str = "A") -> np.ndarray:
+    """Vectorised inverse of SweepIndex.bipartite_iupac_index: indices of the (a, g, b, mod_pos) table ->
+    numpy array of motif strings left + "N" * g + right."""
+    rest = np.asarray(index, dtype=np.int64).copy()
+    offset = mod_pos if mod_pos < a else mod_pos - g
+    halves = np.empty((rest.size, a + b), dtype=np.uint8)
+    for i in reversed(range(a + b)):
+        if i == offset:
+            halves[:, i] = ord(canonical)
+        else:
+            halves[:, i] = _IUPAC_BYTES[rest % 14]
+            rest //= 14
+    letters = np.full((rest.size, a + g + b), ord("N"), dtype=np.uint8)
+    letters[:, :a], letters[:, a + g:] = halves[:, :a], halves[:, a:]
+    return letters.view(f"S{a + g + b}").ravel().astype(str)
+
+
+def bip_iupac_scratch_bytes() -> int:
+    """Device bytes per bin of one degenerate bipartite candidate pass (shape (4, g, 4), the largest): the largest
+    expansion step's input + output, both classes (the fused last step writes no table).  16 x 14^5 + 4 x 14^6
+    entries: 310 MB."""
+    n = 7
+    sizes = [4 ** n] + [4 ** (n - 1 - s) * 14 ** (s + 1) for s in range(n - 1)]
+    return 2 * 4 * max(x + y for x, y in zip(sizes, sizes[1:]))
+
+
 def table_scratch_bytes(k: int) -> int:
     """Device bytes per bin of one (k, mod_pos) candidate pass: the largest expansion step's input + output, both
     classes (the fused last step writes no table).  k = 8: 607.5 MB."""
@@ -408,20 +494,28 @@ class BinSweep:
             return index.bipartite_counts(m.group(1), len(m.group(2)), m.group(3), mod_pos)
         return index.counts(motif_iupac, mod_pos, keep=False)
 
+    def bipartite_iupac_counts(self, bin_name, left: str, gap: int, right: str, mod_pos: int) -> tuple[int, int]:
+        """(n_mod, n_nomod) of the motif left + "N" * gap + right in one bin, halves over BIP_LETTERS."""
+        return self.index(bin_name).bipartite_iupac_counts(left, gap, right, mod_pos, keep=False)
+
     def candidates(self, min_mean: float = 0.7, min_mod: int = 50, ks=range(MIN_K, MAX_K + 1), bipartite: bool = True,
-                   scratch_bytes: int = 8 << 30, capacity: int = 1 << 20):
+                   scratch_bytes: int = 8 << 30, capacity: int = 1 << 20, bipartite_letters: str = "ACGT"):
         """Every bin's motifs with posterior mean (5 + n_mod) / (10 + n_mod + n_nomod) >= min_mean and n_mod >=
         min_mod, as SweepIndex.candidates finds them per (k, mod_pos), plus the bipartite ones whose modified position
         holds the canonical base.  pandas frame with columns bin, mod_type, motif (IUPAC; bipartite as left + "N" *
         gap + right), mod_position, n_mod, n_nomod, mean; rows in bin order, then k, then mod_position, then table
         index, the bipartite shapes after k = 8 (by gap, then (3,3) (3,4) (4,3) (4,4), then mod_position, then
         index).  Bins are processed in chunks of max(1, scratch_bytes // table_scratch_bytes(max k)); `capacity` is
-        the initial number of hit records per pass (a pass with more hits runs again with the exact count)."""
+        the initial number of hit records per pass (a pass with more hits runs again with the exact count).
+        bipartite_letters="IUPAC" enumerates bipartite halves over the 14 letters BIP_LETTERS instead of ACGT (index
+        = SweepIndex.bipartite_iupac_index, bins in chunks of scratch_bytes // bip_iupac_scratch_bytes())."""
         if min_mod < 1:
             raise ValueError("min_mod must be >= 1: every motif without rows has the prior mean 0.5")
         ks = sorted(set(int(k) for k in ks))
         if any(not MIN_K <= k <= MAX_K for k in ks):
             raise ValueError("ks must lie in 4..8")
+        if bipartite_letters not in ("ACGT", "IUPAC"):
+            raise ValueError('bipartite_letters must be "ACGT" or "IUPAC"')
         if bipartite and self.bip_raw is None:
             raise ValueError("this BinSweep was made with bipartite=False")
         groups = [(k, mp) for k in ks for mp in range(k)]
@@ -475,21 +569,59 @@ class BinSweep:
 
                     collect(group, launch, s0)
                     del tab
-        if bipartite and n_bins:
+        bip_groups = None
+        if bipartite and n_bins and bipartite_letters == "IUPAC":
+            bip_groups = [(a, g, b, o if o < a else o + g) for g in range(4, 9) for a, b in _BIP_SHAPES
+                          for o in range(a + b)]
+            chunk = max(1, int(scratch_bytes) // bip_iupac_scratch_bytes())
+            bip = self.bip.view(-1)
+            for s0 in range(0, n_bins, chunk):
+                ns = min(chunk, n_bins - s0)
+                for j, (a, g, b, mp) in enumerate(bip_groups):
+                    n = a + b - 1
+                    with torch.cuda.device(d):
+                        tab = []
+                        for cls in (0, 1):
+                            t = torch.empty(ns * 4 ** n, dtype=torch.int32, device=d)
+                            check(lib.nmb_sweep_bip_iupac_slice(ptr(bip[s0 * BIP_SIZE:]), ns, a, g, b, mp, cls,
+                                                                _BASE_DIGIT[self.canonical], ptr(t), _stream()),
+                                  "nmb_sweep_bip_iupac_slice")
+                            tab.append(t)
+                        for step in range(n - 1):  # every axis but the first, as in bipartite_iupac_table
+                            outer, inner = ns * 4 ** (n - 1 - step), 14 ** step
+                            nxt = []
+                            for t in tab:
+                                e = torch.empty(outer * 14 * inner, dtype=torch.int32, device=d)
+                                check(lib.nmb_sweep_bip_iupac_expand(ptr(t), ptr(e), outer, inner, _stream()),
+                                      "nmb_sweep_bip_iupac_expand")
+                                nxt.append(e)
+                            tab = nxt
+
+                    def launch(out, cap, n_out, tab=tab, ns=ns, n=n):
+                        check(lib.nmb_sweep_bip_iupac_expand_filter(ptr(tab[0]), ptr(tab[1]), ns, 14 ** (n - 1),
+                                                                    float(min_mean), int(min_mod), out, cap, n_out,
+                                                                    _stream()), "nmb_sweep_bip_iupac_expand_filter")
+
+                    collect(len(groups) + j, launch, s0)
+                    del tab
+        elif bipartite and n_bins:
             def launch_bip(out, cap, n_out):
                 check(lib.nmb_sweep_bipartite_filter(ptr(self.bip), n_bins, _BASE_DIGIT[self.canonical],
                                                      float(min_mean), int(min_mod), out, cap, n_out, _stream()),
                       "nmb_sweep_bipartite_filter")
 
             collect(len(groups), launch_bip)
-        return self._frame(parts, groups)
+        return self._frame(parts, groups, bip_groups)
 
-    def _frame(self, parts, groups):
+    def _frame(self, parts, groups, bip_groups=None):
+        """bip_groups: None for the ACGT bipartite records (one group after `groups`), else the (a, g, b, mod_pos)
+        of each degenerate bipartite group, numbered from len(groups) on."""
         import pandas as pd
 
         group = np.concatenate([np.full(len(h), g, dtype=np.int64) for g, h in parts]) if parts else np.zeros(0, np.int64)
         hits = np.concatenate([h for _, h in parts]) if parts else np.zeros(0, _lib.SWEEP_HIT_DTYPE)
-        key = (hits["slot"].astype(np.int64) * (len(groups) + 1) + group) << 32 | hits["index"].astype(np.int64)
+        n_groups = len(groups) + (1 if bip_groups is None else len(bip_groups))
+        key = (hits["slot"].astype(np.int64) * n_groups + group) << 32 | hits["index"].astype(np.int64)
         order = np.argsort(key, kind="stable")
         hits, group = hits[order], group[order]
         motif = np.empty(len(hits), dtype=object)
@@ -500,8 +632,12 @@ class BinSweep:
                 k, mp = groups[g]
                 motif[sel] = decode_motifs(k, mp, hits["index"][sel], self.canonical)
                 mod_position[sel] = mp
-            else:
+            elif bip_groups is None:
                 motif[sel], mod_position[sel] = decode_bipartite(hits["index"][sel])
+            else:
+                a, gap, b, mp = bip_groups[g - len(groups)]
+                motif[sel] = decode_bipartite_iupac(a, gap, b, mp, hits["index"][sel], self.canonical)
+                mod_position[sel] = mp
         n_mod, n_nomod = hits["n_mod"].astype(np.int64), hits["n_nomod"].astype(np.int64)
         names = np.empty(len(self.bins), dtype=object)
         names[:] = self.bins
