@@ -49,7 +49,7 @@
 extern "C" {
 #endif
 
-#define NMB_ABI_VERSION 6 /* 2: lane-interleaved tile records (NMB_WORD_SLOT), chunk_info flag bits 28-30; 3: table ingest; 4: nmb_pack_motifs; 5: per-bin sweep slots; 6: degenerate bipartite sweep */
+#define NMB_ABI_VERSION 7 /* 2: lane-interleaved tile records (NMB_WORD_SLOT), chunk_info flag bits 28-30; 3: table ingest; 4: nmb_pack_motifs; 5: per-bin sweep slots; 6: degenerate bipartite sweep; 7: sweep candidate pruning */
 
 #if defined(__GNUC__)
 #define NMB_API __attribute__((visibility("default")))
@@ -585,6 +585,33 @@ NMB_API int nmb_sweep_bip_iupac_expand(const uint32_t *src, uint32_t *dst, int64
 NMB_API int nmb_sweep_bip_iupac_expand_filter(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots,
                                               int64_t inner, double min_mean, int64_t min_mod, nmb_sweep_hit *out,
                                               int64_t capacity, int64_t *n_out, void *stream);
+
+/* ---- K8 candidate pruning (ABI 7): the three filters above, minus the candidates that are a redundant
+ *      specialisation or a mixture of a one-letter neighbour in the same table ----
+ * For a candidate M and every letter other than the modified one: a widening P puts there a letter of the lattice
+ * that covers M's letter (one more base), a narrowing C one that M's letter covers; Q = P - M or M - C, n_mod and
+ * n_nomod separately, mean(Q) = (5 + q_mod) / (10 + q_mod + q_nomod).  M is pruned when (a) some widening P passes
+ * the filter and mean(Q) >= min_mean, or (b) some narrowing C passes and mean(Q) < min_mean.  Neighbours need not be
+ * candidates themselves (a flanking N, the pseudo-letter *).  Lattices, as sets of letter states (see
+ * nmb_sweep_prune_lattice): contiguous k-mers, the 15 IUPAC letters over A T G C other (N also takes "other");
+ * bipartite ACGT halves, A T G C and * = ACGT; bipartite IUPAC halves, the 14 letters other than N and * = ACGT.
+ * Arguments, records and *n_out / capacity as for the filter each one mirrors; the records are a subset of its. */
+NMB_API int nmb_sweep_expand_filter_prune(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots,
+                                          int64_t inner, int32_t k, int32_t mod_pos, double min_mean, int64_t min_mod,
+                                          nmb_sweep_hit *out, int64_t capacity, int64_t *n_out, void *stream);
+NMB_API int nmb_sweep_bipartite_filter_prune(const uint32_t *hist, int32_t n_slots, int32_t canonical, double min_mean,
+                                             int64_t min_mod, nmb_sweep_hit *out, int64_t capacity, int64_t *n_out,
+                                             void *stream);
+/* inner must be a power of 14: the number of table axes follows from it. */
+NMB_API int nmb_sweep_bip_iupac_expand_filter_prune(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots,
+                                                    int64_t inner, double min_mean, int64_t min_mod,
+                                                    nmb_sweep_hit *out, int64_t capacity, int64_t *n_out,
+                                                    void *stream);
+/* Host query, no device work: the lattice the pruning kernels use (0 contiguous, 1 bipartite ACGT, 2 bipartite
+ * IUPAC), in table letter order with the widest letter (N or *) last.  states[i]: bit s set when letter i stands for
+ * state s (A=0 T=1 G=2 C=3 other=4); widen[i] / narrow[i]: bit j set when letter j covers letter i / letter i covers
+ * letter j.  Writes up to 15 entries per array and returns the number of letters. */
+NMB_API int nmb_sweep_prune_lattice(int32_t lattice, uint32_t *states, uint32_t *widen, uint32_t *narrow);
 
 /* ---- host helper: CPython's random.sample(range(n), k) on a transplanted MT19937 state (the reference draws its
  *      background windows with random.sample, nanomotif/seq.py:202-225; its picks depend only on n, k and the

@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libnmb200.so")
 
 # ---- constants mirrored from include/nmb200.h -------------------------------------------------
-ABI_VERSION = 6
+ABI_VERSION = 7
 CHUNK_WORDS = 16
 CHUNK_BP = 512
 TILE_WORDS = 2048
@@ -122,6 +122,10 @@ SIGNATURES = {
     "nmb_sweep_bip_iupac_slice": (C.c_int, [_P, _I32, _I32, _I32, _I32, _I32, _I32, _I32, _P, _P]),
     "nmb_sweep_bip_iupac_expand": (C.c_int, [_P, _P, _I64, _I64, _P]),
     "nmb_sweep_bip_iupac_expand_filter": (C.c_int, [_P, _P, _I64, _I64, _F64, _I64, _P, _I64, _P, _P]),
+    "nmb_sweep_expand_filter_prune": (C.c_int, [_P, _P, _I64, _I64, _I32, _I32, _F64, _I64, _P, _I64, _P, _P]),
+    "nmb_sweep_bipartite_filter_prune": (C.c_int, [_P, _I32, _I32, _F64, _I64, _P, _I64, _P, _P]),
+    "nmb_sweep_bip_iupac_expand_filter_prune": (C.c_int, [_P, _P, _I64, _I64, _F64, _I64, _P, _I64, _P, _P]),
+    "nmb_sweep_prune_lattice": (C.c_int, [_I32, _P, _P, _P]),
     "nmb_add_class_planes_compact": (C.c_int, [_P, _P, _P, _P, _I64, _I32, _I32, C.POINTER(NmbAssembly), _I32, _P, _P]),
     "nmb_filter_coverage": (C.c_int, [_P, _I64, _I64, _P, _P]),
     "nmb_filter_min_mod_frequency": (C.c_int, [_P, _P, _I64, _I32, _F64, _F64, _I64, _P, _P, _P]),

@@ -523,6 +523,254 @@ __global__ void __launch_bounds__(256) sweep_filter_kernel(const uint32_t *__res
     }
 }
 
+// ---- pruning (ABI 7): drop candidates that are a redundant specialisation or a mixture of a neighbour ----
+// A candidate M (it passes sweep_pass) is widened at one letter other than the modified one by one base (P) or
+// narrowed by one (C); Q is the difference of the counts, P - M or M - C.  M is pruned when
+//   (a) some widening P passes and Q's posterior mean is >= min_mean (the added base is methylated too), or
+//   (b) some narrowing C passes and Q's posterior mean is < min_mean (the removed base is not methylated).
+// Widening and narrowing follow the covering relation of a lattice of letters, each a set of letter states:
+//   contiguous: the 15 IUPAC letters over A T G C other (N = every state: a 3-base letter widens to N, which adds a
+//               base and "other", as iupac_sums counts it);
+//   bipartite ACGT halves: A T G C and the pseudo-letter * = {A, C, G, T}, which is never a row;
+//   bipartite IUPAC halves: the 14 letters other than N and * above the 3-base letters.
+struct PruneLattice {
+    int n;               // letters; index n - 1 is the widest (N or *)
+    uint32_t states[15];  // bit s: the letter stands for state s (A=0 T=1 G=2 C=3 other=4)
+    uint32_t widen[15];   // bit e: letter e covers this letter (the smallest supersets in the lattice)
+    uint32_t narrow[15];  // bit e: this letter covers letter e
+};
+
+__host__ __device__ constexpr bool strict_subset(uint32_t x, uint32_t y) { return x != y && (x & y) == x; }
+
+__host__ __device__ constexpr PruneLattice prune_lattice(int n, const uint32_t (&states)[15]) {
+    PruneLattice L{n, {}, {}, {}};
+    for (int i = 0; i < n; ++i) L.states[i] = states[i];
+    for (int i = 0; i < n; ++i)
+        for (int j = 0; j < n; ++j) {
+            if (!strict_subset(states[i], states[j])) continue;
+            bool between = false;
+            for (int l = 0; l < n; ++l)
+                between = between || (strict_subset(states[i], states[l]) && strict_subset(states[l], states[j]));
+            if (!between) {
+                L.widen[i] |= 1u << j;
+                L.narrow[j] |= 1u << i;
+            }
+        }
+    return L;
+}
+
+// letter states in table order: IUPAC_ORDER (A T G C R Y S W K M B D H V N), the 14 without N + *, A T G C + *
+constexpr uint32_t kPruneStatesIupac[15] = {1, 2, 4, 8, 5, 10, 12, 3, 6, 9, 14, 7, 11, 13, 31};
+constexpr uint32_t kPruneStatesBipIupac[15] = {1, 2, 4, 8, 5, 10, 12, 3, 6, 9, 14, 7, 11, 13, 15};
+constexpr uint32_t kPruneStatesBipAcgt[15] = {1, 2, 4, 8, 15};
+constexpr PruneLattice kPruneLattices[3] = {prune_lattice(15, kPruneStatesIupac), prune_lattice(5, kPruneStatesBipAcgt),
+                                            prune_lattice(15, kPruneStatesBipIupac)};
+enum { kLatticeIupac = 0, kLatticeBipAcgt = 1, kLatticeBipIupac = 2 };
+__constant__ PruneLattice c_prune_lattices[3] = {kPruneLattices[0], kPruneLattices[1], kPruneLattices[2]};
+
+// Q's posterior mean, with the arithmetic of sweep_pass
+__device__ __forceinline__ double prune_q_mean(uint32_t q_mod, uint32_t q_nomod) {
+    return (5.0 + q_mod) / (10.0 + q_mod + q_nomod);
+}
+
+// Whether the candidate (m, u) is pruned by the neighbour (nm, nu) that widens it (`wider`) or that it widens.
+__device__ __forceinline__ bool pruned_by(bool wider, uint32_t m, uint32_t u, uint32_t nm, uint32_t nu, double min_mean,
+                                          uint32_t min_mod) {
+    if (!sweep_pass(nm, nu, min_mean, min_mod)) return false;
+    return wider ? prune_q_mean(nm - m, nu - u) >= min_mean : prune_q_mean(m - nm, u - nu) < min_mean;
+}
+
+// Sum of s[t * inner] over the states t of `states` (the register axis of one table entry).
+template <int S>
+__device__ __forceinline__ uint32_t state_sum(const uint32_t *s, int64_t inner, uint32_t states) {
+    uint32_t v = 0;
+#pragma unroll
+    for (int t = 0; t < S; ++t)
+        if (states >> t & 1) v += s[t * inner];
+    return v;
+}
+
+// v[l] for a letter l known only at run time, without moving v out of registers.
+template <int N>
+__device__ __forceinline__ uint32_t pick(const uint32_t (&v)[N], int l) {
+    uint32_t x = 0;
+#pragma unroll
+    for (int j = 0; j < N; ++j) x = j == l ? v[j] : x;
+    return x;
+}
+
+// Whether letter d of the register axis at entry r of one slot's [S][inner] input is pruned (mb / ub: n_mod / n_nomod
+// of the slot; m / u: the register sums of entry r, index L.n - 1 the widest letter).  The other axes are the base-B
+// digits of r, most significant first; a neighbour letter e >= B on such an axis (*) is the sum of the entries with
+// its states' digits, which are the concrete letters 0..S-1 of the table.
+template <int S, int B>
+__device__ __forceinline__ bool expand_pruned(const PruneLattice &L, const uint32_t *mb, const uint32_t *ub,
+                                              int64_t inner, int64_t r, int d, const uint32_t (&m)[15],
+                                              const uint32_t (&u)[15], double min_mean, uint32_t min_mod) {
+    const uint32_t md = pick(m, d), ud = pick(u, d);
+    for (uint32_t e = L.widen[d] | L.narrow[d]; e; e &= e - 1) {
+        const int l = __ffs(e) - 1;
+        if (pruned_by(L.widen[d] >> l & 1, md, ud, pick(m, l), pick(u, l), min_mean, min_mod)) return true;
+    }
+    const uint32_t sd = L.states[d];
+    for (int64_t pv = inner / B; pv >= 1; pv /= B) {
+        const int c = (int)(r / pv % B);
+        for (uint32_t e = L.widen[c] | L.narrow[c]; e; e &= e - 1) {
+            const int l = __ffs(e) - 1;
+            uint32_t nm = 0, nu = 0;
+            if (l < B) {
+                const int64_t r2 = r + (int64_t)(l - c) * pv;
+                nm = state_sum<S>(mb + r2, inner, sd);
+                nu = state_sum<S>(ub + r2, inner, sd);
+            } else {
+                for (uint32_t t = L.states[l]; t; t &= t - 1) {
+                    const int64_t r2 = r + (int64_t)(__ffs(t) - 1 - c) * pv;
+                    nm += state_sum<S>(mb + r2, inner, sd);
+                    nu += state_sum<S>(ub + r2, inner, sd);
+                }
+            }
+            if (pruned_by(L.widen[c] >> l & 1, md, ud, nm, nu, min_mean, min_mod)) return true;
+        }
+    }
+    return false;
+}
+
+// sweep_expand_filter_kernel with pruning: the same candidates, minus the pruned ones.  Input [slot][5][inner],
+// inner = 15^(k-2): neighbours on the first axis come from the 15 register sums, on the other k - 2 axes from the
+// entry with that base-15 digit of r replaced (a flanking N included: GATCN prunes GATCB).
+__global__ void __launch_bounds__(256) sweep_expand_filter_prune_kernel(
+    const uint32_t *__restrict__ n_mod, const uint32_t *__restrict__ n_nomod, int64_t n_slots, int64_t inner,
+    bool skip_first_n, bool skip_last_n, double min_mean, uint32_t min_mod, nmb_sweep_hit *__restrict__ out,
+    int64_t capacity, unsigned long long *__restrict__ n_out) {
+    const PruneLattice &L = c_prune_lattices[kLatticeIupac];
+    const int64_t n = n_slots * inner;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const int64_t slot = i / inner, r = i - slot * inner;
+        const uint32_t *mb = n_mod + slot * 5 * inner, *ub = n_nomod + slot * 5 * inner;
+        uint32_t m[15], u[15];
+        iupac_sums(mb + r, inner, m);
+        uint32_t hits = 0;
+        const int last = skip_last_n && r % 15 == 14 ? 0 : 15;
+        for (int d = 0; d < last; ++d)
+            if (m[d] >= min_mod) hits |= 1u << d;
+        if (skip_first_n) hits &= ~(1u << 14);
+        if (!hits) continue;
+        iupac_sums(ub + r, inner, u);
+        for (int d = 0; d < 15; ++d)
+            if ((hits >> d & 1) && !sweep_pass(m[d], u[d], min_mean, min_mod)) hits &= ~(1u << d);
+#pragma unroll 1
+        for (uint32_t h = hits; h; h &= h - 1) {  // only candidates that pass look at their neighbours
+            const int d = __ffs(h) - 1;
+            if (expand_pruned<5, 15>(L, mb, ub, inner, r, d, m, u, min_mean, min_mod)) hits &= ~(1u << d);
+        }
+        if (!hits) continue;
+        unsigned long long at = atomicAdd(n_out, (unsigned long long)__popc(hits));
+        for (int d = 0; d < 15; ++d) {
+            if (!(hits >> d & 1)) continue;
+            if ((int64_t)at < capacity)
+                out[at] = nmb_sweep_hit{(int32_t)slot, (uint32_t)(d * inner + r), m[d], u[d]};
+            ++at;
+        }
+    }
+}
+
+// bip_iupac_expand_filter_kernel with pruning.  Input [slot][4][inner], inner = 14^(n-1): every axis uses the
+// 14 letters + * lattice; * on the register axis is the sum of the 4 states, on another axis the sum of the entries
+// with A, T, G and C there.
+__global__ void __launch_bounds__(256) bip_iupac_expand_filter_prune_kernel(
+    const uint32_t *__restrict__ n_mod, const uint32_t *__restrict__ n_nomod, int64_t n_slots, int64_t inner,
+    double min_mean, uint32_t min_mod, nmb_sweep_hit *__restrict__ out, int64_t capacity,
+    unsigned long long *__restrict__ n_out) {
+    const PruneLattice &L = c_prune_lattices[kLatticeBipIupac];
+    const int64_t n = n_slots * inner;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const int64_t slot = i / inner, r = i - slot * inner;
+        const uint32_t *mb = n_mod + slot * 4 * inner, *ub = n_nomod + slot * 4 * inner;
+        uint32_t m[15], u[15];
+        const uint32_t *s = mb + r;
+        acgt_sums(s[0], s[inner], s[2 * inner], s[3 * inner], m);
+        uint32_t hits = 0;
+        for (int d = 0; d < 14; ++d)
+            if (m[d] >= min_mod) hits |= 1u << d;
+        if (!hits) continue;
+        m[14] = s[0] + s[inner] + s[2 * inner] + s[3 * inner];
+        s = ub + r;
+        acgt_sums(s[0], s[inner], s[2 * inner], s[3 * inner], u);
+        u[14] = s[0] + s[inner] + s[2 * inner] + s[3 * inner];
+        for (int d = 0; d < 14; ++d)
+            if ((hits >> d & 1) && !sweep_pass(m[d], u[d], min_mean, min_mod)) hits &= ~(1u << d);
+#pragma unroll 1
+        for (uint32_t h = hits; h; h &= h - 1) {  // only candidates that pass look at their neighbours
+            const int d = __ffs(h) - 1;
+            if (expand_pruned<4, 14>(L, mb, ub, inner, r, d, m, u, min_mean, min_mod)) hits &= ~(1u << d);
+        }
+        if (!hits) continue;
+        unsigned long long at = atomicAdd(n_out, (unsigned long long)__popc(hits));
+        for (int d = 0; d < 14; ++d) {
+            if (!(hits >> d & 1)) continue;
+            if ((int64_t)at < capacity)
+                out[at] = nmb_sweep_hit{(int32_t)slot, (uint32_t)(d * inner + r), m[d], u[d]};
+            ++at;
+        }
+    }
+}
+
+// bip_filter_kernel with pruning: every letter but the modified one widens to *, the sum of the 4 counters whose
+// code differs only in that letter's x and y bits (same block, offset and class).
+__global__ void __launch_bounds__(256) bip_filter_prune_kernel(const uint32_t *__restrict__ hist, int64_t n_slots,
+                                                               int canonical, double min_mean, uint32_t min_mod,
+                                                               nmb_sweep_hit *__restrict__ out, int64_t capacity,
+                                                               unsigned long long *__restrict__ n_out) {
+    const PruneLattice &L = c_prune_lattices[kLatticeBipAcgt];
+    constexpr int64_t b33 = bip_block(3, 3), b34 = bip_block(3, 4), b43 = bip_block(4, 3);
+    constexpr int64_t per_gap = bip_offset(3, kBipMinGap + 1, 3);
+    const int64_t n = n_slots * kBipHistSize;
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const uint32_t m = hist[i];
+        if (m < min_mod) continue;
+        const int64_t slot = i / kBipHistSize, j = i - slot * kBipHistSize;
+        int64_t rem = j % per_gap;
+        int a, b;
+        if (rem < b33) { a = 3; b = 3; }
+        else if (rem < b33 + b34) { a = 3; b = 4; rem -= b33; }
+        else if (rem < b33 + b34 + b43) { a = 4; b = 3; rem -= b33 + b34; }
+        else { a = 4; b = 4; rem -= b33 + b34 + b43; }
+        const int bits = 2 * (a + b);
+        const int oc = (int)(rem >> bits), code = (int)(rem & ((1 << bits) - 1));
+        if (oc & 1) continue;
+        const int o = oc >> 1;
+        auto xbit = [&](int p) { return p < a ? p : 2 * a + (p - a); };
+        auto ybit = [&](int p) { return p < a ? a + p : 2 * a + b + (p - a); };
+        auto letter = [&](int p) { return ((code >> xbit(p)) & 1) << 1 | ((code >> ybit(p)) & 1); };
+        if (letter(o) != canonical) continue;
+        const uint32_t u = hist[i + (1 << bits)];
+        if (!sweep_pass(m, u, min_mean, min_mod)) continue;
+        const uint32_t *block = hist + (i - code);  // code 0 of this (shape, offset, class 0) block
+        bool pruned = false;
+        for (int p = 0; p < a + b && !pruned; ++p) {
+            if (p == o) continue;
+            const int c = letter(p), rest = code & ~(1 << xbit(p) | 1 << ybit(p));
+            for (uint32_t e = L.widen[c] | L.narrow[c]; e && !pruned; e &= e - 1) {
+                const int l = __ffs(e) - 1;
+                uint32_t nm = 0, nu = 0;
+                for (uint32_t t = L.states[l]; t; t &= t - 1) {
+                    const int x = __ffs(t) - 1;
+                    const int c2 = rest | (x >> 1) << xbit(p) | (x & 1) << ybit(p);
+                    nm += block[c2];
+                    nu += block[c2 + (1 << bits)];
+                }
+                pruned = pruned_by(L.widen[c] >> l & 1, m, u, nm, nu, min_mean, min_mod);
+            }
+        }
+        if (pruned) continue;
+        const unsigned long long at = atomicAdd(n_out, 1ull);
+        if ((int64_t)at < capacity) out[at] = nmb_sweep_hit{(int32_t)slot, (uint32_t)j, m, u};
+    }
+}
+
 }  // namespace nmb
 
 extern "C" {
@@ -706,6 +954,76 @@ int nmb_sweep_bip_iupac_expand_filter(const uint32_t *n_mod, const uint32_t *n_n
         n_mod, n_nomod, n_slots, inner, min_mean, clamp_min_mod(min_mod), out, capacity, (unsigned long long *)n_out);
     NMB_CUDA(cudaGetLastError());
     return NMB_OK;
+}
+
+int nmb_sweep_expand_filter_prune(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots, int64_t inner,
+                                  int32_t k, int32_t mod_pos, double min_mean, int64_t min_mod, nmb_sweep_hit *out,
+                                  int64_t capacity, int64_t *n_out, void *stream) {
+    NMB_REQUIRE(n_mod && n_nomod && n_out && n_slots >= 0 && capacity >= 0 && min_mod >= 0 && k >= nmb::kSweepMinK &&
+                    k <= nmb::kSweepMaxK && mod_pos >= 0 && mod_pos < k,
+                "nmb_sweep_expand_filter_prune: bad argument");
+    int64_t want = 1;
+    for (int i = 0; i < k - 2; ++i) want *= 15;
+    NMB_REQUIRE(inner == want, "nmb_sweep_expand_filter_prune: inner %lld is not 15^(k-2) for k = %d", (long long)inner,
+                k);
+    NMB_REQUIRE(capacity == 0 || out, "nmb_sweep_expand_filter_prune: null output");
+    NMB_CUDA(cudaMemsetAsync(n_out, 0, sizeof(int64_t), (cudaStream_t)stream));
+    if (n_slots == 0) return NMB_OK;
+    int64_t blocks = (n_slots * inner + 255) / 256;
+    if (blocks > 148 * 32) blocks = 148 * 32;
+    nmb::sweep_expand_filter_prune_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+        n_mod, n_nomod, n_slots, inner, mod_pos != 0, mod_pos != k - 1, min_mean, clamp_min_mod(min_mod), out, capacity,
+        (unsigned long long *)n_out);
+    NMB_CUDA(cudaGetLastError());
+    return NMB_OK;
+}
+
+int nmb_sweep_bipartite_filter_prune(const uint32_t *hist, int32_t n_slots, int32_t canonical, double min_mean,
+                                     int64_t min_mod, nmb_sweep_hit *out, int64_t capacity, int64_t *n_out,
+                                     void *stream) {
+    NMB_REQUIRE(hist && n_out && n_slots >= 0 && canonical >= 0 && canonical < 4 && capacity >= 0 && min_mod >= 0,
+                "nmb_sweep_bipartite_filter_prune: bad argument");
+    NMB_REQUIRE(capacity == 0 || out, "nmb_sweep_bipartite_filter_prune: null output");
+    NMB_CUDA(cudaMemsetAsync(n_out, 0, sizeof(int64_t), (cudaStream_t)stream));
+    if (n_slots == 0) return NMB_OK;
+    int64_t blocks = ((int64_t)n_slots * nmb::kBipHistSize + 255) / 256;
+    if (blocks > 148 * 32) blocks = 148 * 32;
+    nmb::bip_filter_prune_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+        hist, n_slots, canonical, min_mean, clamp_min_mod(min_mod), out, capacity, (unsigned long long *)n_out);
+    NMB_CUDA(cudaGetLastError());
+    return NMB_OK;
+}
+
+int nmb_sweep_bip_iupac_expand_filter_prune(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots,
+                                            int64_t inner, double min_mean, int64_t min_mod, nmb_sweep_hit *out,
+                                            int64_t capacity, int64_t *n_out, void *stream) {
+    NMB_REQUIRE(n_mod && n_nomod && n_out && n_slots >= 0 && inner > 0 && inner <= 0xFFFFFFFFll / 14 &&
+                    capacity >= 0 && min_mod >= 0,
+                "nmb_sweep_bip_iupac_expand_filter_prune: bad argument");
+    int64_t p = 1;
+    while (p < inner) p *= 14;
+    NMB_REQUIRE(p == inner, "nmb_sweep_bip_iupac_expand_filter_prune: inner %lld is not a power of 14",
+                (long long)inner);
+    NMB_REQUIRE(capacity == 0 || out, "nmb_sweep_bip_iupac_expand_filter_prune: null output");
+    NMB_CUDA(cudaMemsetAsync(n_out, 0, sizeof(int64_t), (cudaStream_t)stream));
+    if (n_slots == 0) return NMB_OK;
+    int64_t blocks = (n_slots * inner + 255) / 256;
+    if (blocks > 148 * 32) blocks = 148 * 32;
+    nmb::bip_iupac_expand_filter_prune_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+        n_mod, n_nomod, n_slots, inner, min_mean, clamp_min_mod(min_mod), out, capacity, (unsigned long long *)n_out);
+    NMB_CUDA(cudaGetLastError());
+    return NMB_OK;
+}
+
+int nmb_sweep_prune_lattice(int32_t lattice, uint32_t *states, uint32_t *widen, uint32_t *narrow) {
+    NMB_REQUIRE(lattice >= 0 && lattice < 3 && states && widen && narrow, "nmb_sweep_prune_lattice: bad argument");
+    const nmb::PruneLattice &L = nmb::kPruneLattices[lattice];
+    for (int i = 0; i < L.n; ++i) {
+        states[i] = L.states[i];
+        widen[i] = L.widen[i];
+        narrow[i] = L.narrow[i];
+    }
+    return L.n;
 }
 
 int nmb_sweep_expand(const uint32_t *src, uint32_t *dst, int64_t outer, int64_t inner, void *stream) {

@@ -15,6 +15,7 @@ The same per bin, for all bins of a MultiBinScorer at once (one histogram launch
     sw.index("bin_3")                                              # SweepIndex over that bin's histograms
     sw.candidates(min_mean=0.7, min_mod=50)                        # pandas frame: every bin's candidates
     sw.candidates(bipartite_letters="IUPAC")                       # bipartite halves over every IUPAC letter but N
+    sw.candidates(prune=True)                                      # minus specialisations and mixtures (GATC, not GATCA)
     sw.bipartite_iupac_counts("bin_3", "GAA", 6, "RTCG", 2)        # GAANNNNNNRTCG, modified A at position 2
 
 Letters of a motif are indexed in the order of nanomotif/constants.py:2 (A T G C R Y S W K M B D H V N); the
@@ -372,6 +373,19 @@ def decode_bipartite_iupac(a: int, g: int, b: int, mod_pos: int, index, canonica
     return letters.view(f"S{a + g + b}").ravel().astype(str)
 
 
+PRUNE_LATTICES = {"contiguous": 0, "bipartite_acgt": 1, "bipartite_iupac": 2}
+
+
+def prune_lattice(name: str) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+    """(states, widen, narrow) of the letter lattice the pruning kernels use (nmb_sweep_prune_lattice), in table
+    letter order with the widest letter (N or *) last: states[i] bit s = letter i stands for state s (A T G C other),
+    widen[i] / narrow[i] bit j = letter j covers letter i / letter i covers letter j."""
+    arrays = [np.zeros(15, dtype=np.uint32) for _ in range(3)]
+    n = lib.nmb_sweep_prune_lattice(PRUNE_LATTICES[name], *(ptr(a) for a in arrays))
+    check(n, "nmb_sweep_prune_lattice")
+    return tuple(a[:n] for a in arrays)
+
+
 def bip_iupac_scratch_bytes() -> int:
     """Device bytes per bin of one degenerate bipartite candidate pass (shape (4, g, 4), the largest): the largest
     expansion step's input + output, both classes (the fused last step writes no table).  16 x 14^5 + 4 x 14^6
@@ -499,7 +513,8 @@ class BinSweep:
         return self.index(bin_name).bipartite_iupac_counts(left, gap, right, mod_pos, keep=False)
 
     def candidates(self, min_mean: float = 0.7, min_mod: int = 50, ks=range(MIN_K, MAX_K + 1), bipartite: bool = True,
-                   scratch_bytes: int = 8 << 30, capacity: int = 1 << 20, bipartite_letters: str = "ACGT"):
+                   scratch_bytes: int = 8 << 30, capacity: int = 1 << 20, bipartite_letters: str = "ACGT",
+                   prune: bool = False):
         """Every bin's motifs with posterior mean (5 + n_mod) / (10 + n_mod + n_nomod) >= min_mean and n_mod >=
         min_mod, as SweepIndex.candidates finds them per (k, mod_pos), plus the bipartite ones whose modified position
         holds the canonical base.  pandas frame with columns bin, mod_type, motif (IUPAC; bipartite as left + "N" *
@@ -508,7 +523,14 @@ class BinSweep:
         index).  Bins are processed in chunks of max(1, scratch_bytes // table_scratch_bytes(max k)); `capacity` is
         the initial number of hit records per pass (a pass with more hits runs again with the exact count).
         bipartite_letters="IUPAC" enumerates bipartite halves over the 14 letters BIP_LETTERS instead of ACGT (index
-        = SweepIndex.bipartite_iupac_index, bins in chunks of scratch_bytes // bip_iupac_scratch_bytes())."""
+        = SweepIndex.bipartite_iupac_index, bins in chunks of scratch_bytes // bip_iupac_scratch_bytes()).
+
+        prune=True drops every candidate that a one-letter neighbour in its own table shows to be a redundant
+        specialisation (a widening P of a letter other than the modified one passes and Q = P - M has posterior mean
+        >= min_mean: GATCA next to GATCM) or a mixture (a narrowing C passes and Q = M - C has mean < min_mean: CCHGG
+        next to CCWGG), in the same passes on the device (nmb_sweep_*_prune); the frame is the matching subsequence
+        of the prune=False one.  Lattices: the 15 IUPAC letters for k-mers, ACGT + * or the 14 letters + * for the
+        bipartite halves (* = any of ACGT, never a row)."""
         if min_mod < 1:
             raise ValueError("min_mod must be >= 1: every motif without rows has the prior mean 0.5")
         ks = sorted(set(int(k) for k in ks))
@@ -520,6 +542,10 @@ class BinSweep:
             raise ValueError("this BinSweep was made with bipartite=False")
         groups = [(k, mp) for k in ks for mp in range(k)]
         d, n_bins = self.asm.device, len(self.bins)
+        suffix = "_prune" if prune else ""  # the same passes, with the neighbour test
+        expand_filter = getattr(lib, "nmb_sweep_expand_filter" + suffix)
+        bip_iupac_filter = getattr(lib, "nmb_sweep_bip_iupac_expand_filter" + suffix)
+        bip_filter = getattr(lib, "nmb_sweep_bipartite_filter" + suffix)
         state = {"cap": max(int(capacity), 1)}
         parts = []  # (group, hit records)
 
@@ -563,9 +589,8 @@ class BinSweep:
                                 nxt.append(e)
                             tab = nxt
                     def launch(out, cap, n_out, tab=tab, ns=ns, k=k, mp=mp):
-                        check(lib.nmb_sweep_expand_filter(ptr(tab[0]), ptr(tab[1]), ns, 15 ** (k - 2), k, mp,
-                                                          float(min_mean), int(min_mod), out, cap, n_out, _stream()),
-                              "nmb_sweep_expand_filter")
+                        check(expand_filter(ptr(tab[0]), ptr(tab[1]), ns, 15 ** (k - 2), k, mp, float(min_mean),
+                                            int(min_mod), out, cap, n_out, _stream()), expand_filter.__name__)
 
                     collect(group, launch, s0)
                     del tab
@@ -598,17 +623,15 @@ class BinSweep:
                             tab = nxt
 
                     def launch(out, cap, n_out, tab=tab, ns=ns, n=n):
-                        check(lib.nmb_sweep_bip_iupac_expand_filter(ptr(tab[0]), ptr(tab[1]), ns, 14 ** (n - 1),
-                                                                    float(min_mean), int(min_mod), out, cap, n_out,
-                                                                    _stream()), "nmb_sweep_bip_iupac_expand_filter")
+                        check(bip_iupac_filter(ptr(tab[0]), ptr(tab[1]), ns, 14 ** (n - 1), float(min_mean),
+                                               int(min_mod), out, cap, n_out, _stream()), bip_iupac_filter.__name__)
 
                     collect(len(groups) + j, launch, s0)
                     del tab
         elif bipartite and n_bins:
             def launch_bip(out, cap, n_out):
-                check(lib.nmb_sweep_bipartite_filter(ptr(self.bip), n_bins, _BASE_DIGIT[self.canonical],
-                                                     float(min_mean), int(min_mod), out, cap, n_out, _stream()),
-                      "nmb_sweep_bipartite_filter")
+                check(bip_filter(ptr(self.bip), n_bins, _BASE_DIGIT[self.canonical], float(min_mean), int(min_mod),
+                                 out, cap, n_out, _stream()), bip_filter.__name__)
 
             collect(len(groups), launch_bip)
         return self._frame(parts, groups, bip_groups)
