@@ -49,7 +49,7 @@
 extern "C" {
 #endif
 
-#define NMB_ABI_VERSION 7 /* 2: lane-interleaved tile records (NMB_WORD_SLOT), chunk_info flag bits 28-30; 3: table ingest; 4: nmb_pack_motifs; 5: per-bin sweep slots; 6: degenerate bipartite sweep; 7: sweep candidate pruning */
+#define NMB_ABI_VERSION 8 /* 2: lane-interleaved tile records (NMB_WORD_SLOT), chunk_info flag bits 28-30; 3: table ingest; 4: nmb_pack_motifs; 5: per-bin sweep slots; 6: degenerate bipartite sweep; 7: sweep candidate pruning; 8: one sweep entry point per filter and histogram kind (slots and prune as arguments) */
 
 #if defined(__GNUC__)
 #define NMB_API __attribute__((visibility("default")))
@@ -469,42 +469,50 @@ NMB_API int nmb_bin_matrix(const int64_t *stats, const double *value, const uint
 
 /* ---- K8: exhaustive candidate sweep (BASELINE.json configs[4]): counts of EVERY IUPAC motif of length 4..8
  *      at every modified position from one pass over the assembly (csrc/sweep.cu) ----
- * hist: nmb_sweep_hist_size() uint32 counters, zeroed by the caller; counters ADD, so several calls (contig
- * ranges, GPUs after an all-reduce) accumulate.  For k = 4..8 the block at sum_{j<k} j*2*5^j holds
- * [o = 0..k-1][class: 0 methylated, 1 unmethylated][5^k windows]; a window's index is its letters as base-5
- * digits, first letter most significant, letter states A=0 T=1 G=2 C=3 other=4.  Counted: every pileup row of
- * the class planes (one mod type) under every window that lies inside one contig of [contig_begin, contig_end);
- * '-' rows count under the reverse complement of the window at the mirrored offset. */
+ * hist: nmb_sweep_hist_size() uint32 counters per slot (a slot is one histogram, e.g. one per bin; n_slots of them
+ * stacked), zeroed by the caller; counters ADD, so several calls (contig ranges, GPUs after an all-reduce)
+ * accumulate.  For k = 4..8 the block at sum_{j<k} j*2*5^j holds [o = 0..k-1][class: 0 methylated, 1
+ * unmethylated][5^k windows]; a window's index is its letters as base-5 digits, first letter most significant, letter
+ * states A=0 T=1 G=2 C=3 other=4.  Counted: every pileup row of the class planes (one mod type) under every window
+ * that lies inside one counted contig; '-' rows count under the reverse complement of the window at the mirrored
+ * offset.  contig_slot == NULL: one histogram (n_slots must be 1), the contigs of [contig_begin, contig_end) counted.
+ * Otherwise contig_slot[c] (device int32, one entry per contig of the assembly) = the slot that the rows under the
+ * windows of contig c count into, -1 (or any value outside [0, n_slots)) skips the contig, and the contig range is
+ * ignored.  A window never leaves its contig, so contigs of different slots may share tiles. */
 NMB_API int64_t nmb_sweep_hist_size(void);
 NMB_API int nmb_sweep_hist(const nmb_assembly *assembly_h, const uint32_t *class_records_of_modtype, int32_t tile_begin,
-                           int32_t tile_count, int32_t contig_begin, int32_t contig_end, uint32_t *hist, void *stream);
-/* nmb_sweep_hist leaves the histogram RAW: only the k = 8 block is counted row by row (8 atomic adds per pileup row
+                           int32_t tile_count, int32_t contig_begin, int32_t contig_end, const int32_t *contig_slot,
+                           int32_t n_slots, uint32_t *hist, void *stream);
+/* nmb_sweep_hist leaves the histograms RAW: only the k = 8 block is counted row by row (8 atomic adds per pileup row
  * instead of 30); the blocks of k < 8 hold just the windows at contig ends that have no one-letter extension inside
- * the contig.  nmb_sweep_finalize completes them in place, hist[k] += marginal of hist[k+1] over the trailing letter,
- * k = 7 .. 4.  Call it ONCE, after every nmb_sweep_hist call (and after the histograms of several GPUs have been
- * summed: raw histograms add, finalized ones must not be finalized again). */
-NMB_API int nmb_sweep_finalize(uint32_t *hist, void *stream);
+ * the contig.  nmb_sweep_finalize completes n_slots (1..65535) stacked histograms in place, hist[k] += marginal of
+ * hist[k+1] over the trailing letter, k = 7 .. 4.  Call it ONCE, after every nmb_sweep_hist call (and after the
+ * histograms of several GPUs have been summed: raw histograms add, finalized ones must not be finalized again). */
+NMB_API int nmb_sweep_finalize(uint32_t *hist, int32_t n_slots, void *stream);
 
 /* The bipartite half of the sweep: shapes X{a} N{g} Y{b}, a, b in {3, 4}, g in 4..8, concrete letters only.
- * hist: nmb_sweep_bipartite_size() uint32 counters (zeroed by the caller, counters add); shapes are stored g major,
- * then (3,3) (3,4) (4,3) (4,4); a shape's block is [o = 0..a+b-1 over the concrete letters][class][4^(a+b)] with
- * window index xL | yL << a | xR << 2a | yR << (2a + b), x / y = high / low code bit of each letter (A=0 T=1 G=2
- * C=3), letter i of a part at bit i. */
+ * hist: nmb_sweep_bipartite_size() uint32 counters per slot (zeroed by the caller, counters add); contig_begin,
+ * contig_end, contig_slot and n_slots as for nmb_sweep_hist.  Shapes are stored g major, then (3,3) (3,4) (4,3)
+ * (4,4); a shape's block is [o = 0..a+b-1 over the concrete letters][class][4^(a+b)] with window index
+ * xL | yL << a | xR << 2a | yR << (2a + b), x / y = high / low code bit of each letter (A=0 T=1 G=2 C=3), letter i of
+ * a part at bit i. */
 NMB_API int64_t nmb_sweep_bipartite_size(void);
 NMB_API int nmb_sweep_bipartite(const nmb_assembly *assembly_h, const uint32_t *class_records_of_modtype,
                                 int32_t tile_begin, int32_t tile_count, int32_t contig_begin, int32_t contig_end,
-                                uint32_t *hist, void *stream);
+                                const int32_t *contig_slot, int32_t n_slots, uint32_t *hist, void *stream);
 
-/* Like nmb_sweep_hist, nmb_sweep_bipartite leaves a RAW histogram: only the shapes (4, g, 4) are counted row by row
+/* Like nmb_sweep_hist, nmb_sweep_bipartite leaves RAW histograms: only the shapes (4, g, 4) are counted row by row
  * (40 atomic adds per pileup row instead of 140); (4,g,3), (3,g,4) and (3,g,3) hold just the windows whose extending
- * letter is not a concrete letter of the same contig.  nmb_sweep_bipartite_finalize completes them in place by summing
- * the longer shapes over the dropped letter.  Call it ONCE after all passes / after summing the GPUs' raw histograms. */
-NMB_API int nmb_sweep_bipartite_finalize(uint32_t *hist, void *stream);
+ * letter is not a concrete letter of the same contig.  nmb_sweep_bipartite_finalize completes n_slots (1..65535)
+ * stacked histograms in place by summing the longer shapes over the dropped letter.  Call it ONCE after all passes /
+ * after summing the GPUs' raw histograms. */
+NMB_API int nmb_sweep_bipartite_finalize(uint32_t *hist, int32_t n_slots, void *stream);
 
-/* dst[hi][lo] = src[hi][digit][lo] with lo < axis_stride: fixes one base-5 axis (the modified position's own
- * letter) and drops it.  n_out = elements of dst. */
-NMB_API int nmb_sweep_slice(const uint32_t *src, uint32_t *dst, int64_t n_out, int64_t axis_stride, int32_t digit,
-                            void *stream);
+/* dst[slot][hi][lo] = src[slot * src_slot_stride + (hi * 5 + digit) * axis_stride + lo] with lo < axis_stride, for
+ * n_slots (1..65535) sources: fixes one base-5 axis (the modified position's own letter) and drops it.  n_out =
+ * elements of dst per slot. */
+NMB_API int nmb_sweep_slice(const uint32_t *src, int64_t src_slot_stride, int32_t n_slots, uint32_t *dst,
+                            int64_t n_out, int64_t axis_stride, int32_t digit, void *stream);
 
 /* dst[outer][15][inner] = sums of src[outer][5][inner] over the letters of each IUPAC code, in the order of
  * nanomotif/constants.py:2 (A T G C R Y S W K M B D H V N; N also takes the "other" state, like the regex
@@ -517,25 +525,6 @@ NMB_API int nmb_sweep_expand(const uint32_t *src, uint32_t *dst, int64_t outer, 
 NMB_API int nmb_sweep_filter(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n, double min_mean,
                              int64_t min_mod, int64_t *out_index, int64_t capacity, int64_t *n_out, void *stream);
 
-/* ---- K8 per bin: many histograms ("slots", e.g. one per bin) from ONE pass, stacked at nmb_sweep_hist_size() /
- *      nmb_sweep_bipartite_size() counters per slot ----
- * contig_slot[c] (device int32, one entry per contig of the assembly) = the slot that the rows under the windows of
- * contig c count into; -1 (or any value outside [0, n_slots)) skips the contig.  A window never leaves its contig, so
- * contigs of different slots may share tiles.  The counters ADD like those of nmb_sweep_hist; nmb_sweep_hist /
- * nmb_sweep_bipartite are the one-slot case of the same kernel (contig range instead of a map). */
-NMB_API int nmb_sweep_hist_slots(const nmb_assembly *assembly_h, const uint32_t *class_records_of_modtype,
-                                 int32_t tile_begin, int32_t tile_count, const int32_t *contig_slot, int32_t n_slots,
-                                 uint32_t *hist, void *stream);
-NMB_API int nmb_sweep_bipartite_slots(const nmb_assembly *assembly_h, const uint32_t *class_records_of_modtype,
-                                      int32_t tile_begin, int32_t tile_count, const int32_t *contig_slot, int32_t n_slots,
-                                      uint32_t *hist, void *stream);
-/* nmb_sweep_finalize / nmb_sweep_bipartite_finalize of n_slots (1..65535) stacked raw histograms, in place. */
-NMB_API int nmb_sweep_finalize_slots(uint32_t *hist, int32_t n_slots, void *stream);
-NMB_API int nmb_sweep_bipartite_finalize_slots(uint32_t *hist, int32_t n_slots, void *stream);
-/* nmb_sweep_slice of n_slots (1..65535) sources src + s * src_slot_stride -> dst stacked [slot][n_out]. */
-NMB_API int nmb_sweep_slice_slots(const uint32_t *src, int64_t src_slot_stride, int32_t n_slots, uint32_t *dst,
-                                  int64_t n_out, int64_t axis_stride, int32_t digit, void *stream);
-
 /* One candidate of the per-slot filters: table index (IUPAC) or counter index in the slot's bipartite histogram. */
 typedef struct nmb_sweep_hit {
     int32_t slot;
@@ -544,23 +533,34 @@ typedef struct nmb_sweep_hit {
     uint32_t n_nomod;
 } nmb_sweep_hit; /* 16 bytes */
 
-/* The LAST nmb_sweep_expand pass of a (k, mod_pos) table fused with nmb_sweep_filter: n_mod / n_nomod are stacked
+/* The three per-slot candidate filters below record every motif with n_mod >= min_mod and posterior mean
+ * (5 + n_mod) / (10 + n_mod + n_nomod) >= min_mean -- nmb_sweep_filter's test, bit for bit -- as nmb_sweep_hit
+ * records.  *n_out (device int64) = number of hits, in no particular order, of which at most `capacity` are written.
+ *
+ * prune (0 or 1): 1 also drops the candidates that are a redundant specialisation or a mixture of a one-letter
+ * neighbour in the same table; the records are then a subset of those with prune = 0.  For a candidate M and every
+ * letter other than the modified one: a widening P puts there a letter of the lattice that covers M's letter (one
+ * more base), a narrowing C one that M's letter covers; Q = P - M or M - C, n_mod and n_nomod separately, mean(Q) =
+ * (5 + q_mod) / (10 + q_mod + q_nomod).  M is pruned when (a) some widening P passes the filter and mean(Q) >=
+ * min_mean, or (b) some narrowing C passes and mean(Q) < min_mean.  Neighbours need not be candidates themselves (a
+ * flanking N, the pseudo-letter *).  Lattices, as sets of letter states (see nmb_sweep_prune_lattice): contiguous
+ * k-mers, the 15 IUPAC letters over A T G C other (N also takes "other"); bipartite ACGT halves, A T G C and * = ACGT;
+ * bipartite IUPAC halves, the 14 letters other than N and * = ACGT. */
+
+/* The LAST nmb_sweep_expand pass of a (k, mod_pos) table fused with the filter: n_mod / n_nomod are stacked
  * [n_slots][5][inner], inner = 15^(k-2) (every axis but the most significant one already expanded); the kernel
- * expands that axis in registers and records every entry with n_mod >= min_mod and posterior mean (5 + n_mod) /
- * (10 + n_mod + n_nomod) >= min_mean -- nmb_sweep_filter's test, bit for bit -- as (slot, table index of the
- * 15^(k-1) table, n_mod, n_nomod).  Motifs in canonical form only: no N as the first or last letter (the modified
- * position's own letter, at mod_pos 0 or k-1, is the fixed base and never N).  The 15^(k-1) table is not written.
- * *n_out (device int64) = number of hits, in no particular order, of which at most `capacity` are written. */
+ * expands that axis in registers and records (slot, table index of the 15^(k-1) table, n_mod, n_nomod).  Motifs in
+ * canonical form only: no N as the first or last letter (the modified position's own letter, at mod_pos 0 or k-1, is
+ * the fixed base and never N).  The 15^(k-1) table is not written. */
 NMB_API int nmb_sweep_expand_filter(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots, int64_t inner,
-                                    int32_t k, int32_t mod_pos, double min_mean, int64_t min_mod, nmb_sweep_hit *out,
-                                    int64_t capacity, int64_t *n_out, void *stream);
+                                    int32_t k, int32_t mod_pos, double min_mean, int64_t min_mod, int32_t prune,
+                                    nmb_sweep_hit *out, int64_t capacity, int64_t *n_out, void *stream);
 /* Candidates of n_slots FINISHED bipartite histograms stacked at nmb_sweep_bipartite_size(): the n_mod counters
- * (class 0) whose concrete letter at the counter's offset o is `canonical` (A=0 T=1 G=2 C=3) and that pass the test
- * above; index = the n_mod counter's position in its slot's histogram (n_nomod sits 4^(a+b) counters later).
- * *n_out / capacity as for nmb_sweep_expand_filter. */
+ * (class 0) whose concrete letter at the counter's offset o is `canonical` (A=0 T=1 G=2 C=3) and that pass the
+ * filter; index = the n_mod counter's position in its slot's histogram (n_nomod sits 4^(a+b) counters later). */
 NMB_API int nmb_sweep_bipartite_filter(const uint32_t *hist, int32_t n_slots, int32_t canonical, double min_mean,
-                                       int64_t min_mod, nmb_sweep_hit *out, int64_t capacity, int64_t *n_out,
-                                       void *stream);
+                                       int64_t min_mod, int32_t prune, nmb_sweep_hit *out, int64_t capacity,
+                                       int64_t *n_out, void *stream);
 
 /* ---- K8 degenerate bipartite motifs (ABI 6): X{a} N{g} Y{b} whose halves use the 14 IUPAC letters other than N
  *      (A T G C R Y S W K M B D H V, the order of nmb_sweep_expand without N), from the FINISHED bipartite
@@ -578,36 +578,14 @@ NMB_API int nmb_sweep_bip_iupac_slice(const uint32_t *hist, int32_t n_slots, int
  * to the a + b - 1 axes of a slice, last axis first, it gives the table of all 14^(a+b-1) motifs, index = the letters
  * other than the modified one as base-14 digits, first letter most significant. */
 NMB_API int nmb_sweep_bip_iupac_expand(const uint32_t *src, uint32_t *dst, int64_t outer, int64_t inner, void *stream);
-/* The last nmb_sweep_bip_iupac_expand pass fused with the filter of nmb_sweep_expand_filter: n_mod / n_nomod stacked
- * [n_slots][4][inner] (inner = 14^(a+b-2), every axis but the first expanded); records (slot, table index, n_mod,
- * n_nomod) of every motif with n_mod >= min_mod and posterior mean >= min_mean; the table is not written.
- * *n_out / capacity as for nmb_sweep_expand_filter. */
+/* The last nmb_sweep_bip_iupac_expand pass fused with the filter (see the candidate filters above): n_mod / n_nomod
+ * stacked [n_slots][4][inner], inner = 14^(a+b-2) (every axis but the first expanded; a power of 14 below 2^32 / 14,
+ * from which the number of axes follows); records (slot, table index, n_mod, n_nomod); the table is not written. */
 NMB_API int nmb_sweep_bip_iupac_expand_filter(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots,
-                                              int64_t inner, double min_mean, int64_t min_mod, nmb_sweep_hit *out,
-                                              int64_t capacity, int64_t *n_out, void *stream);
+                                              int64_t inner, double min_mean, int64_t min_mod, int32_t prune,
+                                              nmb_sweep_hit *out, int64_t capacity, int64_t *n_out, void *stream);
 
-/* ---- K8 candidate pruning (ABI 7): the three filters above, minus the candidates that are a redundant
- *      specialisation or a mixture of a one-letter neighbour in the same table ----
- * For a candidate M and every letter other than the modified one: a widening P puts there a letter of the lattice
- * that covers M's letter (one more base), a narrowing C one that M's letter covers; Q = P - M or M - C, n_mod and
- * n_nomod separately, mean(Q) = (5 + q_mod) / (10 + q_mod + q_nomod).  M is pruned when (a) some widening P passes
- * the filter and mean(Q) >= min_mean, or (b) some narrowing C passes and mean(Q) < min_mean.  Neighbours need not be
- * candidates themselves (a flanking N, the pseudo-letter *).  Lattices, as sets of letter states (see
- * nmb_sweep_prune_lattice): contiguous k-mers, the 15 IUPAC letters over A T G C other (N also takes "other");
- * bipartite ACGT halves, A T G C and * = ACGT; bipartite IUPAC halves, the 14 letters other than N and * = ACGT.
- * Arguments, records and *n_out / capacity as for the filter each one mirrors; the records are a subset of its. */
-NMB_API int nmb_sweep_expand_filter_prune(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots,
-                                          int64_t inner, int32_t k, int32_t mod_pos, double min_mean, int64_t min_mod,
-                                          nmb_sweep_hit *out, int64_t capacity, int64_t *n_out, void *stream);
-NMB_API int nmb_sweep_bipartite_filter_prune(const uint32_t *hist, int32_t n_slots, int32_t canonical, double min_mean,
-                                             int64_t min_mod, nmb_sweep_hit *out, int64_t capacity, int64_t *n_out,
-                                             void *stream);
-/* inner must be a power of 14: the number of table axes follows from it. */
-NMB_API int nmb_sweep_bip_iupac_expand_filter_prune(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots,
-                                                    int64_t inner, double min_mean, int64_t min_mod,
-                                                    nmb_sweep_hit *out, int64_t capacity, int64_t *n_out,
-                                                    void *stream);
-/* Host query, no device work: the lattice the pruning kernels use (0 contiguous, 1 bipartite ACGT, 2 bipartite
+/* Host query, no device work: the lattice the pruning filters use (0 contiguous, 1 bipartite ACGT, 2 bipartite
  * IUPAC), in table letter order with the widest letter (N or *) last.  states[i]: bit s set when letter i stands for
  * state s (A=0 T=1 G=2 C=3 other=4); widen[i] / narrow[i]: bit j set when letter j covers letter i / letter i covers
  * letter j.  Writes up to 15 entries per array and returns the number of letters. */

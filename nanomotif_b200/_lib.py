@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libnmb200.so")
 
 # ---- constants mirrored from include/nmb200.h -------------------------------------------------
-ABI_VERSION = 7
+ABI_VERSION = 8
 CHUNK_WORDS = 16
 CHUNK_BP = 512
 TILE_WORDS = 2048
@@ -104,27 +104,19 @@ SIGNATURES = {
     "nmb_gather_rows": (C.c_int, [_P, _I32, _P, _I64, _P, _P]),
     "nmb_bgzf_inflate": (C.c_int, [_P, _P, _P, _P, _P, _P, _I32, _P, _P, _P]),
     "nmb_sweep_hist_size": (C.c_int64, []),
-    "nmb_sweep_hist": (C.c_int, [C.POINTER(NmbAssembly), _P, _I32, _I32, _I32, _I32, _P, _P]),
-    "nmb_sweep_finalize": (C.c_int, [_P, _P]),
+    "nmb_sweep_hist": (C.c_int, [C.POINTER(NmbAssembly), _P, _I32, _I32, _I32, _I32, _P, _I32, _P, _P]),
+    "nmb_sweep_finalize": (C.c_int, [_P, _I32, _P]),
     "nmb_sweep_bipartite_size": (C.c_int64, []),
-    "nmb_sweep_bipartite": (C.c_int, [C.POINTER(NmbAssembly), _P, _I32, _I32, _I32, _I32, _P, _P]),
-    "nmb_sweep_bipartite_finalize": (C.c_int, [_P, _P]),
-    "nmb_sweep_slice": (C.c_int, [_P, _P, _I64, _I64, _I32, _P]),
+    "nmb_sweep_bipartite": (C.c_int, [C.POINTER(NmbAssembly), _P, _I32, _I32, _I32, _I32, _P, _I32, _P, _P]),
+    "nmb_sweep_bipartite_finalize": (C.c_int, [_P, _I32, _P]),
+    "nmb_sweep_slice": (C.c_int, [_P, _I64, _I32, _P, _I64, _I64, _I32, _P]),
     "nmb_sweep_expand": (C.c_int, [_P, _P, _I64, _I64, _P]),
     "nmb_sweep_filter": (C.c_int, [_P, _P, _I64, _F64, _I64, _P, _I64, _P, _P]),
-    "nmb_sweep_hist_slots": (C.c_int, [C.POINTER(NmbAssembly), _P, _I32, _I32, _P, _I32, _P, _P]),
-    "nmb_sweep_bipartite_slots": (C.c_int, [C.POINTER(NmbAssembly), _P, _I32, _I32, _P, _I32, _P, _P]),
-    "nmb_sweep_finalize_slots": (C.c_int, [_P, _I32, _P]),
-    "nmb_sweep_bipartite_finalize_slots": (C.c_int, [_P, _I32, _P]),
-    "nmb_sweep_slice_slots": (C.c_int, [_P, _I64, _I32, _P, _I64, _I64, _I32, _P]),
-    "nmb_sweep_expand_filter": (C.c_int, [_P, _P, _I64, _I64, _I32, _I32, _F64, _I64, _P, _I64, _P, _P]),
-    "nmb_sweep_bipartite_filter": (C.c_int, [_P, _I32, _I32, _F64, _I64, _P, _I64, _P, _P]),
+    "nmb_sweep_expand_filter": (C.c_int, [_P, _P, _I64, _I64, _I32, _I32, _F64, _I64, _I32, _P, _I64, _P, _P]),
+    "nmb_sweep_bipartite_filter": (C.c_int, [_P, _I32, _I32, _F64, _I64, _I32, _P, _I64, _P, _P]),
     "nmb_sweep_bip_iupac_slice": (C.c_int, [_P, _I32, _I32, _I32, _I32, _I32, _I32, _I32, _P, _P]),
     "nmb_sweep_bip_iupac_expand": (C.c_int, [_P, _P, _I64, _I64, _P]),
-    "nmb_sweep_bip_iupac_expand_filter": (C.c_int, [_P, _P, _I64, _I64, _F64, _I64, _P, _I64, _P, _P]),
-    "nmb_sweep_expand_filter_prune": (C.c_int, [_P, _P, _I64, _I64, _I32, _I32, _F64, _I64, _P, _I64, _P, _P]),
-    "nmb_sweep_bipartite_filter_prune": (C.c_int, [_P, _I32, _I32, _F64, _I64, _P, _I64, _P, _P]),
-    "nmb_sweep_bip_iupac_expand_filter_prune": (C.c_int, [_P, _P, _I64, _I64, _F64, _I64, _P, _I64, _P, _P]),
+    "nmb_sweep_bip_iupac_expand_filter": (C.c_int, [_P, _P, _I64, _I64, _F64, _I64, _I32, _P, _I64, _P, _P]),
     "nmb_sweep_prune_lattice": (C.c_int, [_I32, _P, _P, _P]),
     "nmb_add_class_planes_compact": (C.c_int, [_P, _P, _P, _P, _I64, _I32, _I32, C.POINTER(NmbAssembly), _I32, _P, _P]),
     "nmb_filter_coverage": (C.c_int, [_P, _I64, _I64, _P, _P]),

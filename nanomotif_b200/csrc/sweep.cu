@@ -362,76 +362,6 @@ __global__ void __launch_bounds__(256) sweep_slice_kernel(const uint32_t *__rest
     dst[i] = src[(hi * 5 + digit) * axis_stride + lo];
 }
 
-// The last expansion pass fused with the filter: the most significant table axis of src[slot][5][inner] is expanded to
-// the 15 IUPAC letters in registers and every entry that passes sweep_filter_kernel's test (same arithmetic) is
-// appended as (slot, table index = letter * inner + r, n_mod, n_nomod); the expanded table is never written.  Motifs
-// whose first or last letter is N are skipped (canonical form) unless that letter is the modified position's fixed
-// base.  *n_out counts all hits, at most `capacity` are written.
-__global__ void __launch_bounds__(256) sweep_expand_filter_kernel(const uint32_t *__restrict__ n_mod,
-                                                                  const uint32_t *__restrict__ n_nomod, int64_t n_slots,
-                                                                  int64_t inner, bool skip_first_n, bool skip_last_n,
-                                                                  double min_mean, uint32_t min_mod,
-                                                                  nmb_sweep_hit *__restrict__ out, int64_t capacity,
-                                                                  unsigned long long *__restrict__ n_out) {
-    const int64_t n = n_slots * inner;
-    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-        const int64_t slot = i / inner, r = i - slot * inner;
-        uint32_t m[15], u[15];
-        iupac_sums(n_mod + slot * 5 * inner + r, inner, m);
-        uint32_t hits = 0;  // bit d: letter d passes
-        const int last = skip_last_n && r % 15 == 14 ? 0 : 15;
-        for (int d = 0; d < last; ++d)
-            if (m[d] >= min_mod) hits |= 1u << d;
-        if (skip_first_n) hits &= ~(1u << 14);
-        if (!hits) continue;
-        iupac_sums(n_nomod + slot * 5 * inner + r, inner, u);
-        for (int d = 0; d < 15; ++d)
-            if ((hits >> d & 1) && !sweep_pass(m[d], u[d], min_mean, min_mod)) hits &= ~(1u << d);
-        if (!hits) continue;
-        unsigned long long at = atomicAdd(n_out, (unsigned long long)__popc(hits));
-        for (int d = 0; d < 15; ++d) {
-            if (!(hits >> d & 1)) continue;
-            if ((int64_t)at < capacity)
-                out[at] = nmb_sweep_hit{(int32_t)slot, (uint32_t)(d * inner + r), m[d], u[d]};
-            ++at;
-        }
-    }
-}
-
-// Candidates of finished bipartite histograms stacked [slot][kBipHistSize]: every n_mod counter (class 0) whose
-// concrete letter at the counter's offset is `canonical` (A=0 T=1 G=2 C=3) and that passes the test of
-// sweep_filter_kernel; index = the counter's position in its slot's histogram.
-__global__ void __launch_bounds__(256) bip_filter_kernel(const uint32_t *__restrict__ hist, int64_t n_slots, int canonical,
-                                                         double min_mean, uint32_t min_mod, nmb_sweep_hit *__restrict__ out,
-                                                         int64_t capacity, unsigned long long *__restrict__ n_out) {
-    constexpr int64_t b33 = bip_block(3, 3), b34 = bip_block(3, 4), b43 = bip_block(4, 3);
-    constexpr int64_t per_gap = bip_offset(3, kBipMinGap + 1, 3);
-    const int64_t n = n_slots * kBipHistSize;
-    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-        const uint32_t m = hist[i];
-        if (m < min_mod) continue;
-        const int64_t slot = i / kBipHistSize, j = i - slot * kBipHistSize;
-        int64_t rem = j % per_gap;
-        int a, b;
-        if (rem < b33) { a = 3; b = 3; }
-        else if (rem < b33 + b34) { a = 3; b = 4; rem -= b33; }
-        else if (rem < b33 + b34 + b43) { a = 4; b = 3; rem -= b33 + b34; }
-        else { a = 4; b = 4; rem -= b33 + b34 + b43; }
-        const int bits = 2 * (a + b);
-        const int oc = (int)(rem >> bits), code = (int)(rem & ((1 << bits) - 1));
-        if (oc & 1) continue;  // an n_nomod counter
-        const int o = oc >> 1;
-        const int xbit = o < a ? o : 2 * a + (o - a), ybit = o < a ? a + o : 2 * a + b + (o - a);
-        if ((((code >> xbit) & 1) << 1 | ((code >> ybit) & 1)) != canonical) continue;
-        const uint32_t u = hist[i + (1 << bits)];
-        if (!sweep_pass(m, u, min_mean, min_mod)) continue;
-        const unsigned long long at = atomicAdd(n_out, 1ull);
-        if ((int64_t)at < capacity) out[at] = nmb_sweep_hit{(int32_t)slot, (uint32_t)j, m, u};
-    }
-}
-
 // ---- degenerate bipartite halves: X{a} N{g} Y{b} with any of the 14 IUPAC letters other than N in X and Y ----
 // A half letter other than N matches only the four concrete contig letters, and bip_add skips every window with a
 // non-ACGT letter in a half, so the count of such a motif is the sum of the finished ACGT counters over the concrete
@@ -470,42 +400,6 @@ __global__ void __launch_bounds__(256) bip_iupac_expand_kernel(const uint32_t *_
         acgt_sums(s[0], s[inner], s[2 * inner], s[3 * inner], v);
         uint32_t *d = dst + o * 14 * inner + r;
         for (int l = 0; l < 14; ++l) d[l * inner] = v[l];
-    }
-}
-
-// The last bip_iupac_expand pass fused with the filter, as sweep_expand_filter_kernel does for the contiguous tables:
-// src[slot][4][inner] -> the 14 letters of the most significant axis in registers, every entry that passes
-// sweep_pass appended as (slot, index = letter * inner + r, n_mod, n_nomod).  *n_out counts all hits, at most
-// `capacity` are written.
-__global__ void __launch_bounds__(256) bip_iupac_expand_filter_kernel(const uint32_t *__restrict__ n_mod,
-                                                                      const uint32_t *__restrict__ n_nomod,
-                                                                      int64_t n_slots, int64_t inner, double min_mean,
-                                                                      uint32_t min_mod, nmb_sweep_hit *__restrict__ out,
-                                                                      int64_t capacity,
-                                                                      unsigned long long *__restrict__ n_out) {
-    const int64_t n = n_slots * inner;
-    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-        const int64_t slot = i / inner, r = i - slot * inner;
-        const uint32_t *s = n_mod + slot * 4 * inner + r;
-        uint32_t m[14], u[14];
-        acgt_sums(s[0], s[inner], s[2 * inner], s[3 * inner], m);
-        uint32_t hits = 0;  // bit d: letter d passes
-        for (int d = 0; d < 14; ++d)
-            if (m[d] >= min_mod) hits |= 1u << d;
-        if (!hits) continue;
-        s = n_nomod + slot * 4 * inner + r;
-        acgt_sums(s[0], s[inner], s[2 * inner], s[3 * inner], u);
-        for (int d = 0; d < 14; ++d)
-            if ((hits >> d & 1) && !sweep_pass(m[d], u[d], min_mean, min_mod)) hits &= ~(1u << d);
-        if (!hits) continue;
-        unsigned long long at = atomicAdd(n_out, (unsigned long long)__popc(hits));
-        for (int d = 0; d < 14; ++d) {
-            if (!(hits >> d & 1)) continue;
-            if ((int64_t)at < capacity)
-                out[at] = nmb_sweep_hit{(int32_t)slot, (uint32_t)(d * inner + r), m[d], u[d]};
-            ++at;
-        }
     }
 }
 
@@ -635,95 +529,88 @@ __device__ __forceinline__ bool expand_pruned(const PruneLattice &L, const uint3
     return false;
 }
 
-// sweep_expand_filter_kernel with pruning: the same candidates, minus the pruned ones.  Input [slot][5][inner],
-// inner = 15^(k-2): neighbours on the first axis come from the 15 register sums, on the other k - 2 axes from the
-// entry with that base-15 digit of r replaced (a flanking N included: GATCN prunes GATCB).
-__global__ void __launch_bounds__(256) sweep_expand_filter_prune_kernel(
-    const uint32_t *__restrict__ n_mod, const uint32_t *__restrict__ n_nomod, int64_t n_slots, int64_t inner,
-    bool skip_first_n, bool skip_last_n, double min_mean, uint32_t min_mod, nmb_sweep_hit *__restrict__ out,
-    int64_t capacity, unsigned long long *__restrict__ n_out) {
-    const PruneLattice &L = c_prune_lattices[kLatticeIupac];
+// v[0..14] = the letter sums of the S states s[0], s[inner], ..., s[(S - 1) * inner]: for S = 5 the 15 IUPAC letters
+// (iupac_sums), for S = 4 the 14 letters other than N and, at index 14, the pseudo-letter * = the sum of the 4 states.
+template <int S>
+__device__ __forceinline__ void letter_sums(const uint32_t *s, int64_t inner, uint32_t (&v)[15]) {
+    if constexpr (S == 5) {
+        iupac_sums(s, inner, v);
+    } else {
+        acgt_sums(s[0], s[inner], s[2 * inner], s[3 * inner], v);
+        v[14] = s[0] + s[inner] + s[2 * inner] + s[3 * inner];
+    }
+}
+
+// Appends (slot, index r + d * inner, m[d], u[d]) for every letter d < N set in `hits`.  *n_out counts all hits, at
+// most `capacity` records are written (count-then-fill).
+template <int N>
+__device__ __forceinline__ void append_hits(uint32_t hits, int64_t slot, int64_t inner, int64_t r, const uint32_t *m,
+                                            const uint32_t *u, nmb_sweep_hit *__restrict__ out, int64_t capacity,
+                                            unsigned long long *__restrict__ n_out) {
+    unsigned long long at = atomicAdd(n_out, (unsigned long long)__popc(hits));
+    for (int d = 0; d < N; ++d) {
+        if (!(hits >> d & 1)) continue;
+        if ((int64_t)at < capacity) out[at] = nmb_sweep_hit{(int32_t)slot, (uint32_t)(d * inner + r), m[d], u[d]};
+        ++at;
+    }
+}
+
+// The last expansion pass fused with the filter: the most significant table axis of src[slot][S][inner] is expanded
+// in registers and every entry that passes sweep_filter_kernel's test (same arithmetic) is appended as (slot, table
+// index = letter * inner + r, n_mod, n_nomod); the expanded table is never written.
+//   S = 5: the 15 IUPAC letters of nmb_sweep_expand (contiguous k-mers, inner = 15^(k-2)).  Motifs whose first or
+//          last letter is N are skipped (canonical form) unless that letter is the modified position's fixed base.
+//   S = 4: the 14 letters of nmb_sweep_bip_iupac_expand (degenerate bipartite halves, inner = 14^(a+b-2)).
+// PRUNE drops the candidates that expand_pruned prunes: neighbours on the register axis come from the register sums
+// (index 14: N, or for S = 4 the pseudo-letter * = the sum of the 4 states), those on the other axes from the entry
+// with that digit of r replaced (a flanking N included: GATCN prunes GATCB; * is the sum of the entries with A, T, G
+// and C there).  Only candidates that pass look at their neighbours.
+template <int S, bool PRUNE>
+__global__ void __launch_bounds__(256) expand_filter_kernel(const uint32_t *__restrict__ n_mod,
+                                                            const uint32_t *__restrict__ n_nomod, int64_t n_slots,
+                                                            int64_t inner, bool skip_first_n, bool skip_last_n,
+                                                            double min_mean, uint32_t min_mod,
+                                                            nmb_sweep_hit *__restrict__ out, int64_t capacity,
+                                                            unsigned long long *__restrict__ n_out) {
+    constexpr int L = S == 5 ? 15 : 14;  // letters of the register axis
     const int64_t n = n_slots * inner;
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
         const int64_t slot = i / inner, r = i - slot * inner;
-        const uint32_t *mb = n_mod + slot * 5 * inner, *ub = n_nomod + slot * 5 * inner;
+        const uint32_t *mb = n_mod + slot * S * inner, *ub = n_nomod + slot * S * inner;
         uint32_t m[15], u[15];
-        iupac_sums(mb + r, inner, m);
-        uint32_t hits = 0;
-        const int last = skip_last_n && r % 15 == 14 ? 0 : 15;
+        letter_sums<S>(mb + r, inner, m);
+        uint32_t hits = 0;  // bit d: letter d passes
+        const int last = S == 5 && skip_last_n && r % 15 == 14 ? 0 : L;
         for (int d = 0; d < last; ++d)
             if (m[d] >= min_mod) hits |= 1u << d;
-        if (skip_first_n) hits &= ~(1u << 14);
+        if (S == 5 && skip_first_n) hits &= ~(1u << 14);
         if (!hits) continue;
-        iupac_sums(ub + r, inner, u);
-        for (int d = 0; d < 15; ++d)
+        letter_sums<S>(ub + r, inner, u);
+        for (int d = 0; d < L; ++d)
             if ((hits >> d & 1) && !sweep_pass(m[d], u[d], min_mean, min_mod)) hits &= ~(1u << d);
+        if constexpr (PRUNE) {
+            const PruneLattice &lat = c_prune_lattices[S == 5 ? kLatticeIupac : kLatticeBipIupac];
 #pragma unroll 1
-        for (uint32_t h = hits; h; h &= h - 1) {  // only candidates that pass look at their neighbours
-            const int d = __ffs(h) - 1;
-            if (expand_pruned<5, 15>(L, mb, ub, inner, r, d, m, u, min_mean, min_mod)) hits &= ~(1u << d);
+            for (uint32_t h = hits; h; h &= h - 1) {
+                const int d = __ffs(h) - 1;
+                if (expand_pruned<S, L>(lat, mb, ub, inner, r, d, m, u, min_mean, min_mod)) hits &= ~(1u << d);
+            }
         }
         if (!hits) continue;
-        unsigned long long at = atomicAdd(n_out, (unsigned long long)__popc(hits));
-        for (int d = 0; d < 15; ++d) {
-            if (!(hits >> d & 1)) continue;
-            if ((int64_t)at < capacity)
-                out[at] = nmb_sweep_hit{(int32_t)slot, (uint32_t)(d * inner + r), m[d], u[d]};
-            ++at;
-        }
+        append_hits<L>(hits, slot, inner, r, m, u, out, capacity, n_out);
     }
 }
 
-// bip_iupac_expand_filter_kernel with pruning.  Input [slot][4][inner], inner = 14^(n-1): every axis uses the
-// 14 letters + * lattice; * on the register axis is the sum of the 4 states, on another axis the sum of the entries
-// with A, T, G and C there.
-__global__ void __launch_bounds__(256) bip_iupac_expand_filter_prune_kernel(
-    const uint32_t *__restrict__ n_mod, const uint32_t *__restrict__ n_nomod, int64_t n_slots, int64_t inner,
-    double min_mean, uint32_t min_mod, nmb_sweep_hit *__restrict__ out, int64_t capacity,
-    unsigned long long *__restrict__ n_out) {
-    const PruneLattice &L = c_prune_lattices[kLatticeBipIupac];
-    const int64_t n = n_slots * inner;
-    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
-        const int64_t slot = i / inner, r = i - slot * inner;
-        const uint32_t *mb = n_mod + slot * 4 * inner, *ub = n_nomod + slot * 4 * inner;
-        uint32_t m[15], u[15];
-        const uint32_t *s = mb + r;
-        acgt_sums(s[0], s[inner], s[2 * inner], s[3 * inner], m);
-        uint32_t hits = 0;
-        for (int d = 0; d < 14; ++d)
-            if (m[d] >= min_mod) hits |= 1u << d;
-        if (!hits) continue;
-        m[14] = s[0] + s[inner] + s[2 * inner] + s[3 * inner];
-        s = ub + r;
-        acgt_sums(s[0], s[inner], s[2 * inner], s[3 * inner], u);
-        u[14] = s[0] + s[inner] + s[2 * inner] + s[3 * inner];
-        for (int d = 0; d < 14; ++d)
-            if ((hits >> d & 1) && !sweep_pass(m[d], u[d], min_mean, min_mod)) hits &= ~(1u << d);
-#pragma unroll 1
-        for (uint32_t h = hits; h; h &= h - 1) {  // only candidates that pass look at their neighbours
-            const int d = __ffs(h) - 1;
-            if (expand_pruned<4, 14>(L, mb, ub, inner, r, d, m, u, min_mean, min_mod)) hits &= ~(1u << d);
-        }
-        if (!hits) continue;
-        unsigned long long at = atomicAdd(n_out, (unsigned long long)__popc(hits));
-        for (int d = 0; d < 14; ++d) {
-            if (!(hits >> d & 1)) continue;
-            if ((int64_t)at < capacity)
-                out[at] = nmb_sweep_hit{(int32_t)slot, (uint32_t)(d * inner + r), m[d], u[d]};
-            ++at;
-        }
-    }
-}
-
-// bip_filter_kernel with pruning: every letter but the modified one widens to *, the sum of the 4 counters whose
-// code differs only in that letter's x and y bits (same block, offset and class).
-__global__ void __launch_bounds__(256) bip_filter_prune_kernel(const uint32_t *__restrict__ hist, int64_t n_slots,
-                                                               int canonical, double min_mean, uint32_t min_mod,
-                                                               nmb_sweep_hit *__restrict__ out, int64_t capacity,
-                                                               unsigned long long *__restrict__ n_out) {
-    const PruneLattice &L = c_prune_lattices[kLatticeBipAcgt];
+// Candidates of finished bipartite histograms stacked [slot][kBipHistSize]: every n_mod counter (class 0) whose
+// concrete letter at the counter's offset is `canonical` (A=0 T=1 G=2 C=3) and that passes the test of
+// sweep_filter_kernel; index = the counter's position in its slot's histogram.  PRUNE: every letter but the modified
+// one widens to *, the sum of the 4 counters whose code differs only in that letter's x and y bits (same block,
+// offset and class).
+template <bool PRUNE>
+__global__ void __launch_bounds__(256) bip_filter_kernel(const uint32_t *__restrict__ hist, int64_t n_slots, int canonical,
+                                                         double min_mean, uint32_t min_mod, nmb_sweep_hit *__restrict__ out,
+                                                         int64_t capacity, unsigned long long *__restrict__ n_out) {
     constexpr int64_t b33 = bip_block(3, 3), b34 = bip_block(3, 4), b43 = bip_block(4, 3);
     constexpr int64_t per_gap = bip_offset(3, kBipMinGap + 1, 3);
     const int64_t n = n_slots * kBipHistSize;
@@ -740,7 +627,7 @@ __global__ void __launch_bounds__(256) bip_filter_prune_kernel(const uint32_t *_
         else { a = 4; b = 4; rem -= b33 + b34 + b43; }
         const int bits = 2 * (a + b);
         const int oc = (int)(rem >> bits), code = (int)(rem & ((1 << bits) - 1));
-        if (oc & 1) continue;
+        if (oc & 1) continue;  // an n_nomod counter
         const int o = oc >> 1;
         auto xbit = [&](int p) { return p < a ? p : 2 * a + (p - a); };
         auto ybit = [&](int p) { return p < a ? a + p : 2 * a + b + (p - a); };
@@ -748,26 +635,28 @@ __global__ void __launch_bounds__(256) bip_filter_prune_kernel(const uint32_t *_
         if (letter(o) != canonical) continue;
         const uint32_t u = hist[i + (1 << bits)];
         if (!sweep_pass(m, u, min_mean, min_mod)) continue;
-        const uint32_t *block = hist + (i - code);  // code 0 of this (shape, offset, class 0) block
-        bool pruned = false;
-        for (int p = 0; p < a + b && !pruned; ++p) {
-            if (p == o) continue;
-            const int c = letter(p), rest = code & ~(1 << xbit(p) | 1 << ybit(p));
-            for (uint32_t e = L.widen[c] | L.narrow[c]; e && !pruned; e &= e - 1) {
-                const int l = __ffs(e) - 1;
-                uint32_t nm = 0, nu = 0;
-                for (uint32_t t = L.states[l]; t; t &= t - 1) {
-                    const int x = __ffs(t) - 1;
-                    const int c2 = rest | (x >> 1) << xbit(p) | (x & 1) << ybit(p);
-                    nm += block[c2];
-                    nu += block[c2 + (1 << bits)];
+        if constexpr (PRUNE) {
+            const PruneLattice &L = c_prune_lattices[kLatticeBipAcgt];
+            const uint32_t *block = hist + (i - code);  // code 0 of this (shape, offset, class 0) block
+            bool pruned = false;
+            for (int p = 0; p < a + b && !pruned; ++p) {
+                if (p == o) continue;
+                const int c = letter(p), rest = code & ~(1 << xbit(p) | 1 << ybit(p));
+                for (uint32_t e = L.widen[c] | L.narrow[c]; e && !pruned; e &= e - 1) {
+                    const int l = __ffs(e) - 1;
+                    uint32_t nm = 0, nu = 0;
+                    for (uint32_t t = L.states[l]; t; t &= t - 1) {
+                        const int x = __ffs(t) - 1;
+                        const int c2 = rest | (x >> 1) << xbit(p) | (x & 1) << ybit(p);
+                        nm += block[c2];
+                        nu += block[c2 + (1 << bits)];
+                    }
+                    pruned = pruned_by(L.widen[c] >> l & 1, m, u, nm, nu, min_mean, min_mod);
                 }
-                pruned = pruned_by(L.widen[c] >> l & 1, m, u, nm, nu, min_mean, min_mod);
             }
+            if (pruned) continue;
         }
-        if (pruned) continue;
-        const unsigned long long at = atomicAdd(n_out, 1ull);
-        if ((int64_t)at < capacity) out[at] = nmb_sweep_hit{(int32_t)slot, (uint32_t)j, m, u};
+        append_hits<1>(1u, slot, 0, j, &m, &u, out, capacity, n_out);
     }
 }
 
@@ -779,43 +668,15 @@ int64_t nmb_sweep_hist_size(void) { return nmb::kSweepHistSize; }
 
 int64_t nmb_sweep_bipartite_size(void) { return nmb::kBipHistSize; }
 
-static int sweep_launch(bool bipartite, const nmb_assembly *a, const uint32_t *class_records_of_modtype,
-                        int32_t tile_begin, int32_t tile_count, int32_t contig_begin, int32_t contig_end,
-                        const int32_t *contig_slot, int32_t n_slots, uint32_t *hist, void *stream);
-
-int nmb_sweep_hist(const nmb_assembly *a, const uint32_t *class_records_of_modtype, int32_t tile_begin,
-                   int32_t tile_count, int32_t contig_begin, int32_t contig_end, uint32_t *hist, void *stream) {
-    return sweep_launch(false, a, class_records_of_modtype, tile_begin, tile_count, contig_begin, contig_end, nullptr, 1,
-                        hist, stream);
-}
-
-int nmb_sweep_bipartite(const nmb_assembly *a, const uint32_t *class_records_of_modtype, int32_t tile_begin,
-                        int32_t tile_count, int32_t contig_begin, int32_t contig_end, uint32_t *hist, void *stream) {
-    return sweep_launch(true, a, class_records_of_modtype, tile_begin, tile_count, contig_begin, contig_end, nullptr, 1,
-                        hist, stream);
-}
-
-int nmb_sweep_hist_slots(const nmb_assembly *a, const uint32_t *class_records_of_modtype, int32_t tile_begin,
-                         int32_t tile_count, const int32_t *contig_slot, int32_t n_slots, uint32_t *hist, void *stream) {
-    NMB_REQUIRE(contig_slot && n_slots > 0, "nmb_sweep_hist_slots: bad slot map");
-    return sweep_launch(false, a, class_records_of_modtype, tile_begin, tile_count, 0, 0, contig_slot, n_slots, hist,
-                        stream);
-}
-
-int nmb_sweep_bipartite_slots(const nmb_assembly *a, const uint32_t *class_records_of_modtype, int32_t tile_begin,
-                              int32_t tile_count, const int32_t *contig_slot, int32_t n_slots, uint32_t *hist,
-                              void *stream) {
-    NMB_REQUIRE(contig_slot && n_slots > 0, "nmb_sweep_bipartite_slots: bad slot map");
-    return sweep_launch(true, a, class_records_of_modtype, tile_begin, tile_count, 0, 0, contig_slot, n_slots, hist,
-                        stream);
-}
-
+// One launch of sweep_hist_kernel; SweepParams says how contig_slot / the contig range select the counted contigs.
 static int sweep_launch(bool bipartite, const nmb_assembly *a, const uint32_t *class_records_of_modtype,
                         int32_t tile_begin, int32_t tile_count, int32_t contig_begin, int32_t contig_end,
                         const int32_t *contig_slot, int32_t n_slots, uint32_t *hist, void *stream) {
-    NMB_REQUIRE(a && class_records_of_modtype && hist, "nmb_sweep_hist: null argument");
+    const char *what = bipartite ? "nmb_sweep_bipartite" : "nmb_sweep_hist";
+    NMB_REQUIRE(a && class_records_of_modtype && hist, "%s: null argument", what);
+    NMB_REQUIRE(contig_slot ? n_slots > 0 : n_slots == 1, "%s: bad slot map", what);
     NMB_REQUIRE(tile_begin >= 0 && tile_count >= 0 && tile_begin + tile_count <= a->n_tiles,
-                "nmb_sweep_hist: tiles [%d, %d) outside the assembly", tile_begin, tile_begin + tile_count);
+                "%s: tiles [%d, %d) outside the assembly", what, tile_begin, tile_begin + tile_count);
     if (tile_count == 0) return NMB_OK;
     nmb::SweepParams p{a->seq_records, a->nonacgt, class_records_of_modtype, a->contig_start, a->contig_len, hist,
                        contig_slot, tile_begin, a->n_tiles, contig_begin, contig_end, n_slots};
@@ -827,7 +688,21 @@ static int sweep_launch(bool bipartite, const nmb_assembly *a, const uint32_t *c
     return NMB_OK;
 }
 
-int nmb_sweep_finalize_slots(uint32_t *hist, int32_t n_slots, void *stream) {
+int nmb_sweep_hist(const nmb_assembly *a, const uint32_t *class_records_of_modtype, int32_t tile_begin,
+                   int32_t tile_count, int32_t contig_begin, int32_t contig_end, const int32_t *contig_slot,
+                   int32_t n_slots, uint32_t *hist, void *stream) {
+    return sweep_launch(false, a, class_records_of_modtype, tile_begin, tile_count, contig_begin, contig_end,
+                        contig_slot, n_slots, hist, stream);
+}
+
+int nmb_sweep_bipartite(const nmb_assembly *a, const uint32_t *class_records_of_modtype, int32_t tile_begin,
+                        int32_t tile_count, int32_t contig_begin, int32_t contig_end, const int32_t *contig_slot,
+                        int32_t n_slots, uint32_t *hist, void *stream) {
+    return sweep_launch(true, a, class_records_of_modtype, tile_begin, tile_count, contig_begin, contig_end,
+                        contig_slot, n_slots, hist, stream);
+}
+
+int nmb_sweep_finalize(uint32_t *hist, int32_t n_slots, void *stream) {
     NMB_REQUIRE(hist && n_slots > 0 && n_slots <= 65535, "nmb_sweep_finalize: bad argument");
     for (int k = nmb::kSweepMaxK - 1; k >= nmb::kSweepMinK; --k) {  // 8 -> 7, then 7 -> 6, ... each level complete first
         const int64_t n = (int64_t)k * 2 * nmb::pow5(k);
@@ -838,9 +713,7 @@ int nmb_sweep_finalize_slots(uint32_t *hist, int32_t n_slots, void *stream) {
     return NMB_OK;
 }
 
-int nmb_sweep_finalize(uint32_t *hist, void *stream) { return nmb_sweep_finalize_slots(hist, 1, stream); }
-
-int nmb_sweep_bipartite_finalize_slots(uint32_t *hist, int32_t n_slots, void *stream) {
+int nmb_sweep_bipartite_finalize(uint32_t *hist, int32_t n_slots, void *stream) {
     NMB_REQUIRE(hist && n_slots > 0 && n_slots <= 65535, "nmb_sweep_bipartite_finalize: bad argument");
     auto run = [&](int g, int a, int b, int mode) {
         const int64_t n = (int64_t)(a + b) * 2 * (1ll << (2 * (a + b)));
@@ -856,12 +729,8 @@ int nmb_sweep_bipartite_finalize_slots(uint32_t *hist, int32_t n_slots, void *st
     return NMB_OK;
 }
 
-int nmb_sweep_bipartite_finalize(uint32_t *hist, void *stream) {
-    return nmb_sweep_bipartite_finalize_slots(hist, 1, stream);
-}
-
-int nmb_sweep_slice_slots(const uint32_t *src, int64_t src_slot_stride, int32_t n_slots, uint32_t *dst, int64_t n_out,
-                          int64_t axis_stride, int32_t digit, void *stream) {
+int nmb_sweep_slice(const uint32_t *src, int64_t src_slot_stride, int32_t n_slots, uint32_t *dst, int64_t n_out,
+                    int64_t axis_stride, int32_t digit, void *stream) {
     NMB_REQUIRE(src && dst && n_out > 0 && axis_stride > 0 && digit >= 0 && digit < 5 && n_slots > 0 &&
                     n_slots <= 65535 && src_slot_stride >= 0,
                 "nmb_sweep_slice: bad argument");
@@ -871,27 +740,37 @@ int nmb_sweep_slice_slots(const uint32_t *src, int64_t src_slot_stride, int32_t 
     return NMB_OK;
 }
 
-int nmb_sweep_slice(const uint32_t *src, uint32_t *dst, int64_t n_out, int64_t axis_stride, int32_t digit,
-                    void *stream) {
-    return nmb_sweep_slice_slots(src, 0, 1, dst, n_out, axis_stride, digit, stream);
-}
-
 static uint32_t clamp_min_mod(int64_t min_mod) { return (uint32_t)(min_mod > 0xFFFFFFFFll ? 0xFFFFFFFFll : min_mod); }
 
-int nmb_sweep_expand_filter(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots, int64_t inner, int32_t k,
-                            int32_t mod_pos, double min_mean, int64_t min_mod, nmb_sweep_hit *out, int64_t capacity,
-                            int64_t *n_out, void *stream) {
-    NMB_REQUIRE(n_mod && n_nomod && n_out && n_slots >= 0 && inner >= 15 && capacity >= 0 && min_mod >= 0 &&
-                    k >= nmb::kSweepMinK && k <= nmb::kSweepMaxK && mod_pos >= 0 && mod_pos < k,
-                "nmb_sweep_expand_filter: bad argument");
-    NMB_REQUIRE(capacity == 0 || out, "nmb_sweep_expand_filter: null output");
+// What the three candidate filters share before their launch: the checks of the filter and output arguments, *n_out
+// zeroed, and *blocks = the grid for n entries (0: nothing to launch).
+static int filter_begin(const char *what, int64_t min_mod, int32_t prune, nmb_sweep_hit *out, int64_t capacity,
+                        int64_t *n_out, int64_t n, void *stream, unsigned *blocks) {
+    NMB_REQUIRE(n_out && capacity >= 0 && min_mod >= 0 && (prune == 0 || prune == 1), "%s: bad argument", what);
+    NMB_REQUIRE(capacity == 0 || out, "%s: null output", what);
     NMB_CUDA(cudaMemsetAsync(n_out, 0, sizeof(int64_t), (cudaStream_t)stream));
-    if (n_slots == 0) return NMB_OK;
-    int64_t blocks = (n_slots * inner + 255) / 256;
-    if (blocks > 148 * 32) blocks = 148 * 32;
+    const int64_t grid = (n + 255) / 256;
+    *blocks = (unsigned)(grid < 148 * 32 ? grid : 148 * 32);
+    return NMB_OK;
+}
+
+int nmb_sweep_expand_filter(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots, int64_t inner, int32_t k,
+                            int32_t mod_pos, double min_mean, int64_t min_mod, int32_t prune, nmb_sweep_hit *out,
+                            int64_t capacity, int64_t *n_out, void *stream) {
+    NMB_REQUIRE(n_mod && n_nomod && n_slots >= 0 && k >= nmb::kSweepMinK && k <= nmb::kSweepMaxK && mod_pos >= 0 &&
+                    mod_pos < k,
+                "nmb_sweep_expand_filter: bad argument");
+    int64_t want = 1;
+    for (int i = 0; i < k - 2; ++i) want *= 15;
+    NMB_REQUIRE(inner == want, "nmb_sweep_expand_filter: inner %lld is not 15^(k-2) for k = %d", (long long)inner, k);
+    unsigned blocks;
+    const int rc = filter_begin("nmb_sweep_expand_filter", min_mod, prune, out, capacity, n_out, n_slots * inner,
+                                stream, &blocks);
+    if (rc != NMB_OK || blocks == 0) return rc;
     // the first motif letter is the expanded (most significant) axis unless it is the modified position; the last one
     // is the least significant digit of r unless it is the modified position
-    nmb::sweep_expand_filter_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+    (prune ? nmb::expand_filter_kernel<5, true> : nmb::expand_filter_kernel<5, false>)<<<blocks, 256, 0,
+                                                                                        (cudaStream_t)stream>>>(
         n_mod, n_nomod, n_slots, inner, mod_pos != 0, mod_pos != k - 1, min_mean, clamp_min_mod(min_mod), out, capacity,
         (unsigned long long *)n_out);
     NMB_CUDA(cudaGetLastError());
@@ -899,15 +778,14 @@ int nmb_sweep_expand_filter(const uint32_t *n_mod, const uint32_t *n_nomod, int6
 }
 
 int nmb_sweep_bipartite_filter(const uint32_t *hist, int32_t n_slots, int32_t canonical, double min_mean,
-                               int64_t min_mod, nmb_sweep_hit *out, int64_t capacity, int64_t *n_out, void *stream) {
-    NMB_REQUIRE(hist && n_out && n_slots >= 0 && canonical >= 0 && canonical < 4 && capacity >= 0 && min_mod >= 0,
-                "nmb_sweep_bipartite_filter: bad argument");
-    NMB_REQUIRE(capacity == 0 || out, "nmb_sweep_bipartite_filter: null output");
-    NMB_CUDA(cudaMemsetAsync(n_out, 0, sizeof(int64_t), (cudaStream_t)stream));
-    if (n_slots == 0) return NMB_OK;
-    int64_t blocks = ((int64_t)n_slots * nmb::kBipHistSize + 255) / 256;
-    if (blocks > 148 * 32) blocks = 148 * 32;
-    nmb::bip_filter_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
+                               int64_t min_mod, int32_t prune, nmb_sweep_hit *out, int64_t capacity, int64_t *n_out,
+                               void *stream) {
+    NMB_REQUIRE(hist && n_slots >= 0 && canonical >= 0 && canonical < 4, "nmb_sweep_bipartite_filter: bad argument");
+    unsigned blocks;
+    const int rc = filter_begin("nmb_sweep_bipartite_filter", min_mod, prune, out, capacity, n_out,
+                                (int64_t)n_slots * nmb::kBipHistSize, stream, &blocks);
+    if (rc != NMB_OK || blocks == 0) return rc;
+    (prune ? nmb::bip_filter_kernel<true> : nmb::bip_filter_kernel<false>)<<<blocks, 256, 0, (cudaStream_t)stream>>>(
         hist, n_slots, canonical, min_mean, clamp_min_mod(min_mod), out, capacity, (unsigned long long *)n_out);
     NMB_CUDA(cudaGetLastError());
     return NMB_OK;
@@ -940,77 +818,21 @@ int nmb_sweep_bip_iupac_expand(const uint32_t *src, uint32_t *dst, int64_t outer
 }
 
 int nmb_sweep_bip_iupac_expand_filter(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots, int64_t inner,
-                                      double min_mean, int64_t min_mod, nmb_sweep_hit *out, int64_t capacity,
-                                      int64_t *n_out, void *stream) {
-    NMB_REQUIRE(n_mod && n_nomod && n_out && n_slots >= 0 && inner > 0 && inner <= 0xFFFFFFFFll / 14 &&
-                    capacity >= 0 && min_mod >= 0,
+                                      double min_mean, int64_t min_mod, int32_t prune, nmb_sweep_hit *out,
+                                      int64_t capacity, int64_t *n_out, void *stream) {
+    NMB_REQUIRE(n_mod && n_nomod && n_slots >= 0 && inner > 0 && inner <= 0xFFFFFFFFll / 14,
                 "nmb_sweep_bip_iupac_expand_filter: bad argument");
-    NMB_REQUIRE(capacity == 0 || out, "nmb_sweep_bip_iupac_expand_filter: null output");
-    NMB_CUDA(cudaMemsetAsync(n_out, 0, sizeof(int64_t), (cudaStream_t)stream));
-    if (n_slots == 0) return NMB_OK;
-    int64_t blocks = (n_slots * inner + 255) / 256;
-    if (blocks > 148 * 32) blocks = 148 * 32;
-    nmb::bip_iupac_expand_filter_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
-        n_mod, n_nomod, n_slots, inner, min_mean, clamp_min_mod(min_mod), out, capacity, (unsigned long long *)n_out);
-    NMB_CUDA(cudaGetLastError());
-    return NMB_OK;
-}
-
-int nmb_sweep_expand_filter_prune(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots, int64_t inner,
-                                  int32_t k, int32_t mod_pos, double min_mean, int64_t min_mod, nmb_sweep_hit *out,
-                                  int64_t capacity, int64_t *n_out, void *stream) {
-    NMB_REQUIRE(n_mod && n_nomod && n_out && n_slots >= 0 && capacity >= 0 && min_mod >= 0 && k >= nmb::kSweepMinK &&
-                    k <= nmb::kSweepMaxK && mod_pos >= 0 && mod_pos < k,
-                "nmb_sweep_expand_filter_prune: bad argument");
-    int64_t want = 1;
-    for (int i = 0; i < k - 2; ++i) want *= 15;
-    NMB_REQUIRE(inner == want, "nmb_sweep_expand_filter_prune: inner %lld is not 15^(k-2) for k = %d", (long long)inner,
-                k);
-    NMB_REQUIRE(capacity == 0 || out, "nmb_sweep_expand_filter_prune: null output");
-    NMB_CUDA(cudaMemsetAsync(n_out, 0, sizeof(int64_t), (cudaStream_t)stream));
-    if (n_slots == 0) return NMB_OK;
-    int64_t blocks = (n_slots * inner + 255) / 256;
-    if (blocks > 148 * 32) blocks = 148 * 32;
-    nmb::sweep_expand_filter_prune_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
-        n_mod, n_nomod, n_slots, inner, mod_pos != 0, mod_pos != k - 1, min_mean, clamp_min_mod(min_mod), out, capacity,
-        (unsigned long long *)n_out);
-    NMB_CUDA(cudaGetLastError());
-    return NMB_OK;
-}
-
-int nmb_sweep_bipartite_filter_prune(const uint32_t *hist, int32_t n_slots, int32_t canonical, double min_mean,
-                                     int64_t min_mod, nmb_sweep_hit *out, int64_t capacity, int64_t *n_out,
-                                     void *stream) {
-    NMB_REQUIRE(hist && n_out && n_slots >= 0 && canonical >= 0 && canonical < 4 && capacity >= 0 && min_mod >= 0,
-                "nmb_sweep_bipartite_filter_prune: bad argument");
-    NMB_REQUIRE(capacity == 0 || out, "nmb_sweep_bipartite_filter_prune: null output");
-    NMB_CUDA(cudaMemsetAsync(n_out, 0, sizeof(int64_t), (cudaStream_t)stream));
-    if (n_slots == 0) return NMB_OK;
-    int64_t blocks = ((int64_t)n_slots * nmb::kBipHistSize + 255) / 256;
-    if (blocks > 148 * 32) blocks = 148 * 32;
-    nmb::bip_filter_prune_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
-        hist, n_slots, canonical, min_mean, clamp_min_mod(min_mod), out, capacity, (unsigned long long *)n_out);
-    NMB_CUDA(cudaGetLastError());
-    return NMB_OK;
-}
-
-int nmb_sweep_bip_iupac_expand_filter_prune(const uint32_t *n_mod, const uint32_t *n_nomod, int64_t n_slots,
-                                            int64_t inner, double min_mean, int64_t min_mod, nmb_sweep_hit *out,
-                                            int64_t capacity, int64_t *n_out, void *stream) {
-    NMB_REQUIRE(n_mod && n_nomod && n_out && n_slots >= 0 && inner > 0 && inner <= 0xFFFFFFFFll / 14 &&
-                    capacity >= 0 && min_mod >= 0,
-                "nmb_sweep_bip_iupac_expand_filter_prune: bad argument");
     int64_t p = 1;
     while (p < inner) p *= 14;
-    NMB_REQUIRE(p == inner, "nmb_sweep_bip_iupac_expand_filter_prune: inner %lld is not a power of 14",
-                (long long)inner);
-    NMB_REQUIRE(capacity == 0 || out, "nmb_sweep_bip_iupac_expand_filter_prune: null output");
-    NMB_CUDA(cudaMemsetAsync(n_out, 0, sizeof(int64_t), (cudaStream_t)stream));
-    if (n_slots == 0) return NMB_OK;
-    int64_t blocks = (n_slots * inner + 255) / 256;
-    if (blocks > 148 * 32) blocks = 148 * 32;
-    nmb::bip_iupac_expand_filter_prune_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(
-        n_mod, n_nomod, n_slots, inner, min_mean, clamp_min_mod(min_mod), out, capacity, (unsigned long long *)n_out);
+    NMB_REQUIRE(p == inner, "nmb_sweep_bip_iupac_expand_filter: inner %lld is not a power of 14", (long long)inner);
+    unsigned blocks;
+    const int rc = filter_begin("nmb_sweep_bip_iupac_expand_filter", min_mod, prune, out, capacity, n_out,
+                                n_slots * inner, stream, &blocks);
+    if (rc != NMB_OK || blocks == 0) return rc;
+    (prune ? nmb::expand_filter_kernel<4, true> : nmb::expand_filter_kernel<4, false>)<<<blocks, 256, 0,
+                                                                                        (cudaStream_t)stream>>>(
+        n_mod, n_nomod, n_slots, inner, false, false, min_mean, clamp_min_mod(min_mod), out, capacity,
+        (unsigned long long *)n_out);
     NMB_CUDA(cudaGetLastError());
     return NMB_OK;
 }

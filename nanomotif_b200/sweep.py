@@ -44,6 +44,49 @@ def hist_offset(k: int) -> int:
     return sum(j * 2 * 5 ** j for j in range(MIN_K, k))
 
 
+def _class_records(pileup: DevicePileup, asm: DeviceAssembly, modtype: int) -> int:
+    """Device address of the class records of one mod type (the pileup stacks them per mod type)."""
+    return ptr(pileup.class_records) + modtype * asm.n_tiles * _lib.CLS_REC_WORDS * 4
+
+
+def _slice(hist: torch.Tensor, n_slots: int, k: int, mod_pos: int, cls: int, canonical: str) -> torch.Tensor:
+    """[n_slots][5^(k-1)]: the class-`cls` counters of the (k, mod_pos) block of the finished histograms stacked at
+    HIST_SIZE from `hist` on, with the modified letter fixed to `canonical` (nmb_sweep_slice)."""
+    n = 5 ** (k - 1)
+    t = torch.empty(n_slots * n, dtype=torch.int32, device=hist.device)
+    src = hist[hist_offset(k) + (mod_pos * 2 + cls) * 5 ** k:]
+    check(lib.nmb_sweep_slice(ptr(src), HIST_SIZE, n_slots, ptr(t), n, 5 ** (k - 1 - mod_pos), _BASE_DIGIT[canonical],
+                              _stream()), "nmb_sweep_slice")
+    return t
+
+
+def _bip_iupac_slice(bip: torch.Tensor, n_slots: int, a: int, g: int, b: int, mod_pos: int, cls: int,
+                     canonical: str) -> torch.Tensor:
+    """[n_slots][4^(a+b-1)]: the class-`cls` counters of shape (a, g, b) of the finished bipartite histograms stacked
+    at BIP_SIZE from `bip` on, with the modified letter fixed to `canonical` (nmb_sweep_bip_iupac_slice)."""
+    t = torch.empty(n_slots * 4 ** (a + b - 1), dtype=torch.int32, device=bip.device)
+    check(lib.nmb_sweep_bip_iupac_slice(ptr(bip), n_slots, a, g, b, mod_pos, cls, _BASE_DIGIT[canonical], ptr(t),
+                                        _stream()), "nmb_sweep_bip_iupac_slice")
+    return t
+
+
+def _expand(tables, states: int, steps: int) -> tuple:
+    """Expands the last `steps` axes of each sliced class table, last axis first (the large final passes then run
+    with a long contiguous inner): states = 5 gives the 15 IUPAC letters (nmb_sweep_expand), states = 4 the 14
+    letters other than N (nmb_sweep_bip_iupac_expand)."""
+    letters, fn = (15, lib.nmb_sweep_expand) if states == 5 else (14, lib.nmb_sweep_bip_iupac_expand)
+    out = []
+    for t in tables:
+        for step in range(steps):
+            inner = letters ** step
+            outer = t.numel() // (states * inner)
+            e = torch.empty(outer * letters * inner, dtype=torch.int32, device=t.device)
+            check(fn(ptr(t), ptr(e), outer, inner, _stream()), fn.__name__)
+            t = e
+        out.append(t)
+    return tuple(out)
+
+
 class SweepIndex:
     """Window histograms of one mod type (nmb_sweep_hist), accumulated over the contig ranges added so far."""
 
@@ -66,7 +109,7 @@ class SweepIndex:
         if self._hist is None:
             with torch.cuda.device(self.asm.device):
                 h = self.raw.clone()
-                check(lib.nmb_sweep_finalize(ptr(h), _stream()), "nmb_sweep_finalize")
+                check(lib.nmb_sweep_finalize(ptr(h), 1, _stream()), "nmb_sweep_finalize")
             self._hist = h
         return self._hist
 
@@ -74,12 +117,11 @@ class SweepIndex:
         asm = self.asm
         contig_end = asm.n_contigs if contig_end is None else contig_end
         tile_begin, tile_count = asm.tile_span(contig_begin, contig_end)
-        cls = self.pileup.class_records
         view = asm.view()
         with torch.cuda.device(asm.device):
-            base = ptr(cls) + self.modtype * asm.n_tiles * _lib.CLS_REC_WORDS * 4
-            check(lib.nmb_sweep_hist(C.byref(view), base, tile_begin, tile_count, contig_begin, contig_end, ptr(self.raw),
-                                     _stream()), "nmb_sweep_hist")
+            check(lib.nmb_sweep_hist(C.byref(view), _class_records(self.pileup, asm, self.modtype), tile_begin,
+                                     tile_count, contig_begin, contig_end, None, 1, ptr(self.raw), _stream()),
+                  "nmb_sweep_hist")
         self._tables.clear()
         self._hist = None
         return self
@@ -93,9 +135,9 @@ class SweepIndex:
         with torch.cuda.device(asm.device):
             if self.bip_raw is None:
                 self.bip_raw = torch.zeros(int(lib.nmb_sweep_bipartite_size()), dtype=torch.int32, device=asm.device)
-            base = ptr(self.pileup.class_records) + self.modtype * asm.n_tiles * _lib.CLS_REC_WORDS * 4
-            check(lib.nmb_sweep_bipartite(C.byref(view), base, tile_begin, tile_count, contig_begin, contig_end,
-                                          ptr(self.bip_raw), _stream()), "nmb_sweep_bipartite")
+            check(lib.nmb_sweep_bipartite(C.byref(view), _class_records(self.pileup, asm, self.modtype), tile_begin,
+                                          tile_count, contig_begin, contig_end, None, 1, ptr(self.bip_raw), _stream()),
+                  "nmb_sweep_bipartite")
         self._bip = None
         self._tables = {k: v for k, v in self._tables.items() if k[0] != "bip"}
         return self
@@ -117,7 +159,7 @@ class SweepIndex:
         if self._bip is None and self.bip_raw is not None:
             with torch.cuda.device(self.asm.device):
                 h = self.bip_raw.clone()
-                check(lib.nmb_sweep_bipartite_finalize(ptr(h), _stream()), "nmb_sweep_bipartite_finalize")
+                check(lib.nmb_sweep_bipartite_finalize(ptr(h), 1, _stream()), "nmb_sweep_bipartite_finalize")
             self._bip = h
         return self._bip
 
@@ -170,23 +212,12 @@ class SweepIndex:
         key = ("bip", a, g, b, mod_pos, canonical)
         if key in self._tables:
             return self._tables[key]
-        d, n = self.asm.device, a + b - 1
-        out = []
-        with torch.cuda.device(d):
-            for cls in (0, 1):
-                t = torch.empty(4 ** n, dtype=torch.int32, device=d)
-                check(lib.nmb_sweep_bip_iupac_slice(ptr(self.bip), 1, a, g, b, mod_pos, cls, _BASE_DIGIT[canonical],
-                                                    ptr(t), _stream()), "nmb_sweep_bip_iupac_slice")
-                for step in range(n):  # last axis first, as in table()
-                    outer, inner = 4 ** (n - 1 - step), 14 ** step
-                    e = torch.empty(outer * 14 * inner, dtype=torch.int32, device=d)
-                    check(lib.nmb_sweep_bip_iupac_expand(ptr(t), ptr(e), outer, inner, _stream()),
-                          "nmb_sweep_bip_iupac_expand")
-                    t = e
-                out.append(t)
+        with torch.cuda.device(self.asm.device):
+            out = _expand([_bip_iupac_slice(self.bip, 1, a, g, b, mod_pos, cls, canonical) for cls in (0, 1)], 4,
+                          a + b - 1)
         if keep:
-            self._tables[key] = tuple(out)
-        return tuple(out)
+            self._tables[key] = out
+        return out
 
     @staticmethod
     def bipartite_iupac_index(left: str, right: str, offset: int) -> int:
@@ -230,24 +261,11 @@ class SweepIndex:
         key = (k, mod_pos, canonical)
         if key in self._tables:
             return self._tables[key]
-        d = self.asm.device
-        out = []
-        with torch.cuda.device(d):
-            n5 = 5 ** (k - 1)
-            for cls in (0, 1):
-                src = self.hist[hist_offset(k) + (mod_pos * 2 + cls) * 5 ** k:][:5 ** k]
-                a = torch.empty(n5, dtype=torch.int32, device=d)
-                check(lib.nmb_sweep_slice(ptr(src), ptr(a), n5, 5 ** (k - 1 - mod_pos), _BASE_DIGIT[canonical], _stream()),
-                      "nmb_sweep_slice")
-                for step in range(k - 1):  # last axis first: the big final passes run with a long contiguous inner
-                    outer, inner = 5 ** (k - 2 - step), 15 ** step
-                    b = torch.empty(outer * 15 * inner, dtype=torch.int32, device=d)
-                    check(lib.nmb_sweep_expand(ptr(a), ptr(b), outer, inner, _stream()), "nmb_sweep_expand")
-                    a = b
-                out.append(a)
+        with torch.cuda.device(self.asm.device):
+            out = _expand([_slice(self.hist, 1, k, mod_pos, cls, canonical) for cls in (0, 1)], 5, k - 1)
         if keep:
-            self._tables[key] = tuple(out)
-        return tuple(out)
+            self._tables[key] = out
+        return out
 
     @staticmethod
     def motif_index(motif_iupac: str, mod_pos: int) -> int:
@@ -445,17 +463,16 @@ class BinSweep:
         if bipartite:
             self.add_bipartite()
 
-    def _launch(self, fn, hist, what):
+    def _launch(self, fn, hist):
         if not self.bins:
             return
-        base = ptr(self.pileup.class_records) + self.modtype * self.asm.n_tiles * _lib.CLS_REC_WORDS * 4
         with torch.cuda.device(self.asm.device):
-            check(fn(C.byref(self.asm.view()), base, self.tile_begin, self.tile_count, ptr(self.contig_slot),
-                     len(self.bins), ptr(hist), _stream()), what)
+            check(fn(C.byref(self.asm.view()), _class_records(self.pileup, self.asm, self.modtype), self.tile_begin,
+                     self.tile_count, 0, 0, ptr(self.contig_slot), len(self.bins), ptr(hist), _stream()), fn.__name__)
 
     def add(self) -> "BinSweep":
         """One more pass over the listed bins into the raw IUPAC histograms (counters add)."""
-        self._launch(lib.nmb_sweep_hist_slots, self.raw, "nmb_sweep_hist_slots")
+        self._launch(lib.nmb_sweep_hist, self.raw)
         self._hist = None
         return self
 
@@ -463,18 +480,18 @@ class BinSweep:
         """One more pass into the raw bipartite histograms (counters add)."""
         if self.bip_raw is None:
             raise ValueError("this BinSweep was made with bipartite=False")
-        self._launch(lib.nmb_sweep_bipartite_slots, self.bip_raw, "nmb_sweep_bipartite_slots")
+        self._launch(lib.nmb_sweep_bipartite, self.bip_raw)
         self._bip = None
         return self
 
     @property
     def hist(self) -> torch.Tensor:
-        """Finished IUPAC histograms [bin][HIST_SIZE] (nmb_sweep_finalize_slots on a copy of the raw ones)."""
+        """Finished IUPAC histograms [bin][HIST_SIZE] (nmb_sweep_finalize on a copy of the raw ones)."""
         if self._hist is None:
             with torch.cuda.device(self.asm.device):
                 h = self.raw.clone()
                 if self.bins:
-                    check(lib.nmb_sweep_finalize_slots(ptr(h), len(self.bins), _stream()), "nmb_sweep_finalize_slots")
+                    check(lib.nmb_sweep_finalize(ptr(h), len(self.bins), _stream()), "nmb_sweep_finalize")
             self._hist = h
         return self._hist.view(-1, HIST_SIZE)
 
@@ -487,8 +504,8 @@ class BinSweep:
             with torch.cuda.device(self.asm.device):
                 h = self.bip_raw.clone()
                 if self.bins:
-                    check(lib.nmb_sweep_bipartite_finalize_slots(ptr(h), len(self.bins), _stream()),
-                          "nmb_sweep_bipartite_finalize_slots")
+                    check(lib.nmb_sweep_bipartite_finalize(ptr(h), len(self.bins), _stream()),
+                          "nmb_sweep_bipartite_finalize")
             self._bip = h
         return self._bip.view(-1, BIP_SIZE)
 
@@ -528,9 +545,9 @@ class BinSweep:
         prune=True drops every candidate that a one-letter neighbour in its own table shows to be a redundant
         specialisation (a widening P of a letter other than the modified one passes and Q = P - M has posterior mean
         >= min_mean: GATCA next to GATCM) or a mixture (a narrowing C passes and Q = M - C has mean < min_mean: CCHGG
-        next to CCWGG), in the same passes on the device (nmb_sweep_*_prune); the frame is the matching subsequence
-        of the prune=False one.  Lattices: the 15 IUPAC letters for k-mers, ACGT + * or the 14 letters + * for the
-        bipartite halves (* = any of ACGT, never a row)."""
+        next to CCWGG), in the same passes on the device (the filters' prune flag); the frame is the matching
+        subsequence of the prune=False one.  Lattices: the 15 IUPAC letters for k-mers, ACGT + * or the 14 letters + *
+        for the bipartite halves (* = any of ACGT, never a row)."""
         if min_mod < 1:
             raise ValueError("min_mod must be >= 1: every motif without rows has the prior mean 0.5")
         ks = sorted(set(int(k) for k in ks))
@@ -541,11 +558,11 @@ class BinSweep:
         if bipartite and self.bip_raw is None:
             raise ValueError("this BinSweep was made with bipartite=False")
         groups = [(k, mp) for k in ks for mp in range(k)]
+        bip_groups = None  # None: ACGT halves, one pass over the finished histograms after `groups`
+        if bipartite and bipartite_letters == "IUPAC":
+            bip_groups = [(a, g, b, o if o < a else o + g) for g in range(4, 9) for a, b in _BIP_SHAPES
+                          for o in range(a + b)]
         d, n_bins = self.asm.device, len(self.bins)
-        suffix = "_prune" if prune else ""  # the same passes, with the neighbour test
-        expand_filter = getattr(lib, "nmb_sweep_expand_filter" + suffix)
-        bip_iupac_filter = getattr(lib, "nmb_sweep_bip_iupac_expand_filter" + suffix)
-        bip_filter = getattr(lib, "nmb_sweep_bipartite_filter" + suffix)
         state = {"cap": max(int(capacity), 1)}
         parts = []  # (group, hit records)
 
@@ -564,74 +581,41 @@ class BinSweep:
                 hits["slot"] += slot0
                 parts.append((group, hits))
 
+        # groups read from expanded tables, bins in chunks: (scratch bytes per bin, number of the first group, groups)
+        passes = []
         if groups and n_bins:
-            chunk = max(1, int(scratch_bytes) // table_scratch_bytes(ks[-1]))
-            hist = self.hist.view(-1)
+            passes.append((table_scratch_bytes(ks[-1]), 0, groups))
+        if bip_groups and n_bins:
+            passes.append((bip_iupac_scratch_bytes(), len(groups), bip_groups))
+        for per_bin, first, todo in passes:
+            chunk = max(1, int(scratch_bytes) // per_bin)
             for s0 in range(0, n_bins, chunk):
                 ns = min(chunk, n_bins - s0)
-                for group, (k, mp) in enumerate(groups):
+                for j, group in enumerate(todo):
                     with torch.cuda.device(d):
-                        n5 = 5 ** (k - 1)
-                        tab = []
-                        for cls in (0, 1):
-                            src = hist[s0 * HIST_SIZE + hist_offset(k) + (mp * 2 + cls) * 5 ** k:]
-                            t = torch.empty(ns * n5, dtype=torch.int32, device=d)
-                            check(lib.nmb_sweep_slice_slots(ptr(src), HIST_SIZE, ns, ptr(t), n5, 5 ** (k - 1 - mp),
-                                                            _BASE_DIGIT[self.canonical], _stream()),
-                                  "nmb_sweep_slice_slots")
-                            tab.append(t)
-                        for step in range(k - 2):  # every axis but the most significant one, as in SweepIndex.table
-                            outer, inner = ns * 5 ** (k - 2 - step), 15 ** step
-                            nxt = []
-                            for t in tab:
-                                e = torch.empty(outer * 15 * inner, dtype=torch.int32, device=d)
-                                check(lib.nmb_sweep_expand(ptr(t), ptr(e), outer, inner, _stream()), "nmb_sweep_expand")
-                                nxt.append(e)
-                            tab = nxt
-                    def launch(out, cap, n_out, tab=tab, ns=ns, k=k, mp=mp):
-                        check(expand_filter(ptr(tab[0]), ptr(tab[1]), ns, 15 ** (k - 2), k, mp, float(min_mean),
-                                            int(min_mod), out, cap, n_out, _stream()), expand_filter.__name__)
+                        if len(group) == 2:  # (k, mod_pos): 5 states -> 15 IUPAC letters, every axis but the first
+                            k, mp = group
+                            tab = _expand([_slice(self.hist.view(-1)[s0 * HIST_SIZE:], ns, k, mp, cls, self.canonical)
+                                           for cls in (0, 1)], 5, k - 2)
+                            fn, args = lib.nmb_sweep_expand_filter, (15 ** (k - 2), k, mp)
+                        else:  # (a, g, b, mod_pos): halves from 4 states -> the 14 letters other than N
+                            a, g, b, mp = group
+                            tab = _expand([_bip_iupac_slice(self.bip.view(-1)[s0 * BIP_SIZE:], ns, a, g, b, mp, cls,
+                                                            self.canonical) for cls in (0, 1)], 4, a + b - 2)
+                            fn, args = lib.nmb_sweep_bip_iupac_expand_filter, (14 ** (a + b - 2),)
 
-                    collect(group, launch, s0)
+                    def launch(out, cap, n_out, tab=tab, ns=ns, fn=fn, args=args):
+                        check(fn(ptr(tab[0]), ptr(tab[1]), ns, *args, float(min_mean), int(min_mod), int(prune), out,
+                                 cap, n_out, _stream()), fn.__name__)
+
+                    collect(first + j, launch, s0)
                     del tab
-        bip_groups = None
-        if bipartite and n_bins and bipartite_letters == "IUPAC":
-            bip_groups = [(a, g, b, o if o < a else o + g) for g in range(4, 9) for a, b in _BIP_SHAPES
-                          for o in range(a + b)]
-            chunk = max(1, int(scratch_bytes) // bip_iupac_scratch_bytes())
-            bip = self.bip.view(-1)
-            for s0 in range(0, n_bins, chunk):
-                ns = min(chunk, n_bins - s0)
-                for j, (a, g, b, mp) in enumerate(bip_groups):
-                    n = a + b - 1
-                    with torch.cuda.device(d):
-                        tab = []
-                        for cls in (0, 1):
-                            t = torch.empty(ns * 4 ** n, dtype=torch.int32, device=d)
-                            check(lib.nmb_sweep_bip_iupac_slice(ptr(bip[s0 * BIP_SIZE:]), ns, a, g, b, mp, cls,
-                                                                _BASE_DIGIT[self.canonical], ptr(t), _stream()),
-                                  "nmb_sweep_bip_iupac_slice")
-                            tab.append(t)
-                        for step in range(n - 1):  # every axis but the first, as in bipartite_iupac_table
-                            outer, inner = ns * 4 ** (n - 1 - step), 14 ** step
-                            nxt = []
-                            for t in tab:
-                                e = torch.empty(outer * 14 * inner, dtype=torch.int32, device=d)
-                                check(lib.nmb_sweep_bip_iupac_expand(ptr(t), ptr(e), outer, inner, _stream()),
-                                      "nmb_sweep_bip_iupac_expand")
-                                nxt.append(e)
-                            tab = nxt
-
-                    def launch(out, cap, n_out, tab=tab, ns=ns, n=n):
-                        check(bip_iupac_filter(ptr(tab[0]), ptr(tab[1]), ns, 14 ** (n - 1), float(min_mean),
-                                               int(min_mod), out, cap, n_out, _stream()), bip_iupac_filter.__name__)
-
-                    collect(len(groups) + j, launch, s0)
-                    del tab
-        elif bipartite and n_bins:
+        if bipartite and n_bins and bip_groups is None:
             def launch_bip(out, cap, n_out):
-                check(bip_filter(ptr(self.bip), n_bins, _BASE_DIGIT[self.canonical], float(min_mean), int(min_mod),
-                                 out, cap, n_out, _stream()), bip_filter.__name__)
+                check(lib.nmb_sweep_bipartite_filter(ptr(self.bip), n_bins, _BASE_DIGIT[self.canonical],
+                                                     float(min_mean), int(min_mod), int(prune), out, cap, n_out,
+                                                     _stream()),
+                      "nmb_sweep_bipartite_filter")
 
             collect(len(groups), launch_bip)
         return self._frame(parts, groups, bip_groups)

@@ -1,7 +1,10 @@
 """Host side of the per-bin sweep (sweep.BinSweep): the vectorised decoders of candidate records against the scalar
-SweepIndex helpers they replace (no GPU needed)."""
+SweepIndex helpers they replace, and the argument checks of the histogram entry points (no GPU needed)."""
+import ctypes as C
+
 import numpy as np
 
+from nanomotif_b200 import _lib
 from nanomotif_b200.sweep import IUPAC_ORDER, SweepIndex, decode_bipartite, decode_motifs, table_scratch_bytes
 
 
@@ -38,3 +41,20 @@ def test_scratch_per_bin():
     # k = 8: the 25 x 15^5 input and the 5 x 15^6 output of the last written expansion step, two classes of uint32
     assert table_scratch_bytes(8) == 2 * 4 * (25 * 15 ** 5 + 5 * 15 ** 6) == 607_500_000
     assert all(table_scratch_bytes(k) < table_scratch_bytes(k + 1) for k in range(4, 8))
+
+
+def test_histogram_entry_points_refuse_bad_slot_maps():
+    lib = _lib.lib
+    asm = _lib.NmbAssembly()  # no tiles: an accepted call launches nothing
+    p = np.zeros(16, dtype=np.uint32).ctypes.data
+    slot_map = np.zeros(4, dtype=np.int32).ctypes.data
+    for fn in (lib.nmb_sweep_hist, lib.nmb_sweep_bipartite):
+        # a null map counts the contig range into one histogram; a map routes contigs into n_slots > 0 histograms
+        assert fn(C.byref(asm), p, 0, 0, 0, 0, None, 1, p, None) == 0
+        assert fn(C.byref(asm), p, 0, 0, 0, 0, slot_map, 3, p, None) == 0
+        for contig_slot, n_slots in ((None, 0), (None, 2), (slot_map, 0), (slot_map, -1)):
+            assert fn(C.byref(asm), p, 0, 0, 0, 0, contig_slot, n_slots, p, None) == -1
+            assert b"bad slot map" in lib.nmb_last_error() and fn.__name__.encode() in lib.nmb_last_error()
+        assert fn(C.byref(asm), p, 0, 1, 0, 0, None, 1, p, None) == -1  # tiles outside the assembly
+    assert lib.nmb_sweep_finalize(p, 0, None) == -1 and lib.nmb_sweep_bipartite_finalize(p, 0, None) == -1
+    assert lib.nmb_sweep_slice(p, 0, 0, p, 1, 1, 0, None) == -1

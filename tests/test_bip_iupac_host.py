@@ -97,7 +97,7 @@ def test_scratch_per_bin():
     assert bip_iupac_scratch_bytes() == 2 * 4 * (16 * 14 ** 5 + 4 * 14 ** 6) == 309_786_624
 
 
-def test_entry_points_refuse_bad_arguments():
+def test_slice_expand_and_filter_refuse_bad_arguments():
     lib = _lib.lib
     buf = np.zeros(16, dtype=np.uint32)
     p = buf.ctypes.data
@@ -114,8 +114,9 @@ def test_entry_points_refuse_bad_arguments():
     assert lib.nmb_sweep_bip_iupac_expand(p, p, 0, 1, None) == -1
     f = lib.nmb_sweep_bip_iupac_expand_filter
     n_out = np.zeros(1, dtype=np.int64).ctypes.data
-    assert f(p, p, 1, 14, 0.7, 5, None, 10, n_out, None) == -1  # null output with room for records
-    assert b"null output" in lib.nmb_last_error()
-    assert f(p, p, 1, 14, 0.7, 5, p, 10, None, None) == -1
-    assert f(p, p, 1, 14 ** 9, 0.7, 5, p, 10, n_out, None) == -1  # table index past 32 bits
-    assert f(p, p, 1, 14, 0.7, -1, p, 10, n_out, None) == -1
+    for prune in (0, 1):
+        assert f(p, p, 1, 14, 0.7, 5, prune, None, 10, n_out, None) == -1  # null output with room for records
+        assert b"null output" in lib.nmb_last_error()
+        assert f(p, p, 1, 14, 0.7, 5, prune, p, 10, None, None) == -1
+        assert f(p, p, 1, 14 ** 9, 0.7, 5, prune, p, 10, n_out, None) == -1  # table index past 32 bits
+        assert f(p, p, 1, 14, 0.7, -1, prune, p, 10, n_out, None) == -1

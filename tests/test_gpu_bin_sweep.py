@@ -110,7 +110,7 @@ def test_histograms_equal_one_index_per_bin(world, sweeps, mt):
     assert total > 0
 
 
-def test_subset_and_skipped_slots(world):
+def test_subset_and_skipped_slots_through_the_slot_map(world):
     """bins= sweeps a subset; a contig mapped to -1 counts nowhere, so slots no contig maps to stay zero."""
     import ctypes as C
 
@@ -135,8 +135,8 @@ def test_subset_and_skipped_slots(world):
     hist = torch.zeros(len(BINS) * HIST_SIZE, dtype=torch.int32, device=d)
     cmap = torch.from_numpy(slot_of).to(d)
     base = _lib.ptr(scorer.pileup.class_records)
-    _lib.check(_lib.lib.nmb_sweep_hist_slots(C.byref(asm.view()), base, 0, asm.n_tiles, _lib.ptr(cmap), len(BINS),
-                                             _lib.ptr(hist), None))
+    _lib.check(_lib.lib.nmb_sweep_hist(C.byref(asm.view()), base, 0, asm.n_tiles, 0, 0, _lib.ptr(cmap), len(BINS),
+                                       _lib.ptr(hist), None))
     torch.cuda.synchronize()
     hist = hist.view(len(BINS), HIST_SIZE)
     for s, b in enumerate(BINS):

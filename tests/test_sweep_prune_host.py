@@ -125,49 +125,46 @@ def test_oracle_equals_brute_force(name, n_axes, n_states):
         P.sweep_prune(n_mod[:-1], n_nomod[:-1], lattice, 0.7, 5)
 
 
-def test_entry_points_refuse_bad_arguments():
+def test_filters_refuse_bad_arguments_with_and_without_prune():
     lib = _lib.lib
     buf = np.zeros(16, dtype=np.uint32)
     p = buf.ctypes.data
     n_out = np.zeros(1, dtype=np.int64).ctypes.data
 
-    f = lib.nmb_sweep_expand_filter_prune
+    f = lib.nmb_sweep_expand_filter
+    g = lib.nmb_sweep_bipartite_filter
+    h = lib.nmb_sweep_bip_iupac_expand_filter
+    for prune in (0, 1):
+        def contiguous(nm=p, nu=p, slots=1, inner=15 ** 3, k=5, mp=1, min_mod=5, prune=prune, out=p, cap=10, n=n_out):
+            return f(nm, nu, slots, inner, k, mp, 0.7, min_mod, prune, out, cap, n, None)
 
-    def contiguous(nm=p, nu=p, slots=1, inner=15 ** 3, k=5, mp=1, min_mod=5, out=p, cap=10, n=n_out):
-        return f(nm, nu, slots, inner, k, mp, 0.7, min_mod, out, cap, n, None)
+        for kw in ({"out": None}, {"n": None}, {"nm": None}, {"nu": None}, {"slots": -1}, {"min_mod": -1}, {"cap": -1},
+                   {"k": 3, "inner": 15 ** 1}, {"k": 9, "inner": 15 ** 7}, {"mp": 5}, {"mp": -1},
+                   {"inner": 15 ** 2}, {"inner": 15 ** 4}, {"inner": 15 ** 9}, {"inner": 0}, {"prune": 2}):
+            assert contiguous(**kw) == -1, (prune, kw)
+            assert b"nmb_sweep_expand_filter" in lib.nmb_last_error(), (prune, kw)
+        assert contiguous(out=None) == -1 and b"null output" in lib.nmb_last_error()
+        assert contiguous(inner=15 ** 9) == -1 and b"15^(k-2)" in lib.nmb_last_error()  # table index past 32 bits
 
-    for kw in ({"out": None}, {"n": None}, {"nm": None}, {"nu": None}, {"slots": -1}, {"min_mod": -1}, {"cap": -1},
-               {"k": 3, "inner": 15 ** 1}, {"k": 9, "inner": 15 ** 7}, {"mp": 5}, {"mp": -1},
-               {"inner": 15 ** 2}, {"inner": 15 ** 4}, {"inner": 15 ** 9}, {"inner": 0}):
-        assert contiguous(**kw) == -1, kw
-        assert b"nmb_sweep_expand_filter_prune" in lib.nmb_last_error(), kw
-    assert contiguous(out=None) == -1 and b"null output" in lib.nmb_last_error()
-    assert contiguous(inner=15 ** 9) == -1 and b"15^(k-2)" in lib.nmb_last_error()  # table index past 32 bits
+        def bipartite(hist=p, slots=1, canon=0, min_mod=5, prune=prune, out=p, cap=10, n=n_out):
+            return g(hist, slots, canon, 0.7, min_mod, prune, out, cap, n, None)
 
-    g = lib.nmb_sweep_bipartite_filter_prune
+        for kw in ({"out": None}, {"n": None}, {"hist": None}, {"slots": -1}, {"canon": 4}, {"canon": -1},
+                   {"min_mod": -1}, {"cap": -1}, {"prune": 2}):
+            assert bipartite(**kw) == -1, (prune, kw)
+            assert b"nmb_sweep_bipartite_filter" in lib.nmb_last_error(), (prune, kw)
+        assert bipartite(out=None) == -1 and b"null output" in lib.nmb_last_error()
 
-    def bipartite(hist=p, slots=1, canon=0, min_mod=5, out=p, cap=10, n=n_out):
-        return g(hist, slots, canon, 0.7, min_mod, out, cap, n, None)
+        def iupac(nm=p, nu=p, slots=1, inner=14 ** 4, min_mod=5, prune=prune, out=p, cap=10, n=n_out):
+            return h(nm, nu, slots, inner, 0.7, min_mod, prune, out, cap, n, None)
 
-    for kw in ({"out": None}, {"n": None}, {"hist": None}, {"slots": -1}, {"canon": 4}, {"canon": -1},
-               {"min_mod": -1}, {"cap": -1}):
-        assert bipartite(**kw) == -1, kw
-        assert b"nmb_sweep_bipartite_filter_prune" in lib.nmb_last_error(), kw
-    assert bipartite(out=None) == -1 and b"null output" in lib.nmb_last_error()
-
-    h = lib.nmb_sweep_bip_iupac_expand_filter_prune
-
-    def iupac(nm=p, nu=p, slots=1, inner=14 ** 4, min_mod=5, out=p, cap=10, n=n_out):
-        return h(nm, nu, slots, inner, 0.7, min_mod, out, cap, n, None)
-
-    for kw in ({"out": None}, {"n": None}, {"nm": None}, {"nu": None}, {"slots": -1}, {"min_mod": -1}, {"cap": -1},
-               {"inner": 0}, {"inner": 15}, {"inner": 14 ** 3 + 1}, {"inner": 14 ** 9}):
-        assert iupac(**kw) == -1, kw
-        assert b"nmb_sweep_bip_iupac_expand_filter_prune" in lib.nmb_last_error(), kw
-    assert iupac(out=None) == -1 and b"null output" in lib.nmb_last_error()
-    assert iupac(inner=14 ** 9) == -1 and b"bad argument" in lib.nmb_last_error()  # table index past 32 bits
-    assert iupac(inner=15) == -1 and b"power of 14" in lib.nmb_last_error()
-
+        for kw in ({"out": None}, {"n": None}, {"nm": None}, {"nu": None}, {"slots": -1}, {"min_mod": -1}, {"cap": -1},
+                   {"inner": 0}, {"inner": 15}, {"inner": 14 ** 3 + 1}, {"inner": 14 ** 9}, {"prune": 2}):
+            assert iupac(**kw) == -1, (prune, kw)
+            assert b"nmb_sweep_bip_iupac_expand_filter" in lib.nmb_last_error(), (prune, kw)
+        assert iupac(out=None) == -1 and b"null output" in lib.nmb_last_error()
+        assert iupac(inner=14 ** 9) == -1 and b"bad argument" in lib.nmb_last_error()  # table index past 32 bits
+        assert iupac(inner=15) == -1 and b"power of 14" in lib.nmb_last_error()
     arrays = [np.zeros(15, dtype=np.uint32) for _ in range(3)]
     assert lib.nmb_sweep_prune_lattice(3, *(a.ctypes.data for a in arrays)) == -1
     assert lib.nmb_sweep_prune_lattice(0, None, arrays[1].ctypes.data, arrays[2].ctypes.data) == -1

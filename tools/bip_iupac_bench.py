@@ -58,7 +58,9 @@ def timed(fn):
 
 def phase_passes(sw, ns, min_mean, min_mod):
     """Device time (ms) and bytes of the slice, expansion and fused filter passes of the first `ns` bins over every
-    (gap, shape, modified position) group, each kind summed over the groups; the same launches candidates() makes."""
+    (gap, shape, modified position) group, each kind summed over the groups; the same launches candidates() makes.
+    The buffers are allocated outside the timed windows, so the passes are launched here rather than through
+    sweep._expand."""
     d = sw.asm.device
     canon = {"A": 0, "T": 1, "G": 2, "C": 3}[sw.canonical]
     ms = {"slice": 0.0, "expand": 0.0, "filter": 0.0}
@@ -92,7 +94,7 @@ def phase_passes(sw, ns, min_mean, min_mod):
 
                 def run_filter():
                     check(lib.nmb_sweep_bip_iupac_expand_filter(ptr(tab[0]), ptr(tab[1]), ns, 14 ** (n - 1), min_mean,
-                                                                min_mod, None, 0, ptr(n_out), None))
+                                                                min_mod, 0, None, 0, ptr(n_out), None))
 
                 ms["filter"] += timed(run_filter)
                 nbytes["filter"] += 2 * ns * 4 * 14 ** (n - 1) * 4  # records not counted (count-only run)

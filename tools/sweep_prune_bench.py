@@ -3,7 +3,7 @@
 (synth.cfg3_plan, built by bench.Resident), mod type 'a'.
 
   * BinSweep.candidates() against candidates(prune=True), alternating: wall time (host frame included), device time
-    of the filter passes (CUDA events around every nmb_sweep_*filter* launch), and rows in total, per-bin median and
+    of the filter passes (CUDA events around every nmb_sweep_*filter launch), and rows in total, per-bin median and
     per-bin maximum; the same for bipartite_letters="IUPAC" on the first --iupac-bins bins;
   * planted recovery: how many planted 'a' motifs of sweep shape appear verbatim in their bin's frame, and in how
     many bins where they were not planted;
@@ -51,14 +51,13 @@ def gpu_info() -> dict:
 
 
 class FilterTimer:
-    """Wraps the six filter entry points of the bound library with CUDA events on the current stream; `ms()` is the
+    """Wraps the three filter entry points of the bound library with CUDA events on the current stream; `ms()` is the
     summed device time of the launches since the last reset (call after a synchronize)."""
 
     def __init__(self):
         self.events = []
         for name in FILTERS:
-            for n in (name, name + "_prune"):
-                setattr(lib, n, self._wrap(getattr(lib, n)))
+            setattr(lib, name, self._wrap(getattr(lib, name)))
 
     def _wrap(self, fn):
         def call(*args):
