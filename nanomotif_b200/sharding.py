@@ -214,6 +214,34 @@ class ShardedMultiBinScorer:
                                     self.device, pieces=self.pieces) if mine else None
         self._local_bins = set(mine)
 
+    @classmethod
+    def from_local(cls, local, bins: dict, mod_types, rank: int, world_size: int, device=None, group=None,
+                   split_contigs: bool = True) -> "ShardedMultiBinScorer":
+        """The sharded scorer over a rank's MultiBinScorer built elsewhere -- e.g. MultiBinScorer.from_device over bins
+        generated or parsed on the device, when the host cannot hold the tables.  `bins` = {bin: {contig: sequence or
+        length}} of ALL ranks, the same on every rank; `local` must hold exactly the bins plan(bins, world_size) gives
+        this rank, with as many contigs (or pieces) each, or be None when the plan gives it none."""
+        import torch
+
+        self = cls.__new__(cls)
+        self.rank, self.world_size, self.group = int(rank), int(world_size), group
+        self.owner, per_rank, self.split_bins, self.bin_ranks = self.plan(bins, world_size, split_contigs)
+        mine = per_rank[self.rank]
+        held = {} if local is None else {b: hi - lo for b, (lo, hi) in local._ranges.items()}
+        if held != {b: len(cs) for b, cs in mine.items()}:
+            raise ValueError(f"rank {self.rank}: the local scorer's bins and contig counts are not those the shard plan "
+                             "gives this rank")
+        if local is not None and [str(m) for m in local.mod_types] != [str(m) for m in mod_types]:
+            raise ValueError("the local scorer's mod types differ from mod_types")
+        self.pieces = [(name, seq.name, seq.a, seq.b, seq.shift) for cs in mine.values() for name, seq in cs.items()
+                       if isinstance(seq, ContigPiece)]
+        self.mod_types = list(mod_types)
+        if device is None:
+            device = local.assembly.device if local is not None else torch.device("cuda", torch.cuda.current_device())
+        self.device = torch.device(device)
+        self.local, self._local_bins = local, set(mine)
+        return self
+
     @staticmethod
     def plan(bins: dict, world_size: int, split_contigs: bool = True):
         """The shard plan every rank derives for itself (pure host logic, no device): (owner rank of every contig in
@@ -294,3 +322,140 @@ class ShardedMultiBinScorer:
 
     def score_batch(self, requests) -> list:
         return self.submit(requests).result()
+
+
+def sweep_layout(bins, bin_ranks: Mapping, split_bins, local_bins) -> tuple:
+    """Host logic of ShardedBinSweep for one rank: (designated rank of every bin in `bins` -- the lowest rank holding
+    part of it, 0 for a bin without contigs --; the split bins in `bins` order, which is the row order of the packed
+    all-reduce on every rank; this rank's bins in `bins` order, the slots of its BinSweep; the position in `bins` of
+    each of them, int32)."""
+    designated = {b: min(bin_ranks[b], default=0) for b in bins}
+    split = [b for b in bins if b in split_bins]
+    local = [b for b in bins if b in local_bins]
+    position = {b: i for i, b in enumerate(bins)}
+    return designated, split, local, np.array([position[b] for b in local], dtype=np.int32)
+
+
+def global_parts(parts, global_slot) -> list:
+    """[(group number, hit records)] of a rank's BinSweep -> the same records with slots numbered in the sharded
+    sweep's `bins` (global_slot[local slot]).  Returns new arrays."""
+    out = []
+    for g, h in parts:
+        h = h.copy()
+        h["slot"] = np.asarray(global_slot, dtype=np.int32)[h["slot"]]
+        out.append((g, h))
+    return out
+
+
+class ShardedBinSweep:
+    """The multi-GPU form of sweep.BinSweep over a ShardedMultiBinScorer: every bin's histograms and candidates on the
+    GPUs of one box, with the same candidate frame as one GPU.  Every rank makes every call with the same arguments
+    (like score_batch); the collectives go over scorer.group.
+
+    Each rank fills one BinSweep over the requested bins it holds (one histogram launch per kind).  A bin split over
+    several ranks was counted piecewise: the raw IUPAC and bipartite counters of all split bins are summed by one
+    all-reduce per kind, and the marginalisation runs once on the sum, so the finished histograms are those of one GPU
+    bit for bit (a row lies under windows at most 15 bp from it, less than a piece's 64 bp of halo; DESIGN.md §5).  The
+    bin's designated rank, the lowest holding part of it, keeps the sum; the other holders zero their copy, which then
+    passes no filter (min_mod >= 1).  candidates() gathers every rank's hit records and builds the frame on every rank;
+    counts() and bipartite_iupac_counts() are answered by the designated rank and broadcast.  A bin without contigs
+    has no counters on any rank: its counts are (0, 0) and it has no candidate rows."""
+
+    def __init__(self, scorer, mod_type, bins=None, bipartite: bool = True):
+        from .search import CANONICAL
+        from .sweep import BinSweep
+
+        self.scorer, self.mod_type, self.bipartite = scorer, mod_type, bool(bipartite)
+        scorer.mod_types.index(mod_type)  # an unknown mod type raises ValueError on every rank, as in BinSweep
+        self.canonical = CANONICAL[str(mod_type)]
+        self.bins = list(scorer.bin_ranks) if bins is None else list(bins)
+        for b in self.bins:
+            if b not in scorer.bin_ranks:
+                raise KeyError(b)
+        if len(set(self.bins)) != len(self.bins):
+            raise ValueError("a bin is listed twice")
+        self.designated, split, local_bins, self._global_slot = sweep_layout(self.bins, scorer.bin_ranks,
+                                                                              scorer.split_bins, scorer._local_bins)
+        self.local = BinSweep(scorer.local, mod_type, local_bins, bipartite) if local_bins else None
+        if split:
+            self._merge_split(split)
+
+    def _collective(self) -> bool:
+        import torch.distributed as dist
+
+        return self.scorer.world_size > 1 and dist.is_available() and dist.is_initialized()
+
+    def _merge_split(self, split):
+        """One all-reduce per histogram kind over a packed [n_split][size] int32 tensor, zero rows where this rank holds
+        nothing; the designated rank writes the sums back, the other holders zero their slot."""
+        import torch
+        import torch.distributed as dist
+
+        from .sweep import BIP_SIZE, HIST_SIZE
+
+        sw, d = self.local, self.scorer.device
+        held = [(i, sw.slot[b], self.designated[b] == self.scorer.rank) for i, b in enumerate(split)
+                if sw is not None and b in sw.slot]
+        kinds = [("raw", HIST_SIZE)] + ([("bip_raw", BIP_SIZE)] if self.bipartite else [])
+        for attr, size in kinds:
+            with torch.cuda.device(d):
+                packed = torch.zeros((len(split), size), dtype=torch.int32, device=d)
+                slots = getattr(sw, attr).view(-1, size) if sw is not None else None
+                for i, s, _ in held:
+                    packed[i] = slots[s]
+                if self._collective():
+                    dist.all_reduce(packed, op=dist.ReduceOp.SUM, group=self.scorer.group)
+                for i, s, keep in held:
+                    slots[s] = packed[i] if keep else 0
+        if sw is not None:
+            sw._hist = sw._bip = None
+
+    def candidates(self, min_mean: float = 0.7, min_mod: int = 50, ks=range(4, 9), bipartite: bool = True,
+                   scratch_bytes: int = 8 << 30, capacity: int = 1 << 20, bipartite_letters: str = "ACGT",
+                   prune: bool = False):
+        """BinSweep.candidates over the sharded bins (same arguments, errors and frame): every rank runs its local
+        passes, the hit records of all ranks are gathered, and every rank returns the whole frame."""
+        from .sweep import _candidate_groups, _frame
+
+        # the argument checks run on every rank before any collective, so a bad argument raises everywhere
+        if self.local is not None:
+            groups, bip_groups, parts = self.local._hits(min_mean, min_mod, ks, bipartite, scratch_bytes, capacity,
+                                                         bipartite_letters, prune)
+            parts = global_parts(parts, self._global_slot)
+        else:
+            _, groups, bip_groups = _candidate_groups(min_mod, ks, bipartite, bipartite_letters, self.bipartite)
+            parts = []
+        if self._collective():
+            parts = gather_rows(parts, self.scorer.group)
+        return _frame(parts, groups, bip_groups, self.bins, self.mod_type, self.canonical)
+
+    def _answer(self, bin_name, method: str, *args):
+        """The designated rank's BinSweep.<method>(bin_name, *args), broadcast to every rank; an error raised there is
+        raised on every rank (the others would otherwise wait in the broadcast)."""
+        import torch.distributed as dist
+
+        if bin_name not in self.designated:
+            raise KeyError(bin_name)
+        src = self.designated[bin_name]
+        out = [None]
+        if self.scorer.rank == src:
+            try:
+                if self.local is not None and bin_name in self.local.slot:
+                    out[0] = getattr(self.local, method)(bin_name, *args)
+                else:  # a bin without contigs
+                    out[0] = (0, 0)
+            except Exception as exc:  # noqa: BLE001 -- re-raised below, on every rank
+                out[0] = exc
+        if self._collective():
+            dist.broadcast_object_list(out, group=self.scorer.group, group_src=src)
+        if isinstance(out[0], Exception):
+            raise out[0]
+        return out[0]
+
+    def counts(self, bin_name, motif_iupac: str, mod_pos: int) -> tuple[int, int]:
+        """BinSweep.counts: (n_mod, n_nomod) of one IUPAC 4..8-mer or ACGT bipartite motif in one bin, on every rank."""
+        return self._answer(bin_name, "counts", motif_iupac, mod_pos)
+
+    def bipartite_iupac_counts(self, bin_name, left: str, gap: int, right: str, mod_pos: int) -> tuple[int, int]:
+        """BinSweep.bipartite_iupac_counts: the motif left + "N" * gap + right, halves over the 14 letters but N."""
+        return self._answer(bin_name, "bipartite_iupac_counts", left, gap, right, mod_pos)

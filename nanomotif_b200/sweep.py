@@ -548,20 +548,14 @@ class BinSweep:
         next to CCWGG), in the same passes on the device (the filters' prune flag); the frame is the matching
         subsequence of the prune=False one.  Lattices: the 15 IUPAC letters for k-mers, ACGT + * or the 14 letters + *
         for the bipartite halves (* = any of ACGT, never a row)."""
-        if min_mod < 1:
-            raise ValueError("min_mod must be >= 1: every motif without rows has the prior mean 0.5")
-        ks = sorted(set(int(k) for k in ks))
-        if any(not MIN_K <= k <= MAX_K for k in ks):
-            raise ValueError("ks must lie in 4..8")
-        if bipartite_letters not in ("ACGT", "IUPAC"):
-            raise ValueError('bipartite_letters must be "ACGT" or "IUPAC"')
-        if bipartite and self.bip_raw is None:
-            raise ValueError("this BinSweep was made with bipartite=False")
-        groups = [(k, mp) for k in ks for mp in range(k)]
-        bip_groups = None  # None: ACGT halves, one pass over the finished histograms after `groups`
-        if bipartite and bipartite_letters == "IUPAC":
-            bip_groups = [(a, g, b, o if o < a else o + g) for g in range(4, 9) for a, b in _BIP_SHAPES
-                          for o in range(a + b)]
+        groups, bip_groups, parts = self._hits(min_mean, min_mod, ks, bipartite, scratch_bytes, capacity,
+                                               bipartite_letters, prune)
+        return _frame(parts, groups, bip_groups, self.bins, self.mod_type, self.canonical)
+
+    def _hits(self, min_mean, min_mod, ks, bipartite, scratch_bytes, capacity, bipartite_letters, prune):
+        """(groups, bip_groups, [(group number, hit records)]) of candidates(): every pass's records, with the slots of
+        this sweep."""
+        ks, groups, bip_groups = _candidate_groups(min_mod, ks, bipartite, bipartite_letters, self.bip_raw is not None)
         d, n_bins = self.asm.device, len(self.bins)
         state = {"cap": max(int(capacity), 1)}
         parts = []  # (group, hit records)
@@ -618,36 +612,59 @@ class BinSweep:
                       "nmb_sweep_bipartite_filter")
 
             collect(len(groups), launch_bip)
-        return self._frame(parts, groups, bip_groups)
+        return groups, bip_groups, parts
 
-    def _frame(self, parts, groups, bip_groups=None):
-        """bip_groups: None for the ACGT bipartite records (one group after `groups`), else the (a, g, b, mod_pos)
-        of each degenerate bipartite group, numbered from len(groups) on."""
-        import pandas as pd
 
-        group = np.concatenate([np.full(len(h), g, dtype=np.int64) for g, h in parts]) if parts else np.zeros(0, np.int64)
-        hits = np.concatenate([h for _, h in parts]) if parts else np.zeros(0, _lib.SWEEP_HIT_DTYPE)
-        n_groups = len(groups) + (1 if bip_groups is None else len(bip_groups))
-        key = (hits["slot"].astype(np.int64) * n_groups + group) << 32 | hits["index"].astype(np.int64)
-        order = np.argsort(key, kind="stable")
-        hits, group = hits[order], group[order]
-        motif = np.empty(len(hits), dtype=object)
-        mod_position = np.empty(len(hits), dtype=np.int64)
-        for g in np.unique(group):
-            sel = np.flatnonzero(group == g)
-            if g < len(groups):
-                k, mp = groups[g]
-                motif[sel] = decode_motifs(k, mp, hits["index"][sel], self.canonical)
-                mod_position[sel] = mp
-            elif bip_groups is None:
-                motif[sel], mod_position[sel] = decode_bipartite(hits["index"][sel])
-            else:
-                a, gap, b, mp = bip_groups[g - len(groups)]
-                motif[sel] = decode_bipartite_iupac(a, gap, b, mp, hits["index"][sel], self.canonical)
-                mod_position[sel] = mp
-        n_mod, n_nomod = hits["n_mod"].astype(np.int64), hits["n_nomod"].astype(np.int64)
-        names = np.empty(len(self.bins), dtype=object)
-        names[:] = self.bins
-        return pd.DataFrame({"bin": names[hits["slot"]], "mod_type": np.full(len(hits), self.mod_type, dtype=object),
-                             "motif": motif, "mod_position": mod_position, "n_mod": n_mod, "n_nomod": n_nomod,
-                             "mean": (5.0 + n_mod) / (10.0 + n_mod + n_nomod)})
+def _candidate_groups(min_mod, ks, bipartite: bool, bipartite_letters: str, has_bipartite: bool) -> tuple:
+    """The argument checks of BinSweep.candidates and its record groups: (sorted ks, [(k, mod_pos)], bip_groups),
+    bip_groups None for ACGT halves (one pass over the finished histograms after the (k, mod_pos) groups), else the
+    (a, g, b, mod_pos) of every degenerate bipartite group."""
+    if min_mod < 1:
+        raise ValueError("min_mod must be >= 1: every motif without rows has the prior mean 0.5")
+    ks = sorted(set(int(k) for k in ks))
+    if any(not MIN_K <= k <= MAX_K for k in ks):
+        raise ValueError("ks must lie in 4..8")
+    if bipartite_letters not in ("ACGT", "IUPAC"):
+        raise ValueError('bipartite_letters must be "ACGT" or "IUPAC"')
+    if bipartite and not has_bipartite:
+        raise ValueError("this BinSweep was made with bipartite=False")
+    groups = [(k, mp) for k in ks for mp in range(k)]
+    bip_groups = None
+    if bipartite and bipartite_letters == "IUPAC":
+        bip_groups = [(a, g, b, o if o < a else o + g) for g in range(4, 9) for a, b in _BIP_SHAPES
+                      for o in range(a + b)]
+    return ks, groups, bip_groups
+
+
+def _frame(parts, groups, bip_groups, bins, mod_type, canonical: str):
+    """The candidate frame of hit records [(group number, records)] whose slots index `bins`: rows in slot order, then
+    group, then table index.  bip_groups: None for the ACGT bipartite records (one group after `groups`), else the
+    (a, g, b, mod_pos) of each degenerate bipartite group, numbered from len(groups) on."""
+    import pandas as pd
+
+    group = np.concatenate([np.full(len(h), g, dtype=np.int64) for g, h in parts]) if parts else np.zeros(0, np.int64)
+    hits = np.concatenate([h for _, h in parts]) if parts else np.zeros(0, _lib.SWEEP_HIT_DTYPE)
+    n_groups = len(groups) + (1 if bip_groups is None else len(bip_groups))
+    key = (hits["slot"].astype(np.int64) * n_groups + group) << 32 | hits["index"].astype(np.int64)
+    order = np.argsort(key, kind="stable")
+    hits, group = hits[order], group[order]
+    motif = np.empty(len(hits), dtype=object)
+    mod_position = np.empty(len(hits), dtype=np.int64)
+    for g in np.unique(group):
+        sel = np.flatnonzero(group == g)
+        if g < len(groups):
+            k, mp = groups[g]
+            motif[sel] = decode_motifs(k, mp, hits["index"][sel], canonical)
+            mod_position[sel] = mp
+        elif bip_groups is None:
+            motif[sel], mod_position[sel] = decode_bipartite(hits["index"][sel])
+        else:
+            a, gap, b, mp = bip_groups[g - len(groups)]
+            motif[sel] = decode_bipartite_iupac(a, gap, b, mp, hits["index"][sel], canonical)
+            mod_position[sel] = mp
+    n_mod, n_nomod = hits["n_mod"].astype(np.int64), hits["n_nomod"].astype(np.int64)
+    names = np.empty(len(bins), dtype=object)
+    names[:] = bins
+    return pd.DataFrame({"bin": names[hits["slot"]], "mod_type": np.full(len(hits), mod_type, dtype=object),
+                         "motif": motif, "mod_position": mod_position, "n_mod": n_mod, "n_nomod": n_nomod,
+                         "mean": (5.0 + n_mod) / (10.0 + n_mod + n_nomod)})
