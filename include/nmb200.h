@@ -49,7 +49,7 @@
 extern "C" {
 #endif
 
-#define NMB_ABI_VERSION 8 /* 2: lane-interleaved tile records (NMB_WORD_SLOT), chunk_info flag bits 28-30; 3: table ingest; 4: nmb_pack_motifs; 5: per-bin sweep slots; 6: degenerate bipartite sweep; 7: sweep candidate pruning; 8: one sweep entry point per filter and histogram kind (slots and prune as arguments) */
+#define NMB_ABI_VERSION 9 /* 2: lane-interleaved tile records (NMB_WORD_SLOT), chunk_info flag bits 28-30; 3: table ingest; 4: nmb_pack_motifs; 5: per-bin sweep slots; 6: degenerate bipartite sweep; 7: sweep candidate pruning; 8: one sweep entry point per filter and histogram kind (slots and prune as arguments); 9: nmb_sweep_lookup, motif counts gathered from the finished sweep histograms */
 
 #if defined(__GNUC__)
 #define NMB_API __attribute__((visibility("default")))
@@ -590,6 +590,36 @@ NMB_API int nmb_sweep_bip_iupac_expand_filter(const uint32_t *n_mod, const uint3
  * state s (A=0 T=1 G=2 C=3 other=4); widen[i] / narrow[i]: bit j set when letter j covers letter i / letter i covers
  * letter j.  Writes up to 15 entries per array and returns the number of letters. */
 NMB_API int nmb_sweep_prune_lattice(int32_t lattice, uint32_t *states, uint32_t *widen, uint32_t *narrow);
+
+/* ---- K8 lookup (ABI 9): the counts of any list of motifs in every slot, gathered from the FINISHED histograms ----
+ * A motif's count is the sum of the histogram cells of the concrete motifs it stands for, with the modified letter
+ * fixed.  One record per motif says which cells; the kernel knows no motif layout.  cells = product of n_states[p]
+ * over p < n_pos; cell (d_0, .., d_{n_pos-1}) (mixed radix, the last position the least significant digit) has its
+ * class-0 counter at base + sum_p offset[p][d_p] and its class-1 counter class_step counters later, both relative to
+ * the slot's histogram.  Concrete letters and the modified letter are folded into base, so a concrete motif has
+ * n_pos = 0 and one cell.  Contiguous k-mers (kind 0): base = sum_{j<k} j*2*5^j + mod_pos*2*5^k + the digits of the
+ * concrete letters times 5^(k-1-i), class_step = 5^k, offset = state x 5^(k-1-i) for the states a letter stands for
+ * (N: all five).  Bipartite (kind 1): base = the shape's block + o*2*4^(a+b) + the concrete letters' window bits,
+ * class_step = 4^(a+b), offset = the window index bits of each state (x << xbit | y << ybit, see above). */
+typedef struct nmb_sweep_query {
+    int32_t kind;          /* 0: IUPAC histogram (hist), 1: bipartite histogram (bip) */
+    int32_t n_pos;         /* degenerate positions, 0..7 */
+    int64_t base;          /* class-0 counter of cell 0 */
+    int32_t class_step;    /* class-1 counter - class-0 counter */
+    uint8_t n_states[7];   /* states of degenerate position p: 1..5 (kind 0), 1..4 (kind 1) */
+    uint8_t reserved;      /* 0 */
+    int32_t offset[7][5];  /* counter offset of state d at degenerate position p, >= 0 */
+} nmb_sweep_query; /* 168 bytes */
+
+/* out[r][q][0..1] (device int64, row-major [n_rows][n_queries][2]) = the exact sums of the class-0 (methylated) and
+ * class-1 (unmethylated) counters of query q in slot slots[r] (device int32; NULL: slot r); a negative slot gives a
+ * row of zeros.  hist: finished IUPAC histograms stacked at nmb_sweep_hist_size(); bip: finished bipartite
+ * histograms stacked at nmb_sweep_bipartite_size(), or NULL when no query has kind 1.  queries: device records.
+ * Every existing table entry equals its sum mod 2^32.  A record the kernel cannot read safely (kind, n_pos or
+ * n_states out of range, a negative offset, a counter past the end of its histogram, kind 1 with bip NULL) gives -1
+ * in both entries.  n_rows 0..65535.  Deterministic (no atomics); one launch. */
+NMB_API int nmb_sweep_lookup(const uint32_t *hist, const uint32_t *bip, const int32_t *slots, int32_t n_rows,
+                             const nmb_sweep_query *queries, int64_t n_queries, int64_t *out, void *stream);
 
 /* ---- host helper: CPython's random.sample(range(n), k) on a transplanted MT19937 state (the reference draws its
  *      background windows with random.sample, nanomotif/seq.py:202-225; its picks depend only on n, k and the

@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libnmb200.so")
 
 # ---- constants mirrored from include/nmb200.h -------------------------------------------------
-ABI_VERSION = 8
+ABI_VERSION = 9
 CHUNK_WORDS = 16
 CHUNK_BP = 512
 TILE_WORDS = 2048
@@ -79,6 +79,20 @@ assert JOB_DTYPE.itemsize == 48
 SWEEP_HIT_DTYPE = np.dtype([("slot", np.int32), ("index", np.uint32), ("n_mod", np.uint32), ("n_nomod", np.uint32)])
 assert SWEEP_HIT_DTYPE.itemsize == 16
 
+SWEEP_QUERY_DTYPE = np.dtype(
+    [
+        ("kind", np.int32),
+        ("n_pos", np.int32),
+        ("base", np.int64),
+        ("class_step", np.int32),
+        ("n_states", np.uint8, (7,)),
+        ("reserved", np.uint8),
+        ("offset", np.int32, (7, 5)),
+    ],
+    align=True,
+)
+assert SWEEP_QUERY_DTYPE.itemsize == 168
+
 _P = C.c_void_p
 _I32 = C.c_int32
 _I64 = C.c_int64
@@ -118,6 +132,7 @@ SIGNATURES = {
     "nmb_sweep_bip_iupac_expand": (C.c_int, [_P, _P, _I64, _I64, _P]),
     "nmb_sweep_bip_iupac_expand_filter": (C.c_int, [_P, _P, _I64, _I64, _F64, _I64, _I32, _P, _I64, _P, _P]),
     "nmb_sweep_prune_lattice": (C.c_int, [_I32, _P, _P, _P]),
+    "nmb_sweep_lookup": (C.c_int, [_P, _P, _P, _I32, _P, _I64, _P, _P]),
     "nmb_add_class_planes_compact": (C.c_int, [_P, _P, _P, _P, _I64, _I32, _I32, C.POINTER(NmbAssembly), _I32, _P, _P]),
     "nmb_filter_coverage": (C.c_int, [_P, _I64, _I64, _P, _P]),
     "nmb_filter_min_mod_frequency": (C.c_int, [_P, _P, _I64, _I32, _F64, _F64, _I64, _P, _P, _P]),

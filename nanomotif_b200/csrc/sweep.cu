@@ -660,6 +660,110 @@ __global__ void __launch_bounds__(256) bip_filter_kernel(const uint32_t *__restr
     }
 }
 
+// ---- lookup (ABI 9): the counts of listed motifs, gathered from the finished histograms (nmb_sweep_query) ----
+// One warp per (query, run of kLookupRun output rows).  A query of >= 32 cells spreads its cells over the 32 lanes and
+// takes the run's rows one after the other; a smaller one puts 32 / cells rows side by side, one cell per lane.  Each
+// lane sums its cells in uint64, the lanes of a row are reduced with shuffles and the row's first lane writes the pair:
+// no atomics, so the sums do not depend on the schedule.  The cost is proportional to the cells read.
+constexpr int kLookupRun = 32, kLookupWarps = 8;
+constexpr int kLookupMaxPos = 7, kLookupQueryWords = (int)(sizeof(nmb_sweep_query) / 4);
+static_assert(sizeof(nmb_sweep_query) == 168, "nmb_sweep_query layout is fixed by the header");
+
+// Whether every counter the record addresses lies inside its slot's histogram (both classes).
+__device__ __forceinline__ bool lookup_readable(const nmb_sweep_query &q, const uint32_t *table, int64_t size) {
+    if (!table || q.kind < 0 || q.kind > 1 || q.n_pos < 0 || q.n_pos > kLookupMaxPos || q.base < 0 || q.class_step < 0)
+        return false;
+    const int max_states = q.kind == 0 ? 5 : 4;
+    int64_t last = q.base + q.class_step;
+    for (int p = 0; p < q.n_pos; ++p) {
+        if (q.n_states[p] < 1 || q.n_states[p] > max_states) return false;
+        int32_t hi = 0;
+        for (int d = 0; d < q.n_states[p]; ++d) {
+            if (q.offset[p][d] < 0) return false;
+            hi = max(hi, q.offset[p][d]);
+        }
+        last += hi;
+    }
+    return last < size;
+}
+
+__global__ void __launch_bounds__(kLookupWarps * 32) sweep_lookup_kernel(const uint32_t *__restrict__ hist,
+                                                                          const uint32_t *__restrict__ bip,
+                                                                          const int32_t *__restrict__ slots, int n_rows,
+                                                                          const nmb_sweep_query *__restrict__ queries,
+                                                                          int64_t n_queries, int64_t *__restrict__ out) {
+    __shared__ nmb_sweep_query sq[kLookupWarps];
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const nmb_sweep_query &q = sq[w];
+    const int runs = (n_rows + kLookupRun - 1) / kLookupRun;
+    const int64_t items = n_queries * runs, warps = (int64_t)gridDim.x * kLookupWarps;
+    for (int64_t item = (int64_t)blockIdx.x * kLookupWarps + w; item < items; item += warps) {
+        const int64_t qi = item / runs;
+        const int r0 = (int)(item - qi * runs) * kLookupRun, r1 = min(r0 + kLookupRun, n_rows);
+        __syncwarp();  // the lanes are done with the previous record
+        const uint32_t *src = reinterpret_cast<const uint32_t *>(queries + qi);
+        for (int i = lane; i < kLookupQueryWords; i += 32) reinterpret_cast<uint32_t *>(&sq[w])[i] = __ldg(src + i);
+        __syncwarp();
+        const uint32_t *table = q.kind == 1 ? bip : hist;
+        const int64_t size = q.kind == 1 ? kBipHistSize : kSweepHistSize;
+        if (!lookup_readable(q, table, size)) {
+            for (int r = r0 + lane; r < r1; r += 32) {
+                int64_t *o = out + ((int64_t)r * n_queries + qi) * 2;
+                o[0] = o[1] = -1;
+            }
+            continue;
+        }
+        const int n_pos = q.n_pos;
+        uint32_t radix[kLookupMaxPos], magic[kLookupMaxPos];
+        int cells = 1;
+#pragma unroll
+        for (int p = 0; p < kLookupMaxPos; ++p) {
+            radix[p] = p < n_pos ? q.n_states[p] : 1u;
+            magic[p] = 0xFFFFFFFFu / radix[p] + 1u;  // x / radix = umulhi(x, magic), exact for x < 2^17 (radix > 1)
+            cells *= (int)radix[p];
+        }
+        const int span = min(cells, 32), per = 32 / span, seg = lane / span, j0 = lane - seg * span;
+        const uint32_t *base = table + q.base;
+        const int64_t step = q.class_step;
+        for (int r = r0; r < r1; r += per) {  // uniform over the warp: the shuffles below see every lane
+            const int row = r + seg;
+            const bool mine = seg < per && row < r1;
+            uint64_t s0 = 0, s1 = 0;
+            const int slot = mine ? (slots ? __ldg(slots + row) : row) : -1;
+            if (slot >= 0) {
+                const uint32_t *h = base + (int64_t)slot * size;
+                for (int c = j0; c < cells; c += span) {
+                    uint32_t x = (uint32_t)c;
+                    int32_t off = 0;
+#pragma unroll
+                    for (int p = kLookupMaxPos - 1; p >= 0; --p) {  // the last position is the least significant digit
+                        if (p >= n_pos) continue;
+                        const uint32_t qt = radix[p] == 1u ? x : __umulhi(x, magic[p]);
+                        off += q.offset[p][x - qt * radix[p]];
+                        x = qt;
+                    }
+                    s0 += __ldg(h + off);
+                    s1 += __ldg(h + off + step);
+                }
+            }
+            // segmented tree reduction: after offset o, lane j0 of a row holds the sum of its row's lanes [j0, j0 + 2o)
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const uint64_t t0 = __shfl_down_sync(0xFFFFFFFFu, s0, o), t1 = __shfl_down_sync(0xFFFFFFFFu, s1, o);
+                if (j0 + o < span) {
+                    s0 += t0;
+                    s1 += t1;
+                }
+            }
+            if (mine && j0 == 0) {
+                int64_t *o = out + ((int64_t)row * n_queries + qi) * 2;
+                o[0] = (int64_t)s0;
+                o[1] = (int64_t)s1;
+            }
+        }
+    }
+}
+
 }  // namespace nmb
 
 extern "C" {
@@ -833,6 +937,22 @@ int nmb_sweep_bip_iupac_expand_filter(const uint32_t *n_mod, const uint32_t *n_n
                                                                                         (cudaStream_t)stream>>>(
         n_mod, n_nomod, n_slots, inner, false, false, min_mean, clamp_min_mod(min_mod), out, capacity,
         (unsigned long long *)n_out);
+    NMB_CUDA(cudaGetLastError());
+    return NMB_OK;
+}
+
+int nmb_sweep_lookup(const uint32_t *hist, const uint32_t *bip, const int32_t *slots, int32_t n_rows,
+                     const nmb_sweep_query *queries, int64_t n_queries, int64_t *out, void *stream) {
+    NMB_REQUIRE(hist && n_rows >= 0 && n_rows <= 65535 && n_queries >= 0 && n_queries <= ((int64_t)1 << 40),
+                "nmb_sweep_lookup: bad argument");
+    NMB_REQUIRE(n_queries == 0 || queries, "nmb_sweep_lookup: null queries");
+    NMB_REQUIRE(n_rows == 0 || n_queries == 0 || out, "nmb_sweep_lookup: null output");
+    if (n_rows == 0 || n_queries == 0) return NMB_OK;
+    const int64_t items = n_queries * ((n_rows + nmb::kLookupRun - 1) / nmb::kLookupRun);
+    int64_t blocks = (items + nmb::kLookupWarps - 1) / nmb::kLookupWarps;
+    if (blocks > 148 * 64) blocks = 148 * 64;
+    nmb::sweep_lookup_kernel<<<(unsigned)blocks, nmb::kLookupWarps * 32, 0, (cudaStream_t)stream>>>(
+        hist, bip, slots, n_rows, queries, n_queries, out);
     NMB_CUDA(cudaGetLastError());
     return NMB_OK;
 }

@@ -459,3 +459,27 @@ class ShardedBinSweep:
     def bipartite_iupac_counts(self, bin_name, left: str, gap: int, right: str, mod_pos: int) -> tuple[int, int]:
         """BinSweep.bipartite_iupac_counts: the motif left + "N" * gap + right, halves over the 14 letters but N."""
         return self._answer(bin_name, "bipartite_iupac_counts", left, gap, right, mod_pos)
+
+    def count_matrix(self, motifs, mod_positions, bins=None):
+        """BinSweep.count_matrix over the sharded bins (same arguments, errors and result, on every rank): each rank
+        gathers the rows of the bins it is the designated rank for (a split bin's sum is there) in one launch, every
+        other row is zero, and one all-reduce of the int64 [bin][motif][2] matrix adds the ranks' rows."""
+        import torch
+        import torch.distributed as dist
+
+        from .sweep import _bin_rows, _lookup_records
+
+        # the checks run on every rank before the collective, so a bad argument raises everywhere
+        records = _lookup_records(motifs, mod_positions, self.bipartite, "this BinSweep was made with bipartite=False")
+        rows = _bin_rows(self.designated, bins)
+        d, sw = self.scorer.device, self.local
+        mine = [i for i, b in enumerate(rows)
+                if self.designated[b] == self.scorer.rank and sw is not None and b in sw.slot]
+        with torch.cuda.device(d):
+            out = torch.zeros((len(rows), len(records), 2), dtype=torch.int64, device=d)
+            if mine:
+                out[torch.tensor(mine, device=d)] = sw._count_device(records, [sw.slot[rows[i]] for i in mine])
+            if out.numel() and self._collective():
+                dist.all_reduce(out, op=dist.ReduceOp.SUM, group=self.scorer.group)
+            out = out.cpu().numpy()
+        return out[..., 0], out[..., 1]

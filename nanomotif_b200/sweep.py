@@ -17,6 +17,7 @@ The same per bin, for all bins of a MultiBinScorer at once (one histogram launch
     sw.candidates(bipartite_letters="IUPAC")                       # bipartite halves over every IUPAC letter but N
     sw.candidates(prune=True)                                      # minus specialisations and mixtures (GATC, not GATCA)
     sw.bipartite_iupac_counts("bin_3", "GAA", 6, "RTCG", 2)        # GAANNNNNNRTCG, modified A at position 2
+    sw.count_matrix(["GATC", "CCWGG", "GAANNNNNNRTCG"], [1, 1, 2])  # (n_mod, n_nomod) [bin][motif], one gather launch
 
 Letters of a motif are indexed in the order of nanomotif/constants.py:2 (A T G C R Y S W K M B D H V N); the
 modified position's own letter is fixed to the concrete canonical base and left out of the table index (a pileup
@@ -295,6 +296,17 @@ class SweepIndex:
         i = self.motif_index(motif_iupac, mod_pos)
         return int(n_mod[i].item()) & 0xFFFFFFFF, int(n_nomod[i].item()) & 0xFFFFFFFF
 
+    def count_many(self, motifs, mod_positions) -> tuple[np.ndarray, np.ndarray]:
+        """(n_mod, n_nomod): int64 arrays [len(motifs)], the exact counts of every listed motif (IUPAC 4..8-mers and
+        X{3,4} N{4..8} Y{3,4} motifs with halves over BIP_LETTERS, see pack_queries) from one nmb_sweep_lookup launch;
+        no table is expanded.  Every table entry equals its count mod 2^32."""
+        records = _lookup_records(motifs, mod_positions, self.bip_raw is not None or self._bip is not None,
+                                  "no bipartite histogram: call add_bipartite() first")
+        with torch.cuda.device(self.asm.device):
+            bip = self.bip if (records["kind"] == 1).any() else None
+            out = _lookup(self.hist, bip, None, 1, records).cpu().numpy()
+        return out[0, :, 0], out[0, :, 1]
+
     def candidates(self, k: int, mod_pos: int, canonical: str = "A", min_mean: float = 0.7, min_mod: int = 50,
                    canonical_form: bool = True) -> list[tuple[str, int, int]]:
         """[(motif, n_mod, n_nomod)] of length k with posterior mean >= min_mean and n_mod >= min_mod; with
@@ -402,6 +414,175 @@ def prune_lattice(name: str) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
     n = lib.nmb_sweep_prune_lattice(PRUNE_LATTICES[name], *(ptr(a) for a in arrays))
     check(n, "nmb_sweep_prune_lattice")
     return tuple(a[:n] for a in arrays)
+
+
+# ---- lookup: the counts of any list of motifs, gathered from the finished histograms (nmb_sweep_lookup) ----
+LOOKUP_REASONS = {
+    1: "a letter outside the 15 IUPAC letters",
+    2: "not a shape of the sweep tables (a 4..8-mer, or X{3,4} N{4..8} Y{3,4} without N in X and Y)",
+    3: "the modified position lies outside the motif",
+    4: "the modified position lies in the gap",
+    5: "the modified position must hold A, C, G or T",
+}
+_LETTER_INDEX = np.full(256, -1, dtype=np.int64)  # byte -> IUPAC_ORDER index
+_LETTER_INDEX[_IUPAC_BYTES] = np.arange(15)
+
+
+def _letter_states(lattice: str, n: int) -> tuple[np.ndarray, np.ndarray]:
+    """([n] number of states, [n][5] the state digits, padded with 0) of the first n letters of a prune lattice."""
+    count = np.zeros(n, dtype=np.int64)
+    digits = np.zeros((n, 5), dtype=np.int64)
+    for i, m in enumerate(prune_lattice(lattice)[0][:n].tolist()):
+        ds = [s for s in range(5) if m >> s & 1]
+        count[i], digits[i, :len(ds)] = len(ds), ds
+    return count, digits
+
+
+_CONTIG_STATES = _letter_states("contiguous", 15)  # A T G C other; N also takes "other"
+_BIP_STATES = _letter_states("bipartite_iupac", 14)  # the last letter of that lattice is the pseudo-letter *
+
+
+def pack_queries(motifs, mod_positions) -> tuple[np.ndarray, np.ndarray]:
+    """(records, status): one nmb_sweep_query per motif (_lib.SWEEP_QUERY_DTYPE) and int8 status, 0 when the tables
+    hold the motif, else a key of LOOKUP_REASONS (its record then has kind -1, which nmb_sweep_lookup answers with -1).
+    Covered: a contiguous motif of 4..8 of the 15 letters IUPAC_ORDER, or a motif of > 8 letters that fully matches
+    [BIP_LETTERS]{3,4} N{4,8} [BIP_LETTERS]{3,4}; the modified position inside the motif (inside a half for bipartite
+    motifs) and holding A, C, G or T -- what SweepIndex.counts and bipartite_iupac_counts accept."""
+    text = np.asarray(list(motifs), dtype=str)
+    mods = np.asarray(mod_positions, dtype=np.int64).reshape(-1)
+    if mods.size != text.size:
+        raise ValueError(f"{text.size} motifs but {mods.size} modified positions")
+    n = text.size
+    records = np.zeros(n, dtype=_lib.SWEEP_QUERY_DTYPE)
+    records["kind"] = -1
+    status = np.zeros(n, dtype=np.int8)
+    lengths = np.char.str_len(text) if n else np.zeros(0, np.int64)
+    for L in np.unique(lengths).tolist():
+        sel = np.flatnonzero(lengths == L)
+        if L < MIN_K or L == MAX_K + 1:
+            status[sel] = 2
+            continue
+        code = text[sel].astype(f"U{L}").view(np.uint32).reshape(-1, L)
+        letter = _LETTER_INDEX[np.minimum(code, 255)]
+        mp = mods[sel]
+        st = np.where((letter < 0).any(1), 1, 0)
+        if L <= MAX_K:
+            st, rec = _pack_contiguous(L, letter, mp, st)
+        else:
+            st, rec = _pack_bipartite(L, letter, mp, st)
+        status[sel] = st
+        records[sel[st == 0]] = rec
+    return records, status
+
+
+def _mod_status(st, letter, mp, L, in_gap):
+    """Status of the modified positions of one length group whose letters and shape were checked (st)."""
+    inside = (mp >= 0) & (mp < L)
+    at = letter[np.arange(len(mp)), np.clip(mp, 0, L - 1)]
+    st = np.where(st != 0, st, np.where(~inside, 3, np.where(in_gap, 4, np.where((at < 0) | (at > 3), 5, 0))))
+    return st
+
+
+def _place(records, deg, count, digits, strides, rank):
+    """Fills n_states / offset of the degenerate positions (deg[:, i]) at their rank in the record."""
+    for i in range(deg.shape[1]):
+        rows = np.flatnonzero(deg[:, i])
+        r = rank[rows, i]
+        records["n_states"][rows, r] = count[rows, i]
+        records["offset"][rows, r, :] = strides(i, digits[rows, i, :])
+    records["n_pos"] = deg.sum(1)
+
+
+def _pack_contiguous(L, letter, mp, st):
+    st = _mod_status(st, letter, mp, L, np.zeros(len(mp), bool))
+    ok = st == 0
+    lid, mpo = letter[ok], mp[ok]
+    count, digits = _CONTIG_STATES[0][lid], _CONTIG_STATES[1][lid]  # [m][L], [m][L][5]
+    stride = 5 ** (L - 1 - np.arange(L))
+    deg = count > 1  # the modified letter is concrete, so it goes into base
+    rec = np.zeros(len(lid), dtype=_lib.SWEEP_QUERY_DTYPE)
+    rec["base"] = hist_offset(L) + mpo * 2 * 5 ** L + (np.where(deg, 0, digits[..., 0]) * stride).sum(1)
+    rec["class_step"] = 5 ** L
+    # motif order: the last degenerate letter, the one with the smallest stride, is the least significant digit
+    _place(rec, deg, count, digits, lambda i, d: d * stride[i], np.cumsum(deg, 1) - 1)
+    return st, rec
+
+
+def _pack_bipartite(L, letter, mp, st):
+    half = (letter >= 0) & (letter < 14)  # BIP_LETTERS: IUPAC_ORDER without N (index 14)
+    shape = np.full(len(mp), -1, dtype=np.int64)  # index in _BIP_SHAPES; the run of N fixes a, g and b
+    for j, (a, b) in enumerate(_BIP_SHAPES):
+        g = L - a - b
+        if 4 <= g <= 8:
+            shape[half[:, :a].all(1) & (letter[:, a:a + g] == 14).all(1) & half[:, a + g:].all(1)] = j
+    st = np.where((st == 0) & (shape < 0), 2, st)
+    a_of, b_of = (np.array(x)[shape] for x in zip(*_BIP_SHAPES))
+    st = _mod_status(st, letter, mp, L, (mp >= a_of) & (mp < L - b_of))
+    ok = np.flatnonzero(st == 0)
+    rec = np.zeros(len(ok), dtype=_lib.SWEEP_QUERY_DTYPE)
+    for j, (a, b) in enumerate(_BIP_SHAPES):
+        at = np.flatnonzero(shape[ok] == j)
+        if not at.size:
+            continue
+        g, rows = L - a - b, ok[at]
+        halves = np.concatenate([letter[rows, :a], letter[rows, a + g:]], axis=1)  # [m][a + b]
+        o = np.where(mp[rows] < a, mp[rows], mp[rows] - g)
+        count, digits = _BIP_STATES[0][halves], _BIP_STATES[1][halves]
+        p = np.arange(a + b)
+        xbit, ybit = np.where(p < a, p, a + p), np.where(p < a, a + p, a + b + p)  # the header's window index
+        bits = lambda i, d: (d >> 1) << xbit[i] | (d & 1) << ybit[i]
+        deg = count > 1
+        first, n = SweepIndex.bipartite_block(a, g, b)
+        r = np.zeros(len(rows), dtype=_lib.SWEEP_QUERY_DTYPE)
+        r["kind"] = 1
+        r["base"] = first + o * 2 * n + np.where(deg, 0, bits(p, digits[..., 0])).sum(1)
+        r["class_step"] = n
+        # reversed motif order: the first letter of the left half, at the lowest window bits, is the least significant
+        _place(r, deg, count, digits, bits, np.cumsum(deg[:, ::-1], 1)[:, ::-1] - 1)
+        rec[at] = r
+    return st, rec
+
+
+def covers(motifs, mod_positions) -> np.ndarray:
+    """bool per motif: whether the sweep tables hold it (pack_queries' status 0).  Motifs with N inside a bipartite
+    half or gaps of more than 8 do not occur in the tables; filter a motif list with this before counting it."""
+    return pack_queries(motifs, mod_positions)[1] == 0
+
+
+def _lookup_records(motifs, mod_positions, has_bipartite: bool, missing: str) -> np.ndarray:
+    """pack_queries, raising ValueError for the first uncovered motif, and `missing` when a bipartite motif is asked
+    of histograms without the bipartite kind."""
+    motifs, mod_positions = list(motifs), np.asarray(mod_positions).reshape(-1)
+    records, status = pack_queries(motifs, mod_positions)
+    bad = np.flatnonzero(status)
+    if bad.size:
+        i = int(bad[0])
+        raise ValueError(f"motif {i} ({motifs[i]!r}, mod_position {mod_positions[i]}): {LOOKUP_REASONS[int(status[i])]}")
+    if not has_bipartite and (records["kind"] == 1).any():
+        raise ValueError(missing)
+    return records
+
+
+def _bin_rows(known, bins) -> list:
+    """The rows of a count matrix: `bins`, or every bin of `known` for None; KeyError for an unknown bin."""
+    rows = list(known) if bins is None else list(bins)
+    for b in rows:
+        if b not in known:
+            raise KeyError(b)
+    if len(set(rows)) != len(rows):
+        raise ValueError("a bin is listed twice")
+    return rows
+
+
+def _lookup(hist: torch.Tensor, bip, slots, n_rows: int, records: np.ndarray) -> torch.Tensor:
+    """[n_rows][len(records)][2] int64 device tensor: nmb_sweep_lookup over the stacked finished histograms."""
+    d = hist.device
+    out = torch.empty((n_rows, len(records), 2), dtype=torch.int64, device=d)
+    if n_rows and len(records):
+        q = torch.from_numpy(records.view(np.uint8)).to(d)
+        check(lib.nmb_sweep_lookup(ptr(hist), ptr(bip), ptr(slots), n_rows, ptr(q), len(records), ptr(out),
+                                   _stream()), "nmb_sweep_lookup")
+    return out
 
 
 def bip_iupac_scratch_bytes() -> int:
@@ -528,6 +709,27 @@ class BinSweep:
     def bipartite_iupac_counts(self, bin_name, left: str, gap: int, right: str, mod_pos: int) -> tuple[int, int]:
         """(n_mod, n_nomod) of the motif left + "N" * gap + right in one bin, halves over BIP_LETTERS."""
         return self.index(bin_name).bipartite_iupac_counts(left, gap, right, mod_pos, keep=False)
+
+    def count_matrix(self, motifs, mod_positions, bins=None) -> tuple[np.ndarray, np.ndarray]:
+        """(n_mod, n_nomod): int64 arrays [len(bins)][len(motifs)], the exact counts of every listed motif in every
+        listed bin (rows follow `bins`, default the sweep's bins), from ONE nmb_sweep_lookup launch over the finished
+        histograms: a motif costs the cells it stands for, not a table expansion.  Motifs as SweepIndex.count_many
+        takes them (covers() tells which a list holds); BinSweep.counts(b, m, p) is the entry mod 2^32."""
+        records = _lookup_records(motifs, mod_positions, self.bip_raw is not None,
+                                  "this BinSweep was made with bipartite=False")
+        rows = _bin_rows(self.slot, bins)
+        out = self._count_device(records, [self.slot[b] for b in rows]).cpu().numpy()
+        return out[..., 0], out[..., 1]
+
+    def _count_device(self, records: np.ndarray, slots) -> torch.Tensor:
+        """[len(slots)][len(records)][2] int64 device tensor of checked records in the given slots of this sweep."""
+        d = self.asm.device
+        with torch.cuda.device(d):
+            if not len(slots) or not len(records):
+                return torch.zeros((len(slots), len(records), 2), dtype=torch.int64, device=d)
+            slot = torch.tensor(slots, dtype=torch.int32, device=d)
+            bip = self.bip if (records["kind"] == 1).any() else None
+            return _lookup(self.hist, bip, slot, len(slots), records)
 
     def candidates(self, min_mean: float = 0.7, min_mod: int = 50, ks=range(MIN_K, MAX_K + 1), bipartite: bool = True,
                    scratch_bytes: int = 8 << 30, capacity: int = 1 << 20, bipartite_letters: str = "ACGT",
