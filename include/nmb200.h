@@ -49,7 +49,7 @@
 extern "C" {
 #endif
 
-#define NMB_ABI_VERSION 9 /* 2: lane-interleaved tile records (NMB_WORD_SLOT), chunk_info flag bits 28-30; 3: table ingest; 4: nmb_pack_motifs; 5: per-bin sweep slots; 6: degenerate bipartite sweep; 7: sweep candidate pruning; 8: one sweep entry point per filter and histogram kind (slots and prune as arguments); 9: nmb_sweep_lookup, motif counts gathered from the finished sweep histograms */
+#define NMB_ABI_VERSION 10 /* 2: lane-interleaved tile records (NMB_WORD_SLOT), chunk_info flag bits 28-30; 3: table ingest; 4: nmb_pack_motifs; 5: per-bin sweep slots; 6: degenerate bipartite sweep; 7: sweep candidate pruning; 8: one sweep entry point per filter and histogram kind (slots and prune as arguments); 9: nmb_sweep_lookup, motif counts gathered from the finished sweep histograms; 10: sibling runs (nmb_compile_motifs_siblings, nmb_scan_count_siblings) replace the family finder */
 
 #if defined(__GNUC__)
 #define NMB_API __attribute__((visibility("default")))
@@ -301,17 +301,24 @@ NMB_API int nmb_scan_count_balanced(const nmb_assembly *assembly_h, const uint32
                                     int32_t max_motif_len, const int32_t *contig_group, int64_t *out, int32_t grid_ctas,
                                     int32_t *work_counter, void *stream);
 
-/* nmb_scan_count with FAMILY sharing: inside every work item's block of motifs_per_item motifs, runs of consecutive
- * motifs that share all constrained positions but one -- the children of one search expansion,
- * find_motifs_bin.py:1116-1145 -- are found on the device (from the raw motif records the programs were compiled
- * from) and evaluated as ONE parent chain plus one shifted indicator plane per member.  Same counts as nmb_scan_count,
- * bit for bit.  motifs: the n_motifs records in the order of `programs`; family_scratch: nmb_family_scratch_bytes(
- * n_motifs) bytes of device memory, overwritten. */
-NMB_API int64_t nmb_family_scratch_bytes(int32_t n_motifs);
-NMB_API int nmb_scan_count_families(const nmb_assembly *assembly_h, const uint32_t *class_records, const void *programs,
-                                    const nmb_job *jobs, int32_t n_jobs, int32_t n_items, int32_t motifs_per_item,
-                                    int32_t max_motif_len, const int32_t *contig_group, int64_t *out, int32_t grid_ctas,
-                                    const nmb_motif *motifs, int32_t n_motifs, void *family_scratch, void *stream);
+/* nmb_compile_motifs that also groups the motifs into SIBLINGS: siblings (nmb_sibling_bytes(n_motifs) bytes of device
+ * memory, overwritten) receives per motif its link to the previous motif -- same len and mod_pos, the same allowed set
+ * at every position but at most one -- and the program of the motif with the position where it differs from the next
+ * motif made a wildcard (the parent of a search expansion's children, find_motifs_bin.py:1116-1145).  Same launch. */
+NMB_API int64_t nmb_sibling_bytes(int32_t n_motifs);
+NMB_API int nmb_compile_motifs_siblings(const nmb_motif *motifs, int32_t n_motifs, void *programs, void *siblings,
+                                        void *stream);
+
+/* nmb_scan_count with SIBLING RUNS: inside every work item's block of motifs_per_item motifs, runs of consecutive
+ * linked motifs that differ at one common position are scored as ONE parent chain plus a four-base split of the parent's
+ * occurrences at that position (warps with a non-ACGT letter in reach score the members one by one).  Same counts as
+ * nmb_scan_count, bit for bit.  programs / siblings: from nmb_compile_motifs_siblings over the same n_motifs records;
+ * work_counter: as for nmb_scan_count_balanced, or NULL for the static item split. */
+NMB_API int nmb_scan_count_siblings(const nmb_assembly *assembly_h, const uint32_t *class_records, const void *programs,
+                                    const void *siblings, int32_t n_motifs, const nmb_job *jobs, int32_t n_jobs,
+                                    int32_t n_items, int32_t motifs_per_item, int32_t max_motif_len,
+                                    const int32_t *contig_group, int64_t *out, int32_t grid_ctas, int32_t *work_counter,
+                                    void *stream);
 
 /* ---- K3: occurrence positions (subseq_indices output and the save_motif_positions=True lists
  *      of motif_model_contig, find_motifs_bin.py:1322-1329) ---- */

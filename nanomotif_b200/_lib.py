@@ -14,7 +14,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libnmb200.so")
 
 # ---- constants mirrored from include/nmb200.h -------------------------------------------------
-ABI_VERSION = 9
+ABI_VERSION = 10
 CHUNK_WORDS = 16
 CHUNK_BP = 512
 TILE_WORDS = 2048
@@ -140,8 +140,9 @@ SIGNATURES = {
     "nmb_compile_motifs": (C.c_int, [_P, _I32, _P, _P]),
     "nmb_scan_count": (C.c_int, [C.POINTER(NmbAssembly), _P, _P, _P, _I32, _I32, _I32, _I32, _P, _P, _I32, _P]),
     "nmb_scan_count_balanced": (C.c_int, [C.POINTER(NmbAssembly), _P, _P, _P, _I32, _I32, _I32, _I32, _P, _P, _I32, _P, _P]),
-    "nmb_family_scratch_bytes": (C.c_int64, [_I32]),
-    "nmb_scan_count_families": (C.c_int, [C.POINTER(NmbAssembly), _P, _P, _P, _I32, _I32, _I32, _I32, _P, _P, _I32, _P, _I32, _P, _P]),
+    "nmb_sibling_bytes": (C.c_int64, [_I32]),
+    "nmb_compile_motifs_siblings": (C.c_int, [_P, _I32, _P, _P, _P]),
+    "nmb_scan_count_siblings": (C.c_int, [C.POINTER(NmbAssembly), _P, _P, _P, _I32, _P, _I32, _I32, _I32, _I32, _P, _P, _I32, _P, _P]),
     "nmb_match_plane": (C.c_int, [C.POINTER(NmbAssembly), _P, _I32, _I32, _I32, _I32, _I32, _P, _P]),
     "nmb_letter_plane": (C.c_int, [_P, _I64, _I32, _I64, _P, _I64, _P]),
     "nmb_compact_positions": (C.c_int, [_P, _P, _I64, _I64, _P, _P, _I64, _P, _P]),

@@ -20,19 +20,20 @@ namespace nmb {
 constexpr int kScanThreads = kTileChunks;                                       // 128
 constexpr int kMaxMpi = NMB_MAX_MOTIFS_PER_ITEM;
 
-// A FAMILY is a run of consecutive motifs of one work item that share all constrained positions but one -- the children
-// of one search expansion (find_motifs_bin.py:1116-1145 adds one base at one position to the same parent).  The parent's
-// two chains are evaluated once; a child is then one indicator plane, shifted to the modified base's alignment, ANDed
-// with the parent's aligned planes: ~6 logic ops per word and strand instead of 4 per word, strand and constrained
-// position.  Offsets are relative to the modified base, which all members share.
-struct FamInfo {
-    uint8_t n;      // at the first member (leader): members in the run (>= 2); 0 elsewhere / for single motifs
-    uint8_t set;    // allowed-set of the member's extra position
-    int8_t delta;   // its offset from the modified base, |delta| <= 31
-    uint8_t pad;
-};
-static_assert(sizeof(FamInfo) == 4, "FamInfo is 4 bytes");
-static_assert(NMB_MAX_MOTIFS_PER_ITEM == 32, "one lane per motif of a block holds its family word");
+// A SIBLING RUN is a maximal sequence (>= 2) of consecutive motifs of one work item's block that have the same len and
+// mod_pos and the same allowed set at every position but one common position j -- the children of one search expansion
+// (find_motifs_bin.py:1116-1145 adds one base at one position to the same parent).  The run is scored as ONE parent
+// chain pair (a member with j made a wildcard, same len and mod_pos, so run_chain_pair's clip keeps exactly the members'
+// starts, contig edges included) plus a four-base split: every parent occurrence is counted by the base it has at j.
+// A member with set S at j counts the sum over S.  Exact wherever every in-contig position holds one of A, C, G, T, i.e.
+// in all but the non-ACGT warps, which score the members one by one.
+//
+// Sibling word of motif i (written by the motif compiler; link = motif i against motif i - 1 in the motif array):
+//   bits 0-5 j, bits 6-7 link (0 none, kSibSame identical, kSibDiff differ at j only, both sets there non-empty),
+//   bits 8-11 motif i's set at j, bits 12-15 motif i-1's set at j.
+// parents[i] is motif i with the position where it differs from motif i + 1 made a wildcard (when they are linked).
+constexpr uint32_t kSibSame = 1, kSibDiff = 2;
+static_assert(NMB_MAX_MOTIFS_PER_ITEM == 32, "one lane per motif of a block holds its sibling word");
 
 struct ScanParams {
     const uint32_t *seq_records;
@@ -44,8 +45,8 @@ struct ScanParams {
     const int64_t *contig_start, *contig_len;
     unsigned long long *out;
     int *counter;             // dynamic item scheduling: {next item, finished CTAs}, zero at launch and at exit; or null
-    const FamInfo *fam;       // per motif: family run length at a leader, the member's extra (set, offset); or null
-    const Program *parents;   // per motif: the family's parent program (valid at leaders)
+    const uint32_t *sib;      // per motif: sibling word; or null (every motif scored on its own)
+    const Program *parents;   // per motif: parent program towards the right neighbour
     int n_jobs, n_items, mpi, n_tiles;
 };
 
@@ -76,54 +77,114 @@ __device__ __forceinline__ int group_of(const nmb_job &job, int contig, const in
     return __ldg(contig_group + contig);
 }
 
-// Indicator plane of allowed-set `code` over the lane's words [-H, NW + H) (all fourteen sets; 0 for anything else).
-template <int H, bool HASN>
-__device__ __forceinline__ void set_indicator(const LaneSeq<H, HASN> &q, int code, uint32_t (&ind)[NW + 2 * H]) {
-    switch (code) {
-#define NMB_CASE(m)                                                                            \
-    case m:                                                                                    \
-        _Pragma("unroll") for (int i = 0; i < NW + 2 * H; ++i) ind[i] = q.template and_code<m>(i, 0xFFFFFFFFu); \
-        break;
-        NMB_CASE(1) NMB_CASE(2) NMB_CASE(3) NMB_CASE(4) NMB_CASE(5) NMB_CASE(6) NMB_CASE(7)
-        NMB_CASE(8) NMB_CASE(9) NMB_CASE(10) NMB_CASE(11) NMB_CASE(12) NMB_CASE(13) NMB_CASE(14)
-#undef NMB_CASE
-        default:
+// Run of siblings that starts at block lane `a` (warp-uniform), formed from the block's sibling words (lane l holds
+// motif l's word, 0 past the block) with ballots: the lanes after `a` that are linked to their left neighbour, cut at
+// the first one that differs at another position.  Identical motifs carry their neighbour's set along.
+struct SibRun {
+    int run;    // members; 1 = motif a scored on its own
+    int first;  // first lane whose link differs at j: parents[first - 1] is the parent
+    int j;      // the split position
+    int set;    // this lane's allowed set at j (lanes of the run)
+};
+
+__device__ __forceinline__ SibRun sibling_run(uint32_t sw, int a) {
+    SibRun r = {1, 0, 0, 0};
+    const int lane = threadIdx.x & 31;
+    const uint32_t link = (sw >> 6) & 3;
+    const unsigned gt = ~((2u << a) - 1u);  // lanes after a
+    const unsigned linked = __ballot_sync(0xFFFFFFFFu, link != 0) & gt;
+    const unsigned diff = __ballot_sync(0xFFFFFFFFu, link == kSibDiff) & linked;
+    const unsigned stop = ~linked & gt;
+    unsigned span = stop ? gt & ((1u << (__ffs(stop) - 1)) - 1u) : gt;
+    if (!(diff & span)) return r;  // nothing linked, or identical motifs only: no position to split at
+    r.first = __ffs(diff & span) - 1;
+    r.j = __shfl_sync(0xFFFFFFFFu, sw & 63, r.first);
+    const unsigned bad = __ballot_sync(0xFFFFFFFFu, link == kSibDiff && (int)(sw & 63) != r.j) & span;
+    if (bad) span &= (1u << (__ffs(bad) - 1)) - 1u;
+    r.run = 1 + __popc(span);
+    // up to the first differing link a member has that link's left set at j, after it the set of its last one
+    const unsigned upto = diff & span & ((2u << lane) - 1u);
+    const uint32_t ws = __shfl_sync(0xFFFFFFFFu, sw, upto ? 31 - __clz(upto) : r.first);
+    r.set = (ws >> (upto ? 8 : 12)) & 0xF;
+    return r;
+}
+
+// Word k of a sequence plane seen o positions to the right (0 <= o < 32 * H): bit b = plane[32 k + b + o].
+template <int H>
+__device__ __forceinline__ uint32_t plane_right(const uint32_t (&w)[NW + 2 * H], int k, int o) {
+    if (H == 1 || o < 32) return __funnelshift_r(w[k + H], w[k + H + 1], o);
+    return __funnelshift_r(w[k + H + 1], w[k + H + 2], o);
+}
+// ... o positions to the left (0 <= o < 32 * H): bit b = plane[32 k + b - o] (the clamped shift of 32 is the word itself).
+template <int H>
+__device__ __forceinline__ uint32_t plane_left(const uint32_t (&w)[NW + 2 * H], int k, int o) {
+    if (H == 1 || o <= 32) return __funnelshift_rc(w[k + H - 1], w[k + H], 32 - o);
+    return __funnelshift_rc(w[k + H - 2], w[k + H - 1], 64 - o);
+}
+
+// Popcounts of P, P & x, P & y, P & x & y: by inclusion-exclusion the occurrences in P with each base (x, y) at j.
+__device__ __forceinline__ void tally(uint32_t pw, uint32_t xs, uint32_t ys, uint32_t *t) {
+    t[0] += __popc(pw);
+    t[1] += __popc(pw & xs);
+    t[2] += __popc(pw & ys);
+    t[3] += __popc(lop3<0x80>(pw, xs, ys));
+}
+
+// Four-base split of a parent's finished chains: for each of the four counters (n_mod / n_nomod per strand) the number
+// of the lane's parent occurrences with A, T, G, C at the split position, delta = j - mod_pos positions from the
+// modified base on the forward strand and -delta on the reverse strand (the reverse-complement occurrence sees the
+// complementary base there).  base[col][b]: b = set bit (A, T, G, C), forward coordinates.
+template <int H>
+__device__ __forceinline__ void split_counts(const LaneSeq<H, false> &q, const uint32_t (&c)[NW + 2 * H],
+                                             const uint32_t (&d)[NW + 2 * H], int sh, bool far, int delta,
+                                             const uint32_t *cl, uint32_t (&base)[4][4]) {
+    // the strand that looks right (delta >= 0: forward) and the one that looks left, so that one pair of windows
+    // serves both signs of delta
+    const bool neg = delta < 0;
+    const int o = neg ? -delta : delta;
+    const uint32_t *cr = neg ? cl + 2 * kTileWords : cl, *cf = neg ? cl : cl + 2 * kTileWords;
+    uint32_t t[4][4] = {};  // [right mod, right nomod, left mod, left nomod][all, x, y, xy]
 #pragma unroll
-            for (int i = 0; i < NW + 2 * H; ++i) ind[i] = 0u;
-            break;
+    for (int h = 0; h < NW; h += 4) {
+        const uint4 r0 = *reinterpret_cast<const uint4 *>(cr + (h >> 2) * kSlotStride);
+        const uint4 r1 = *reinterpret_cast<const uint4 *>(cr + kTileWords + (h >> 2) * kSlotStride);
+        const uint4 l0 = *reinterpret_cast<const uint4 *>(cf + (h >> 2) * kSlotStride);
+        const uint4 l1 = *reinterpret_cast<const uint4 *>(cf + kTileWords + (h >> 2) * kSlotStride);
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+            const uint32_t mf = aligned_word<H>(c, h + k, sh, far);
+            const uint32_t mr = aligned_word_rc<H>(d, h + k, sh, far);
+            const uint32_t mR = neg ? mr : mf, mL = neg ? mf : mr;
+            const uint32_t xr = plane_right<H>(q.x, h + k, o), yr = plane_right<H>(q.y, h + k, o);
+            const uint32_t xl = plane_left<H>(q.x, h + k, o), yl = plane_left<H>(q.y, h + k, o);
+            const uint32_t w0 = k == 0 ? r0.x : k == 1 ? r0.y : k == 2 ? r0.z : r0.w;
+            const uint32_t w1 = k == 0 ? r1.x : k == 1 ? r1.y : k == 2 ? r1.z : r1.w;
+            const uint32_t w2 = k == 0 ? l0.x : k == 1 ? l0.y : k == 2 ? l0.z : l0.w;
+            const uint32_t w3 = k == 0 ? l1.x : k == 1 ? l1.y : k == 2 ? l1.z : l1.w;
+            tally(mR & w0, xr, yr, t[0]);
+            tally(mR & w1, xr, yr, t[1]);
+            tally(mL & w2, xl, yl, t[2]);
+            tally(mL & w3, xl, yl, t[3]);
+        }
+    }
+#pragma unroll
+    for (int col = 0; col < 4; ++col) {
+        uint32_t u[4];  // right = forward unless delta < 0
+#pragma unroll
+        for (int e = 0; e < 4; ++e) u[e] = neg ? t[col ^ 2][e] : t[col][e];
+        base[col][0] = u[0] - u[1] - u[2] + u[3];               // A = (0, 0)
+        base[col][1] = u[2] - u[3];                             // T = (0, 1)
+        base[col][2] = u[1] - u[3];                             // G = (1, 0)
+        base[col][3] = u[3];                                    // C = (1, 1)
     }
 }
 
-// One strand of one family member: the parent's aligned match words m[0..NW) ANDed with the indicator of the extra
-// position's set seen `shift` positions to the right (negative: to the left), popcounted against two class planes.
-template <int H, bool HASN>
-__device__ __forceinline__ void count_member_strand(const LaneSeq<H, HASN> &q, const uint32_t (&m)[NW], int code, int shift,
-                                                    const uint32_t *cl_a, const uint32_t *cl_b, uint32_t &cnt_a,
-                                                    uint32_t &cnt_b) {
-    constexpr int CW = NW + 2 * H;
-    uint32_t ind[CW];
-    set_indicator<H, HASN>(q, code, ind);
-    if (shift < 0) {  // warp-uniform: look one word to the left, then shift right by 32 - |shift|
-#pragma unroll
-        for (int i = CW - 1; i > 0; --i) ind[i] = ind[i - 1];
-        ind[0] = 0u;
-    }
-    const int s = shift & 31;
-#pragma unroll
-    for (int h = 0; h < NW; h += 4) {
-        const uint4 pa = *reinterpret_cast<const uint4 *>(cl_a + (h >> 2) * kSlotStride);
-        const uint4 pb = *reinterpret_cast<const uint4 *>(cl_b + (h >> 2) * kSlotStride);
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-            const uint32_t w = m[h + k] & __funnelshift_r(ind[h + k + H], ind[h + k + H + 1], s);
-            cnt_a += __popc(w & (k == 0 ? pa.x : k == 1 ? pa.y : k == 2 ? pa.z : pa.w));
-            cnt_b += __popc(w & (k == 0 ? pb.x : k == 1 ? pb.y : k == 2 ? pb.z : pb.w));
-        }
-    }
+__device__ __forceinline__ uint32_t sum_over_set(const uint32_t (&b)[4], int s) {
+    return ((s & 1) ? b[0] : 0u) + ((s & 2) ? b[1] : 0u) + ((s & 4) ? b[2] : 0u) + ((s & 8) ? b[3] : 0u);
 }
 
 // Evaluate the item's motifs on this lane's chunk and accumulate the four counters.
-template <int H, bool PLANES, bool FAM>
+template <int H, bool PLANES>
 __device__ __forceinline__ void score_motifs(const ScanParams &p, const nmb_job &job, const ItemMeta &meta,
                                              const LaneSeq<H, PLANES> &q, const LaneEdge &edge, const uint32_t *cl,
                                              bool valid,
@@ -131,11 +192,12 @@ __device__ __forceinline__ void score_motifs(const ScanParams &p, const nmb_job 
                                              uint32_t (*acc)[4]) {
     const int m_begin = job.motif_begin + meta.mblk * p.mpi;
     const int m_count = min(p.mpi, job.motif_count - meta.mblk * p.mpi);
-    // family table of the whole block in ONE coalesced load (lane l holds motif l's word; kMaxMpi == 32): looked up
-    // with shuffles below, so no motif waits for a dependent global load before its program can be fetched
-    uint32_t fam_w = 0;
-    if (FAM && !PLANES && !edge.edge && (int)(threadIdx.x & 31) < m_count)
-        fam_w = __ldg(reinterpret_cast<const uint32_t *>(p.fam + m_begin) + (threadIdx.x & 31));
+    // sibling words of the whole block in ONE coalesced load (lane l holds motif l's word; kMaxMpi == 32): the runs
+    // are formed with ballots and shuffles below, so no motif waits for a dependent global load before its program
+    // can be fetched.  Warps with a non-ACGT letter in reach score every motif on its own.
+    const bool siblings = !PLANES && p.sib != nullptr;  // warp-uniform
+    uint32_t sw = 0;
+    if (siblings && (int)(threadIdx.x & 31) < m_count) sw = __ldg(p.sib + m_begin + (threadIdx.x & 31));
 
     // per-lane counts of one motif -> warp sums -> the CTA's accumulators / the output
     auto flush = [&](int mi, uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3) {
@@ -168,73 +230,53 @@ __device__ __forceinline__ void score_motifs(const ScanParams &p, const nmb_job 
     int mi = 0;
 #pragma unroll 1
     while (mi < m_count) {
-        // A family (see FamInfo) is taken as one parent + members only by warps without non-ACGT letters or contig
-        // edges in reach; the other warps take the members one by one (every member keeps its own program).
-        int run = 1;
-        const Program *prog = p.programs + (size_t)(m_begin + mi) * 2;
-        if (FAM && !PLANES && !edge.edge) {  // warp-uniform
-            const int n = __shfl_sync(0xFFFFFFFFu, fam_w, mi) & 0xFF;
-            if (n >= 2) {
-                run = n;
-                prog = p.parents + (m_begin + mi);
-            }
-        }
-        // ONE program serves both strands (scan.cuh: run_chain_pair) -- the motif's own, or the family's parent
-        const ProgramView pv = load_program(prog);
+        SibRun sr = {1, 0, 0, 0};
+        if (siblings) sr = sibling_run(sw, mi);
+        // ONE program serves both strands (scan.cuh: run_chain_pair) -- the motif's own, or the run's parent
+        const ProgramView pv = load_program(sr.run > 1 ? p.parents + (m_begin + sr.first - 1)
+                                                       : p.programs + (size_t)(m_begin + mi) * 2);
         uint32_t c[NW + 2 * H], d[NW + 2 * H];
         if (run_chain_pair<H, PLANES>(pv, q, c, d, edge)) {  // else: no occurrence in this warp's chunks
             const bool far = pv.mod_pos >= 32;  // only possible when H == 2
             const int sh = pv.mod_pos & 31;
-            if (!FAM || run == 1) {
-                uint32_t cnt[4] = {0, 0, 0, 0};  // n_mod '+', n_nomod '+', n_mod '-', n_nomod '-'
-#pragma unroll
-                for (int h = 0; h < NW; h += 4) {
-                    uint4 pl[4];
-#pragma unroll
-                    for (int k = 0; k < 4; ++k)
-                        pl[k] = *reinterpret_cast<const uint4 *>(cl + k * kTileWords + (h >> 2) * kSlotStride);
-#pragma unroll
-                    for (int k = 0; k < 4; ++k) {
-                        const uint32_t mf = aligned_word<H>(c, h + k, sh, far);
-                        const uint32_t mr = aligned_word_rc<H>(d, h + k, sh, far);
-                        const uint32_t w0 = k == 0 ? pl[0].x : k == 1 ? pl[0].y : k == 2 ? pl[0].z : pl[0].w;
-                        const uint32_t w1 = k == 0 ? pl[1].x : k == 1 ? pl[1].y : k == 2 ? pl[1].z : pl[1].w;
-                        const uint32_t w2 = k == 0 ? pl[2].x : k == 1 ? pl[2].y : k == 2 ? pl[2].z : pl[2].w;
-                        const uint32_t w3 = k == 0 ? pl[3].x : k == 1 ? pl[3].y : k == 2 ? pl[3].z : pl[3].w;
-                        cnt[0] += __popc(mf & w0);  // occurrences whose modified base is methylated, '+'
-                        cnt[1] += __popc(mf & w1);  // ... unmethylated, '+'
-                        cnt[2] += __popc(mr & w2);  // reverse-complement occurrences, '-' strand rows
-                        cnt[3] += __popc(mr & w3);
-                    }
-                }
-                flush(mi, cnt[0], cnt[1], cnt[2], cnt[3]);
-            } else {
-                // the parent's two match planes aligned at the modified base; the chains are dead after this
-                uint32_t mf[NW], mr[NW], any = 0;
-#pragma unroll
-                for (int k = 0; k < NW; ++k) {
-                    mf[k] = aligned_word<H>(c, k, sh, far);
-                    mr[k] = aligned_word_rc<H>(d, k, sh, far);
-                    any |= mf[k] | mr[k];
-                }
-                if (__any_sync(0xFFFFFFFFu, any != 0)) {  // else every member counts 0 in this warp
+            if constexpr (!PLANES) {
+                if (sr.run > 1) {
+                    uint32_t base[4][4];
+                    split_counts<H>(q, c, d, sh, far, sr.j - pv.mod_pos, cl, base);
 #pragma unroll 1
-                    for (int k = 0; k < run; ++k) {
-                        const uint32_t fi = __shfl_sync(0xFFFFFFFFu, fam_w, mi + k);
-                        const int code = (fi >> 8) & 0xF;
-                        const int delta = (int)(int8_t)((fi >> 16) & 0xFF);
-                        uint32_t c0 = 0, c1 = 0, c2 = 0, c3 = 0;
-                        // forward: the member occurs at p iff the parent does and base[p + delta] is in the set;
-                        // reverse complement (aligned at ITS modified base q): base[q - delta] in the complementary set
-                        count_member_strand<H, PLANES>(q, mf, code, delta, cl, cl + kTileWords, c0, c1);
-                        count_member_strand<H, PLANES>(q, mr, comp_set(code), -delta, cl + 2 * kTileWords,
-                                                       cl + 3 * kTileWords, c2, c3);
-                        flush(mi + k, c0, c1, c2, c3);
+                    for (int k = 0; k < sr.run; ++k) {
+                        const int s = __shfl_sync(0xFFFFFFFFu, sr.set, mi + k);
+                        flush(mi + k, sum_over_set(base[0], s), sum_over_set(base[1], s),
+                              sum_over_set(base[2], comp_set(s)), sum_over_set(base[3], comp_set(s)));
                     }
+                    mi += sr.run;
+                    continue;
                 }
             }
+            uint32_t cnt[4] = {0, 0, 0, 0};  // n_mod '+', n_nomod '+', n_mod '-', n_nomod '-'
+#pragma unroll
+            for (int h = 0; h < NW; h += 4) {
+                uint4 pl[4];
+#pragma unroll
+                for (int k = 0; k < 4; ++k)
+                    pl[k] = *reinterpret_cast<const uint4 *>(cl + k * kTileWords + (h >> 2) * kSlotStride);
+#pragma unroll
+                for (int k = 0; k < 4; ++k) {
+                    const uint32_t mf = aligned_word<H>(c, h + k, sh, far);
+                    const uint32_t mr = aligned_word_rc<H>(d, h + k, sh, far);
+                    const uint32_t w0 = k == 0 ? pl[0].x : k == 1 ? pl[0].y : k == 2 ? pl[0].z : pl[0].w;
+                    const uint32_t w1 = k == 0 ? pl[1].x : k == 1 ? pl[1].y : k == 2 ? pl[1].z : pl[1].w;
+                    const uint32_t w2 = k == 0 ? pl[2].x : k == 1 ? pl[2].y : k == 2 ? pl[2].z : pl[2].w;
+                    const uint32_t w3 = k == 0 ? pl[3].x : k == 1 ? pl[3].y : k == 2 ? pl[3].z : pl[3].w;
+                    cnt[0] += __popc(mf & w0);  // occurrences whose modified base is methylated, '+'
+                    cnt[1] += __popc(mf & w1);  // ... unmethylated, '+'
+                    cnt[2] += __popc(mr & w2);  // reverse-complement occurrences, '-' strand rows
+                    cnt[3] += __popc(mr & w3);
+                }
+            }
+            flush(mi, cnt[0], cnt[1], cnt[2], cnt[3]);
         }
-        mi += run;
+        mi += sr.run;
     }
 }
 
@@ -250,7 +292,7 @@ __device__ __forceinline__ void bar_sync_1(int n_threads) { asm volatile("bar.sy
 // sequence record is already on its way while this item's motifs are evaluated; only the class record (2/3 of the
 // bytes) has to wait for the end of the item.  ncu's source view had 19 % of all warp samples on the mbarrier spin in
 // front of a tile (profiles/r02_notes.md).
-template <int H, int STAGES, bool FAM>
+template <int H, int STAGES>
 __global__ void __launch_bounds__(kScanThreads, 4) scan_count_kernel(const ScanParams p) {
     static_assert(STAGES == 1, "one tile buffer per CTA");
     extern __shared__ __align__(128) uint8_t smem[];
@@ -358,14 +400,14 @@ __global__ void __launch_bounds__(kScanThreads, 4) scan_count_kernel(const ScanP
             load_xyn<H>(sx, sy, tid, p.nonacgt + kHalo + (size_t)meta.tile * kTileWords + tid * NW - H, q);
             seq_done_prefetch_next();
             const LaneEdge edge = {0, false, false};
-            score_motifs<H, true, FAM>(p, job, meta, q, edge, cl, valid, uniform, peers, leader, g, primary, s_acc[par]);
+            score_motifs<H, true>(p, job, meta, q, edge, cl, valid, uniform, peers, leader, g, primary, s_acc[par]);
         } else {
             LaneSeq<H, false> q;
             load_xy<H>(sx, sy, tid, q);
             seq_done_prefetch_next();
             const LaneEdge edge = lane_edge(warp_edge, info, (int64_t)meta.tile * kTileChunks + tid,
                                             p.contig_start, p.contig_len);
-            score_motifs<H, false, FAM>(p, job, meta, q, edge, cl, valid, uniform, peers, leader, g, primary, s_acc[par]);
+            score_motifs<H, false>(p, job, meta, q, edge, cl, valid, uniform, peers, leader, g, primary, s_acc[par]);
         }
         __syncthreads();  // everyone is done with the class record and with s_acc[par]
         if (tid == 0) issue_cls(par ^ 1);
@@ -409,15 +451,48 @@ __device__ void build_program(const uint8_t *allowed, int len, int mp, Program &
     pr.n = (uint8_t)n; pr.mod_pos = (uint8_t)mp; pr.len = (uint8_t)len;
 }
 
+__device__ __forceinline__ bool motif_ok(const nmb_motif &m) { return m.len >= 1 && m.len <= kMaxLen && m.mod_pos < m.len; }
+
+// Link of motif b to its left neighbour a (sibling word layout above; 0 = not siblings): same len and mod_pos, the same
+// allowed set at every position but at most one, and there both sets non-empty.
+__device__ uint32_t sibling_link(const nmb_motif &a, const nmb_motif &b) {
+    if (!motif_ok(a) || !motif_ok(b) || a.len != b.len || a.mod_pos != b.mod_pos) return 0;
+    int j = -1;
+    for (int i = 0; i < a.len; ++i) {
+        if ((a.allowed[i] & 0xF) == (b.allowed[i] & 0xF)) continue;
+        if (j >= 0) return 0;
+        j = i;
+    }
+    if (j < 0) return kSibSame << 6;
+    const uint32_t sa = a.allowed[j] & 0xF, sb = b.allowed[j] & 0xF;
+    if (!sa || !sb) return 0;
+    return (uint32_t)j | kSibDiff << 6 | sb << 8 | sa << 12;
+}
+
+// Two threads per motif (forward and reverse-complement program); with `siblings`, the forward thread also writes the
+// motif's sibling word and its parent program towards the right neighbour.
 __global__ void compile_motifs_kernel(const nmb_motif *__restrict__ motifs, int n_motifs,
-                                      Program *__restrict__ programs) {
+                                      Program *__restrict__ programs, uint32_t *__restrict__ siblings,
+                                      Program *__restrict__ parents) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= 2 * n_motifs) return;
-    const nmb_motif mt = motifs[t >> 1];
+    const int m = t >> 1;
+    const nmb_motif mt = motifs[m];
     const bool rc = t & 1;
     Program pr;
     int len = mt.len, mp = mt.mod_pos;
-    if (len < 1 || len > kMaxLen || mp >= len) {  // invalid: compile to "never matches"
+    if (siblings && !rc) {
+        siblings[m] = m > 0 ? sibling_link(motifs[m - 1], mt) : 0u;
+        const uint32_t right = m + 1 < n_motifs ? sibling_link(mt, motifs[m + 1]) : 0u;
+        if (((right >> 6) & 3) == kSibDiff) {
+            uint8_t allowed[kMaxLen];
+            for (int j = 0; j < len; ++j) allowed[j] = mt.allowed[j] & 0xF;
+            allowed[right & 63] = 0xF;
+            build_program(allowed, len, mp, pr);
+            parents[m] = pr;
+        }
+    }
+    if (!motif_ok(mt)) {  // invalid: compile to "never matches"
         for (int i = 0; i < kMaxLen; ++i) pr.ent[i] = 0;
         pr.reserved = 0;
         pr.n = 1; pr.mod_pos = 0; pr.len = 1;
@@ -435,146 +510,49 @@ __global__ void compile_motifs_kernel(const nmb_motif *__restrict__ motifs, int 
     programs[t] = pr;
 }
 
-// ---------------------------------------------------------------------------------------------
-// family finder: runs of consecutive motifs inside one work item's motif block that share a parent
-// ---------------------------------------------------------------------------------------------
-// One WARP per motif block, lane l = motif l of the block (<= 32).  Offsets are relative to the modified base and
-// limited to [-31, 31] (a member's extra position must be reachable with one halo word and the parent must fit one
-// word span); motifs reaching further are never family members.  Pass 1: every lane tests whether it and its right
-// neighbour are siblings (same number of constrained positions, all but one shared).  Then leaders are walked left
-// to right: without a sibling to the right a motif is single; otherwise every lane to the right tests itself
-// against the parent P = (leader AND leader + 1) and the run extends while consecutive lanes pass.
-constexpr int kFamReach = 31;
-
-__device__ __forceinline__ int fam_set_at(const nmb_motif *m, int len, int mod, int o) {  // 0xF outside / wildcard
-    const int j = o + mod;
-    return (j >= 0 && j < len) ? (__ldg(&m->allowed[j]) & 0xF) : 0xF;
-}
-
-__global__ void __launch_bounds__(256) find_families_kernel(const nmb_motif *__restrict__ motifs,
-                                                            const nmb_job *__restrict__ jobs, int mpi,
-                                                            FamInfo *__restrict__ fam, Program *__restrict__ parents) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, wpc = blockDim.x >> 5;
-    const int motif_begin = __ldg(&jobs[blockIdx.x].motif_begin), motif_count = __ldg(&jobs[blockIdx.x].motif_count);
-    const int n_blocks = (motif_count + mpi - 1) / mpi;
-    for (int blk = blockIdx.y * wpc + warp; blk < n_blocks; blk += gridDim.y * wpc) {
-        const int m0 = motif_begin + blk * mpi;
-        const int cnt = min(mpi, motif_count - blk * mpi);
-        const bool have = lane < cnt;
-        const nmb_motif *me = motifs + m0 + (have ? lane : 0);
-        const int len = have ? __ldg(&me->len) : 0, mod = have ? __ldg(&me->mod_pos) : 0;
-        // eligible: valid record whose positions all lie within [-31, 31] of the modified base
-        const bool elig = have && len >= 1 && len <= kMaxLen && mod < len && mod <= kFamReach && len - 1 - mod <= kFamReach;
-        FamInfo mine = {0, 0, 0, 0};
-        // ---- pass 1: sibling of the right neighbour? ----
-        bool sib = false;
-        {
-            const nmb_motif *nb = me + 1;
-            const bool nb_have = lane + 1 < cnt;
-            const int nlen = nb_have ? __ldg(&nb->len) : 0, nmod = nb_have ? __ldg(&nb->mod_pos) : 0;
-            const bool nelig = nb_have && nlen >= 1 && nlen <= kMaxLen && nmod < nlen && nmod <= kFamReach &&
-                               nlen - 1 - nmod <= kFamReach;
-            if (elig && nelig) {
-                int ka = 0, kb = 0, common = 0, lo = 99, hi = -99;
-                bool bad = false;
-                for (int o = -kFamReach; o <= kFamReach; ++o) {
-                    const int a = fam_set_at(me, len, mod, o), b = fam_set_at(nb, nlen, nmod, o);
-                    bad |= a == 0 || b == 0;  // an empty set never matches: leave such motifs to the general path
-                    ka += a != 0xF;
-                    kb += b != 0xF;
-                    if (a != 0xF && a == b) { ++common; lo = min(lo, o); hi = max(hi, o); }
-                }
-                sib = !bad && ka == kb && ka >= 2 && common == ka - 1 && lo <= 0 && hi >= 0 && hi - lo + 1 <= 32 &&
-                      fam_set_at(me, len, mod, 0) != 0xF && fam_set_at(me, len, mod, 0) == fam_set_at(nb, nlen, nmod, 0);
-            }
-        }
-        const unsigned adj = __ballot_sync(0xFFFFFFFFu, sib);
-        // ---- walk the leaders ----
-        int leader = 0;
-        while (leader < cnt) {  // warp-uniform
-            int run = 1;
-            if ((adj >> leader) & 1u) {
-                const nmb_motif *A = motifs + m0 + leader, *B = A + 1;
-                const int alen = __ldg(&A->len), amod = __ldg(&A->mod_pos), blen = __ldg(&B->len), bmod = __ldg(&B->mod_pos);
-                // does this lane's motif hold every position of P = A & B, plus exactly one more?
-                bool ok = elig && lane >= leader;
-                int extra_set = 0, extra_o = 0, n_extra = 0, k_me = 0, k_par = 0;
-                if (ok) {
-                    for (int o = -kFamReach; o <= kFamReach; ++o) {
-                        const int a = fam_set_at(A, alen, amod, o), b = fam_set_at(B, blen, bmod, o);
-                        const int c = fam_set_at(me, len, mod, o);
-                        const bool in_par = a != 0xF && a == b;
-                        k_par += in_par;
-                        k_me += c != 0xF;
-                        if (in_par) ok &= c == a;
-                        else if (c != 0xF) { ++n_extra; extra_set = c; extra_o = o; }
-                        ok &= c != 0;
-                    }
-                    ok &= n_extra == 1 && k_me == k_par + 1;
-                }
-                const unsigned pass = __ballot_sync(0xFFFFFFFFu, ok) >> leader;  // bit 0 = the leader itself
-                run = pass == 0xFFFFFFFFu ? 32 : __ffs(~pass) - 1;                // consecutive members from the leader on
-                if (run < 2) run = 1;
-                else {
-                    if (lane >= leader && lane < leader + run) {
-                        mine.n = lane == leader ? (uint8_t)run : 0;
-                        mine.set = (uint8_t)extra_set;
-                        mine.delta = (int8_t)extra_o;
-                    }
-                    if (lane == leader) {  // the parent's program: positions of P over its span, modified base inside
-                        uint8_t allowed[32];
-                        int lo = 99, hi = -99;
-                        for (int o = -kFamReach; o <= kFamReach; ++o) {
-                            const int a = fam_set_at(A, alen, amod, o), b = fam_set_at(B, blen, bmod, o);
-                            if (a != 0xF && a == b) { lo = min(lo, o); hi = max(hi, o); }
-                        }
-                        for (int o = lo; o <= hi; ++o) {
-                            const int a = fam_set_at(A, alen, amod, o), b = fam_set_at(B, blen, bmod, o);
-                            allowed[o - lo] = (uint8_t)((a != 0xF && a == b) ? a : 0xF);
-                        }
-                        Program pr;
-                        build_program(allowed, hi - lo + 1, -lo, pr);
-                        parents[m0 + leader] = pr;
-                    }
-                }
-            }
-            leader += run;
-        }
-        if (have) fam[m0 + lane] = mine;
-    }
-}
-
 }  // namespace nmb
 
 extern "C" {
 
-int nmb_compile_motifs(const nmb_motif *motifs, int32_t n_motifs, void *programs, void *stream) {
+static int compile_impl(const nmb_motif *motifs, int32_t n_motifs, void *programs, void *siblings, void *stream) {
     NMB_REQUIRE(n_motifs >= 0, "nmb_compile_motifs: n_motifs=%d", n_motifs);
     if (n_motifs == 0) return NMB_OK;
     NMB_REQUIRE(motifs && programs, "nmb_compile_motifs: null argument");
+    nmb::Program *parents =
+        siblings ? (nmb::Program *)((uint8_t *)siblings + ((n_motifs * (int64_t)sizeof(uint32_t) + 127) / 128) * 128)
+                 : nullptr;
     nmb::compile_motifs_kernel<<<(2 * n_motifs + 127) / 128, 128, 0, (cudaStream_t)stream>>>(
-        motifs, n_motifs, (nmb::Program *)programs);
+        motifs, n_motifs, (nmb::Program *)programs, (uint32_t *)siblings, parents);
     NMB_CUDA(cudaGetLastError());
     return NMB_OK;
 }
 
-int64_t nmb_family_scratch_bytes(int32_t n_motifs) {
+int nmb_compile_motifs(const nmb_motif *motifs, int32_t n_motifs, void *programs, void *stream) {
+    return compile_impl(motifs, n_motifs, programs, nullptr, stream);
+}
+
+int64_t nmb_sibling_bytes(int32_t n_motifs) {
     const int64_t n = n_motifs > 0 ? n_motifs : 0;
-    return ((n * (int64_t)sizeof(nmb::FamInfo) + 127) / 128) * 128 + n * (int64_t)sizeof(nmb::Program);
+    return ((n * (int64_t)sizeof(uint32_t) + 127) / 128) * 128 + n * (int64_t)sizeof(nmb::Program);
+}
+
+int nmb_compile_motifs_siblings(const nmb_motif *motifs, int32_t n_motifs, void *programs, void *siblings,
+                                void *stream) {
+    NMB_REQUIRE(siblings || n_motifs == 0, "nmb_compile_motifs_siblings: null siblings");
+    return compile_impl(motifs, n_motifs, programs, siblings, stream);
 }
 
 static int scan_count_impl(const nmb_assembly *a, const uint32_t *class_records, const void *programs,
                            const nmb_job *jobs, int32_t n_jobs, int32_t n_items, int32_t motifs_per_item,
                            int32_t max_motif_len, const int32_t *contig_group, int64_t *out, int32_t grid_ctas,
-                           const nmb_motif *motifs, int32_t n_motifs, void *family_scratch, int32_t *work_counter,
-                           void *stream);
+                           const void *siblings, int32_t n_motifs, int32_t *work_counter, void *stream);
 
 int nmb_scan_count(const nmb_assembly *a, const uint32_t *class_records, const void *programs,
                    const nmb_job *jobs, int32_t n_jobs, int32_t n_items, int32_t motifs_per_item,
                    int32_t max_motif_len, const int32_t *contig_group, int64_t *out,
                    int32_t grid_ctas, void *stream) {
     return scan_count_impl(a, class_records, programs, jobs, n_jobs, n_items, motifs_per_item, max_motif_len,
-                           contig_group, out, grid_ctas, nullptr, 0, nullptr, nullptr, stream);
+                           contig_group, out, grid_ctas, nullptr, 0, nullptr, stream);
 }
 
 int nmb_scan_count_balanced(const nmb_assembly *a, const uint32_t *class_records, const void *programs,
@@ -583,23 +561,23 @@ int nmb_scan_count_balanced(const nmb_assembly *a, const uint32_t *class_records
                             int32_t *work_counter, void *stream) {
     NMB_REQUIRE(work_counter, "nmb_scan_count_balanced: null work counter");
     return scan_count_impl(a, class_records, programs, jobs, n_jobs, n_items, motifs_per_item, max_motif_len,
-                           contig_group, out, grid_ctas, nullptr, 0, nullptr, work_counter, stream);
+                           contig_group, out, grid_ctas, nullptr, 0, work_counter, stream);
 }
 
-int nmb_scan_count_families(const nmb_assembly *a, const uint32_t *class_records, const void *programs,
-                            const nmb_job *jobs, int32_t n_jobs, int32_t n_items, int32_t motifs_per_item,
-                            int32_t max_motif_len, const int32_t *contig_group, int64_t *out, int32_t grid_ctas,
-                            const nmb_motif *motifs, int32_t n_motifs, void *family_scratch, void *stream) {
-    NMB_REQUIRE(motifs && family_scratch && n_motifs > 0, "nmb_scan_count_families: null argument");
+int nmb_scan_count_siblings(const nmb_assembly *a, const uint32_t *class_records, const void *programs,
+                            const void *siblings, int32_t n_motifs, const nmb_job *jobs, int32_t n_jobs,
+                            int32_t n_items, int32_t motifs_per_item, int32_t max_motif_len,
+                            const int32_t *contig_group, int64_t *out, int32_t grid_ctas, int32_t *work_counter,
+                            void *stream) {
+    NMB_REQUIRE(siblings && n_motifs > 0, "nmb_scan_count_siblings: null argument");
     return scan_count_impl(a, class_records, programs, jobs, n_jobs, n_items, motifs_per_item, max_motif_len,
-                           contig_group, out, grid_ctas, motifs, n_motifs, family_scratch, nullptr, stream);
+                           contig_group, out, grid_ctas, siblings, n_motifs, work_counter, stream);
 }
 
 static int scan_count_impl(const nmb_assembly *a, const uint32_t *class_records, const void *programs,
                            const nmb_job *jobs, int32_t n_jobs, int32_t n_items, int32_t motifs_per_item,
                            int32_t max_motif_len, const int32_t *contig_group, int64_t *out, int32_t grid_ctas,
-                           const nmb_motif *motifs, int32_t n_motifs, void *family_scratch, int32_t *work_counter,
-                           void *stream) {
+                           const void *siblings, int32_t n_motifs, int32_t *work_counter, void *stream) {
     NMB_REQUIRE(a && class_records && programs && jobs && out, "nmb_scan_count: null argument");
     NMB_REQUIRE(n_jobs > 0 && n_items >= 0, "nmb_scan_count: n_jobs=%d n_items=%d", n_jobs, n_items);
     NMB_REQUIRE(motifs_per_item >= 1 && motifs_per_item <= NMB_MAX_MOTIFS_PER_ITEM,
@@ -623,16 +601,10 @@ static int scan_count_impl(const nmb_assembly *a, const uint32_t *class_records,
     p.mpi = motifs_per_item;
     p.n_tiles = a->n_tiles;
     p.counter = work_counter;
-    p.fam = nullptr;
-    p.parents = nullptr;
-    if (family_scratch && motifs_per_item >= 2) {  // group the motif blocks into families (device, one block per job)
-        p.fam = (const nmb::FamInfo *)family_scratch;
-        p.parents = (const nmb::Program *)((uint8_t *)family_scratch +
-                                           ((n_motifs * (int64_t)sizeof(nmb::FamInfo) + 127) / 128) * 128);
-        nmb::find_families_kernel<<<dim3(n_jobs, 4), 256, 0, (cudaStream_t)stream>>>(
-            motifs, jobs, motifs_per_item, (nmb::FamInfo *)p.fam, (nmb::Program *)p.parents);
-        NMB_CUDA(cudaGetLastError());
-    }
+    p.sib = siblings ? (const uint32_t *)siblings : nullptr;
+    p.parents = siblings ? (const nmb::Program *)((const uint8_t *)siblings +
+                                                  ((n_motifs * (int64_t)sizeof(uint32_t) + 127) / 128) * 128)
+                         : nullptr;
 
     int grid = grid_ctas;
     if (grid <= 0) {
@@ -643,18 +615,14 @@ static int scan_count_impl(const nmb_assembly *a, const uint32_t *class_records,
     if (grid > n_items) grid = n_items;
     cudaStream_t s = (cudaStream_t)stream;
     const int smem_bytes = nmb::kScanSmemBytes;
-#define NMB_LAUNCH_SCAN(H, S, F)                                                                                      \
+#define NMB_LAUNCH_SCAN(H, S)                                                                                         \
     do {                                                                                                              \
-        NMB_CUDA(cudaFuncSetAttribute(nmb::scan_count_kernel<H, S, F>, cudaFuncAttributeMaxDynamicSharedMemorySize,   \
+        NMB_CUDA(cudaFuncSetAttribute(nmb::scan_count_kernel<H, S>, cudaFuncAttributeMaxDynamicSharedMemorySize,      \
                                       smem_bytes));                                                                   \
-        nmb::scan_count_kernel<H, S, F><<<grid, nmb::kScanThreads, smem_bytes, s>>>(p);                                \
+        nmb::scan_count_kernel<H, S><<<grid, nmb::kScanThreads, smem_bytes, s>>>(p);                                   \
     } while (0)
-    const bool fam = p.fam != nullptr;
-    if (max_motif_len <= 32) {  // one halo word covers a total shift (and a mod_pos) of at most 31
-        if (fam) NMB_LAUNCH_SCAN(1, 1, true); else NMB_LAUNCH_SCAN(1, 1, false);
-    } else {
-        if (fam) NMB_LAUNCH_SCAN(2, 1, true); else NMB_LAUNCH_SCAN(2, 1, false);
-    }
+    if (max_motif_len <= 32) NMB_LAUNCH_SCAN(1, 1);  // one halo word covers a total shift (and a mod_pos) of at most 31
+    else NMB_LAUNCH_SCAN(2, 1);
 #undef NMB_LAUNCH_SCAN
     NMB_CUDA(cudaGetLastError());
     return NMB_OK;

@@ -380,12 +380,11 @@ def compact_rows(contig_id, position, strand, fraction_mod, mod_type=None, n_con
 
 import os as _os
 
-# Family sharing in K2 (nmb_scan_count_families: the children of one search expansion evaluated as one parent chain +
-# one indicator plane each).  OFF by default: exact (tests/test_gpu_scan.py) and 17 % fewer instructions on the cfg3
-# search-shaped work list, but the extra code takes the kernel's hot path past the SM's instruction cache
-# (stalled_no_instruction 0.4 -> 4.2 per issue, profiles/r02_scan_families_experiment.txt) and the launch gets
-# SLOWER (1.59 -> 1.99 ms; 1.30 -> 2.23 ms with the final split-barrier kernel).  NMB_FAMILIES=1 enables it.
-FAMILIES = _os.environ.get("NMB_FAMILIES", "0") == "1"
+# Sibling runs in K2 (nmb_scan_count_siblings): the children of one search expansion -- consecutive motifs of a work
+# item that differ at one common position -- are scored as one parent chain pair plus a four-base split of the parent's
+# occurrences at that position, instead of one chain pair each.  Same counts (tests/test_gpu_siblings.py); motifs
+# without siblings take the general path inside the same kernel.  NMB_FAMILIES=0 selects the general path everywhere.
+FAMILIES = _os.environ.get("NMB_FAMILIES", "1") != "0"
 
 
 BALANCED = _os.environ.get("NMB_BALANCED", "1") != "0"  # dynamic item scheduling in K2 (nmb_scan_count_balanced)
@@ -440,11 +439,15 @@ class MotifPrograms:
         with torch.cuda.device(device):
             self.motifs_d = _to_device(packed.view(np.uint8).reshape(-1), device)
             self.programs = torch.empty(max(1, self.n) * lib.nmb_program_bytes(), dtype=torch.uint8, device=device)
+            # per motif: link to the previous motif and the parent program of a sibling run (nmb_compile_motifs_siblings)
+            self.siblings = torch.empty(max(128, int(lib.nmb_sibling_bytes(self.n))), dtype=torch.uint8, device=device)
             self.compile()
 
     def compile(self) -> None:
-        """(Re)run the motif compiler on the device-resident motif records (one small launch, no copies)."""
-        check(lib.nmb_compile_motifs(ptr(self.motifs_d), self.n, ptr(self.programs), _stream()), "nmb_compile_motifs")
+        """(Re)run the motif compiler on the device-resident motif records (one small launch, no copies): the scan
+        programs and the sibling words and parent programs of K2's sibling runs."""
+        check(lib.nmb_compile_motifs_siblings(ptr(self.motifs_d), self.n, ptr(self.programs), ptr(self.siblings),
+                                              _stream()), "nmb_compile_motifs_siblings")
 
 
 class PreparedJobs:
@@ -503,16 +506,14 @@ def scan_count(assembly: DeviceAssembly, pileup: DevicePileup, programs: MotifPr
         if out is None:
             out = torch.zeros((n_out_rows, 4), dtype=torch.int64, device=d)
         view = assembly.view()
-        if FAMILIES and prepared.mpi >= 2 and programs.n >= 2:
-            # motifs that share all positions but one (the children of a search expansion) are evaluated as one parent
-            # chain + one indicator plane each; the grouping runs on the device inside the call
-            scratch = torch.empty(int(lib.nmb_family_scratch_bytes(programs.n)), dtype=torch.uint8, device=d)
+        if FAMILIES and prepared.mpi >= 2 and programs.n >= 2:  # sibling runs need blocks of two or more motifs
             check(
-                lib.nmb_scan_count_families(C.byref(view), ptr(pileup.class_records), ptr(programs.programs),
-                                            ptr(prepared.jobs_d), prepared.n_jobs, prepared.n_items, prepared.mpi,
-                                            programs.max_len, ptr(contig_group), ptr(out), grid_ctas, ptr(programs.motifs_d),
-                                            programs.n, ptr(scratch), _stream()),
-                "nmb_scan_count_families",
+                lib.nmb_scan_count_siblings(C.byref(view), ptr(pileup.class_records), ptr(programs.programs),
+                                            ptr(programs.siblings), programs.n, ptr(prepared.jobs_d), prepared.n_jobs,
+                                            prepared.n_items, prepared.mpi, programs.max_len, ptr(contig_group),
+                                            ptr(out), grid_ctas, ptr(_work_counter(d)) if BALANCED else None,
+                                            _stream()),
+                "nmb_scan_count_siblings",
             )
             return out
         if BALANCED:  # items drawn from a device counter (one pair per device and stream, re-armed by the kernel)

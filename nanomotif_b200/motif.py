@@ -319,6 +319,54 @@ def _pack_motifs_numpy(motifs, strip: bool = True, mod_pos_override: int | None 
     return out
 
 
+SIB_SAME, SIB_DIFF = 1, 2  # sibling link kinds (csrc/scan.cu)
+
+
+def sibling_links(packed: np.ndarray) -> np.ndarray:
+    """Sibling word of every packed motif, as the device motif compiler writes it (nmb_compile_motifs_siblings): the
+    link to the previous motif -- same len and mod_pos and the same allowed set at every position but at most one j,
+    where both sets are non-empty -- as j | kind << 6 | own set at j << 8 | previous motif's set at j << 12."""
+    out = np.zeros(len(packed), dtype=np.uint32)
+    for i in range(1, len(packed)):
+        a, b = packed[i - 1], packed[i]
+        la, lb = int(a["len"]), int(b["len"])
+        ok = all(1 <= int(m["len"]) <= _lib.MAX_MOTIF_LEN and int(m["mod_pos"]) < int(m["len"]) for m in (a, b))
+        if not ok or la != lb or a["mod_pos"] != b["mod_pos"]:
+            continue
+        sa, sb = a["allowed"][:la] & 0xF, b["allowed"][:lb] & 0xF
+        d = np.flatnonzero(sa != sb)
+        if len(d) == 0:
+            out[i] = SIB_SAME << 6
+        elif len(d) == 1 and sa[d[0]] and sb[d[0]]:
+            j = int(d[0])
+            out[i] = j | SIB_DIFF << 6 | int(sb[j]) << 8 | int(sa[j]) << 12
+    return out
+
+
+def sibling_runs(links: np.ndarray, begin: int, count: int) -> list[tuple[int, int, int]]:
+    """The sibling runs K2 scores inside the motif block [begin, begin + count), from sibling_links: (first motif,
+    members, split position j) per run of >= 2 members, left to right.  A run takes the following motifs while they
+    are linked to their left neighbour and any differing link is at the run's j; identical motifs alone form no run."""
+    kind = (links[begin:begin + count] >> 6) & 3
+    jj = links[begin:begin + count] & 63
+    runs, a = [], 0
+    while a < count:
+        e = a + 1
+        while e < count and kind[e]:
+            e += 1
+        diff = [i for i in range(a + 1, e) if kind[i] == SIB_DIFF]
+        if not diff:
+            a += 1
+            continue
+        j = int(jj[diff[0]])
+        end = a + 1
+        while end < e and not (kind[end] == SIB_DIFF and jj[end] != j):
+            end += 1
+        runs.append((begin + a, end - a, j))
+        a = end
+    return runs
+
+
 def window_masks(motifs, width: int) -> np.ndarray:
     """Full-width (not stripped) masks for the window filter (DNAarray.filter_sequence_matches)."""
     out = np.zeros(len(motifs), dtype=_lib.MOTIF_DTYPE)
