@@ -54,13 +54,42 @@ def test_single_base_counts_equal_plane_popcounts(W):
 
 
 def test_linearity_over_allowed_sets(W):
-    c = _scan(W, [("GA.C", 1), ("GAAC", 1), ("GATC", 1), ("GAGC", 1), ("GACC", 1), ("G[AT]TC", 1), ("GTTC", 1),
-                  ("GA[CGT]C", 1), ("CA......TG", 1), ("CA...[AC]..TG", 1), ("CA...[GT]..TG", 1)], mpi=4)[:, 0]
+    from test_gpu_sibling_fuzz import _k2
+
+    motifs = [("GA.C", 1), ("GAAC", 1), ("GATC", 1), ("GAGC", 1), ("GACC", 1), ("G[AT]TC", 1), ("GTTC", 1),
+              ("GA[CGT]C", 1), ("CA......TG", 1), ("CA...[AC]..TG", 1), ("CA...[GT]..TG", 1)]
+    # GA.C .. GAGC form one sibling run at 4 motifs per item, and the split is built on the identity checked here: take
+    # the identity on the general path, then hold the split to it
+    with _k2(False):
+        c = _scan(W, motifs, mpi=4)[:, 0]
+    with _k2(True):
+        np.testing.assert_array_equal(_scan(W, motifs, mpi=4)[:, 0], c)
     np.testing.assert_array_equal(c[0], c[1] + c[2] + c[3] + c[4])      # wildcard = sum over the four bases
     np.testing.assert_array_equal(c[5][[0, 1]], (c[2] + c[6])[[0, 1]])  # '+' strand: [AT] at a non-modified position
     np.testing.assert_array_equal(c[7], c[2] + c[3] + c[4])              # three-letter class
     np.testing.assert_array_equal(c[8], c[9] + c[10])                    # complementary classes inside a gap
     assert c[2].min() > 1e5
+
+
+def test_sibling_runs_equal_general_path(W):
+    """Four search-shaped work lists and a fuzz list whose members keep the canonical A at the modified base (the class
+    planes hold A/T sites only), scored with sibling runs and on the general path: whole assembly and per bin (group
+    mode 2 over the 300-bin map below), automatic / 4 / 32 motifs per item -- bit for bit."""
+    from nanomotif_b200 import synth
+    from test_gpu_sibling_fuzz import _k2, fuzz_list
+
+    torch, asm = W["torch"], W["asm"]
+    motifs = [kid for seed in range(4) for kids in synth.frontier_worklist(seed, "A", rounds=64) for kid in kids]
+    motifs += fuzz_list(7, 62, canonical="A")[0]
+    bins = np.random.default_rng(0).integers(-1, 300, size=asm.n_contigs).astype(np.int32)
+    for mode, cg, groups in ((0, None, 1), (2, torch.from_numpy(bins).to(W["dev"]), 300)):
+        with _k2(False):
+            general = _scan(W, motifs, mode, cg, groups, mpi=4)
+        assert general.sum() > 1e8
+        for mpi in (None, 4, 32):
+            with _k2(True):
+                got = _scan(W, motifs, mode, cg, groups, mpi=mpi)
+            np.testing.assert_array_equal(got, general, err_msg=f"group mode {mode}, mpi={mpi}")
 
 
 def test_group_modes_are_consistent(W):

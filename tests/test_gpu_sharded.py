@@ -11,7 +11,13 @@ import pytest
 pytestmark = pytest.mark.gpu
 
 MOD_TYPES = ("a", "m")
-MOTIFS = {"a": [("GATC", 1), ("A", 0), ("GCAC......GTT", 2)], "m": [("CC[AT]GG", 1), ("C", 0)]}
+MOTIFS = {"a": [("GATC", 1), ("A", 0), ("GCAC......GTT", 2),
+              # a frontier round (synth.frontier_worklist(1, "A")[5]) and a run split 61 right of the modified base: K2
+              # scores each as one parent chain pair plus a four-base split, next to the pieces' artificial ends too
+              ("C...G....A.G.G....TC", 9), ("G...G....A.G.G....TC", 9), ("T...G....A.G.G....TC", 9),
+              ("A...G....A.G.G....TC", 9),
+              ("A" + "." * 60 + "C", 0), ("A" + "." * 60 + "G", 0), ("A" + "." * 60 + "[CT]", 0)],
+          "m": [("CC[AT]GG", 1), ("C", 0)]}
 
 
 def _free_port():
@@ -66,7 +72,12 @@ def _worker(rank, world, port, backend, q, layout="bins"):
     dist.init_process_group(backend, rank=rank, world_size=world)
     try:
         import nanomotif_b200 as nmb
+        from nanomotif_b200 import device as D
         from nanomotif_b200.sharding import ShardedMultiBinScorer
+
+        # blocks of 32 motifs, as in a search round over many bins: at this size the automatic choice is one motif per
+        # item, where no sibling run forms (the unsharded scorer below keeps it: the general path is the reference)
+        D.choose_motifs_per_item = lambda jobs, sm_count: 32
 
         bins, pile = _make(layout)
         # every rank knows all lengths; sequences only of the contigs it may own -- here simply all of them
