@@ -602,9 +602,10 @@ def load_contigs_pileup_bgzip(path: str, contigs, mod_types=("a", "m", "21839"),
     text, _ = fetch_contigs_device(path, contigs, d, index)
     if int(text.numel()) == 0:
         new = lambda dt: torch.empty(0, dtype=dt, device=d)
+        counts = dict(n_mod=new(torch.int64), n_diff=new(torch.int64)) if with_counts else {}
         return DeviceRows(contigs, mod_types, d, contig_id=new(torch.int32), position=new(torch.int64), strand=new(torch.uint8),
                           mod_type=new(torch.uint8), Nvalid_cov=new(torch.int64), fraction_mod=new(torch.float64),
-                          percent_x100=new(torch.uint16))
+                          percent_x100=new(torch.uint16), **counts)
     # merged block ranges may carry neighbouring contigs (two requested contigs with others between them never do:
     # ranges are per contig span); rows of unknown contigs are dropped by the parser
     return parse_bedmethyl(text, contigs, mod_types, with_counts, d)

@@ -174,52 +174,112 @@ def pattern_table(index: PatternIndex, motifs, median: bool = True, batch: int =
     return stats_out, value_out
 
 
+def load_contigs(assembly) -> dict:
+    """{name: sequence str} of a FASTA path or of a {name: str or DNAsequence-like} mapping."""
+    from . import dataload
+
+    if isinstance(assembly, str):
+        return dataload.load_fasta(assembly)
+    return {k: (v if isinstance(v, str) else v.sequence) for k, v in assembly.items()}
+
+
+def pileup_rows(pileup, names, mod_types, allow_assembly_pileup_mismatch: bool, device, renumber=None):
+    """(rows, mismatch) of methylation_pattern: `rows` = the device columns PatternIndex takes, contig ids indexing
+    `names`, mod_type indexing `mod_types`; `mismatch` = with allow_assembly_pileup_mismatch=False, whether a row names a
+    contig absent from `names` (always False otherwise).  `pileup`: a bedMethyl path (parsed on the device, K6) or a table
+    with n_mod and n_diff.  `renumber` (int32 [len(names)], optional): the new id of every contig, -1 to drop its rows --
+    a table is cut on the host before the copy, parsed rows are renumbered and compacted on the device."""
+    from . import dataload
+
+    d = device
+    if isinstance(pileup, str):
+        dr = dataload.load_pileup_device(pileup, names, mod_types, with_counts=True, device=d,
+                                         keep_unknown_contigs=not allow_assembly_pileup_mismatch)
+        mismatch = not allow_assembly_pileup_mismatch and bool((dr.contig_id < 0).any())
+        if renumber is not None:
+            with torch.cuda.device(d):
+                lut = _to_device(np.append(np.asarray(renumber, dtype=np.int32), np.int32(-1)), d)
+                dr.contig_id = lut[torch.where(dr.contig_id < 0, len(names), dr.contig_id).long()]
+                dr = dr.take_mask((dr.contig_id >= 0).to(torch.uint8))
+        return dict(contig_id=dr.contig_id, position=dr.position, strand=dr.strand, mod_type=dr.mod_type, n_mod=dr.n_mod,
+                    Nvalid_cov=dr.Nvalid_cov, n_diff=dr.n_diff), mismatch
+    table = PileupTable.from_frame(pileup)
+    counts = {}
+    for k in ("n_mod", "n_diff"):  # in `extra` of a PileupTable, plain columns of a pandas / pyarrow / polars frame
+        col = table.extra.get(k)
+        if col is None:
+            col = dataload._frame_column(pileup, k)
+        if col is None:
+            raise KeyError("methylation_pattern needs the n_mod and n_diff pileup columns")
+        counts[k] = dataload._numeric_column(col, np.int64)
+    index = {n: i for i, n in enumerate(names)}
+    contig = np.asarray(table.contig).astype(str)
+    uniq, inv = np.unique(contig, return_inverse=True)
+    lut = np.fromiter((index.get(u, -1) for u in uniq), dtype=np.int32, count=len(uniq))
+    cid = lut[inv] if len(uniq) else np.zeros(0, dtype=np.int32)
+    mismatch = not allow_assembly_pileup_mismatch and bool((cid < 0).any())
+    take = slice(None)
+    if renumber is not None:
+        cid = np.append(np.asarray(renumber, dtype=np.int32), np.int32(-1))[cid]
+        take = np.flatnonzero(cid >= 0)
+        cid = cid[take]
+    mt_names = np.asarray(table.mod_type).astype(str)[take]
+    mt_code = np.full(len(mt_names), 255, dtype=np.uint8)
+    for i, m in enumerate(mod_types):
+        mt_code[mt_names == m] = i
+    with torch.cuda.device(d):
+        rows = dict(contig_id=_to_device(cid.astype(np.int32), d),
+                    position=_to_device(np.asarray(table.position, dtype=np.int64)[take], d),
+                    strand=_to_device(strand_codes(table.strand)[take], d), mod_type=_to_device(mt_code, d),
+                    n_mod=_to_device(counts["n_mod"][take], d),
+                    Nvalid_cov=_to_device(np.asarray(table.Nvalid_cov, dtype=np.int64)[take], d),
+                    n_diff=_to_device(counts["n_diff"][take], d))
+    return rows, mismatch
+
+
+MISMATCH_ERROR = "pileup contains contigs that are absent from the assembly"
+
+
+def pattern_frame(stats: np.ndarray, value, specs, names, median: bool):
+    """The methylation_pattern DataFrame of the [n_motifs, n_contigs] arrays of pattern_table over ALL contigs (`names`
+    order): rows motif-major, contigs ascending, pairs without observations omitted.  `specs` = parse_motif_spec of each
+    motif; `value` is ignored unless `median` (the weighted mean is sum n_mod / sum n_valid_cov)."""
+    import pandas as pd
+
+    if not median:
+        with np.errstate(divide="ignore", invalid="ignore"):
+            value = stats[:, :, 1] / stats[:, :, 2]
+    mi, ci = np.nonzero(stats[:, :, 0] > 0)  # motif-major, contigs ascending; pairs without observations are omitted
+    obs = stats[mi, ci, 0]
+    return pd.DataFrame({
+        "contig": np.array(names, dtype=object)[ci],
+        "motif": np.array([s[0] for s in specs], dtype=object)[mi],
+        "mod_type": np.array([s[1] for s in specs], dtype=object)[mi],
+        "mod_position": np.array([s[2] for s in specs], dtype=np.int8)[mi],
+        "methylation_value": value[mi, ci].astype(np.float64),
+        "mean_read_cov": stats[mi, ci, 2] / obs,
+        "n_motif_obs": obs.astype(np.int32),
+    }, columns=COLUMNS)
+
+
 def methylation_pattern(pileup, assembly, motifs, threads: int = 1, min_valid_read_coverage: int = 3,
                         batch_size: int = 1000, min_valid_cov_to_diff_fraction: float = 0.8, output: str | None = None,
                         allow_assembly_pileup_mismatch: bool = True,
                         output_type: MethylationOutput = MethylationOutput.Median, device=None):
-    """Same keyword arguments as ``epymetheus.methylation_pattern``.  `pileup`: path to a bedMethyl file or a
-    table with n_mod / n_diff in ``extra``; `assembly`: FASTA path or {name: sequence}.  Returns a pandas
-    DataFrame with the columns of nanomotif/main.py:157-161 (and writes it as TSV to `output`).
+    """Same keyword arguments as ``epymetheus.methylation_pattern``.  `pileup`: path to a bedMethyl file, a
+    pandas / pyarrow / polars frame with n_mod and n_diff columns, or a PileupTable with them in ``extra``;
+    `assembly`: FASTA path or {name: sequence}.  Returns a pandas DataFrame with the columns of
+    nanomotif/main.py:157-161 (and writes it as TSV to `output`).
     `threads` and `batch_size` are accepted for signature compatibility (the GPU needs neither)."""
-    import pandas as pd
-
-    from . import dataload
-
-    contigs = dataload.load_fasta(assembly) if isinstance(assembly, str) else {k: (v if isinstance(v, str) else v.sequence) for k, v in assembly.items()}
+    contigs = load_contigs(assembly)
     asm = DeviceAssembly.from_sequences(contigs, device)
     d = asm.device
     motifs = [str(m) for m in motifs]
     specs = [parse_motif_spec(m) for m in motifs]
     mod_types = sorted({mt for _, mt, _ in specs})
-    if isinstance(pileup, str):  # bedMethyl text parsed on the device (K6)
-        dr = dataload.load_pileup_device(pileup, asm.names, mod_types, with_counts=True, device=d,
-                                         keep_unknown_contigs=not allow_assembly_pileup_mismatch)
-        if not allow_assembly_pileup_mismatch and bool((dr.contig_id < 0).any()):
-            raise ValueError("pileup contains contigs that are absent from the assembly")
-        rows = dict(contig_id=dr.contig_id, position=dr.position, strand=dr.strand, mod_type=dr.mod_type, n_mod=dr.n_mod,
-                    Nvalid_cov=dr.Nvalid_cov, n_diff=dr.n_diff)
-    else:
-        table = PileupTable.from_frame(pileup)
-        if "n_mod" not in table.extra or "n_diff" not in table.extra:
-            raise KeyError("methylation_pattern needs the n_mod and n_diff pileup columns")
-        names = np.asarray(table.contig).astype(str)
-        uniq, inv = np.unique(names, return_inverse=True)
-        lut = np.fromiter((asm.index.get(u, -1) for u in uniq), dtype=np.int32, count=len(uniq))
-        cid = lut[inv] if len(uniq) else np.zeros(0, dtype=np.int32)
-        if not allow_assembly_pileup_mismatch and (cid < 0).any():
-            raise ValueError("pileup contains contigs that are absent from the assembly")
-        mt_names = np.asarray(table.mod_type).astype(str)
-        mt_code = np.full(len(mt_names), 255, dtype=np.uint8)
-        for i, m in enumerate(mod_types):
-            mt_code[mt_names == m] = i
-        with torch.cuda.device(d):
-            rows = dict(contig_id=_to_device(cid.astype(np.int32), d),
-                        position=_to_device(np.asarray(table.position, dtype=np.int64), d),
-                        strand=_to_device(strand_codes(table.strand), d), mod_type=_to_device(mt_code, d),
-                        n_mod=_to_device(np.asarray(table.extra["n_mod"], dtype=np.int64), d),
-                        Nvalid_cov=_to_device(np.asarray(table.Nvalid_cov, dtype=np.int64), d),
-                        n_diff=_to_device(np.asarray(table.extra["n_diff"], dtype=np.int64), d))
+    rows, mismatch = pileup_rows(pileup, asm.names, mod_types, allow_assembly_pileup_mismatch, d)
+    if mismatch:
+        raise ValueError(MISMATCH_ERROR)
 
     median = output_type == MethylationOutput.Median
     nc = asm.n_contigs
@@ -233,20 +293,7 @@ def methylation_pattern(pileup, assembly, motifs, threads: int = 1, min_valid_re
         if median:
             value[sel] = val
         del index
-    if not median:
-        with np.errstate(divide="ignore", invalid="ignore"):
-            value = stats[:, :, 1] / stats[:, :, 2]
-    mi, ci = np.nonzero(stats[:, :, 0] > 0)  # motif-major, contigs ascending; pairs without observations are omitted
-    obs = stats[mi, ci, 0]
-    df = pd.DataFrame({
-        "contig": np.array(asm.names, dtype=object)[ci],
-        "motif": np.array([s[0] for s in specs], dtype=object)[mi],
-        "mod_type": np.array([s[1] for s in specs], dtype=object)[mi],
-        "mod_position": np.array([s[2] for s in specs], dtype=np.int8)[mi],
-        "methylation_value": value[mi, ci].astype(np.float64),
-        "mean_read_cov": stats[mi, ci, 2] / obs,
-        "n_motif_obs": obs.astype(np.int32),
-    }, columns=COLUMNS)
+    df = pattern_frame(stats, value, specs, asm.names, median)
     if output is not None:
         df.to_csv(output, sep="\t", index=False)
     return df

@@ -21,6 +21,8 @@ from typing import Mapping, Sequence
 
 import numpy as np
 
+from .pattern import MethylationOutput
+
 
 def plan_shards(lengths: Sequence[int], world_size: int, groups: Sequence[int] | None = None) -> np.ndarray:
     """Rank of every contig.  Longest-first greedy packing balances total bp per rank.  With `groups`
@@ -483,3 +485,234 @@ class ShardedBinSweep:
                 dist.all_reduce(out, op=dist.ReduceOp.SUM, group=self.scorer.group)
             out = out.cpu().numpy()
         return out[..., 0], out[..., 1]
+
+
+# ---------------------------------------------------------------------------------------------
+# The contig x motif methylation-pattern table (K5) over the GPUs of one box.
+# ---------------------------------------------------------------------------------------------
+def _collective(world_size: int) -> bool:
+    import torch.distributed as dist
+
+    return world_size > 1 and dist.is_available() and dist.is_initialized()
+
+
+def rank_extremes(values, device, world_size: int, group=None) -> tuple[np.ndarray, np.ndarray]:
+    """(maximum, minimum) over the ranks of each of the small int64 `values`, on every rank, with ONE all-reduce (MAX
+    over the values and their negations).  Every rank must call it with as many values."""
+    import torch
+
+    v = np.asarray(values, dtype=np.int64)
+    t = torch.from_numpy(np.concatenate([v, -v])).to(device)
+    if _collective(world_size):
+        import torch.distributed as dist
+
+        dist.all_reduce(t, op=dist.ReduceOp.MAX, group=group)
+    t = t.cpu().numpy()
+    return t[:len(v)], -t[len(v):]
+
+
+def motif_list_key(motifs) -> tuple[int, int]:
+    """(count, 62-bit hash) of a list of motif strings -- a hash that does not depend on the process (unlike hash())."""
+    import hashlib
+
+    digest = hashlib.blake2b("\n".join(str(m) for m in motifs).encode(), digest_size=8).digest()
+    return len(motifs), int.from_bytes(digest, "little") >> 2
+
+
+def check_same_motifs(motifs, device, world_size: int, group=None) -> None:
+    """Raise ValueError on every rank unless every rank passed the same motif list (count and hash compared)."""
+    hi, lo = rank_extremes(motif_list_key(motifs), device, world_size, group)
+    if (hi != lo).any():
+        raise ValueError("the ranks were given different motif lists")
+
+
+def place_columns(stats, value, columns, n_contigs: int):
+    """Zero-filled [n_motifs, n_contigs, 3] int64 and [n_motifs, n_contigs] float64 tensors holding this rank's columns
+    at their global contig index `columns` (stats / value: [n_motifs, len(columns)(, 3)] of the rank's contigs in local
+    order; value may be None).  A cell without observations gets value 0.0, so that the ranks' tensors can be added."""
+    import torch
+
+    idx = torch.as_tensor(np.asarray(columns, dtype=np.int64), device=stats.device)
+    out_s = torch.zeros((stats.shape[0], n_contigs, 3), dtype=torch.int64, device=stats.device)
+    out_s[:, idx] = stats
+    out_v = None
+    if value is not None:
+        out_v = torch.zeros((stats.shape[0], n_contigs), dtype=torch.float64, device=stats.device)
+        out_v[:, idx] = torch.where(stats[:, :, 0] > 0, value, torch.zeros_like(value))
+    return out_s, out_v
+
+
+def gather_columns(stats, value, columns, n_contigs: int, world_size: int, group=None):
+    """The whole table on every rank from each rank's own contig columns (place_columns): one all-reduce (sum) per
+    tensor, then NaN where n_motif_obs == 0.  Exact: every cell has one owner and the other ranks add integer zeros or
+    +0.0 to it."""
+    out_s, out_v = place_columns(stats, value, columns, n_contigs)
+    if _collective(world_size):
+        import torch.distributed as dist
+
+        dist.all_reduce(out_s, op=dist.ReduceOp.SUM, group=group)
+        if out_v is not None:
+            dist.all_reduce(out_v, op=dist.ReduceOp.SUM, group=group)
+    if out_v is not None:
+        out_v[out_s[:, :, 0] == 0] = float("nan")
+    return out_s, out_v
+
+
+class ShardedPatternTable:
+    """The multi-GPU form of the K5 contig x motif table (pattern.methylation_pattern, the table detect_contamination
+    and include_contigs read, nanomotif/main.py:167-178).  Every rank passes the same arguments.
+
+    Whole contigs are assigned to ranks by plan_shards (greedy on bp, no bins); each rank packs only its own contigs and
+    builds one PatternIndex per mod type over them, so the K5 kernels run unchanged on every rank.  Contigs are never
+    cut: counts of pieces would add, medians would not (an exact merge needs every fraction of the contig in one place),
+    and a contig larger than one rank's share only occurs in assemblies small enough for one GPU.  A rank without
+    contigs still takes part in every collective.
+
+    Rows each rank reads: a table (pandas / pyarrow / polars-like, with n_mod and n_diff) is cut to the rank's contigs
+    on the host before the copy; a bgzip pileup with a tabix index (.tbi next to it) is read member by member for the
+    rank's contigs only (dataload.load_contigs_pileup_bgzip); plain text, or bgzip without an index, is parsed whole on
+    every rank against all contig names and then cut -- that path does not split the parse cost.
+
+    With allow_assembly_pileup_mismatch=False a pileup row of a contig absent from the whole assembly raises the same
+    ValueError on every rank, after one all-reduce of the flag (the first collective)."""
+
+    def __init__(self, pileup, assembly, mod_types, rank: int, world_size: int, device=None, group=None,
+                 min_valid_read_coverage: int = 3, min_valid_cov_to_diff_fraction: float = 0.8,
+                 allow_assembly_pileup_mismatch: bool = True):
+        import torch
+
+        from .device import DeviceAssembly
+        from .pattern import MISMATCH_ERROR, load_contigs, pileup_rows
+
+        contigs = load_contigs(assembly)
+        self._plan(list(contigs), [len(s) for s in contigs.values()], mod_types, rank, world_size, group)
+        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        asm, rows, mismatch = None, None, False
+        if len(self.columns):  # the rank holding the longest contig (rank 0) always reads, so it sees any mismatch
+            asm = DeviceAssembly.from_sequences({n: contigs[n] for n in self.local_names}, self.device)
+            if isinstance(pileup, str) and _tabix_indexed(pileup):
+                rows, mismatch = self._tabix_rows(pileup, allow_assembly_pileup_mismatch)
+            else:
+                renumber = np.full(len(self.names), -1, dtype=np.int32)
+                renumber[self.columns] = np.arange(len(self.columns), dtype=np.int32)
+                rows, mismatch = pileup_rows(pileup, self.names, self.mod_types, allow_assembly_pileup_mismatch,
+                                             self.device, renumber)
+        if rank_extremes([int(mismatch)], self.device, self.world_size, group)[0][0]:
+            raise ValueError(MISMATCH_ERROR)
+        self._index(asm, rows, min_valid_read_coverage, min_valid_cov_to_diff_fraction)
+
+    @classmethod
+    def from_local(cls, assembly, rows, contigs, mod_types, rank: int, world_size: int, device=None, group=None,
+                   min_valid_read_coverage: int = 3, min_valid_cov_to_diff_fraction: float = 0.8) -> "ShardedPatternTable":
+        """The sharded table over a rank's DeviceAssembly and pileup rows built elsewhere -- e.g. generated or parsed on
+        the device, when the rows cannot go through host text.  `contigs` = {name: sequence or length} of ALL ranks, the
+        same on every rank; `assembly` must hold exactly the contigs plan_shards gives this rank, in `contigs` order, or
+        be None when it gives none.  `rows`: device tensors as PatternIndex takes them, contig ids indexing `assembly`."""
+        import torch
+
+        self = cls.__new__(cls)
+        self._plan(list(contigs), [_contig_length(s) for s in contigs.values()], mod_types, rank, world_size, group)
+        held = [] if assembly is None else list(assembly.names)
+        if held != self.local_names:
+            raise ValueError(f"rank {self.rank}: the local assembly's contigs are not those the shard plan gives this rank")
+        if assembly is not None:
+            device = assembly.device
+        self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+        self._index(assembly, rows, min_valid_read_coverage, min_valid_cov_to_diff_fraction)
+        return self
+
+    def _plan(self, names, lengths, mod_types, rank, world_size, group):
+        self.rank, self.world_size, self.group = int(rank), int(world_size), group
+        self.names, self.mod_types = list(names), [str(m) for m in mod_types]
+        self.owner = plan_shards(lengths, self.world_size)
+        self.columns = np.flatnonzero(self.owner == self.rank)  # global index of every local contig, ascending
+        self.local_names = [self.names[i] for i in self.columns]
+
+    def _tabix_rows(self, path, allow_assembly_pileup_mismatch):
+        from .bgzf import tabix_contigs
+        from .dataload import load_contigs_pileup_bgzip
+
+        mismatch = not allow_assembly_pileup_mismatch and bool(set(tabix_contigs(path)) - set(self.names))
+        dr = load_contigs_pileup_bgzip(path, self.local_names, self.mod_types, with_counts=True, device=self.device)
+        return dict(contig_id=dr.contig_id, position=dr.position, strand=dr.strand, mod_type=dr.mod_type, n_mod=dr.n_mod,
+                    Nvalid_cov=dr.Nvalid_cov, n_diff=dr.n_diff), mismatch
+
+    def _index(self, asm, rows, min_valid_read_coverage, min_valid_cov_to_diff_fraction):
+        from .pattern import PatternIndex
+
+        self.assembly = asm
+        self.indices = [] if asm is None else [
+            PatternIndex(asm, rows, ti, min_valid_read_coverage, min_valid_cov_to_diff_fraction)
+            for ti in range(len(self.mod_types))]
+
+    def table(self, motifs, median: bool = True, on_device: bool = False):
+        """(stats int64 [n_motifs, n_contigs, 3], value float64 [n_motifs, n_contigs] or None) over ALL contigs in the
+        assembly's order, on every rank: the arrays pattern.pattern_table returns for an index over the whole assembly,
+        bit for bit (NaN where a cell has no observation).  `motifs`: strings <IUPAC>_<mod_type>_<mod_position>, the
+        same list on every rank (checked; a difference raises ValueError on every rank).  on_device=True returns device
+        tensors (for tables.bin_feature_matrix_device)."""
+        import torch
+
+        from .motif import Motif
+        from .pattern import parse_motif_spec, pattern_table
+
+        motifs = [str(m) for m in motifs]
+        check_same_motifs(motifs, self.device, self.world_size, self.group)
+        specs = [parse_motif_spec(m) for m in motifs]
+        for _, mt, _ in specs:
+            if mt not in self.mod_types:
+                raise KeyError(f"mod type {mt!r} is not one of {self.mod_types}")
+        nl, d = len(self.columns), self.device
+        with torch.cuda.device(d):
+            stats = torch.zeros((len(specs), nl, 3), dtype=torch.int64, device=d)
+            value = torch.full((len(specs), nl), float("nan"), dtype=torch.float64, device=d) if median else None
+            for ti, mt in enumerate(self.mod_types):
+                sel = [i for i, s in enumerate(specs) if s[1] == mt]
+                if not sel or self.assembly is None:
+                    continue
+                st, val = pattern_table(self.indices[ti], [Motif(specs[i][0], specs[i][2]).from_iupac() for i in sel],
+                                        median, on_device=True)
+                sel_d = torch.tensor(sel, dtype=torch.int64, device=d)
+                stats[sel_d] = st
+                if median:
+                    value[sel_d] = val
+            stats, value = gather_columns(stats, value, self.columns, len(self.names), self.world_size, self.group)
+            if on_device:
+                return stats, value
+            return stats.cpu().numpy(), (value.cpu().numpy() if median else None)
+
+
+def _tabix_indexed(path: str) -> bool:
+    """A bgzip pileup with its tabix index next to it."""
+    import os
+
+    with open(path, "rb") as f:
+        magic = f.read(2)
+    return magic == b"\x1f\x8b" and os.path.exists(path + ".tbi")
+
+
+def methylation_pattern(pileup, assembly, motifs, rank: int, world_size: int, group=None, threads: int = 1,
+                        min_valid_read_coverage: int = 3, batch_size: int = 1000,
+                        min_valid_cov_to_diff_fraction: float = 0.8, output: str | None = None,
+                        allow_assembly_pileup_mismatch: bool = True,
+                        output_type: MethylationOutput = MethylationOutput.Median, device=None):
+    """pattern.methylation_pattern over the GPUs of one box (ShardedPatternTable): the same keyword arguments, and on
+    every rank the DataFrame one GPU returns (same rows, order, values and dtypes).  Every rank passes the same
+    arguments; only rank 0 writes `output`."""
+    import torch
+
+    from .pattern import load_contigs, parse_motif_spec, pattern_frame
+
+    motifs = [str(m) for m in motifs]
+    median = output_type == MethylationOutput.Median
+    device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    check_same_motifs(motifs, device, world_size, group)  # the mod types below are derived from the motifs
+    specs = [parse_motif_spec(m) for m in motifs]
+    tab = ShardedPatternTable(pileup, load_contigs(assembly), sorted({mt for _, mt, _ in specs}), rank, world_size,
+                              device, group, min_valid_read_coverage, min_valid_cov_to_diff_fraction,
+                              allow_assembly_pileup_mismatch)
+    stats, value = tab.table(motifs, median)
+    df = pattern_frame(stats, value, specs, tab.names, median)
+    if output is not None and int(rank) == 0:
+        df.to_csv(output, sep="\t", index=False)
+    return df

@@ -191,25 +191,45 @@ def device_workload(device, total_bp: int = 1_500_000_000, n_contigs: int = 1700
     return asm, pile
 
 
-def device_pattern_workload(device, total_bp: int = 1_500_000_000, n_contigs: int = 50_000, seed: int = 4, depth: int = 30):
+def pattern_workload_lengths(total_bp: int = 1_500_000_000, n_contigs: int = 50_000, seed: int = 4) -> np.ndarray:
+    """Contig lengths of device_pattern_workload (host only: what every rank needs to derive a shard plan)."""
+    rng = np.random.default_rng(seed)
+    lens = rng.lognormal(mean=0.0, sigma=1.0, size=n_contigs)
+    return np.maximum(2500, (lens / lens.sum() * total_bp).astype(np.int64))
+
+
+def device_pattern_workload(device, total_bp: int = 1_500_000_000, n_contigs: int = 50_000, seed: int = 4, depth: int = 30,
+                            keep=None):
     """cfg4-shaped input of the contig x motif table built ON the device: `n_contigs` lognormal contigs and one
     read-level pileup row (n_mod, Nvalid_cov, n_diff) for every A on '+' and every T on '-' (mod type 'a').
     Returns (DeviceAssembly, rows) with rows = device tensors contig_id int32, position int64, strand uint8,
-    n_mod / Nvalid_cov / n_diff int64 in (strand, contig, position) order."""
+    n_mod / Nvalid_cov / n_diff int64 in (strand, contig, position) order.  `keep` (ascending contig indices): only
+    those contigs, with the letters and rows they have in the whole workload; contig ids then index `keep` (one rank's
+    share of a sharded run, the same data at every world size)."""
     import torch
 
     from .device import DeviceAssembly
 
     g = torch.Generator(device=device)
     g.manual_seed(seed)
-    rng = np.random.default_rng(seed)
-    lens = rng.lognormal(mean=0.0, sigma=1.0, size=n_contigs)
-    lens = np.maximum(2500, (lens / lens.sum() * total_bp).astype(np.int64))
+    lens = pattern_workload_lengths(total_bp, n_contigs, seed)
     off = np.zeros(n_contigs, dtype=np.int64)
     off[1:] = np.cumsum(lens)[:-1]
     codes = torch.randint(0, 4, (int(lens.sum()),), dtype=torch.uint8, device=device, generator=g)
     ascii_d = 65 + (codes == 1).to(torch.uint8) * 19 + (codes == 2).to(torch.uint8) * 6 + (codes == 3).to(torch.uint8) * 2
-    asm = DeviceAssembly([f"c{i}" for i in range(n_contigs)], lens, ascii_d, off, device)
+    names = [f"c{i}" for i in range(n_contigs)]
+    if keep is None:
+        asm = DeviceAssembly(names, lens, ascii_d, off, device)
+    else:
+        keep = np.asarray(keep, dtype=np.int64)
+        sel = torch.zeros(n_contigs, dtype=torch.bool, device=device)
+        sel[torch.from_numpy(keep).to(device)] = True
+        sub_off = np.zeros(len(keep), dtype=np.int64)
+        sub_off[1:] = np.cumsum(lens[keep])[:-1]
+        asm = DeviceAssembly([names[i] for i in keep], lens[keep], ascii_d[torch.repeat_interleave(
+            sel, torch.from_numpy(lens).to(device))], sub_off, device)
+        renumber = torch.full((n_contigs,), -1, dtype=torch.int32, device=device)
+        renumber[torch.from_numpy(keep).to(device)] = torch.arange(len(keep), dtype=torch.int32, device=device)
     del ascii_d
     bounds = torch.from_numpy(off[1:].copy()).to(device)
     off_d = torch.from_numpy(off).to(device)
@@ -219,13 +239,18 @@ def device_pattern_workload(device, total_bp: int = 1_500_000_000, n_contigs: in
         cid = torch.bucketize(idx, bounds, right=True)
         n = int(idx.numel())
         cov = torch.randint(1, 2 * depth, (n,), dtype=torch.int64, device=device, generator=g)
-        cols["contig_id"].append(cid.to(torch.int32))
-        cols["position"].append(idx - off_d[cid])
-        cols["strand"].append(torch.full((n,), strand, dtype=torch.uint8, device=device))
-        cols["n_mod"].append((torch.rand(n, device=device, generator=g) * (cov + 1).to(torch.float32)).to(torch.int64).clamp_(max=cov))
-        cols["Nvalid_cov"].append(cov)
-        cols["n_diff"].append(torch.randint(0, depth // 3, (n,), dtype=torch.int64, device=device, generator=g))
-        del idx, cid
+        part = dict(contig_id=cid.to(torch.int32), position=idx - off_d[cid],
+                    strand=torch.full((n,), strand, dtype=torch.uint8, device=device),
+                    n_mod=(torch.rand(n, device=device, generator=g) * (cov + 1).to(torch.float32)).to(torch.int64).clamp_(max=cov),
+                    Nvalid_cov=cov,
+                    n_diff=torch.randint(0, depth // 3, (n,), dtype=torch.int64, device=device, generator=g))
+        if keep is not None:
+            mine = sel[cid]
+            part = {k: v[mine] for k, v in part.items()}
+            part["contig_id"] = renumber[part["contig_id"].long()]
+        for k, v in part.items():
+            cols[k].append(v)
+        del idx, cid, part
     del codes
     return asm, {k: torch.cat(v) for k, v in cols.items()}
 
