@@ -165,7 +165,8 @@ NMB_API int nmb_add_class_planes(const int32_t *contig_id, const int64_t *pos, c
  * A row is methylated iff key >= key_high and unmethylated iff key <= key_low, where the keys are the
  * integer images of the reference's float64 tests fl(fl(key/100)/100) >= high / <= low computed by the
  * caller over the 10001 grid values (nanomotif_b200.device.threshold_keys) -- bit-equivalent to
- * nmb_build_class_planes on pileups whose column 11 has two decimals. */
+ * nmb_build_class_planes on pileups whose column 11 has two decimals.  A key above 10000 (nmb_bed_parse's
+ * 0xFFFF: not on the grid, or not a number) puts the row in neither class. */
 NMB_API int nmb_build_class_planes_compact(const int32_t *pos, const uint8_t *flags, const uint16_t *percent_x100,
                                    const int64_t *contig_row_off, int64_t n_rows, int32_t key_low,
                                    int32_t key_high, const nmb_assembly *assembly_h, int32_t n_modtypes,

@@ -148,7 +148,8 @@ __global__ void __launch_bounds__(128) bed_parse_kernel(
                 case 16: if (ok && !point) n_diff = v; else if (out.n_diff) ++n_notnum; break;
                 case 10:
                     if (ok && nd <= 15) {
-                        percent = (double)v / kPow10[fd];
+                        // sign applied to the double, not to iv: "-0.00" is -0.0 like the reference's reader
+                        percent = (neg ? -(double)iv : (double)iv) / kPow10[fd];
                         if (!neg && fd <= 2) {
                             const int64_t k = iv * (fd == 0 ? 100 : fd == 1 ? 10 : 1);
                             if (k <= 10000) key = (int)k;

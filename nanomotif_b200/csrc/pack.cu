@@ -176,6 +176,7 @@ __global__ void __launch_bounds__(256) class_planes_compact_kernel(
     const int64_t stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; r < n_rows; r += stride) {
         const int k = key[r];
+        if (k > 10000) continue;  // off the two-decimal grid (nmb_bed_parse writes 0xFFFF): neither class
         const bool is_mod = k >= key_high, is_non = k <= key_low;
         if (!is_mod && !is_non) continue;
         int lo = 0, hi = n_contigs;  // largest c with row_off[c] <= r

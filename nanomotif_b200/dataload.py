@@ -224,7 +224,7 @@ class DeviceRows:
         return int(self.position.numel())
 
     def take_mask(self, keep: torch.Tensor) -> "DeviceRows":
-        """Rows with keep != 0, in order (nmb_index_bytes + nmb_gather_rows)."""
+        """Rows with keep == 1 (a 0/1 uint8 mask), in order (nmb_index_bytes + nmb_gather_rows)."""
         n = len(self)
         with torch.cuda.device(self.device):
             scratch = torch.empty((n + 4095) // 4096 + 2, dtype=torch.int64, device=self.device)

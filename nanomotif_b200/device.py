@@ -367,7 +367,9 @@ def compact_rows(contig_id, position, strand, fraction_mod, mod_type=None, n_con
         mt = np.where(mt > 127, 127, mt)  # out-of-range types are ignored by the kernel (>= n_modtypes)
     strand = np.asarray(strand, dtype=np.uint8)
     flags = (strand & 1) | (mt << 1)
-    keep = (cid >= 0) & (strand <= 1)  # strand code 2 = neither '+' nor '-': dropped like the reference does
+    # strand code 2 = neither '+' nor '-': dropped like the reference does.  Ids past the contig list are dropped too
+    # (from_columns ignores them): grouped after the last contig, the kernel would take them for rows of that contig
+    keep = (cid >= 0) & (cid < n_contigs) & (strand <= 1)
     if not keep.all():
         cid, position, flags, key = cid[keep], position[keep], flags[keep], key[keep]
     if len(cid) > 1 and np.any(cid[1:] < cid[:-1]):

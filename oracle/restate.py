@@ -340,7 +340,12 @@ def filter_pileup_adjacency_filter(contig, strand, position, fraction_mod, methy
     polars rolling(index_column=position, period=window, offset=-(window//2+1)) looks at rows with
     position in (p - window//2 - 1, p - window//2 - 1 + window] = [p - d, p + d] for window = 2d+1,
     over ALL mod types of the (contig, strand) group.  A row is kept when its fraction equals the
-    window maximum or is below the threshold."""
+    window maximum or is below the threshold.
+
+    Null fractions ("NA" / "null" in column 11, NaN here): polars' rolling max skips nulls, so a NaN
+    neighbour does not take part in the window maximum (np.max would return NaN and drop every
+    above-threshold row whose window holds one).  A NaN row itself is dropped: both of its tests are
+    null in polars, which filter() treats as false."""
     contig, strand = np.asarray(contig), np.asarray(strand)
     position = np.asarray(position, dtype=np.int64)
     fraction_mod = np.asarray(fraction_mod, dtype=np.float64)
@@ -355,7 +360,9 @@ def filter_pileup_adjacency_filter(contig, strand, position, fraction_mod, methy
         left = np.searchsorted(p, p + lo_off, side="right")  # first index with pos > p + lo_off
         right = np.searchsorted(p, p + lo_off + window, side="right")  # one past last pos <= upper
         for k in range(len(order)):
-            roll_max = f[left[k] : right[k]].max()
+            w = f[left[k] : right[k]]
+            w = w[~np.isnan(w)]
+            roll_max = w.max() if len(w) else np.nan
             keep[order[k]] = (f[k] == roll_max) or (f[k] < methylation_threshold)
     return keep
 
