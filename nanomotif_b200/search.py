@@ -21,7 +21,7 @@ a search visits exactly the motifs the reference visits.
 from __future__ import annotations
 
 import heapq
-from typing import Iterable
+from typing import Iterable, Mapping
 
 import numpy as np
 
@@ -418,6 +418,90 @@ def run(coroutine, backend):
             request = coroutine.send(backend.handle(request))
     except StopIteration as stop:
         return stop.value
+
+
+DISCOVERY_COLUMNS = ("bin", "mod_type", "motif", "mod_position", "n_mod", "n_nomod", "score")
+
+
+def candidate_rows(bin_name, mod_type, result) -> list:
+    """Rows of one (bin, mod type) search: `result` = find_candidates' (graph, best) or None.  One row per best
+    candidate, in the order of `best` (found, then missed): the motif and mod_position after new_stripped_motif(),
+    n_mod / n_nomod = the node model's alpha - alpha0 and beta - beta0, score = the node's score in the graph."""
+    if result is None:
+        return []
+    graph, best = result
+    rows = []
+    for motif in best:
+        node = graph.nodes[motif]
+        n_mod, n_nomod = node["model"].get_raw_counts()
+        stripped = motif.new_stripped_motif()
+        rows.append(dict(bin=bin_name, mod_type=mod_type, motif=stripped.string, mod_position=int(stripped.mod_position),
+                         n_mod=int(n_mod), n_nomod=int(n_nomod), score=float(node["score"])))
+    return rows
+
+
+def discovery_frame(rows):
+    """pandas frame of candidate_rows (DISCOVERY_COLUMNS, in the order given; int64 counts, float64 score)."""
+    import pandas as pd
+
+    df = pd.DataFrame(list(rows), columns=list(DISCOVERY_COLUMNS))
+    return df.astype({"bin": object, "mod_type": object, "motif": object, "mod_position": np.int64, "n_mod": np.int64,
+                      "n_nomod": np.int64, "score": np.float64})
+
+
+def discover(scorer, mod_types=None, bins=None, padding: int = 20, min_kl: float = 0.05, min_motif_score: float = 1.5,
+             seed=1):
+    """The motif search of every (bin, mod type) pair of a MultiBinScorer on its GPU, all pairs in lock-step: the
+    candidate loop of find_best_candidates (find_motifs_bin.py:330-372 + process_subpileup up to find_best_candidates)
+    for a whole metagenome.  Returns a pandas frame with DISCOVERY_COLUMNS, one row per best candidate of every pair:
+    bins in `bins` order (default: the scorer's), then `mod_types` order (default: the scorer's), then the order of
+    find_candidates' `best` (found, then missed).  Defaults are the reference CLI's (search_frame_size 40 -> padding
+    20, minimum_kl_divergence 0.05, min_motif_score 1.5, seed 1); the high methylation threshold is the scorer's.
+
+    One growth.prepare_searches per mod type builds every pair's windows and background PSSM; then every score round
+    of all pairs is ONE K2 launch, every expand / remove round one K4 launch per mod type.  Like the reference's
+    per-worker set_seed(seed) (find_motifs_bin.py:171), the background draws of every pair start from random.seed(seed),
+    so a pair's rows depend only on its own bin: not on the other bins, their order or a `bins` subset.  `seed` may
+    also be a {bin: seed} mapping.  The caller's `random` state is restored afterwards.  A pair without methylation
+    windows starts no search and has no rows.  Errors of prepare_searches (a contig too short for its background
+    samples, a scorer without kept rows) pass through."""
+    import random
+
+    from . import growth
+
+    mod_types = list(scorer.mod_types) if mod_types is None else list(mod_types)
+    names = list(scorer._ranges) if bins is None else list(bins)
+    for b in names:
+        if b not in scorer._ranges:
+            raise KeyError(b)
+    if len(set(names)) != len(names):
+        raise ValueError("a bin is listed twice")
+    if len(set(mod_types)) != len(mod_types):
+        raise ValueError("a mod type is listed twice")
+    for mt in mod_types:
+        scorer.mod_types.index(mt)  # ValueError for a mod type the scorer does not hold
+    seeds = [seed[b] for b in names] if isinstance(seed, Mapping) else [seed] * len(names)
+    if not names or not mod_types:
+        return discovery_frame([])
+    high = scorer.pileup.high
+    pairs = []  # ((bin index, mod type index), coroutine, backend)
+    state = random.getstate()
+    try:
+        for j, mt in enumerate(mod_types):
+            pool, pssms, totals = growth.prepare_searches(scorer, mt, padding, high, bin_names=names, seeds=seeds)
+            for i, b in enumerate(names):
+                if totals[i] == 0:
+                    continue
+                co = find_candidates(mt, padding, pssms[i], totals[i], min_kl=min_kl, score_threshold=min_motif_score)
+                pairs.append(((i, j), co, PoolBackend(scorer.context(b, mt), pool, i)))
+    finally:
+        random.setstate(state)
+    results = run_lockstep([(co, be) for _, co, be in pairs], gpu_batch_score, gpu_batch_expand, gpu_batch_remove)
+    by_pair = {key: res for (key, _, _), res in zip(pairs, results)}
+    rows = []
+    for key in sorted(by_pair):
+        rows += candidate_rows(names[key[0]], mod_types[key[1]], by_pair[key])
+    return discovery_frame(rows)
 
 
 def run_lockstep(searches: list, batch_score=None, batch_expand=None, batch_remove=None) -> list:

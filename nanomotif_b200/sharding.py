@@ -488,6 +488,128 @@ class ShardedBinSweep:
 
 
 # ---------------------------------------------------------------------------------------------
+# Motif discovery (search.discover) over the GPUs of one box.
+# ---------------------------------------------------------------------------------------------
+def discovery_plan(bins: dict, world_size: int) -> dict:
+    """{bin: rank} of sharding.discover, from the bins' lengths alone (contigs given by sequence or length): plan_shards
+    over every bin's total bp with one unit per bin, so a bin is never spread over ranks, whatever its size (its windows
+    and search state live on one GPU).  Every rank derives the same plan."""
+    lengths = [sum(_contig_length(s) for s in cs.values()) for cs in bins.values()]
+    return {b: int(r) for b, r in zip(bins, plan_shards(lengths, world_size))}
+
+
+def merge_discovery_rows(rows, bins, mod_types) -> list:
+    """The rows of all ranks in the order of one GPU: bins in `bins` order, then `mod_types` order; the rows of one
+    (bin, mod type) pair keep their order (a pair's rows come from one rank)."""
+    bin_at = {b: i for i, b in enumerate(bins)}
+    mt_at = {m: i for i, m in enumerate(mod_types)}
+    return sorted(rows, key=lambda r: (bin_at[r["bin"]], mt_at[r["mod_type"]]))
+
+
+def agree_on_error(error, device, world_size: int, rank: int, group=None) -> None:
+    """Raise on every rank the exception of the lowest rank whose `error` is not None (one all-reduce of the flag, then
+    one broadcast of that exception); return when no rank failed.  Every rank must call it."""
+    _, low = rank_extremes([rank if error is not None else world_size], device, world_size, group)
+    src = int(low[0])
+    if src >= world_size:
+        return
+    if rank == src:
+        import pickle
+
+        try:
+            pickle.dumps(error)
+        except Exception:  # noqa: BLE001 -- the other ranks must receive something they can raise
+            error = RuntimeError(f"rank {rank}: {error!r}")
+    out = [error]
+    if _collective(world_size):
+        import torch.distributed as dist
+
+        dist.broadcast_object_list(out, group=group, group_src=src)
+    raise out[0]
+
+
+def discover(pileup, bins: dict, mod_types, low_meth_threshold: float, high_meth_threshold: float, rank: int,
+             world_size: int, padding: int = 20, min_kl: float = 0.05, min_motif_score: float = 1.5, seed=1,
+             device=None, group=None):
+    """search.discover over the GPUs of one box: on every rank, the frame one GPU returns for all `bins` (same rows,
+    order and values).  Every rank passes the same arguments.
+
+    The searches of different bins never communicate (the reference's process pool over bins does the same), so each
+    rank searches its own whole bins (discovery_plan) with search.discover and one object all-gather joins the rows.
+    `pileup`: one table, or the partitioned {(bin, mod_type): frame} dict whose other-rank partitions are skipped before
+    any copy; `bins` = {bin: {contig: sequence or length}} of ALL ranks (a rank needs the sequences of its own bins
+    only).  An error on any rank (bad input, a contig too short for its background samples) raises on every rank."""
+    import torch
+
+    device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    plan = discovery_plan(bins, world_size)
+    mine = {b: cs for b, cs in bins.items() if plan[b] == int(rank)}
+    local, error = None, None
+    try:
+        for b, cs in mine.items():
+            for name, seq in cs.items():
+                if isinstance(seq, (int, np.integer)):
+                    raise ValueError(f"bin {b}: this rank owns contig {name}, which was given by length only")
+        if mine:
+            from .api import MultiBinScorer
+
+            tables = pileup
+            if isinstance(pileup, dict) and "position" not in pileup:  # partitioned {(bin, mod_type): frame}
+                tables = {k: v for k, v in pileup.items() if not (isinstance(k, tuple) and k[0] in bins and k[0] not in mine)}
+            local = MultiBinScorer(tables, mine, list(mod_types), low_meth_threshold, high_meth_threshold, device)
+    except Exception as exc:  # noqa: BLE001 -- raised on every rank by gather_discovery
+        error = exc
+    return _discover_local(local, bins, mod_types, rank, world_size, plan, padding, min_kl, min_motif_score, seed,
+                           device, group, error)
+
+
+def discover_local(local, bins: dict, mod_types, rank: int, world_size: int, padding: int = 20, min_kl: float = 0.05,
+                   min_motif_score: float = 1.5, seed=1, device=None, group=None):
+    """sharding.discover over a rank's MultiBinScorer built elsewhere -- e.g. MultiBinScorer.from_device with the rows
+    kept, over bins generated or parsed on the device.  `bins` = {bin: {contig: sequence or length}} of ALL ranks, the
+    same on every rank; `local` must hold exactly the bins discovery_plan(bins, world_size) gives this rank, or be None
+    when it gives none.  The high methylation threshold is the local scorer's."""
+    import torch
+
+    if device is None:
+        device = local.assembly.device if local is not None else torch.device("cuda", torch.cuda.current_device())
+    plan = discovery_plan(bins, world_size)
+    held = set() if local is None else set(local._ranges)
+    error = None
+    if held != {b for b in bins if plan[b] == int(rank)}:
+        error = ValueError(f"rank {int(rank)}: the local scorer's bins are not those the discovery plan gives this rank")
+    return _discover_local(local, bins, mod_types, rank, world_size, plan, padding, min_kl, min_motif_score, seed,
+                           torch.device(device), group, error)
+
+
+def _discover_local(local, bins, mod_types, rank, world_size, plan, padding, min_kl, min_motif_score, seed, device,
+                    group, error):
+    """search.discover on the rank's bins (in `bins` order), the error agreement, then the gather."""
+    from .search import discover as discover_one
+
+    rows = []
+    if error is None and local is not None:
+        try:
+            df = discover_one(local, mod_types, [b for b in bins if plan[b] == int(rank)], padding, min_kl,
+                              min_motif_score, seed)
+            rows = df.to_dict("records")
+        except Exception as exc:  # noqa: BLE001 -- raised on every rank by gather_discovery
+            error = exc
+    return gather_discovery(rows, error, bins, mod_types, rank, world_size, device, group)
+
+
+def gather_discovery(rows, error, bins, mod_types, rank: int, world_size: int, device, group=None):
+    """The end of sharding.discover on every rank: agree_on_error, then one object all-gather of the rank's rows
+    (search.candidate_rows dicts) and the frame of all of them in the order of one GPU (merge_discovery_rows)."""
+    from .search import discovery_frame
+
+    agree_on_error(error, device, world_size, int(rank), group)
+    if _collective(world_size):
+        rows = gather_rows(rows, group)
+    return discovery_frame(merge_discovery_rows(rows, list(bins), list(mod_types)))
+
+
+# ---------------------------------------------------------------------------------------------
 # The contig x motif methylation-pattern table (K5) over the GPUs of one box.
 # ---------------------------------------------------------------------------------------------
 def _collective(world_size: int) -> bool:

@@ -1,12 +1,22 @@
 #!/usr/bin/env python
-"""Lock-step motif search over many bins (scaled-down BASELINE cfg 3): every (bin, mod type) search advances together,
-one K2 launch per score round and one K4 launch per expand / remove round (development tool).
+"""Lock-step motif search over many bins (scaled-down BASELINE cfg 3) through search.discover: every (bin, mod type)
+search advances together, one K2 launch per score round and one K4 launch per expand / remove round (development tool).
 
     python tools/search_bench.py [--bins 16] [--bin-bp 1000000] [--cpu-bins 1]
+    python tools/search_bench.py --cfg3 [--bins 300]
+    python -m torch.distributed.run --nproc-per-node N tools/search_bench.py --cfg3 [--json out.json]
+
+--cfg3 runs sharding.discover_local: every rank generates only the cfg3 bins the discovery plan gives it, on its own
+GPU, and searches them; one gather joins the rows.  Reported as the maximum over ranks: ingest, setup
+(growth.prepare_searches), search (search.run_lockstep) and gather time, the rounds of each kind; the motifs scored per
+rank; the SHA-256 of the frame (the same at every GPU count); the card name and power limit.
 """
 import argparse
+import hashlib
+import json
 import os
 import random
+import subprocess
 import sys
 import time
 
@@ -17,10 +27,68 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 import nanomotif_b200 as nmb  # noqa: E402
-from nanomotif_b200 import growth, search, synth  # noqa: E402
+from nanomotif_b200 import growth, search, sharding, synth  # noqa: E402
 
 PLANTED = [("GATC", 1), ("CTGCAG", 4), ("GA[AG]TC", 1), ("GCAC......GTT", 2), ("CAA..[AT]TG", 2), ("TTAA", 3), ("ACC.GT", 0),
            ("GAAG[CT]", 2)]
+
+
+class Probe:
+    """Counts and times the parts of a discover call by wrapping the module functions it calls: the hook calls of
+    search.run_lockstep (one per round of a kind that more than one search has pending), the motifs of the score
+    rounds, and the wall time (between device synchronises) of run_lockstep, growth.prepare_searches and
+    sharding.gather_rows."""
+
+    def __init__(self):
+        self.counts = {"score": 0, "expand": 0, "remove": 0, "motifs": 0}
+        self.seconds = {"setup": 0.0, "search": 0.0, "gather": 0.0}
+        self.windows = 0
+        run, prepare, gather = search.run_lockstep, growth.prepare_searches, sharding.gather_rows
+
+        def counting(kind, fn):
+            def hook(reqs):
+                self.counts[kind] += 1
+                if kind == "score":
+                    self.counts["motifs"] += sum(len(m) for _, m in reqs)
+                return fn(reqs)
+            return hook
+
+        def run_counted(searches, batch_score=None, batch_expand=None, batch_remove=None):
+            return self._timed("search", run, searches, counting("score", batch_score), counting("expand", batch_expand),
+                               counting("remove", batch_remove))
+
+        def prepare_timed(*args, **kw):
+            out = self._timed("setup", prepare, *args, **kw)
+            self.windows += int(out[0].n_total)
+            return out
+
+        search.run_lockstep = run_counted
+        growth.prepare_searches = prepare_timed
+        sharding.gather_rows = lambda *args, **kw: self._timed("gather", gather, *args, **kw)
+
+    def _timed(self, key, fn, *args, **kw):
+        torch.cuda.synchronize()
+        t0 = time.perf_counter()
+        out = fn(*args, **kw)
+        torch.cuda.synchronize()
+        self.seconds[key] += time.perf_counter() - t0
+        return out
+
+
+def expansions(m):
+    """Concrete strings of a planted motif: the search reports bracket classes as separate motifs."""
+    out = [""]
+    for t in nmb.motif.tokenize(m):
+        out = [o + c for o in out for c in (t[1:-1] if t.startswith("[") else t)]
+    return out
+
+
+def found_by_pair(df) -> dict:
+    """{(bin, mod type): set of motif strings} of a discover frame."""
+    best = {}
+    for b, mt, motif in zip(df["bin"], df["mod_type"], df["motif"]):
+        best.setdefault((b, mt), set()).add(motif)
+    return best
 
 
 def build_bin(b, rng, bin_bp, depth):
@@ -55,19 +123,18 @@ def windows_for(asm, contigs, pile, pad, high):
     return growth.DeviceDNAarray.from_positions(asm, np.concatenate(ci), np.concatenate(pos), np.concatenate(st), pad)
 
 
-def cfg3_main(args):
-    """--cfg3: the lock-step search of EVERY (bin, mod type) of the cfg3 metagenome (bench.py's generator: 300 bins x
-    5 Mbp, three mod types, planted motifs per bin), all on one GPU."""
-    import bench
+def gpu_info(n: int) -> list:
+    out = subprocess.run(["nvidia-smi", "--query-gpu=index,name,power.limit", "--format=csv,noheader"],
+                         capture_output=True, text=True).stdout.strip().splitlines()
+    return out[:n] if out else [torch.cuda.get_device_name(0)]
+
+
+def cfg3_scorer(synth_m, plan, bins, dev, mod_types):
+    """MultiBinScorer.from_device over cfg3 bins `bins` (generated on `dev`), with the rows the window step needs."""
     from nanomotif_b200.dataload import DeviceRows
     from nanomotif_b200.device import DeviceAssembly, DevicePileup
 
-    synth_m = bench.load_synth()
-    plan = synth_m.cfg3_plan(bench.N_BINS + bench.SWEEP_EXTRA_BINS, bench.BIN_BP)
-    dev = torch.device("cuda", 0)
-    pad, low, high, min_kl, thr = 20, 0.3, 0.7, 0.05, 1.5
-    bins = list(range(args.bins))
-    t0 = time.perf_counter()
+    low, high = 0.3, 0.7
     names, lens, ranges, parts = [], [], {}, []
     for b in bins:
         d = synth_m.cfg3_bin_device(plan, b, dev, ascii_only=True)
@@ -81,63 +148,91 @@ def cfg3_main(args):
     off[1:] = np.cumsum(lens)[:-1]
     asm = DeviceAssembly(names, lens, torch.cat(parts), off, dev)
     del parts
-    pile = DevicePileup(asm, 3, low, high).clear()
+    pile = DevicePileup(asm, len(mod_types), low, high).clear()
     rows = []
     for b in bins:
         d = synth_m.cfg3_bin_device(plan, b, dev)
         cid = (d["contig"] + ranges[f"bin_{b}"][0]).to(torch.int32)
         pile.add_columns(cid, d["position"], d["strand"], d["fraction_mod"], d["mod_type"], sync=False)
-        rows.append(DeviceRows(names, bench.MOD_TYPES, dev, contig_id=cid, position=d["position"], strand=d["strand"],
+        rows.append(DeviceRows(names, mod_types, dev, contig_id=cid, position=d["position"], strand=d["strand"],
                                mod_type=d["mod_type"], fraction_mod=d["fraction_mod"]))
     torch.cuda.synchronize()
-    t_gen = time.perf_counter() - t0
-    multi = nmb.MultiBinScorer.from_device(asm, pile, ranges, bench.MOD_TYPES, rows)
-    n_rows = sum(len(r) for r in rows)
-    print(f"cfg3: {len(bins)} bins, {asm.total_bp / 1e9:.2f} Gbp, {asm.n_contigs} contigs, {n_rows / 1e9:.2f} G pileup rows "
-          f"(device generation + packing + class planes {t_gen:.1f} s)")
-    searches, t_prep = [], 0.0
-    pools = {}
-    for mt in bench.MOD_TYPES:
-        t0 = time.perf_counter()
-        pool, pssms, totals = growth.prepare_searches(multi, mt, pad, high, seeds=[1 + b for b in bins])
-        torch.cuda.synchronize()
-        t_prep += time.perf_counter() - t0
-        pools[mt] = pool
-        for slot, b in enumerate(bins):
-            co = search.find_candidates(mt, pad, pssms[slot], totals[slot], min_kl=min_kl, score_threshold=thr)
-            searches.append((co, search.PoolBackend(multi.context(f"bin_{b}", mt), pool, slot), b, mt))
-    print(f"windows + background PSSMs of all {len(searches)} searches (growth.prepare_searches, host random.sample stream kept) "
-          f"{t_prep:.1f} s; windows: {sum(int(p.n_total) for p in pools.values())}")
-    counts = {"score": 0, "expand": 0, "remove": 0, "motifs": 0}
+    return nmb.MultiBinScorer.from_device(asm, pile, ranges, mod_types, rows), sum(len(r) for r in rows)
 
-    def counting(kind, fn):
-        def hook(reqs):
-            counts[kind] += 1
-            if kind == "score":
-                counts["motifs"] += sum(len(m) for _, m in reqs)
-            return fn(reqs)
-        return hook
 
+def cfg3_main(args):
+    """--cfg3: the lock-step search of EVERY (bin, mod type) of the cfg3 metagenome (bench.py's generator: 300 bins x
+    5 Mbp, three mod types, planted motifs per bin), one GPU per rank."""
+    import torch.distributed as dist
+
+    import bench
+
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    rank = int(os.environ.get("RANK", "0"))
+    dev = torch.device("cuda", int(os.environ.get("LOCAL_RANK", "0")))
+    torch.cuda.set_device(dev)
+    if world > 1:
+        dist.init_process_group("nccl", device_id=dev)
+
+    def gather(x):
+        if world == 1:
+            return [x]
+        out = [None] * world
+        dist.all_gather_object(out, x)
+        return out
+
+    synth_m = bench.load_synth()
+    plan = synth_m.cfg3_plan(bench.N_BINS + bench.SWEEP_EXTRA_BINS, bench.BIN_BP)
+    pad, min_kl, thr = 20, 0.05, 1.5
+    bins = {f"bin_{b}": {f"contig_{i}": int(plan["lengths"][i]) for i in range(*plan["ranges"][b])} for b in range(args.bins)}
+    owner = sharding.discovery_plan(bins, world)
+    mine = [b for b in range(args.bins) if owner[f"bin_{b}"] == rank]
     t0 = time.perf_counter()
-    results = search.run_lockstep([(co, be) for co, be, _, _ in searches], counting("score", search.gpu_batch_score),
-                                  counting("expand", search.gpu_batch_expand),
-                                  counting("remove", search.gpu_batch_remove))
-    torch.cuda.synchronize()
-    t_search = time.perf_counter() - t0
+    local, n_rows = cfg3_scorer(synth_m, plan, mine, dev, bench.MOD_TYPES) if mine else (None, 0)
+    t_gen = time.perf_counter() - t0
+    asm_bp = local.assembly.total_bp if local is not None else 0
+    n_contigs = local.assembly.n_contigs if local is not None else 0
+    probe = Probe()
+    df = sharding.discover_local(local, bins, bench.MOD_TYPES, rank, world, padding=pad, min_kl=min_kl,
+                                 min_motif_score=thr, seed={f"bin_{b}": 1 + b for b in range(args.bins)}, device=dev)
     found = total = 0
-    for (co, be, b, mt), res in zip(searches, results):
-        best = set() if res is None else {m.string.strip(".") for m in res[1]}
-        for motif, _, mtype in plan["planted"][b]:
-            if mtype != mt:
-                continue
+    best = found_by_pair(df)
+    for b in range(args.bins):
+        for motif, _, mt in plan["planted"][b]:
+            got = best.get((f"bin_{b}", mt), set())
             total += 1
-            out = [""]
-            for t in nmb.motif.tokenize(motif):
-                out = [o + c for o in out for c in (t[1:-1] if t.startswith("[") else t)]
-            found += motif in best or all(e in best for e in out)
-    print(f"lock-step search of {len(searches)} (bin, mod type) pairs: {t_search:.1f} s; rounds: score {counts['score']} "
-          f"({counts['motifs']} motifs), expand {counts['expand']}, remove {counts['remove']}")
-    print(f"planted motifs recovered: {found} / {total}")
+            found += motif in got or all(e in got for e in expansions(motif))
+    per_rank = gather({"bins": len(mine), "bp": int(asm_bp), "contigs": int(n_contigs), "rows": int(n_rows),
+                       "ingest_s": t_gen, "windows": probe.windows, "counts": probe.counts, **probe.seconds})
+    sha = hashlib.sha256(df.to_csv(index=False).encode()).hexdigest()
+    shas = gather(sha)
+    assert len(set(shas)) == 1, shas
+    if rank == 0:
+        top = lambda k: max(r[k] for r in per_rank)
+        rounds = {k: max(r["counts"][k] for r in per_rank) for k in ("score", "expand", "remove")}
+        motifs = [r["counts"]["motifs"] for r in per_rank]
+        n_pairs = args.bins * len(bench.MOD_TYPES)
+        print(f"cfg3: {args.bins} bins, {sum(r['bp'] for r in per_rank) / 1e9:.2f} Gbp, "
+              f"{sum(r['contigs'] for r in per_rank)} contigs, {sum(r['rows'] for r in per_rank) / 1e9:.2f} G pileup rows "
+              f"(device generation + packing + class planes {top('ingest_s'):.1f} s)")
+        print(f"windows + background PSSMs of all {n_pairs} searches (growth.prepare_searches, host random.sample stream "
+              f"kept) {top('setup'):.1f} s; windows: {sum(r['windows'] for r in per_rank)}")
+        print(f"lock-step search of {n_pairs} (bin, mod type) pairs: {top('search'):.1f} s; rounds: score {rounds['score']} "
+              f"({sum(motifs)} motifs), expand {rounds['expand']}, remove {rounds['remove']}")
+        print(f"planted motifs recovered: {found} / {total}")
+        result = {"gpus": gpu_info(world), "world_size": world, "bins": args.bins, "pairs": n_pairs,
+                  "bins_per_rank": [r["bins"] for r in per_rank], "bp_per_rank": [r["bp"] for r in per_rank],
+                  "ingest_s": round(top("ingest_s"), 3), "setup_s": round(top("setup"), 3),
+                  "search_s": round(top("search"), 3), "gather_s": round(top("gather"), 4), "rounds": rounds,
+                  "motifs_per_rank": motifs, "frame_rows": len(df), "planted_recovered": [found, total],
+                  "frame_sha256": sha}
+        print(json.dumps(result), flush=True)
+        if args.json:
+            os.makedirs(os.path.dirname(os.path.abspath(args.json)), exist_ok=True)
+            with open(args.json, "w") as f:
+                f.write(json.dumps(result) + "\n")
+    if world > 1:
+        dist.destroy_process_group()
 
 
 def main():
@@ -148,6 +243,7 @@ def main():
     ap.add_argument("--depth", type=int, default=20)
     ap.add_argument("--cpu-bins", type=int, default=1, help="bins also searched with the CPU oracle backend (slow)")
     ap.add_argument("--check-setup", action="store_true", help="compare the batched setup with the per-bin host-driven one")
+    ap.add_argument("--json", default=None, help="--cfg3: rank 0 also writes the result line here")
     args = ap.parse_args()
     if args.cfg3:
         if args.bins == 16:
@@ -180,47 +276,27 @@ def main():
     multi = nmb.MultiBinScorer(table, bins, ["a"], low, high)
     torch.cuda.synchronize()
     t_ingest = time.perf_counter() - t0
-    # windows of every bin + every bin's background PSSM, batched on the device (growth.prepare_searches)
-    pool, pssms, totals = growth.prepare_searches(multi, "a", pad, high, seeds=[1 + b for b in range(args.bins)])
-    torch.cuda.synchronize()
-    t_setup = time.perf_counter() - t0
+    seeds = {f"bin{b}": 1 + b for b in range(args.bins)}
     if args.check_setup:  # the old per-bin host-driven setup must give the same windows and backgrounds
+        pool, pssms, _ = growth.prepare_searches(multi, "a", pad, high, seeds=list(seeds.values()))
         asm = multi.assembly
         for b in range(args.bins):
             random.seed(1 + b)
             w = windows_for(asm, bins[f"bin{b}"], piles[b], pad, high)
             bg = growth.background_pssm(asm, bins[f"bin{b}"], "A", pad)
             assert torch.equal(pool.windows[pool.begin[b]:pool.end[b]], w.windows) and np.array_equal(bg, pssms[b])
-    setups = list(zip(totals, pssms))
-    counts = {"score": 0, "expand": 0, "remove": 0, "motifs": 0}
-
-    def counting(kind, fn):
-        def hook(reqs):
-            counts[kind] += 1
-            if kind == "score":
-                counts["motifs"] += sum(len(m) for _, m in reqs)
-            return fn(reqs)
-        return hook
-
-    searches = []
-    for b, (total, bg) in enumerate(setups):
-        co = search.find_candidates("a", pad, bg, total, min_kl=min_kl, score_threshold=thr)
-        searches.append((co, search.PoolBackend(multi.context(f"bin{b}", "a"), pool, b)))
-    t0 = time.perf_counter()
-    results = search.run_lockstep(searches, counting("score", search.gpu_batch_score), counting("expand", search.gpu_batch_expand),
-                                  counting("remove", search.gpu_batch_remove))
-    torch.cuda.synchronize()
-    t_search = time.perf_counter() - t0
-    def expansions(m):  # concrete strings of a planted motif: the search reports bracket classes as separate motifs
-        out = [""]
-        for t in nmb.motif.tokenize(m):
-            out = [o + c for o in out for c in (t[1:-1] if t.startswith("[") else t)]
-        return out
-
+    probe = Probe()
+    # windows of every bin + every bin's background PSSM, batched on the device (growth.prepare_searches), then the
+    # lock-step search of all bins
+    df = search.discover(multi, ["a"], padding=pad, min_kl=min_kl, min_motif_score=thr, seed=seeds)
+    t_setup = t_ingest + probe.seconds["setup"]
+    t_search = probe.seconds["search"]
+    counts = probe.counts
+    best = found_by_pair(df)
     found = 0
-    for b, res in enumerate(results):
-        best = set() if res is None else {m.string.strip(".") for m in res[1]}
-        found += all(p[0] in best or all(e in best for e in expansions(p[0])) for p in truth[f"bin{b}"])
+    for b in range(args.bins):
+        got = best.get((f"bin{b}", "a"), set())
+        found += all(p[0] in got or all(e in got for e in expansions(p[0])) for p in truth[f"bin{b}"])
     total_bp = sum(len(s) for cs in bins.values() for s in cs.values())
     print(f"{args.bins} bins, {total_bp / 1e6:.1f} Mbp, {len(pile['position']) / 1e6:.1f} M pileup rows (host generation {t_gen:.1f} s)")
     print(f"device setup from the Arrow table (ingest {t_ingest:.3f} s + windows / backgrounds of all bins) {t_setup:7.3f} s")
